@@ -1,7 +1,10 @@
 #!/usr/bin/env python3
 """bench.py -- throughput of the stereo front-end hot path on synthetic data, one JSON line per run.
 
-  python bench.py [--config c1|c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--config c1|c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs writes the results of the last timed step as .npy files; the inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
 
 Configurations (BASELINE.json `configs`, SURVEY.md section 8):
   c1  one KITTI-00-shaped 1241x376 pair per step, maxCorners 1000 (the reference's own CPU-runnable case)
@@ -37,6 +40,7 @@ from types import SimpleNamespace
 
 ROOT = pathlib.Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # a run leaves the tree as build() left it (it may be read-only)
 
 BYTES_PER_KEYPOINT = 113  # uvL 8 + uvR 8 + xyz 24 + descL 32 + descR 32 + dist 4 + idx 4 + status 1
 CALIB = ROOT / "tests" / "golden" / "calib"
@@ -71,13 +75,68 @@ def parse():
     ap.add_argument("--device-only", action="store_true", help="tuning aid: only the device-resident measurement; not a bench line")
     ap.add_argument("--device-order", default=None, help="comma list: CUDA device of local rank i (placement experiments)")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not bind the rank to its GPU's NUMA node (placement experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 / float64, "
+                         "under 64 MB: a fixed sample of the frames of a larger batch); rank 0 only")
     a = ap.parse_args()
     a.cfg = dict(CONFIGS[a.config])
     if a.frames is not None:
         a.cfg["frames"] = a.frames
     if a.steps is None:
         a.steps = a.cfg["steps"]
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     return a
+
+
+# ----------------------------------------------------------------------------- --dump-outputs
+# svi_stereo_result field -> the name of the same array in run_batch's output tensors
+RESULT_FIELDS = {"n_keypoints": "n_kp", "n_detected": "n_det", "uv_left": "uv_l", "uv_right": "uv_r", "xyz_left": "xyz",
+                 "desc_left": "dl", "desc_right": "dr", "distance": "dist", "match_index": "idx", "status": "st"}
+DUMP_BYTES = 60_000_000   # the arrays of the sampled frames; the .npy headers and per-frame counts stay well inside 64 MB
+
+
+def dump_frame_sample(n_frames: int, cap: int):
+    """Frames whose results --dump-outputs writes: all of them when they fit DUMP_BYTES, else a fixed seeded sample."""
+    import numpy as np
+    per_frame = cap * (2 * 4 + 2 * 4 + 3 * 8 + 2 * 32 * 4 + 3 * 4)   # uv x2, xyz, two descriptors (one float per byte), distance, index, status
+    n = min(n_frames, max(1, DUMP_BYTES // per_frame))
+    return np.arange(n_frames) if n == n_frames else np.sort(np.random.default_rng(0).choice(n_frames, n, replace=False))
+
+
+def write_stereo_dump(out_dir, r: dict, frames) -> None:
+    """svi_stereo_result arrays of the given frames (field names of include/svi_gpu.h) as float32, xyz as float64; every
+    integer converts exactly.  What the C API leaves unspecified is written as 0: the slots past n_keypoints, and uv_right,
+    xyz_left and desc_right of key-points whose status is not SVI_OK."""
+    import numpy as np
+    cap = r["status"].shape[1]
+    live = np.arange(cap)[None, :] < r["n_keypoints"][:, None]
+    matched = live & (r["status"] == 0)
+    out = {"frame_index": np.asarray(frames, np.float64)}
+    for k in ("n_keypoints", "n_detected"):
+        out[k] = r[k].astype(np.float64)
+    for k in ("uv_left", "uv_right", "xyz_left", "desc_left", "desc_right", "distance", "match_index", "status"):
+        a = r[k].astype(np.float64 if k == "xyz_left" else np.float32)
+        a[~(matched if k in ("uv_right", "xyz_left", "desc_right") else live)] = 0
+        out[k] = a
+    write_arrays(out_dir, out)
+
+
+def write_sequence_dump(out_dir, trk) -> None:
+    """The tracker after a whole sequence: its landmark state (one row per active landmark) and its per-frame record
+    (tracked, visible, new, active, motion scaling, landmarks per tracking stage 0-5), all float64 (exact)."""
+    import numpy as np
+    out = {f"landmark_{k}": np.asarray(v, np.float64) for k, v in trk.s.items()}
+    out["frame_log"] = np.array([[r["tracked"], r["visible"], r["new"], r["active"], r["scaling"], *r["stages"]] for r in trk.log], np.float64)
+    write_arrays(out_dir, out)
+
+
+def write_arrays(out_dir, arrays: dict) -> None:
+    import numpy as np
+    d = pathlib.Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", np.ascontiguousarray(a))
 
 
 def cameras(cfg):
@@ -194,12 +253,16 @@ def metric_name(name, cams):
 
 # ----------------------------------------------------------------------------- CPU arm (reference / baseline)
 def load_oracle():
+    """The checker built with -march=native for this host, as the reference builds itself, in a temporary directory so that
+    the tree stays as build() left it; the portable build of build() when that fails.  Returns (module, `native` argument)."""
+    import tempfile
     from oracle import c_oracle as co
-    native = True
-    try:
-        co.load(native=True)
-    except Exception:
-        native = False
+    with tempfile.TemporaryDirectory(prefix="svi_oracle_") as d:
+        try:
+            native = co.build(native=True, out=pathlib.Path(d) / "libsvi_oracle_native.so")
+            co.load(native)   # mapped (and cached by path) before the directory goes
+        except Exception:
+            native = False
     return co, native
 
 
@@ -276,7 +339,7 @@ def run_reference(args, rank: int):
         from svi_mapper_b200.sequence import SequenceTracker, render_sequence
         n = min(cfg["frames"], 24)
         L, R, T = render_sequence(cams[0], cams[1], n, cfg["seed"])
-        steps = max(1, min(args.steps, 3))
+        steps = args.steps
         t_sum, lm_sum = 0.0, 0
         for _ in range(steps):
             be = CpuSequenceBackend(co, native, ocfg, threads)
@@ -284,6 +347,8 @@ def run_reference(args, rank: int):
             for t in range(n):
                 lm_sum += trk.process(L[t], R[t], T[t])["tracked"]
             t_sum += be.seconds
+        if args.dump_outputs:
+            write_sequence_dump(args.dump_outputs, trk)
         fps = steps * n / t_sum
         sample = (f"first {n} frames of the sequence per step x {steps} steps, landmark-parallel over {threads} threads, "
                   f"{build} build of oracle/svi_oracle.c")
@@ -296,13 +361,16 @@ def run_reference(args, rank: int):
         sample_n = max(2, min(threads, 4)) if big else max(threads, 8)
         L = np.stack([pairs[i % n_unique][0] for i in range(sample_n)])
         R = np.stack([pairs[i % n_unique][1] for i in range(sample_n)])
-        steps = max(1, min(args.steps, 3 if big else 10))
+        steps = args.steps
         for _ in range(min(args.warmup, 1)):
             co.stereo_frames(ocfg, L, R, n_threads=threads, native=native)
         t0 = time.perf_counter()
         for _ in range(steps):
-            co.stereo_frames(ocfg, L, R, n_threads=threads, native=native)
+            out = co.stereo_frames(ocfg, L, R, n_threads=threads, native=native)
         dt = time.perf_counter() - t0
+        if args.dump_outputs:
+            frames = dump_frame_sample(sample_n, cfg["max_corners"])
+            write_stereo_dump(args.dump_outputs, {k: v[frames] for k, v in out.items()}, frames)
         fps = sample_n * steps / dt
         sample = f"{sample_n} frames/step x {steps} steps, {min(threads, sample_n)} threads (one frame per thread), {build} build of oracle/svi_oracle.c"
         ms_step = dt / steps * 1e3
@@ -387,6 +455,10 @@ def run_batch(args, rank, world, dev_index):
     ms_max = float(t_ms.item())
     total_frames = cfg["frames"] if cfg["scaling"] == "strong" else world * F
     value = total_frames * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs and rank == 0:   # before the profiled step below writes into the same buffers
+        frames = dump_frame_sample(F, cap)
+        sel = torch.as_tensor(frames, device=dev)
+        write_stereo_dump(args.dump_outputs, {k: dout[v].index_select(0, sel).cpu().numpy() for k, v in RESULT_FIELDS.items()}, f_lo + frames)
 
     # ---- one extra step with every chunk on ONE stream: exclusive per-kernel durations for the roofline record
     fe.set_profiling(2)
@@ -630,6 +702,8 @@ def run_sequence(args, rank, world, dev_index):
         dist.all_reduce(t_e, op=dist.ReduceOp.MAX)
     dt_max = float(t_e.item())
     value = world * n * args.steps / dt_max
+    if args.dump_outputs and rank == 0:
+        write_sequence_dump(args.dump_outputs, trk)
     log = trk.log
     tracked = sum(r["tracked"] for r in log)
     stages = np.sum([r["stages"] for r in log], axis=0)

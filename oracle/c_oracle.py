@@ -40,12 +40,17 @@ class TrackResult(C.Structure):
                 ("desc_left", C.c_void_p), ("desc_right", C.c_void_p)]
 
 
-def build(native: bool = False) -> pathlib.Path:
-    target = "libsvi_oracle_native.so" if native else "libsvi_oracle.so"
-    r = subprocess.run(["make", "-C", str(HERE), "native" if native else "all"], capture_output=True, text=True)
+def build(native: bool = False, out: pathlib.Path | None = None) -> pathlib.Path:
+    """make the portable or the -march=native library; `out` is where the native one goes instead of oracle/."""
+    target = HERE / ("libsvi_oracle_native.so" if native else "libsvi_oracle.so")
+    cmd = ["make", "-C", str(HERE), "native" if native else "all"]
+    if native and out is not None:
+        target = pathlib.Path(out).resolve()
+        cmd.append(f"NATIVE={target}")
+    r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("oracle build failed:\n" + r.stdout + r.stderr)
-    return HERE / target
+    return target
 
 
 def build_variant(pattern_header: pathlib.Path, out: pathlib.Path) -> pathlib.Path:

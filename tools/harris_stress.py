@@ -1,9 +1,9 @@
-import sys; sys.path.insert(0,'/root/repo')
+import pathlib, sys; ROOT=pathlib.Path(__file__).resolve().parents[1]; sys.path.insert(0,str(ROOT))
 import numpy as np, cv2
 from svi_mapper_b200 import StereoFrontend, load_camera
 from svi_mapper_b200.synth import stereo_pair
 from oracle import frontend_np as o, c_oracle as co
-cl=load_camera('tests/golden/calib/kitti_00_left.txt'); cr=load_camera('tests/golden/calib/kitti_00_right.txt')
+cl=load_camera(str(ROOT/'tests/golden/calib/kitti_00_left.txt')); cr=load_camera(str(ROOT/'tests/golden/calib/kitti_00_right.txt'))
 def variants(seed):
     L,R=stereo_pair(1241,376,seed)
     yield 'tex',L,R
