@@ -354,8 +354,44 @@ int svi_config(const svi_ctx* ctx, int32_t* chunk_frames, int32_t* n_lanes, int3
 
 /* Number of kernels the new-landmark path launches for one chunk of a call with n_frames frames: 4 (detector, RIGHT box
  * sums, corner selection, matcher) on the small-call path, 5 when the LEFT descriptors are a kernel of their own (batch
- * path), 6 when the batch path also sorts the key-points into image bins (dense frames).  For launch accounting. */
+ * path), 6 when the batch path also sorts the key-points into image bins (dense frames); one more while rectification is
+ * set (svi_set_rectification).  For launch accounting. */
 int svi_kernels_per_chunk(const svi_ctx* ctx, int n_frames);
+
+/* ---- undistortion + rectification of raw camera images (CStereoCamera.h:102-107, CStereoCameraIMU.h:36-51: the reference
+ * builds cv::initUndistortRectifyMap(matIntrinsic, vecDistortionCoefficients, matRectification, matProjection, (W, H), m1type)
+ * per camera and runs cv::remap(raw, rectified, map1, map2, INTER_LINEAR) on every frame).  The new camera matrix is the
+ * first 3 x 3 of the svi_camera's P the ctx was created with. */
+typedef struct svi_rectification {
+    double K[9];          /* matIntrinsic, row-major                                                      */
+    double D[4];          /* vecDistortionCoefficients k1 k2 p1 p2                                        */
+    double R[9];          /* matRectification, row-major                                                  */
+    int32_t float_maps;   /* 0: maps as cv::initUndistortRectifyMap(..., CV_16SC2) (default)               */
+                          /* 1: CV_32FC1 maps handed to cv::remap (which rounds float32(u) * 32, not u * 32) */
+} svi_rectification;
+
+/* The map of one camera in cv2's CV_16SC2 layout: xy = W x H x 2 int16 (integer source column, row), frac = W x H uint16
+ * (5-bit row fraction * 32 + 5-bit column fraction).  Host only, needs no ctx and no GPU; the library builds its device
+ * maps with this function.  SVI_ERR_INVALID for a singular K or P[:3,:3] * R (e.g. an all-zero matIntrinsic). */
+int svi_rectify_map(const svi_camera* cam, const svi_rectification* r, int16_t* xy, uint16_t* frac);
+
+/* Switches rectification on (both non-NULL) or off (both NULL) for every later call on ctx.  Waits for the ctx to go idle,
+ * builds both maps, uploads them and allocates the raw-image staging once.  While it is set, EVERY image argument of every
+ * entry point is a RAW image of the camera it belongs to -- svi_stereo_frames, svi_stereo_frames_device,
+ * svi_stereo_frame_masked, svi_triangulate_right (RIGHT), svi_triangulate_left (LEFT), svi_track_landmarks[_stages], and
+ * svi_harris_response / svi_detect / svi_describe (LEFT) -- and is rectified on the device with cv::remap(INTER_LINEAR,
+ * BORDER_CONSTANT 0) arithmetic, bit for bit.  Masks, key-point coordinates and every other coordinate in and out stay in
+ * the RECTIFIED frame.  Off (the default) costs nothing: no launch, copy or allocation. */
+int svi_set_rectification(svi_ctx* ctx, const svi_rectification* left, const svi_rectification* right);
+
+/* The rectified images themselves (display, key-frame images, inspection): n_frames raw host images of camera `side`
+ * (0 = LEFT, 1 = RIGHT), height x pitch bytes, frame_stride apart -> n_frames rectified images of height x out_pitch
+ * bytes, densely stacked.  Needs svi_set_rectification. */
+int svi_rectify(svi_ctx* ctx, int side, const uint8_t* raw, size_t pitch, size_t frame_stride, int n_frames, uint8_t* out,
+                size_t out_pitch);
+
+/* svi_set_rectification on every context of the multi-GPU driver. */
+int svi_multi_set_rectification(svi_multi* m, const svi_rectification* left, const svi_rectification* right);
 
 #ifdef __cplusplus
 }

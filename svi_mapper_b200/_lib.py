@@ -25,7 +25,7 @@ EXPORTS = (
     "svi_match_hamming", "svi_match_epipolar", "svi_triangulate_right", "svi_triangulate_left", "svi_point_in_left",
     "svi_track_landmarks", "svi_track_landmarks_stages", "svi_set_profiling", "svi_stage_timings", "svi_config", "svi_kernels_per_chunk", "svi_optimize_landmarks",
     "svi_multi_create", "svi_multi_destroy", "svi_multi_last_error", "svi_multi_device_count", "svi_multi_frame_range",
-    "svi_multi_stereo_frames",
+    "svi_multi_stereo_frames", "svi_rectify_map", "svi_set_rectification", "svi_rectify", "svi_multi_set_rectification",
 )
 
 u8p, i32p, f32p, f64p = C.POINTER(C.c_uint8), C.POINTER(C.c_int32), C.POINTER(C.c_float), C.POINTER(C.c_double)
@@ -79,6 +79,11 @@ class LandmarkMeasurements(C.Structure):
 
 class OptimizeResult(C.Structure):
     _fields_ = [("xyz_world", C.c_void_p), ("outcome", C.c_void_p), ("average_squared_error", C.c_void_p), ("iterations", C.c_void_p)]
+
+
+class Rectification(C.Structure):
+    """svi_rectification: matIntrinsic, vecDistortionCoefficients (k1 k2 p1 p2), matRectification, map type."""
+    _fields_ = [("K", C.c_double * 9), ("D", C.c_double * 4), ("R", C.c_double * 9), ("float_maps", C.c_int32)]
 
 
 (SVI_OPT_SKIPPED, SVI_OPT_CONVERGED, SVI_OPT_OPTIMAL, SVI_OPT_REJECTED, SVI_OPT_NOT_CONVERGED) = range(5)
@@ -141,6 +146,10 @@ def load(path=None):
     lib.svi_multi_device_count.argtypes = [vp]
     lib.svi_multi_frame_range.argtypes = [vp, ci, ci, i32p, i32p]
     lib.svi_multi_stereo_frames.argtypes = [vp, vp, vp, sz, sz, ci, vp, C.POINTER(StereoResult)]
+    lib.svi_rectify_map.argtypes = [C.POINTER(Camera), C.POINTER(Rectification), vp, vp]
+    lib.svi_set_rectification.argtypes = [vp, C.POINTER(Rectification), C.POINTER(Rectification)]
+    lib.svi_rectify.argtypes = [vp, ci, vp, sz, sz, ci, vp, sz]
+    lib.svi_multi_set_rectification.argtypes = [vp, C.POINTER(Rectification), C.POINTER(Rectification)]
     for name in EXPORTS:
         getattr(lib, name)  # AttributeError here = header/library mismatch
     if path is None:

@@ -25,6 +25,7 @@
 #include "binned.cuh"
 #include "harris.cuh"
 #include "landmark_opt.cuh"
+#include "rectify.cuh"
 #include "select.cuh"
 #include "track_plan.cuh"
 
@@ -63,6 +64,9 @@ struct Lane {
     uint8_t* img_l = nullptr;
     uint8_t* img_r = nullptr;
     uint8_t* mask = nullptr;
+    // raw images while rectification is set (svi_set_rectification): rectify_kernel reads these and writes img_l / img_r
+    uint8_t* raw_l = nullptr;
+    uint8_t* raw_r = nullptr;
     CUtensorMap map_l{}, map_r{}, map_ls{}, map_rs{};  // TMA views of the four planes: (W, chunk*H) u16, row pitch box_pitch
     CUtensorMap map_l_patch{};                          // LEFT plane again, box = the 56 x 49 patch of one descriptor
     // binned matcher (binned.cuh): key-points sorted by image bin, one tile of the planes per bin
@@ -151,6 +155,11 @@ struct svi_ctx {
     bool profiling = false;
     bool batch_uploads = false;   // upload(): stage into the pinned mirror only (svi_track_landmarks sends one copy)
     bool serial = false;   // profiling mode 2: every chunk on lane 0, so that the stage events bracket ONE kernel each
+    // rectification (svi_set_rectification): both cameras' maps in one device block, [camera][xy short2 | frac uint16]
+    // with rect_npad (W * H rounded up to 4) entries each; off = all null, no launch, copy or allocation anywhere
+    bool rect = false;
+    unsigned char* rect_map = nullptr;
+    int rect_npad = 0;
     double stage_ms[kStages] = {};
     long stage_launches[kStages] = {};
     std::string err;
@@ -407,6 +416,107 @@ int sync_lanes(svi_ctx* ctx) {
 template <typename T>
 cudaError_t dmalloc(T** p, size_t count) { return cudaMalloc(reinterpret_cast<void**>(p), count * sizeof(T)); }
 
+// ---- rectification
+// cvRound of OpenCV's x86 build (cvtsd2si / cvtss2si): half to even, and INT_MIN for NaN or anything outside int
+int cv_round_host(double v) {
+    if (!(v >= -2147483648.0 && v < 2147483648.0)) return INT32_MIN;
+    return (int)std::nearbyint(v);
+}
+int16_t saturate_short(int v) { return (int16_t)std::min(32767, std::max(-32768, v)); }
+
+// The numbers of Matx33d::determinant / Matx33d::inv (the cofactor form OpenCV uses for 3 x 3).
+double det33(const double* a) {
+    return a[0] * (a[4] * a[8] - a[7] * a[5]) - a[1] * (a[3] * a[8] - a[6] * a[5]) + a[2] * (a[3] * a[7] - a[6] * a[4]);
+}
+
+// cv::initUndistortRectifyMap(K, D, R, P, (W, H), CV_16SC2) -- or, with float_maps, CV_32FC1 followed by the conversion
+// cv::remap applies to float maps (cv::convertMaps to CV_16SC2) -- in OpenCV's scalar operation order, fp64 without
+// contraction (the library is built with -ffp-contract=off).  Empty string on success.
+std::string rectify_map_host(const svi_camera* cam, const svi_rectification* r, int16_t* xy, uint16_t* frac) {
+    if (!cam || !r || !xy || !frac) return "svi_rectify_map: null argument";
+    if (cam->width == 0 || cam->height == 0 || cam->width > 65535 || cam->height > 65535) return "svi_rectify_map: bad image size";
+    if (r->float_maps != 0 && r->float_maps != 1) return "svi_rectify_map: float_maps must be 0 or 1";
+    const double dk = det33(r->K);
+    if (!(dk != 0.0) || !std::isfinite(dk)) return "svi_rectify_map: matIntrinsic K is singular";
+    double a[9];   // P[:3,:3] * R, Matx product order
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) {
+            double acc = 0.0;
+            for (int k = 0; k < 3; ++k) acc += cam->P[i * 4 + k] * r->R[k * 3 + j];
+            a[i * 3 + j] = acc;
+        }
+    double d = det33(a);
+    if (!(d != 0.0) || !std::isfinite(d)) return "svi_rectify_map: P[:3,:3] * matRectification is singular";
+    d = 1.0 / d;
+    const double ir[9] = {(a[4] * a[8] - a[5] * a[7]) * d, (a[2] * a[7] - a[1] * a[8]) * d, (a[1] * a[5] - a[2] * a[4]) * d,
+                          (a[5] * a[6] - a[3] * a[8]) * d, (a[0] * a[8] - a[2] * a[6]) * d, (a[2] * a[3] - a[0] * a[5]) * d,
+                          (a[3] * a[7] - a[4] * a[6]) * d, (a[1] * a[6] - a[0] * a[7]) * d, (a[0] * a[4] - a[1] * a[3]) * d};
+    const double u0 = r->K[2], v0 = r->K[5], fx = r->K[0], fy = r->K[4];
+    const double k1 = r->D[0], k2 = r->D[1], p1 = r->D[2], p2 = r->D[3], k3 = 0.0, k4 = 0.0, k5 = 0.0, k6 = 0.0;
+    const double s1 = 0.0, s2 = 0.0, s3 = 0.0, s4 = 0.0;
+    const int W = (int)cam->width, H = (int)cam->height;
+    for (int i = 0; i < H; ++i) {
+        double _x = i * ir[1] + ir[2], _y = i * ir[4] + ir[5], _w = i * ir[7] + ir[8];
+        for (int j = 0; j < W; ++j, _x += ir[0], _y += ir[3], _w += ir[6]) {
+            const double w = 1. / _w, x = _x * w, y = _y * w;
+            const double x2 = x * x, y2 = y * y;
+            const double r2 = x2 + y2, _2xy = 2 * x * y;
+            const double kr = (1 + ((k3 * r2 + k2) * r2 + k1) * r2) / (1 + ((k6 * r2 + k5) * r2 + k4) * r2);
+            const double xd = (x * kr + p1 * _2xy + p2 * (r2 + 2 * x2) + s1 * r2 + s2 * r2 * r2);
+            const double yd = (y * kr + p1 * (r2 + 2 * y2) + p2 * _2xy + s3 * r2 + s4 * r2 * r2);
+            // the identity tilt matrix of the 4-coefficient model, applied as OpenCV applies it
+            double t0 = 0.0, t1 = 0.0, t2 = 0.0;
+            t0 += 1.0 * xd; t0 += 0.0 * yd; t0 += 0.0 * 1.0;
+            t1 += 0.0 * xd; t1 += 1.0 * yd; t1 += 0.0 * 1.0;
+            t2 += 0.0 * xd; t2 += 0.0 * yd; t2 += 1.0 * 1.0;
+            const double inv_proj = t2 ? 1. / t2 : 1;
+            const double u = fx * inv_proj * t0 + u0, v = fy * inv_proj * t1 + v0;
+            int iu, iv;
+            if (r->float_maps) {
+                iu = cv_round_host((double)((float)u * 32.f));
+                iv = cv_round_host((double)((float)v * 32.f));
+            } else {
+                iu = cv_round_host(u * 32.0);
+                iv = cv_round_host(v * 32.0);
+            }
+            const size_t o = (size_t)i * W + j;
+            xy[2 * o] = saturate_short(iu >> 5);
+            xy[2 * o + 1] = saturate_short(iv >> 5);
+            frac[o] = (uint16_t)((iv & 31) * 32 + (iu & 31));
+        }
+    }
+    return std::string();
+}
+
+const short2* rect_xy(const svi_ctx* c, int cam) { return reinterpret_cast<const short2*>(c->rect_map + (size_t)cam * c->rect_npad * 6); }
+const uint16_t* rect_frac(const svi_ctx* c, int cam) {
+    return reinterpret_cast<const uint16_t*>(c->rect_map + (size_t)cam * c->rect_npad * 6 + (size_t)c->rect_npad * 4);
+}
+
+// One rectify_kernel launch for n_cams images of nf frames each: raw src[i] (src_pitch bytes per row, src_stride per
+// frame) through the map of camera cams[i] into the dense plane stack dst[i] (W bytes per row, H * W per frame).
+int launch_rectify(svi_ctx* ctx, int n_cams, const int* cams, const uint8_t* const* src, uint8_t* const* dst, size_t src_pitch,
+                   size_t src_stride, int nf, cudaStream_t s) {
+    RectifyArgs a{};
+    for (int i = 0; i < n_cams; ++i) a.cam[i] = RectifySide{rect_xy(ctx, cams[i]), rect_frac(ctx, cams[i]), src[i], dst[i]};
+    a.W = ctx->W; a.H = ctx->H; a.n_pix = ctx->W * ctx->H; a.n_pad = ctx->rect_npad; a.nf = nf;
+    a.src_pitch = src_pitch; a.src_stride = src_stride; a.dst_stride = (size_t)ctx->H * ctx->dev_pitch;
+    const int quads = (a.n_pix + RECT_PX - 1) / RECT_PX;
+    rectify_kernel<<<dim3((quads + RECT_THREADS - 1) / RECT_THREADS, n_cams, (nf + RECT_FRAMES - 1) / RECT_FRAMES), RECT_THREADS, 0, s>>>(a);
+    CK(cudaGetLastError());
+    return SVI_SUCCESS;
+}
+int rectify_pair(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t stride, uint8_t* d_left, uint8_t* d_right,
+                 int nf, cudaStream_t s) {
+    const int cams[2] = {0, 1};
+    const uint8_t* src[2] = {left, right};
+    uint8_t* dst[2] = {d_left, d_right};
+    return launch_rectify(ctx, 2, cams, src, dst, pitch, stride, nf, s);
+}
+int rectify_one(svi_ctx* ctx, int cam, const uint8_t* raw, size_t pitch, size_t stride, uint8_t* d_out, int nf, cudaStream_t s) {
+    return launch_rectify(ctx, 1, &cam, &raw, &d_out, pitch, stride, nf, s);
+}
+
 }  // namespace
 
 // ---- per-query entry points: one image (or pair) staged in lane 0, queries in the arena ----
@@ -421,10 +531,14 @@ bool host_is_pinned(const void* p) {
     return a.type == cudaMemoryTypeHost;
 }
 
+// One image of camera `cam` (0 = LEFT, 1 = RIGHT) into d_img plus its box sums.  While rectification is set the image is
+// raw: it goes up into lane 0's raw plane of that camera and rectify_kernel writes d_img.
 int stage_box(svi_ctx* ctx, const uint8_t* img, size_t pitch, uint8_t* d_img, uint16_t* d_box, uint16_t* d_box_shift,
-              cudaStream_t s, int pin_plane = 0) {
+              cudaStream_t s, int cam, int pin_plane = 0) {
     const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
     const size_t plane = (size_t)ctx->H * ctx->dev_pitch;
+    uint8_t* const d_rect = d_img;
+    if (ctx->rect) d_img = cam ? ctx->lanes[0].raw_r : ctx->lanes[0].raw_l;
     if (host_is_pinned(img)) {
         if ((int)pitch == ctx->dev_pitch) CK(cudaMemcpyAsync(d_img, img, plane, cudaMemcpyHostToDevice, s));
         else CK(cudaMemcpy2DAsync(d_img, ctx->dev_pitch, img, pitch, ctx->W, ctx->H, cudaMemcpyHostToDevice, s));
@@ -436,8 +550,12 @@ int stage_box(svi_ctx* ctx, const uint8_t* img, size_t pitch, uint8_t* d_img, ui
     } else {
         CK(cudaMemcpy2DAsync(d_img, ctx->dev_pitch, img, pitch, ctx->W, ctx->H, cudaMemcpyHostToDevice, s));
     }
+    if (ctx->rect) {
+        const int rc = rectify_one(ctx, cam, d_img, ctx->dev_pitch, plane, d_rect, 1, s);
+        if (rc != SVI_SUCCESS) return rc;
+    }
     const dim3 tiles((g.W + HT_W - 1) / HT_W, (g.H + HT_H - 1) / HT_H, 1);
-    boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, d_box, d_box_shift);
+    boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_rect, g, d_box, d_box_shift);
     CK(cudaGetLastError());
     return SVI_SUCCESS;
 }
@@ -522,7 +640,7 @@ int small_call(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t p
             CK(cudaStreamWaitEvent(side, ctx->fork, 0));
         }
         const uint8_t* srcs[3] = {left, masks, right};
-        uint8_t* dsts[3] = {l.img_l, l.mask, l.img_r};
+        uint8_t* dsts[3] = {ctx->rect ? l.raw_l : l.img_l, l.mask, ctx->rect ? l.raw_r : l.img_r};
         auto upload_plane = [&](int k, cudaStream_t sk) -> int {
             if (!srcs[k]) return SVI_SUCCESS;
             if (host_is_pinned(srcs[k])) {   // the caller's buffer is page-locked: DMA straight from it
@@ -549,6 +667,22 @@ int small_call(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t p
             if (rc != SVI_SUCCESS) return rc;
         }
         const std::function<int(cudaStream_t)> upload_right = [&](cudaStream_t sk) { return upload_plane(2, sk); };
+        if (ctx->rect) {
+            // raw images: RIGHT goes up on the side stream beside LEFT, one launch rectifies both into img_l / img_r, and the
+            // RIGHT box sums still run on the side stream beside the detector
+            const int rc = upload_plane(2, side ? side : s);
+            if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); if (side) cudaStreamSynchronize(side); return rc; }
+            if (side) {
+                CK(cudaEventRecord(ctx->side_done, side));
+                CK(cudaStreamWaitEvent(s, ctx->side_done, 0));
+            }
+            const int rr = rectify_pair(ctx, l.raw_l, l.raw_r, ctx->dev_pitch, dstride, l.img_l, l.img_r, nf, s);
+            if (rr != SVI_SUCCESS) return rr;
+            if (side) {
+                CK(cudaEventRecord(ctx->fork, s));
+                CK(cudaStreamWaitEvent(side, ctx->fork, 0));
+            }
+        }
         bool have_mask = masks != nullptr;
         if (centres) {
             int rc = build_mask(ctx, l, centres, n_centres);
@@ -556,7 +690,7 @@ int small_call(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t p
             have_mask = true;
         }
         int rc = run_pipeline(ctx, l, l.img_l, l.img_r, have_mask ? l.mask : nullptr, g, nf, ctx->small_out, 0, ctx->small_n_kp, ctx->small_n_det, side,
-                              &upload_right);
+                              ctx->rect ? nullptr : &upload_right);
         if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); if (side) cudaStreamSynchronize(side); return rc; }
         // one copy brings the whole result block back; only the live slots are scattered to the caller's arrays
         CK(cudaMemcpyAsync(pin_out, ctx->small_block, ctx->small_bytes, cudaMemcpyDeviceToHost, s));
@@ -591,7 +725,7 @@ int triangulate_common(svi_ctx* ctx, bool left_search, const uint8_t* img, size_
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
     ctx->arena_used = 0; ctx->pending.clear();
-    int rc = stage_box(ctx, img, pitch, l.img_l, l.box_l, l.box_ls, s);
+    int rc = stage_box(ctx, img, pitch, l.img_l, l.box_l, l.box_ls, s, left_search ? 0 : 1);
     if (rc != SVI_SUCCESS) return rc;
     float* d_range = nullptr; float* d_tl; float* d_uv; uint8_t* d_desc;
     TriOutDev o;
@@ -808,7 +942,8 @@ void svi_destroy(svi_ctx* ctx) {
         if (l.stream) cudaStreamSynchronize(l.stream);
         void* ptrs[] = {l.box_l, l.box_r, l.box_ls, l.box_rs, l.frame_max, l.cand_count, l.cand, l.det_xy, l.kp_xy, l.n_det, l.n_kp,
                         l.g_head, l.g_next, l.g_state, l.img_l, l.img_r, l.mask, l.out.uv_l, l.out.uv_r, l.out.xyz,
-                        l.out.desc_l, l.out.desc_r, l.out.dist, l.out.idx, l.out.status, l.bin_start, l.bin_slot, l.bin_kp};
+                        l.out.desc_l, l.out.desc_r, l.out.dist, l.out.idx, l.out.status, l.bin_start, l.bin_slot, l.bin_kp,
+                        l.raw_l, l.raw_r};
         for (void* p : ptrs) if (p) cudaFree(p);
         for (cudaEvent_t e : l.ev) cudaEventDestroy(e);
         if (l.done) cudaEventDestroy(l.done);
@@ -826,6 +961,7 @@ void svi_destroy(svi_ctx* ctx) {
     if (ctx->trk_img) cudaFree(ctx->trk_img);
     if (ctx->s3_items) cudaFree(ctx->s3_items);
     if (ctx->resp_one) cudaFree(ctx->resp_one);
+    if (ctx->rect_map) cudaFree(ctx->rect_map);
     {
         void* rp[] = {ctx->roi.max, ctx->roi.cand, ctx->roi.det, ctx->roi.kp, ctx->roi.n_det, ctx->roi.n_kp, ctx->roi.rois, ctx->roi.s2};
         for (void* q : rp) if (q) cudaFree(q);
@@ -988,7 +1124,7 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
                                  (const void*)triangulate_kernel<false>, (const void*)track_stage1_kernel,
                                  (const void*)track_stage2_kernel<true>, (const void*)track_stage2_kernel<false>,
                                  (const void*)track_stage3_kernel, (const void*)fast_candidates_kernel,
-                                 (const void*)describe_kernel, (const void*)hamming_match_kernel};
+                                 (const void*)describe_kernel, (const void*)hamming_match_kernel, (const void*)rectify_kernel};
         for (const void* k : kernels)
             CK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
@@ -1111,6 +1247,8 @@ int svi_stereo_frames_device(svi_ctx* ctx, const uint8_t* left, const uint8_t* r
     CK(cudaEventRecord(ctx->fork, user));
     for (int i = 0; i < ctx->n_lanes; ++i) CK(cudaStreamWaitEvent(ctx->lanes[i].stream, ctx->fork, 0));
     const FrameGeom g = make_geom(ctx, (int)pitch, frame_stride);
+    const size_t dstride = (size_t)ctx->H * ctx->dev_pitch;
+    const FrameGeom g_rect = make_geom(ctx, ctx->dev_pitch, dstride);   // rectified planes in the lane's staging
     StereoOutDev o;
     o.cap = out->capacity_per_frame;
     o.uv_l = out->uv_left; o.uv_r = out->uv_right; o.xyz = out->xyz_left;
@@ -1121,8 +1259,24 @@ int svi_stereo_frames_device(svi_ctx* ctx, const uint8_t* left, const uint8_t* r
         Lane& l = ctx->lanes[ctx->serial ? 0 : chunk_id % ctx->n_lanes];
         const int nf = std::min(ctx->chunk, n_frames - f0);
         int* n_det = out->n_detected ? out->n_detected + f0 : l.n_det;
-        rc = run_pipeline(ctx, l, left + (size_t)f0 * frame_stride, right + (size_t)f0 * frame_stride,
-                          masks ? masks + (size_t)f0 * frame_stride : nullptr, g, nf, o, f0, out->n_keypoints + f0, n_det);
+        const uint8_t* m = masks ? masks + (size_t)f0 * frame_stride : nullptr;
+        if (ctx->rect) {   // the caller's raw frames are read in place; the pipeline reads the rectified planes
+            rc = rectify_pair(ctx, left + (size_t)f0 * frame_stride, right + (size_t)f0 * frame_stride, pitch, frame_stride, l.img_l, l.img_r, nf,
+                              l.stream);
+            if (rc != SVI_SUCCESS) break;
+            if (m && ((int)pitch != ctx->dev_pitch || frame_stride != dstride)) {   // the masks follow the planes' layout
+                for (int f = 0; f < nf && rc == SVI_SUCCESS; ++f)
+                    if (cudaMemcpy2DAsync(l.mask + f * dstride, ctx->dev_pitch, m + (size_t)f * frame_stride, pitch, ctx->W, ctx->H,
+                                          cudaMemcpyDeviceToDevice, l.stream) != cudaSuccess)
+                        rc = fail(ctx, SVI_ERR_CUDA, "svi_stereo_frames_device: mask copy failed");
+                if (rc != SVI_SUCCESS) break;
+                m = l.mask;
+            }
+            rc = run_pipeline(ctx, l, l.img_l, l.img_r, m, g_rect, nf, o, f0, out->n_keypoints + f0, n_det);
+        } else {
+            rc = run_pipeline(ctx, l, left + (size_t)f0 * frame_stride, right + (size_t)f0 * frame_stride, m, g, nf, o, f0, out->n_keypoints + f0,
+                              n_det);
+        }
         if (rc != SVI_SUCCESS) break;
     }
     // join the lanes back into the caller's stream -- also after a failure, so that nothing queued so far can outlive
@@ -1156,7 +1310,7 @@ int svi_stereo_frames(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, s
         cudaStream_t s = l.stream;
         const int nf = std::min(ctx->chunk, n_frames - f0);
         const uint8_t* srcs[3] = {left, right, masks};
-        uint8_t* dsts[3] = {l.img_l, l.img_r, l.mask};
+        uint8_t* dsts[3] = {ctx->rect ? l.raw_l : l.img_l, ctx->rect ? l.raw_r : l.img_r, l.mask};
         for (int k = 0; k < 3; ++k) {
             if (!srcs[k]) continue;
             if (dense && (int)pitch == ctx->dev_pitch) {
@@ -1169,6 +1323,10 @@ int svi_stereo_frames(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, s
                     CK(cudaMemcpy2DAsync(dsts[k] + f * dstride, ctx->dev_pitch, srcs[k] + (size_t)(f0 + f) * frame_stride,
                                          pitch, W, H, cudaMemcpyHostToDevice, s));
             }
+        }
+        if (ctx->rect) {
+            const int rr = rectify_pair(ctx, l.raw_l, l.raw_r, ctx->dev_pitch, dstride, l.img_l, l.img_r, nf, s);
+            if (rr != SVI_SUCCESS) return rr;
         }
         int rc = run_pipeline(ctx, l, l.img_l, l.img_r, masks ? l.mask : nullptr, g, nf, l.out, 0, l.n_kp, l.n_det);
         if (rc != SVI_SUCCESS) return rc;
@@ -1238,7 +1396,11 @@ int svi_harris_response(svi_ctx* ctx, const uint8_t* img, size_t pitch, float* r
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
     const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
-    CK(cudaMemcpy2DAsync(l.img_l, ctx->dev_pitch, img, pitch, ctx->W, ctx->H, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpy2DAsync(ctx->rect ? l.raw_l : l.img_l, ctx->dev_pitch, img, pitch, ctx->W, ctx->H, cudaMemcpyHostToDevice, s));
+    if (ctx->rect) {
+        const int rc = rectify_one(ctx, 0, l.raw_l, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch, l.img_l, 1, s);
+        if (rc != SVI_SUCCESS) return rc;
+    }
     CK(cudaMemsetAsync(l.frame_max, 0, sizeof(uint32_t), s));
     if (!ctx->resp_one) CK(dmalloc(&ctx->resp_one, (size_t)ctx->H * ctx->resp_pitch));
     harris_box_kernel<<<harris_grid(g.W, g.H, 1), HT_THREADS, sizeof(HarrisSmem), s>>>(
@@ -1265,11 +1427,15 @@ int svi_detect(svi_ctx* ctx, const uint8_t* img, size_t pitch, size_t frame_stri
     for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk) {
         const int nf = std::min(ctx->chunk, n_frames - f0);
         for (int f = 0; f < nf; ++f) {
-            CK(cudaMemcpy2DAsync(l.img_l + f * dstride, ctx->dev_pitch, img + (size_t)(f0 + f) * frame_stride, pitch, W, H,
+            CK(cudaMemcpy2DAsync((ctx->rect ? l.raw_l : l.img_l) + f * dstride, ctx->dev_pitch, img + (size_t)(f0 + f) * frame_stride, pitch, W, H,
                                  cudaMemcpyHostToDevice, s));
             if (masks)
                 CK(cudaMemcpy2DAsync(l.mask + f * dstride, ctx->dev_pitch, masks + (size_t)(f0 + f) * frame_stride, pitch, W, H,
                                      cudaMemcpyHostToDevice, s));
+        }
+        if (ctx->rect) {
+            const int rc = rectify_one(ctx, 0, l.raw_l, ctx->dev_pitch, dstride, l.img_l, nf, s);
+            if (rc != SVI_SUCCESS) return rc;
         }
         const uint8_t* d_mask = masks ? l.mask : nullptr;
         CK(cudaMemsetAsync(l.frame_max, 0, sizeof(uint32_t) * nf, s));
@@ -1314,7 +1480,7 @@ int svi_describe(svi_ctx* ctx, const uint8_t* img, size_t pitch, const float* xy
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
     ctx->arena_used = 0; ctx->pending.clear();
-    int rc = stage_box(ctx, img, pitch, l.img_l, l.box_l, l.box_ls, s);
+    int rc = stage_box(ctx, img, pitch, l.img_l, l.box_l, l.box_ls, s, 0);
     if (rc != SVI_SUCCESS) return rc;
     float* d_xy; uint8_t* d_desc; uint8_t* d_kept;
     UP(d_xy, xy, (size_t)n * 2);
@@ -1461,8 +1627,8 @@ int svi_track_landmarks_stages(svi_ctx* ctx, const uint8_t* img_left, const uint
     // (RIGHT goes up and gets its box sums on the side stream, beside LEFT's)
     CK(cudaEventRecord(ctx->fork, s));
     CK(cudaStreamWaitEvent(ctx->side, ctx->fork, 0));
-    rc = stage_box(ctx, img_right, pitch, ctx->trk_img + plane, l.box_r, l.box_rs, ctx->side, 1);
-    if (rc == SVI_SUCCESS) rc = stage_box(ctx, img_left, pitch, ctx->trk_img, l.box_l, l.box_ls, s);
+    rc = stage_box(ctx, img_right, pitch, ctx->trk_img + plane, l.box_r, l.box_rs, ctx->side, 1, 1);
+    if (rc == SVI_SUCCESS) rc = stage_box(ctx, img_left, pitch, ctx->trk_img, l.box_l, l.box_ls, s, 0);
     if (cudaEventRecord(ctx->side_done, ctx->side) != cudaSuccess || cudaStreamWaitEvent(s, ctx->side_done, 0) != cudaSuccess)
         rc = rc == SVI_SUCCESS ? fail(ctx, SVI_ERR_CUDA, "svi_track_landmarks: joining the side stream failed") : rc;
     if (rc != SVI_SUCCESS) { cudaStreamSynchronize(ctx->side); cudaStreamSynchronize(s); return rc; }
@@ -1684,6 +1850,85 @@ int svi_stage_timings(svi_ctx* ctx, const char** names, double* total_ms, int64_
     return n;
 }
 
+// ---- undistortion + rectification of raw images (CStereoCamera.h:102-107: cv::initUndistortRectifyMap + cv::remap)
+int svi_rectify_map(const svi_camera* cam, const svi_rectification* r, int16_t* xy, uint16_t* frac) {
+    const std::string e = rectify_map_host(cam, r, xy, frac);
+    return e.empty() ? SVI_SUCCESS : fail(nullptr, SVI_ERR_INVALID, e);
+}
+
+int svi_set_rectification(svi_ctx* ctx, const svi_rectification* left, const svi_rectification* right) {
+    if (!ctx) return SVI_ERR_INVALID;
+    if (!left != !right) return fail(ctx, SVI_ERR_INVALID, "svi_set_rectification: give both cameras or neither");
+    CK(cudaSetDevice(ctx->device));
+    const size_t npix = (size_t)ctx->W * ctx->H, npad = (npix + 7) & ~size_t(7);   // 8: camera 1's xy block stays 16-byte aligned
+    std::vector<int16_t> xy;
+    std::vector<uint16_t> frac;
+    if (left) {   // both maps first: a rejected calibration leaves the ctx as it was
+        xy.assign(2 * 2 * npad, 0);
+        frac.assign(2 * npad, 0);
+        for (int c = 0; c < 2; ++c) {
+            const std::string e = rectify_map_host(c ? &ctx->cam_r : &ctx->cam_l, c ? right : left, xy.data() + c * 2 * npad, frac.data() + c * npad);
+            if (!e.empty()) return fail(ctx, SVI_ERR_INVALID, e + (c ? " (right camera)" : " (left camera)"));
+        }
+    }
+    // nothing queued may still read the maps or the raw planes that are replaced below
+    for (int i = 0; i < ctx->n_lanes; ++i) CK(cudaStreamSynchronize(ctx->lanes[i].stream));
+    CK(cudaStreamSynchronize(ctx->side));
+    if (ctx->profiling) collect_timings(ctx);
+    if (!left) {
+        for (int i = 0; i < ctx->n_lanes; ++i) {
+            Lane& l = ctx->lanes[i];
+            if (l.raw_l) cudaFree(l.raw_l);
+            if (l.raw_r) cudaFree(l.raw_r);
+            l.raw_l = l.raw_r = nullptr;
+        }
+        if (ctx->rect_map) cudaFree(ctx->rect_map);
+        ctx->rect_map = nullptr;
+        ctx->rect_npad = 0;
+        ctx->rect = false;
+        return SVI_SUCCESS;
+    }
+    ctx->rect = false;   // until everything below is in place
+    const size_t raw = (size_t)ctx->chunk * ctx->H * ctx->dev_pitch;   // allocated once, kept until rectification is switched off
+    for (int i = 0; i < ctx->n_lanes; ++i) {
+        if (!ctx->lanes[i].raw_l) CK(dmalloc(&ctx->lanes[i].raw_l, raw));
+        if (!ctx->lanes[i].raw_r) CK(dmalloc(&ctx->lanes[i].raw_r, raw));
+    }
+    if (!ctx->rect_map) CK(cudaMalloc(reinterpret_cast<void**>(&ctx->rect_map), 2 * npad * 6));
+    ctx->rect_npad = (int)npad;
+    for (int c = 0; c < 2; ++c) {
+        CK(cudaMemcpy(ctx->rect_map + c * npad * 6, xy.data() + c * 2 * npad, npad * 4, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(ctx->rect_map + c * npad * 6 + npad * 4, frac.data() + c * npad, npad * 2, cudaMemcpyHostToDevice));
+    }
+    ctx->rect = true;
+    return SVI_SUCCESS;
+}
+
+int svi_rectify(svi_ctx* ctx, int side, const uint8_t* raw, size_t pitch, size_t frame_stride, int n_frames, uint8_t* out, size_t out_pitch) {
+    if (!ctx) return SVI_ERR_INVALID;
+    if (!raw || !out || (side != 0 && side != 1) || n_frames < 0 || (int)pitch < ctx->W || (int)out_pitch < ctx->W ||
+        (n_frames > 1 && frame_stride < pitch * (size_t)ctx->H))
+        return fail(ctx, SVI_ERR_INVALID, "svi_rectify: bad argument");
+    if (!ctx->rect) return fail(ctx, SVI_ERR_INVALID, "svi_rectify: no rectification set (svi_set_rectification)");
+    CK(cudaSetDevice(ctx->device));
+    Lane& l = ctx->lanes[0];
+    cudaStream_t s = l.stream;
+    const size_t dstride = (size_t)ctx->H * ctx->dev_pitch;
+    uint8_t* d_raw = side ? l.raw_r : l.raw_l;
+    for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk) {
+        const int nf = std::min(ctx->chunk, n_frames - f0);
+        for (int f = 0; f < nf; ++f)
+            CK(cudaMemcpy2DAsync(d_raw + f * dstride, ctx->dev_pitch, raw + (size_t)(f0 + f) * frame_stride, pitch, ctx->W, ctx->H,
+                                 cudaMemcpyHostToDevice, s));
+        const int rc = rectify_one(ctx, side, d_raw, ctx->dev_pitch, dstride, l.img_l, nf, s);
+        if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); return rc; }
+        CK(cudaMemcpy2DAsync(out + (size_t)f0 * ctx->H * out_pitch, out_pitch, l.img_l, ctx->dev_pitch, ctx->W, (size_t)ctx->H * nf,
+                             cudaMemcpyDeviceToHost, s));
+    }
+    CK(cudaStreamSynchronize(s));
+    return check_overflow(ctx);
+}
+
 // ---- frame-partitioned batches over several GPUs (SURVEY.md 8e): stereo pairs are independent, so a batch of F
 // frames is cut into contiguous ranges [g*F/G, (g+1)*F/G), one per device; each range runs through its own svi_ctx on
 // its own host thread and writes a disjoint slice of the caller's arrays.  No collective, no peer access: the result is
@@ -1771,12 +2016,24 @@ int svi_multi_stereo_frames(svi_multi* m, const uint8_t* left, const uint8_t* ri
     return SVI_SUCCESS;
 }
 
+int svi_multi_set_rectification(svi_multi* m, const svi_rectification* left, const svi_rectification* right) {
+    if (!m) return SVI_ERR_INVALID;
+    for (size_t g = 0; g < m->ctx.size(); ++g) {
+        const int rc = svi_set_rectification(m->ctx[g], left, right);
+        if (rc != SVI_SUCCESS) {
+            m->err = "device " + std::to_string(m->devices[g]) + ": " + svi_last_error(m->ctx[g]);
+            return rc;
+        }
+    }
+    return SVI_SUCCESS;
+}
+
 int svi_kernels_per_chunk(const svi_ctx* ctx, int n_frames) {
     if (!ctx || n_frames <= 0) return SVI_ERR_INVALID;
     const long long slots = (long long)std::min(n_frames, ctx->chunk) * ctx->p.max_corners;
     const bool pre = ctx->match_pre && slots / (2LL * ctx->n_sm * 9) >= MATCH_KP_PER_WARP;
     // detector, RIGHT box sums, corner selection, matcher (+ LEFT descriptors as a kernel of their own, + the bin sort)
-    return 4 + (pre ? 1 : 0) + (pre && ctx->match_binned ? 1 : 0);
+    return 4 + (pre ? 1 : 0) + (pre && ctx->match_binned ? 1 : 0) + (ctx->rect ? 1 : 0);
 }
 
 int svi_config(const svi_ctx* ctx, int32_t* chunk_frames, int32_t* n_lanes, int32_t* select_in_smem) {

@@ -56,6 +56,30 @@ def _ptr(a) -> int:
     return a.ctypes.data if a is not None else None
 
 
+def rectification(cam, float_maps: bool = False) -> _lib.Rectification:
+    """svi_rectification of a calib.PinholeCamera: matIntrinsic, vecDistortionCoefficients, matRectification."""
+    r = _lib.Rectification()
+    for dst, src, n in ((r.K, cam.K, 9), (r.D, cam.distortion, 4), (r.R, cam.rectification, 9)):
+        v = np.asarray(src, np.float64).reshape(n)
+        for i in range(n):
+            dst[i] = float(v[i])
+    r.float_maps = 1 if float_maps else 0
+    return r
+
+
+def rectify_map(cam, float_maps: bool = False):
+    """svi_rectify_map: the map of one camera as cv::initUndistortRectifyMap(K, D, R, P, (W, H), CV_16SC2) returns it
+    -- (xy (H, W, 2) int16, frac (H, W) uint16); with float_maps, the CV_16SC2 form of the CV_32FC1 maps.  Host only."""
+    c, r = _cam(cam), rectification(cam, float_maps)
+    xy = np.zeros((int(cam.height), int(cam.width), 2), np.int16)
+    frac = np.zeros((int(cam.height), int(cam.width)), np.uint16)
+    lib = _lib.load()
+    rc = lib.svi_rectify_map(C.byref(c), C.byref(r), _ptr(xy), _ptr(frac))
+    if rc != _lib.SVI_SUCCESS:
+        raise SviError(rc, lib.svi_last_error(None).decode())
+    return xy, frac
+
+
 @dataclass
 class StereoFrames:
     """SoA result of the new-landmark path (svi_stereo_result); arrays are (n_frames, capacity, ...)."""
@@ -145,6 +169,26 @@ class StereoFrontend:
         if a.ndim != 3 or a.shape[1] != self.height or a.shape[2] != self.width:
             raise ValueError(f"{name}: expected (n, {self.height}, {self.width}) uint8, got {a.shape}")
         return np.ascontiguousarray(a)
+
+    # -- raw camera images: undistortion + rectification on the device (CStereoCamera.h:102-107)
+    def set_rectification(self, cam_left, cam_right, float_maps: bool = False):
+        """svi_set_rectification from the two calib.PinholeCamera (K / distortion / rectification; the new camera matrix is
+        the P this front-end was created with).  From now on every image argument of every method is a RAW image;
+        masks and coordinates stay in the rectified frame.  float_maps: CV_32FC1 maps instead of CV_16SC2."""
+        rl, rr = rectification(cam_left, float_maps), rectification(cam_right, float_maps)
+        self._check(self._lib.svi_set_rectification(self._ctx, C.byref(rl), C.byref(rr)))
+
+    def clear_rectification(self):
+        """Images are rectified already again (the default)."""
+        self._check(self._lib.svi_set_rectification(self._ctx, None, None))
+
+    def rectify(self, images, side: int) -> np.ndarray:
+        """svi_rectify: raw images (n, H, W) or (H, W) of camera `side` (0 = LEFT, 1 = RIGHT) -> rectified, same shape."""
+        a = np.asarray(images)
+        A = self._images(a, "images")
+        out = np.empty_like(A)
+        self._check(self._lib.svi_rectify(self._ctx, int(side), _ptr(A), self.width, self.width * self.height, A.shape[0], _ptr(out), self.width))
+        return out[0] if a.ndim == 2 else out
 
     # -- CFundamentalMatcher::addNewLandmarks for a batch of independent pairs
     def stereo_frames(self, left, right, masks=None, capacity: int | None = None) -> StereoFrames:

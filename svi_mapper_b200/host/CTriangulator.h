@@ -36,6 +36,17 @@ public:
     CGpuContext(const CGpuContext&) = delete;
     CGpuContext& operator=(const CGpuContext&) = delete;
     void check(int rc) const { if (SVI_SUCCESS != rc) throw std::runtime_error(std::string("libsvi_gpu: ") + svi_last_error(ctx)); }
+    // CStereoCamera.h:102-107: from here on every image handed to the library is a RAW camera image, undistorted and
+    // rectified on the GPU with the maps cv::initUndistortRectifyMap builds from the members CPinholeCamera holds
+    // (m_matIntrinsic, m_vecDistortionCoefficients, m_matRectification; new camera matrix m_matProjection).
+    // p_bFloatMaps: the CV_32FC1 maps instead of CV_16SC2.
+    void setRectification(const CStereoCamera& p_cCamera, bool p_bFloatMaps = false) {
+        svi_rectification rL, rR;
+        fill(rL, *p_cCamera.m_pCameraLEFT, p_bFloatMaps);
+        fill(rR, *p_cCamera.m_pCameraRIGHT, p_bFloatMaps);
+        check(svi_set_rectification(ctx, &rL, &rR));
+    }
+    void clearRectification() { check(svi_set_rectification(ctx, nullptr, nullptr)); }
     svi_ctx* ctx = nullptr;
     svi_params params;
 private:
@@ -43,6 +54,12 @@ private:
         c.width = cam.m_uWidthPixel;
         c.height = cam.m_uHeightPixel;
         for (int i = 0; i < 12; ++i) c.P[i] = cam.m_matProjection.m[i];
+    }
+    static void fill(svi_rectification& r, const CPinholeCamera& cam, bool p_bFloatMaps) {
+        for (int i = 0; i < 9; ++i) r.K[i] = cam.m_matIntrinsic.m[i];
+        for (int i = 0; i < 4; ++i) r.D[i] = cam.m_vecDistortionCoefficients.v[i];
+        for (int i = 0; i < 9; ++i) r.R[i] = cam.m_matRectification.m[i];
+        r.float_maps = p_bFloatMaps ? 1 : 0;
     }
 };
 

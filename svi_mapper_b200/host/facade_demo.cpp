@@ -195,9 +195,10 @@ static int maskMain(char** argv) {
 // planes) through CTrackerGT::process (track -> optimise -> re-detect), the per-frame relative motion LEFTLAST->LEFTNOW as
 // 12 numbers + the rotation norm per line.  Prints, per frame, the counters, every visible landmark's measurement and the
 // state of every active landmark after the frame -- compared line by line with the CPU restatement of the same loop.
+// --sequence --rectify <left_calib> ...: the frames are RAW camera images, rectified on the GPU (CGpuContext::setRectification).
 // With SVI_DEMO_TIMING set the per-frame dump is skipped and ONE line goes to stdout instead: the wall time of every
 // process() call (frames after the first three), split into trackManual / landmark optimisation / re-detection.
-static int sequenceMain(char** argv) {
+static int sequenceMain(char** argv, bool p_bRectify) {
     try {
         CParameterBase::loadCameraLEFT(argv[2]);
         CParameterBase::loadCameraRIGHT(argv[3]);
@@ -210,6 +211,7 @@ static int sequenceMain(char** argv) {
         svi_params_default(&p);
         p.max_corners = std::atoi(argv[8]);
         auto pGpu = std::make_shared<CGpuContext>(CParameterBase::pCameraSTEREO, &p);
+        if (p_bRectify) pGpu->setRectification(*CParameterBase::pCameraSTEREO);
         CTrackerGT cTracker(CParameterBase::pCameraSTEREO, pGpu);
         const bool bTiming = std::getenv("SVI_DEMO_TIMING") != nullptr;
         std::FILE* out = bTiming ? nullptr : std::fopen(argv[9], "w");
@@ -266,7 +268,10 @@ static int sequenceMain(char** argv) {
 }
 
 int main(int argc, char** argv) {
-    if (argc == 10 && std::string(argv[1]) == "--sequence") return sequenceMain(argv);
+    if (argc == 10 && std::string(argv[1]) == "--sequence") return sequenceMain(argv, false);
+    if (argc == 11 && std::string(argv[1]) == "--sequence" && std::string(argv[2]) == "--rectify") {
+        return sequenceMain(argv + 1, true);   // the remaining arguments keep their positions
+    }
     if (argc == 5 && std::string(argv[1]) == "--solver") return solverMain(argv);
     if (argc == 6 && std::string(argv[1]) == "--mask") return maskMain(argv);
     if (argc == 3 && std::string(argv[1]) == "--landmark") return landmarkMain(argv);

@@ -71,6 +71,19 @@ class MultiFrontend:
         except Exception:
             pass
 
+    def set_rectification(self, cam_left, cam_right, float_maps: bool = False):
+        """svi_multi_set_rectification: StereoFrontend.set_rectification on every context."""
+        from .frontend import rectification
+        rl, rr = rectification(cam_left, float_maps), rectification(cam_right, float_maps)
+        rc = self._lib.svi_multi_set_rectification(self._m, C.byref(rl), C.byref(rr))
+        if rc != _lib.SVI_SUCCESS:
+            raise SviError(rc, self._lib.svi_multi_last_error(self._m).decode())
+
+    def clear_rectification(self):
+        rc = self._lib.svi_multi_set_rectification(self._m, None, None)
+        if rc != _lib.SVI_SUCCESS:
+            raise SviError(rc, self._lib.svi_multi_last_error(self._m).decode())
+
     def frame_range(self, n_frames: int, part: int) -> tuple[int, int]:
         a, b = C.c_int32(), C.c_int32()
         rc = self._lib.svi_multi_frame_range(self._m, int(n_frames), int(part), C.byref(a), C.byref(b))

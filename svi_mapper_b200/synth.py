@@ -74,6 +74,24 @@ def stereo_pair(width: int, height: int, seed: int, d_min=1, d_max=55):
     return np.ascontiguousarray(left), np.ascontiguousarray(right)
 
 
+def unrectify(img: np.ndarray, cam) -> np.ndarray:
+    """The raw image a distorted, unrectified camera would have seen of a rectified image `img` (H, W) u8: every raw pixel
+    takes the rectified position cv2.undistortPoints(pixel, K, D, R=R, P=P) of calib.PinholeCamera `cam` and samples `img`
+    there bilinearly (0 outside).  For raw test sequences; rectifying the result gives `img` back up to the two
+    interpolations."""
+    import cv2
+
+    H, W = img.shape
+    K = np.asarray(cam.K, np.float64).reshape(3, 3)
+    D = np.asarray(cam.distortion, np.float64).reshape(4)
+    R = np.asarray(cam.rectification, np.float64).reshape(3, 3)
+    P = np.asarray(cam.P, np.float64).reshape(3, 4)
+    u, v = np.meshgrid(np.arange(W, dtype=np.float64), np.arange(H, dtype=np.float64))
+    pts = np.stack([u, v], -1).reshape(-1, 1, 2)
+    rect = cv2.undistortPoints(pts, K, D, R=R, P=P).reshape(H, W, 2).astype(np.float32)
+    return cv2.remap(img, rect[..., 0], rect[..., 1], cv2.INTER_LINEAR, borderMode=cv2.BORDER_CONSTANT, borderValue=0)
+
+
 def stereo_batch_torch(n_frames: int, width: int, height: int, seed: int, device="cuda", d_max: int = 55):
     """Batch of n_frames distinct pairs generated on `device` with torch ops.
 
