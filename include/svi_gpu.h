@@ -319,6 +319,42 @@ typedef struct svi_optimize_result {
 } svi_optimize_result;
 int svi_optimize_landmarks(svi_ctx* ctx, const svi_landmark_measurements* in, int n, svi_optimize_result* out);
 
+/* ---- pose from the stereo measurements of one frame.
+ * CSolverStereoPosit::getTransformationWORLDtoLEFT (src/optimization/CSolverStereoPosit.cpp:8-170), what
+ * CFundamentalMatcher::getPoseStereoPosit hands the measurements of tracking stages 1 and 2 to: robust Gauss-Newton on the
+ * stereo re-projection error of the WORLD->LEFT pose from the prior T_estimate (constants of CSolverStereoPosit.h:89-99: more
+ * than 25 points, at most 1000 iterations, convergence 1e-5 on the total squared error, kernel 10 px^2; a converged pose with
+ * an average error above 9 px^2 AND fewer than 15 inliers is inaccurate; a translation within 1 mm (squared 0.001 m^2) of
+ * T_last keeps T_last's translation; a camera position more than 2 m^2 (squared) away from the prior's plus t_imu is a high
+ * risk).  The projection matrices are the P of the ctx's two cameras.  One launch, the whole iteration loop on the device,
+ * fp64 without contraction in the host's operation order: the results equal the C++ host implementation of the same loop bit
+ * for bit.  Per-problem failures are the outcome, not the return code; n <= 25 is answered without touching the GPU. */
+enum svi_posit_outcome {
+    SVI_POSIT_OK = 0,               /* T_world_to_left is the solution                                              */
+    SVI_POSIT_TOO_FEW_POINTS = 1,   /* "insufficient number of points: <n>"                                          */
+    SVI_POSIT_INACCURATE = 2,       /* "insufficient accuracy (average error: <average_squared_error> inliers: <inliers>)" */
+    SVI_POSIT_HIGH_RISK = 3,        /* "inconsistent with prior (HIGH RISK: <risk>)"                                 */
+    SVI_POSIT_NOT_CONVERGED = 4     /* "system did not converge" (1000 iterations)                                   */
+};
+typedef struct svi_posit_problem {   /* one frame's CSolverStereoPosit::CMatch list + the solver's other arguments */
+    int32_t n;                       /* measurements                                                               */
+    const double* xyz_world;         /* n x 3 vecPointXYZWORLD                                                     */
+    const float* uv_left;            /* n x 2 ptUVLEFT                                                             */
+    const float* uv_right;           /* n x 2 ptUVRIGHT                                                            */
+    double T_estimate[16];           /* p_matTransformationWORLDtoLEFTESTIMATE, row-major                          */
+    double T_last[16];               /* p_matTransformationWORLDtoLEFTLAST                                         */
+    double t_imu[3];                 /* p_vecTranslationIMU                                                        */
+} svi_posit_problem;
+typedef struct svi_posit_result {
+    double T_world_to_left[16];      /* the solution when SVI_POSIT_OK, else T_estimate                            */
+    uint8_t outcome;                 /* svi_posit_outcome                                                          */
+    int32_t iterations;              /* iterations run (0 for SVI_POSIT_TOO_FEW_POINTS)                            */
+    int32_t inliers;                 /* inliers of the last iteration                                              */
+    double average_squared_error;    /* of the converged iteration (0 if it did not converge)                      */
+    double risk;                     /* squared distance to the prior's position (0 unless the risk test ran)      */
+} svi_posit_result;
+int svi_solve_stereo_posit(svi_ctx* ctx, const svi_posit_problem* in, svi_posit_result* out);
+
 /* Stage profiling: when enabled, every kernel of the new-landmark path is bracketed by CUDA events
  * on the stream it is launched on (the events come from a pool filled here, none is created while
  * work is being timed).  enable = 1: the lanes keep overlapping, a bracket also contains other lanes'

@@ -24,6 +24,7 @@ EXPORTS = (
     "svi_stereo_frames", "svi_stereo_frames_device", "svi_check_overflow", "svi_mask_active_landmarks", "svi_stereo_frame_masked", "svi_harris_response", "svi_detect", "svi_describe",
     "svi_match_hamming", "svi_match_epipolar", "svi_triangulate_right", "svi_triangulate_left", "svi_point_in_left",
     "svi_track_landmarks", "svi_track_landmarks_stages", "svi_set_profiling", "svi_stage_timings", "svi_config", "svi_kernels_per_chunk", "svi_optimize_landmarks",
+    "svi_solve_stereo_posit",
     "svi_multi_create", "svi_multi_destroy", "svi_multi_last_error", "svi_multi_device_count", "svi_multi_frame_range",
     "svi_multi_stereo_frames", "svi_rectify_map", "svi_set_rectification", "svi_rectify", "svi_multi_set_rectification",
 )
@@ -81,12 +82,24 @@ class OptimizeResult(C.Structure):
     _fields_ = [("xyz_world", C.c_void_p), ("outcome", C.c_void_p), ("average_squared_error", C.c_void_p), ("iterations", C.c_void_p)]
 
 
+class PositProblem(C.Structure):
+    """svi_posit_problem: one frame's measurements (WORLD points, LEFT / RIGHT image points) and the solver's priors."""
+    _fields_ = [("n", C.c_int32), ("xyz_world", C.c_void_p), ("uv_left", C.c_void_p), ("uv_right", C.c_void_p),
+                ("T_estimate", C.c_double * 16), ("T_last", C.c_double * 16), ("t_imu", C.c_double * 3)]
+
+
+class PositResult(C.Structure):
+    _fields_ = [("T_world_to_left", C.c_double * 16), ("outcome", C.c_uint8), ("iterations", C.c_int32), ("inliers", C.c_int32),
+                ("average_squared_error", C.c_double), ("risk", C.c_double)]
+
+
 class Rectification(C.Structure):
     """svi_rectification: matIntrinsic, vecDistortionCoefficients (k1 k2 p1 p2), matRectification, map type."""
     _fields_ = [("K", C.c_double * 9), ("D", C.c_double * 4), ("R", C.c_double * 9), ("float_maps", C.c_int32)]
 
 
 (SVI_OPT_SKIPPED, SVI_OPT_CONVERGED, SVI_OPT_OPTIMAL, SVI_OPT_REJECTED, SVI_OPT_NOT_CONVERGED) = range(5)
+(SVI_POSIT_OK, SVI_POSIT_TOO_FEW_POINTS, SVI_POSIT_INACCURATE, SVI_POSIT_HIGH_RISK, SVI_POSIT_NOT_CONVERGED) = range(5)
 
 _lib = None
 _others: dict = {}
@@ -138,6 +151,7 @@ def load(path=None):
     lib.svi_config.argtypes = [vp, i32p, i32p, i32p]
     lib.svi_kernels_per_chunk.argtypes = [vp, ci]
     lib.svi_optimize_landmarks.argtypes = [vp, C.POINTER(LandmarkMeasurements), ci, C.POINTER(OptimizeResult)]
+    lib.svi_solve_stereo_posit.argtypes = [vp, C.POINTER(PositProblem), C.POINTER(PositResult)]
     lib.svi_multi_create.argtypes = [C.POINTER(Camera), C.POINTER(Camera), C.POINTER(Params), i32p, ci, C.POINTER(vp)]
     lib.svi_multi_destroy.argtypes = [vp]
     lib.svi_multi_destroy.restype = None

@@ -25,6 +25,7 @@
 #include "binned.cuh"
 #include "harris.cuh"
 #include "landmark_opt.cuh"
+#include "posit.cuh"
 #include "rectify.cuh"
 #include "select.cuh"
 #include "track_plan.cuh"
@@ -1111,6 +1112,7 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     CK(cudaFuncSetAttribute(track_stage2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
     CK(cudaFuncSetAttribute(track_stage2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
     CK(cudaFuncSetAttribute(track_stage3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
+    CK(cudaFuncSetAttribute(stereo_posit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPositSmemBytes));
     // one shared-memory carve-out for every kernel of the pipeline: back-to-back kernels with different
     // carve-outs make the SMs drain and reconfigure between launches
     {
@@ -1732,6 +1734,22 @@ int svi_track_landmarks_stages(svi_ctx* ctx, const uint8_t* img_left, const uint
     return rd;
 }
 
+namespace {
+// the staging pair of svi_optimize_landmarks / svi_solve_stereo_posit: one device buffer + its pinned mirror, grown to
+// twice the need (a tracker's measurement lists get longer frame by frame)
+int reserve_opt(svi_ctx* ctx, size_t total) {
+    if (total <= ctx->opt_bytes) return SVI_SUCCESS;
+    if (ctx->opt_dev) cudaFree(ctx->opt_dev);
+    if (ctx->opt_pin) cudaFreeHost(ctx->opt_pin);
+    ctx->opt_dev = nullptr; ctx->opt_pin = nullptr; ctx->opt_bytes = 0;
+    const size_t want = std::max<size_t>(2 * total, 1u << 20);
+    CK(cudaMalloc(reinterpret_cast<void**>(&ctx->opt_dev), want));
+    CK(cudaMallocHost(reinterpret_cast<void**>(&ctx->opt_pin), want));
+    ctx->opt_bytes = want;
+    return SVI_SUCCESS;
+}
+}  // namespace
+
 int svi_optimize_landmarks(svi_ctx* ctx, const svi_landmark_measurements* in, int n, svi_optimize_result* out) {
     if (!ctx) return SVI_ERR_INVALID;
     if (!in || !out || n < 0 || !out->xyz_world || !out->outcome || !out->average_squared_error)
@@ -1759,15 +1777,7 @@ int svi_optimize_landmarks(svi_ctx* ctx, const svi_landmark_measurements* in, in
     const size_t in_bytes = off;
     const size_t o_xyz = take(sizeof(double) * 3 * n), o_avg = take(sizeof(double) * n), o_it = take(sizeof(int) * (size_t)n), o_out = take((size_t)n);
     const size_t total = off;
-    if (total > ctx->opt_bytes) {   // grows to twice the need: a tracker's measurement lists get longer frame by frame
-        if (ctx->opt_dev) cudaFree(ctx->opt_dev);
-        if (ctx->opt_pin) cudaFreeHost(ctx->opt_pin);
-        ctx->opt_dev = nullptr; ctx->opt_pin = nullptr; ctx->opt_bytes = 0;
-        const size_t want = std::max<size_t>(2 * total, 1u << 20);
-        CK(cudaMalloc(reinterpret_cast<void**>(&ctx->opt_dev), want));
-        CK(cudaMallocHost(reinterpret_cast<void**>(&ctx->opt_pin), want));
-        ctx->opt_bytes = want;
-    }
+    if (const int rc = reserve_opt(ctx, total)) return rc;
     unsigned char* hp = ctx->opt_pin;
     std::memcpy(hp + o_guess, in->xyz_world_guess, sizeof(double) * 3 * n);
     std::memcpy(hp + o_first, in->first, sizeof(int) * ((size_t)n + 1));
@@ -1814,6 +1824,68 @@ int svi_optimize_landmarks(svi_ctx* ctx, const svi_landmark_measurements* in, in
         auto us = [](clk::time_point a, clk::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
         std::fprintf(stderr, "svi_optimize_landmarks n=%d m=%d poses=%d: check + stage inputs %.0f us | copy up, kernel, copy back %.0f us | total %.0f us\n",
                      n, m, in->n_poses, us(t_begin, t_staged), us(t_staged, t_end), us(t_begin, t_end));
+    }
+    return check_overflow(ctx);
+}
+
+int svi_solve_stereo_posit(svi_ctx* ctx, const svi_posit_problem* in, svi_posit_result* out) {
+    if (!ctx) return SVI_ERR_INVALID;
+    if (!in || !out || in->n < 0) return fail(ctx, SVI_ERR_INVALID, "svi_solve_stereo_posit: bad argument");
+    const int n = in->n;
+    if (n > 0 && (!in->xyz_world || !in->uv_left || !in->uv_right)) return fail(ctx, SVI_ERR_INVALID, "svi_solve_stereo_posit: null array");
+    std::memcpy(out->T_world_to_left, in->T_estimate, sizeof(out->T_world_to_left));
+    out->iterations = 0;
+    out->inliers = 0;
+    out->average_squared_error = 0.0;
+    out->risk = 0.0;
+    if (n <= kPositMinimumPoints) {   // !(m_uMinimumPointsForPoseOptimization < uNumberOfMeasurements): fails before any iteration
+        out->outcome = SVI_POSIT_TOO_FEW_POINTS;
+        return SVI_SUCCESS;
+    }
+    CK(cudaSetDevice(ctx->device));
+    using clk = std::chrono::steady_clock;
+    const clk::time_point t_begin = clk::now();
+    // layout: [xyz | uv_left | uv_right] -> [PositOut]
+    size_t off = 0;
+    auto take = [&off](size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
+    const size_t o_xyz = take(sizeof(double) * 3 * (size_t)n), o_uvl = take(sizeof(float) * 2 * (size_t)n), o_uvr = take(sizeof(float) * 2 * (size_t)n);
+    const size_t in_bytes = off;
+    const size_t o_out = take(sizeof(PositOut));
+    if (const int rc = reserve_opt(ctx, off)) return rc;
+    unsigned char* hp = ctx->opt_pin;
+    std::memcpy(hp + o_xyz, in->xyz_world, sizeof(double) * 3 * (size_t)n);
+    std::memcpy(hp + o_uvl, in->uv_left, sizeof(float) * 2 * (size_t)n);
+    std::memcpy(hp + o_uvr, in->uv_right, sizeof(float) * 2 * (size_t)n);
+    PositIn pi{};
+    unsigned char* d = ctx->opt_dev;
+    pi.xyz_world = reinterpret_cast<const double*>(d + o_xyz);
+    pi.uv_left = reinterpret_cast<const float*>(d + o_uvl);
+    pi.uv_right = reinterpret_cast<const float*>(d + o_uvr);
+    std::memcpy(pi.P_left, ctx->cam_l.P, sizeof(pi.P_left));
+    std::memcpy(pi.P_right, ctx->cam_r.P, sizeof(pi.P_right));
+    std::memcpy(pi.T_estimate, in->T_estimate, sizeof(pi.T_estimate));
+    std::memcpy(pi.T_last, in->T_last, sizeof(pi.T_last));
+    std::memcpy(pi.t_imu, in->t_imu, sizeof(pi.t_imu));
+    cudaStream_t s = ctx->lanes[0].stream;
+    const clk::time_point t_staged = clk::now();
+    CK(cudaMemcpyAsync(d, hp, in_bytes, cudaMemcpyHostToDevice, s));
+    stereo_posit_kernel<<<1, kPositThreads, kPositSmemBytes, s>>>(pi, n, reinterpret_cast<PositOut*>(d + o_out));
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(hp + o_out, d + o_out, sizeof(PositOut), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    PositOut po;
+    std::memcpy(&po, hp + o_out, sizeof(po));
+    std::memcpy(out->T_world_to_left, po.T, sizeof(out->T_world_to_left));
+    out->outcome = (uint8_t)po.outcome;
+    out->iterations = po.iterations;
+    out->inliers = po.inliers;
+    out->average_squared_error = po.average_squared_error;
+    out->risk = po.risk;
+    if (ctx->trace) {
+        const clk::time_point t_end = clk::now();
+        auto us = [](clk::time_point a, clk::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
+        std::fprintf(stderr, "svi_solve_stereo_posit n=%d: outcome %d after %d iterations | check + stage inputs %.0f us | copy up, kernel, copy back %.0f us | total %.0f us\n",
+                     n, po.outcome, po.iterations, us(t_begin, t_staged), us(t_staged, t_end), us(t_begin, t_end));
     }
     return check_overflow(ctx);
 }

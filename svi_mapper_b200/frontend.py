@@ -6,6 +6,7 @@ The method names follow the reference's interface for this path
   CTriangulator::getPointTriangulatedInRIGHT  -> StereoFrontend.get_point_triangulated_in_right
   CTriangulator::getPointTriangulatedInLEFT   -> StereoFrontend.get_point_triangulated_in_left
   CTriangulator::getPointInLEFT               -> StereoFrontend.get_point_in_left
+  CSolverStereoPosit::getTransformationWORLDtoLEFT -> StereoFrontend.solve_stereo_posit
   cv::GFTTDetector::detect / BRIEF::compute / BFMatcher::match -> detect / describe / match_hamming
 Every call goes to the GPU through ctypes; nothing here computes on the CPU."""
 from __future__ import annotations
@@ -412,6 +413,36 @@ class StereoFrontend:
         r = _lib.OptimizeResult(_ptr(out["xyz"]), _ptr(out["outcome"]), _ptr(out["average_squared_error"]), _ptr(out["iterations"]))
         self._check(self._lib.svi_optimize_landmarks(self._ctx, C.byref(a), n, C.byref(r)))
         return out
+
+    # reason strings of the outcomes (svi_posit_outcome), as the CPU restatement of the solver names them
+    POSIT_REASONS = {_lib.SVI_POSIT_OK: None, _lib.SVI_POSIT_TOO_FEW_POINTS: "insufficient number of points",
+                     _lib.SVI_POSIT_INACCURATE: "insufficient accuracy", _lib.SVI_POSIT_HIGH_RISK: "inconsistent with prior",
+                     _lib.SVI_POSIT_NOT_CONVERGED: "system did not converge"}
+
+    def solve_stereo_posit(self, xyz_world, uv_left, uv_right, T_estimate, T_last=None, t_imu=None) -> dict:
+        """svi_solve_stereo_posit: CSolverStereoPosit::getTransformationWORLDtoLEFT on the GPU -- the WORLD->LEFT pose from n
+        stereo measurements (xyz_world (n, 3) float64, uv_left / uv_right (n, 2) float32) starting at the prior T_estimate (4, 4).
+        T_last: the previous frame's pose, whose translation a solution within 1 mm of it keeps (default: T_estimate);
+        t_imu: the expected translation for the risk test (default: zero).  Returns dict(T (4, 4): the solution, or T_estimate
+        when the solve failed; outcome (svi_posit_outcome); reason (None or the failure); iterations; inliers;
+        average_squared_error; risk)."""
+        xw = np.ascontiguousarray(np.asarray(xyz_world, np.float64).reshape(-1, 3))
+        n = len(xw)
+        ul = np.ascontiguousarray(np.asarray(uv_left, np.float32).reshape(n, 2))
+        ur = np.ascontiguousarray(np.asarray(uv_right, np.float32).reshape(n, 2))
+        Te = np.asarray(T_estimate, np.float64).reshape(16)
+        Tl = Te if T_last is None else np.asarray(T_last, np.float64).reshape(16)
+        ti = np.zeros(3) if t_imu is None else np.asarray(t_imu, np.float64).reshape(3)
+        prob = _lib.PositProblem(n, _ptr(xw) if n else None, _ptr(ul) if n else None, _ptr(ur) if n else None)
+        for i in range(16):
+            prob.T_estimate[i], prob.T_last[i] = float(Te[i]), float(Tl[i])
+        for i in range(3):
+            prob.t_imu[i] = float(ti[i])
+        res = _lib.PositResult()
+        self._check(self._lib.svi_solve_stereo_posit(self._ctx, C.byref(prob), C.byref(res)))
+        return dict(T=np.array(res.T_world_to_left[:], np.float64).reshape(4, 4), outcome=int(res.outcome),
+                    reason=self.POSIT_REASONS[int(res.outcome)], iterations=int(res.iterations), inliers=int(res.inliers),
+                    average_squared_error=float(res.average_squared_error), risk=float(res.risk))
 
     # -- profiling
     def set_profiling(self, enable):

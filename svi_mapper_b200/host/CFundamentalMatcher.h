@@ -252,7 +252,7 @@ public:
         : m_pGpu(p_pGpu), m_pTriangulator(std::make_shared<CTriangulator>(p_pCameraSTEREO, p_pGpu)), m_pCameraLEFT(p_pCameraSTEREO->m_pCameraLEFT),
           m_pCameraRIGHT(p_pCameraSTEREO->m_pCameraRIGHT), m_pCameraSTEREO(p_pCameraSTEREO), m_dMinimumDepthMeters(m_pTriangulator->dDepthMinimumMeters),
           m_dMaximumDepthMeters(m_pTriangulator->dDepthMaximumMeters),
-          m_cSolverSterePosit(p_pCameraSTEREO->m_pCameraLEFT->m_matProjection, p_pCameraSTEREO->m_pCameraRIGHT->m_matProjection) {}
+          m_cSolverSterePosit(p_pCameraSTEREO->m_pCameraLEFT->m_matProjection, p_pCameraSTEREO->m_pCameraRIGHT->m_matProjection, p_pGpu) {}
     ~CFundamentalMatcher() { for (CLandmark* p : m_vecLandmarksWINDOW) delete p; }
 
     const std::shared_ptr<CTriangulator> getTriangulator() const { return m_pTriangulator; }
@@ -508,7 +508,7 @@ public:
     }
 
     // getPoseStereoPosit :338-757: stages 1 and 2 on every OPTIMAL landmark around the pose estimate (one GPU call), the
-    // measurements go to CSolverStereoPosit (CExceptionPoseOptimization on failure, as in the reference), then the
+    // measurements go to CSolverStereoPosit (one more GPU call; CExceptionPoseOptimization on failure, as in the reference), then the
     // landmarks receive their measurement under the optimised pose.
     const Isometry3d getPoseStereoPosit(const UIDFrame p_uFrame, const ImageView& p_matImageLEFT, const ImageView& p_matImageRIGHT,
                                         const Isometry3d& p_matTransformationEstimateWORLDtoLEFT, const Isometry3d& p_matTransformationWORLDtoLEFTLAST,
@@ -545,6 +545,7 @@ public:
         return matTransformationWORLDtoLEFT;
     }
     const std::vector<CSolverStereoPosit::CMatch>& getMeasurementsStereoPositLAST() const { return m_vecMeasurementsStereoPositLAST; }
+    const CSolverStereoPosit& getSolverStereoPosit() const { return m_cSolverSterePosit; }
 
     // trackEpipolar :760-1332: the landmarks getPoseStereoPosit did not see.  Where the camera has moved since the
     // landmark's detection: the epipolar search (stage 3) alone; otherwise: the regional search (stage 2) behind the

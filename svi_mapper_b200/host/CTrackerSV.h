@@ -7,6 +7,8 @@
 #ifndef SVI_HOST_CTRACKERSV_H
 #define SVI_HOST_CTRACKERSV_H
 
+#include <chrono>
+
 #include "CFundamentalMatcher.h"
 
 // Pinned arithmetic: every product and sum below rounds on its own, in the written order (the GPU kernels and the CPU
@@ -48,6 +50,7 @@ public:
         auto norm = [](const CPoint3D& v) { return std::sqrt(v.x() * v.x() + v.y() * v.y() + v.z() * v.z()); };
         const double dMotionScaling = std::min(1.0 + (10.0 * norm(vecRotationTotal) + 0.5 * norm(vecTranslationTotal)), 5.0);   // :254
 
+        const auto tStart = std::chrono::steady_clock::now();
         m_cMatcher.resetVisibilityActiveLandmarks();                                                                           // :257
         Isometry3d matTransformationWORLDtoLEFT(matEstimate);
         m_strPoseSource = "posit";
@@ -68,6 +71,7 @@ public:
                 matTransformationWORLDtoLEFT = matEstimateParallel;                                                            // :313
             }
         }
+        const auto tPose = std::chrono::steady_clock::now();
         const Isometry3d matTransformationLEFTtoWORLD(inverseIsometry(matTransformationWORLDtoLEFT));
         m_cMatcher.trackEpipolar(m_uFrameCount, p_matImageLEFT, p_matImageRIGHT, matTransformationWORLDtoLEFT, matTransformationLEFTtoWORLD,
                                  dMotionScaling);                                                                              // :320-327
@@ -76,7 +80,9 @@ public:
             0.75 < (double)((int64_t)m_uNumberofVisibleLandmarksLAST - iVisible) / (double)m_uNumberofVisibleLandmarksLAST && 20 > m_uCountInstability)
             m_uCountInstability += 5;                                                                                          // :333-349
         m_uNumberofVisibleLandmarksLAST = (uint64_t)iVisible;
+        const auto tEpipolar = std::chrono::steady_clock::now();
         if (0 == m_uFrameCount % m_uLandmarkOptimizationEveryNFrames) m_cMatcher.optimizeActiveLandmarks(m_uFrameCount);       // :362-365
+        const auto tOptimized = std::chrono::steady_clock::now();
         if (m_uVisibleLandmarksMinimum > m_uNumberofVisibleLandmarksLAST || m_uMaximumNumberOfFramesWithoutDetection < m_uNumberOfFramesWithoutDetection) {
             m_uNumberofVisibleLandmarksLAST = m_cMatcher.addNewLandmarks(p_matImageLEFT, p_matImageRIGHT, matTransformationWORLDtoLEFT,
                                                                          matTransformationLEFTtoWORLD, m_uFrameCount);         // :468-473
@@ -85,10 +91,24 @@ public:
         } else {
             ++m_uNumberOfFramesWithoutDetection;
         }
+        // the reference keeps such timers too (m_dDurationTotalSeconds*), see CTrackerGT
+        const auto tEnd = std::chrono::steady_clock::now();
+        m_dDurationPoseSeconds += std::chrono::duration<double>(tPose - tStart).count();
+        m_dDurationTrackEpipolarSeconds += std::chrono::duration<double>(tEpipolar - tPose).count();
+        m_dDurationOptimizationSeconds += std::chrono::duration<double>(tOptimized - tEpipolar).count();
+        m_dDurationDetectionSeconds += std::chrono::duration<double>(tEnd - tOptimized).count();
         ++m_uFrameCount;
         m_matTransformationLEFTLASTtoLEFTNOW = matTransformationWORLDtoLEFT * inverseIsometry(m_matTransformationWORLDtoLEFTLAST);   // :547
         m_matTransformationWORLDtoLEFTLAST = matTransformationWORLDtoLEFT;                                                     // :548
     }
+
+    // wall time: the pose stage (getPoseStereoPosit incl. its fallback: stages 1-2 tracking and the solves), the solves alone
+    // (CSolverStereoPosit, failed ones included), trackEpipolar, landmark optimisation, re-detection
+    double getDurationPoseSeconds() const { return m_dDurationPoseSeconds; }
+    double getDurationPoseSolverSeconds() const { return m_cMatcher.getSolverStereoPosit().getDurationSeconds(); }
+    double getDurationTrackEpipolarSeconds() const { return m_dDurationTrackEpipolarSeconds; }
+    double getDurationOptimizationSeconds() const { return m_dDurationOptimizationSeconds; }
+    double getDurationDetectionSeconds() const { return m_dDurationDetectionSeconds; }
 
     CFundamentalMatcher& getMatcher() { return m_cMatcher; }
     UIDFrame getFrameCount() const { return m_uFrameCount; }
@@ -109,6 +129,7 @@ private:
     const UIDFrame m_uMaximumNumberOfFramesWithoutDetection = 2;     // CTrackerSV.h:62
     const uint8_t m_uLandmarkOptimizationEveryNFrames = 10;          // CTrackerSV.h:79
     UIDFrame m_uNumberOfFramesWithoutDetection = 0;
+    double m_dDurationPoseSeconds = 0.0, m_dDurationTrackEpipolarSeconds = 0.0, m_dDurationOptimizationSeconds = 0.0, m_dDurationDetectionSeconds = 0.0;
 };
 
 #if defined(__GNUC__) && !defined(__clang__)

@@ -5,6 +5,12 @@
 // drives the SV/SVI entry points getPoseStereoPosit and trackEpipolar (src/core/CTrackerSV.cpp:274,324).
 //        facade_demo --solver <left_calib> <right_calib> <matches.txt>
 // CSolverStereoPosit alone (no GPU work): matches.txt holds "x y z uL vL uR vR" per line, the pose goes to stdout.
+//        facade_demo --posit <left_calib> <right_calib> <problem.txt>
+// CSolverStereoPosit with arbitrary priors, on the GPU (SVI_HOST_POSIT=cpu: the CPU loop, no GPU needed): problem.txt holds
+// T_estimate (16 numbers), T_last (16), t_imu (3), then "x y z uL vL uR vR" per line; prints the 12 pose numbers and the
+// iteration count, or FAILED <what()>.
+//        facade_demo --sequence-sv <left_calib> <right_calib> <n> <L.raw> <R.raw> <max_corners> <out.txt>
+// CTrackerSV::process over n frames without any pose given (see sequenceSVMain).
 //        facade_demo --landmark <measurements.txt>
 // CLandmark::optimize alone (no GPU work): first line "x y z" = first triangulation in the camera frame of measurement 0,
 // then per line 16 numbers of LEFTtoWORLD... see landmarkMain; prints "x y z optimal successful failed".
@@ -45,6 +51,51 @@ static int solverMain(char** argv) {
         for (int i = 0; i < 12; ++i) std::printf("%.17g%c", T.m[i], i == 11 ? '\n' : ' ');
     } catch (const CExceptionPoseOptimization& e) {
         std::printf("FAILED %s\n", e.what());
+    } catch (const std::exception& e) {
+        std::fprintf(stderr, "facade_demo failed: %s\n", e.what());
+        return 1;
+    }
+    return 0;
+}
+
+static int positMain(char** argv) {
+    try {
+        CParameterBase::loadCameraLEFT(argv[2]);
+        CParameterBase::loadCameraRIGHT(argv[3]);
+        CParameterBase::constructCameraSTEREO(CPoint3D(-0.54, 0.0, 0.0));
+        const char* e = std::getenv("SVI_HOST_POSIT");
+        const bool bCPU = e && std::string(e) == "cpu";
+        const std::shared_ptr<CGpuContext> pGpu(bCPU ? nullptr : std::make_shared<CGpuContext>(CParameterBase::pCameraSTEREO));
+        CSolverStereoPosit cSolver(CParameterBase::pCameraLEFT->m_matProjection, CParameterBase::pCameraRIGHT->m_matProjection, pGpu);
+        std::ifstream f(argv[4]);
+        Isometry3d matEstimate, matLast;
+        CPoint3D vecTranslationIMU;
+        for (double& d : matEstimate.m) f >> d;
+        for (double& d : matLast.m) f >> d;
+        for (double& d : vecTranslationIMU.v) f >> d;
+        if (!f) throw std::invalid_argument("malformed problem file");
+        std::vector<CSolverStereoPosit::CMatch> vecMatches;
+        double x, y, z;
+        float uL, vL, uR, vR;
+        while (f >> x >> y >> z >> uL >> vL >> uR >> vR)
+            vecMatches.push_back(CSolverStereoPosit::CMatch(nullptr, CPoint3D(x, y, z), CPoint3D(), Point2f(uL, vL), Point2f(uR, vR), CDescriptor(), CDescriptor()));
+        try {
+            const Isometry3d T(cSolver.getTransformationWORLDtoLEFT(matLast, vecTranslationIMU, matEstimate, vecMatches));
+            for (int i = 0; i < 12; ++i) std::printf("%.17g ", T.m[i]);
+            std::printf("%u\n", cSolver.getIterationsLAST());
+        } catch (const CExceptionPoseOptimization& e) {
+            std::printf("FAILED %s\n", e.what());
+        }
+        if (const char* pTiming = std::getenv("SVI_DEMO_TIMING")) {   // the same solve SVI_DEMO_TIMING more times: median wall time of one call
+            std::vector<double> vecMicroseconds;
+            for (int k = std::max(1, std::atoi(pTiming)); k > 0; --k) {
+                const auto t0 = std::chrono::steady_clock::now();
+                try { cSolver.getTransformationWORLDtoLEFT(matLast, vecTranslationIMU, matEstimate, vecMatches); } catch (const CExceptionPoseOptimization&) {}
+                vecMicroseconds.push_back(std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t0).count());
+            }
+            std::sort(vecMicroseconds.begin(), vecMicroseconds.end());
+            std::printf("{\"calls\": %zu, \"median_us\": %.3f, \"min_us\": %.3f}\n", vecMicroseconds.size(), vecMicroseconds[vecMicroseconds.size() / 2], vecMicroseconds[0]);
+        }
     } catch (const std::exception& e) {
         std::fprintf(stderr, "facade_demo failed: %s\n", e.what());
         return 1;
@@ -267,12 +318,89 @@ static int sequenceMain(char** argv, bool p_bRectify) {
     return 0;
 }
 
+// --sequence-sv <left_calib> <right_calib> <n> <L.raw> <R.raw> <max_corners> <out.txt>: n frames through CTrackerSV::process --
+// the stereo-only tracker, no pose given: each frame's pose comes from getPoseStereoPosit (CSolverStereoPosit on the GPU;
+// SVI_HOST_POSIT=cpu: the CPU loop).  Prints, per frame, the pose source, the counters and the 12 numbers of T_WORLDtoLEFT,
+// then the M / A lines of --sequence.  With SVI_DEMO_TIMING set ONE line goes to stdout instead: the wall time of every
+// process() call (frames after the first three), split into pose stage (tracking + solves), solves alone, trackEpipolar,
+// landmark optimisation and re-detection.
+static int sequenceSVMain(char** argv) {
+    try {
+        CParameterBase::loadCameraLEFT(argv[2]);
+        CParameterBase::loadCameraRIGHT(argv[3]);
+        CParameterBase::constructCameraSTEREO(CPoint3D(-0.54, 0.0, 0.0));
+        const int W = (int)CParameterBase::pCameraLEFT->m_uWidthPixel, H = (int)CParameterBase::pCameraLEFT->m_uHeightPixel;
+        const int n = std::atoi(argv[4]);
+        const std::vector<uint8_t> L = readRaw(argv[5], (size_t)n * W * H), R = readRaw(argv[6], (size_t)n * W * H);
+        svi_params p;
+        svi_params_default(&p);
+        p.max_corners = std::atoi(argv[7]);
+        auto pGpu = std::make_shared<CGpuContext>(CParameterBase::pCameraSTEREO, &p);
+        CTrackerSV cTracker(CParameterBase::pCameraSTEREO, pGpu);
+        const bool bTiming = std::getenv("SVI_DEMO_TIMING") != nullptr;
+        std::FILE* out = bTiming ? nullptr : std::fopen(argv[8], "w");
+        std::vector<double> vecFrameMilliseconds;
+        double dWarm[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+        auto durations = [&cTracker](double (&d)[5]) {
+            d[0] = cTracker.getDurationPoseSeconds(); d[1] = cTracker.getDurationPoseSolverSeconds(); d[2] = cTracker.getDurationTrackEpipolarSeconds();
+            d[3] = cTracker.getDurationOptimizationSeconds(); d[4] = cTracker.getDurationDetectionSeconds();
+        };
+        size_t uMeasurementsPosit = 0, uFramesPosit = 0;
+        for (int t = 0; t < n; ++t) {
+            if (t == 3) durations(dWarm);
+            const auto t0 = std::chrono::steady_clock::now();
+            cTracker.process(ImageView(L.data() + (size_t)t * W * H, W, H), ImageView(R.data() + (size_t)t * W * H, W, H));
+            CFundamentalMatcher& m = cTracker.getMatcher();
+            if (t >= 3) {
+                vecFrameMilliseconds.push_back(std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
+                uMeasurementsPosit += m.getMeasurementsStereoPositLAST().size();
+                ++uFramesPosit;
+            }
+            if (bTiming) continue;
+            const Isometry3d& T = cTracker.getTransformationWORLDtoLEFT();
+            std::fprintf(out, "F %d POSE %s VISIBLE %lu ACTIVE %zu S1 %lu S2 %lu S3 %lu S22 %lu DETECTIONS %lu INSTABILITY %d POSIT %zu T", t,
+                         cTracker.getPoseSource().c_str(), (unsigned long)cTracker.getNumberOfVisibleLandmarksLAST(), m.getNumberOfActiveLandmarks(),
+                         (unsigned long)m.getNumberOfTracksStage1(), (unsigned long)m.getNumberOfTracksStage2_1(), (unsigned long)m.getNumberOfTracksStage3(),
+                         (unsigned long)m.getNumberOfTracksStage2_2(), (unsigned long)cTracker.getNumberOfDetections(), (int)cTracker.getCountInstability(),
+                         m.getMeasurementsStereoPositLAST().size());
+            for (int i = 0; i < 12; ++i) std::fprintf(out, " %.17g", T.m[i]);
+            std::fprintf(out, "\n");
+            for (const CMeasurementLandmark* q : m.getMeasurementsForVisibleLandmarks())
+                std::fprintf(out, "M %lu %.9g %.9g %.9g %.9g %.17g %.17g %.17g\n", (unsigned long)q->uID, q->ptUVLEFT.x, q->ptUVLEFT.y, q->ptUVRIGHT.x,
+                             q->ptUVRIGHT.y, q->vecPointXYZLEFT.x(), q->vecPointXYZLEFT.y(), q->vecPointXYZLEFT.z());
+            for (const CLandmark* q : m.getActiveLandmarks())
+                std::fprintf(out, "A %lu %.17g %.17g %.17g %d %d %u %u %u %zu\n", (unsigned long)q->uID, q->vecPointXYZOptimized.x(), q->vecPointXYZOptimized.y(),
+                             q->vecPointXYZOptimized.z(), (int)q->bIsOptimal, (int)q->bIsCurrentlyVisible, q->uOptimizationsSuccessful, q->uOptimizationsFailed,
+                             (unsigned)q->uFailedSubsequentTrackings, q->getNumberOfMeasurements());
+        }
+        if (out) std::fclose(out);
+        if (bTiming && !vecFrameMilliseconds.empty()) {
+            double dTotal = 0.0, dNow[5];
+            for (const double d : vecFrameMilliseconds) dTotal += d;
+            std::vector<double> vecSorted(vecFrameMilliseconds);
+            std::sort(vecSorted.begin(), vecSorted.end());
+            durations(dNow);
+            std::printf("{\"frames\": %zu, \"total_ms\": %.4f, \"median_ms\": %.4f, \"pose_ms\": %.4f, \"pose_solver_ms\": %.4f, \"track_epipolar_ms\": %.4f, "
+                        "\"optimize_ms\": %.4f, \"add_new_landmarks_ms\": %.4f, \"posit_measurements_mean\": %.1f, \"detections\": %lu}\n",
+                        vecFrameMilliseconds.size(), dTotal, vecSorted[vecSorted.size() / 2], 1e3 * (dNow[0] - dWarm[0]), 1e3 * (dNow[1] - dWarm[1]),
+                        1e3 * (dNow[2] - dWarm[2]), 1e3 * (dNow[3] - dWarm[3]), 1e3 * (dNow[4] - dWarm[4]),
+                        (double)uMeasurementsPosit / (double)std::max<size_t>(1, uFramesPosit), (unsigned long)cTracker.getNumberOfDetections());
+        }
+    } catch (const std::exception& e) {
+        std::fprintf(stderr, "facade_demo failed: %s\n", e.what());
+        return 1;
+    }
+    return 0;
+}
+
 int main(int argc, char** argv) {
     if (argc == 10 && std::string(argv[1]) == "--sequence") return sequenceMain(argv, false);
     if (argc == 11 && std::string(argv[1]) == "--sequence" && std::string(argv[2]) == "--rectify") {
         return sequenceMain(argv + 1, true);   // the remaining arguments keep their positions
     }
     if (argc == 5 && std::string(argv[1]) == "--solver") return solverMain(argv);
+    if (argc == 5 && std::string(argv[1]) == "--posit") return positMain(argv);
+    if (argc == 9 && std::string(argv[1]) == "--sequence-sv") return sequenceSVMain(argv);
     if (argc == 6 && std::string(argv[1]) == "--mask") return maskMain(argv);
     if (argc == 3 && std::string(argv[1]) == "--landmark") return landmarkMain(argv);
     if (argc == 5 && std::string(argv[1]) == "--cloud") return cloudMain(argv);
