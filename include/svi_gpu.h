@@ -355,6 +355,52 @@ typedef struct svi_posit_result {
 } svi_posit_result;
 int svi_solve_stereo_posit(svi_ctx* ctx, const svi_posit_problem* in, svi_posit_result* out);
 
+/* ---- one frame of the stereo-only tracker in one call.
+ * CTrackerSV::process (src/core/CTrackerSV.cpp:143-172, :234-552) between the pose prior and the landmark bookkeeping, with exactly
+ * the semantics of the composed calls CFundamentalMatcher::getPoseStereoPosit / trackEpipolar make:
+ *   1. stages 1 and 2 (svi_track_landmarks_stages, SVI_STAGE_1 | SVI_STAGE_2) around T_estimate on the pose candidates (flags bit 0,
+ *      in caller order), then svi_solve_stereo_posit on their hits in that order;
+ *   2. if that solve fails, the same with T_estimate_damped; if that fails too, the pose is T_estimate_damped;
+ *   3. every landmark that is neither a pose hit of an accepted solve nor flagged bit 1 goes to the epipolar stage: stage 3 alone
+ *      when the translation of T_world_to_left * T_left_to_world_at_detection has a non-zero squared norm (evaluated as the host's
+ *      Isometry3d::operator* and CFundamentalMatcher.h:561-563 do it: fp64, no contraction), else, and for stage-3 items that come
+ *      back SVI_EPI_NO_TRANSLATION, stage 2 alone (the regional search, behind its field-of-view gate).
+ * The images are staged (and rectified, while svi_set_rectification is set) once, the landmark arrays go up in one copy and the
+ * results come back in one copy.  The subsets are index lists built on the device.  The host waits for the outcome of each solve
+ * that runs (a few hundred bytes: one or two waits), once for the size of the regional set, and once at the end for the results. */
+enum { SVI_SV_POSE_CANDIDATE = 1,   /* flags bit 0: bIsOptimal                                                           */
+       SVI_SV_LEAVES = 2 };         /* flags bit 1: leaves in trackEpipolar (uOptimizationsFailed > 0, or
+                                       uOptimizationsSuccessful > 0 && !bIsOptimal, :808-825)                             */
+enum svi_sv_source { SVI_SV_POSIT = 0, SVI_SV_POSIT_DAMPED = 1, SVI_SV_PRIOR = 2 };
+enum svi_sv_route {                 /* one per landmark                                                                  */
+    SVI_SV_ROUTE_POSE = 1,          /* stage-1/2 hit of the accepted solve: measured in the pose stage (also if bit 1)    */
+    SVI_SV_ROUTE_EPIPOLAR = 2,      /* stage 3                                                                           */
+    SVI_SV_ROUTE_REGIONAL = 3,      /* stage 2: no translation since detection                                          */
+    SVI_SV_ROUTE_REGIONAL_NO_TRANSLATION = 4, /* stage 2 after stage 3 returned SVI_EPI_NO_TRANSLATION                    */
+    SVI_SV_ROUTE_DROPPED = 5        /* bit 1 and not a pose hit: not tracked                                             */
+};
+typedef struct svi_sv_frame {
+    svi_landmarks landmarks;        /* all active landmarks, in the tracker's order; the three stage-3 arrays are required */
+    const uint8_t* flags;           /* [n] SVI_SV_POSE_CANDIDATE | SVI_SV_LEAVES; other bits are refused                 */
+    double T_estimate[16];          /* constant-velocity prior, row-major                                               */
+    double T_estimate_damped[16];   /* rotation-only prior: the second attempt, and the pose when both solves fail       */
+    double T_last[16];              /* pose of the previous frame (the solver's translation clamp)                      */
+    double t_imu[3];                /* the solver's risk test                                                           */
+    double motion_scaling;
+} svi_sv_frame;
+typedef struct svi_sv_frame_result {
+    double T_world_to_left[16];     /* the frame's pose                                                                 */
+    uint8_t source;                 /* svi_sv_source                                                                    */
+    int32_t attempts;               /* solves that ran: 1 or 2                                                          */
+    svi_posit_result attempt[2];    /* as svi_solve_stereo_posit returns them; fields an outcome does not compute are 0  */
+    int32_t measurements[2];        /* stage-1/2 hits of each attempt: the problem size of its solve                    */
+    svi_track_result pose_stage;    /* [n] stages 1-2 of the LAST attempt that ran (all zero for non-candidates)        */
+    uint8_t* route;                 /* [n] svi_sv_route                                                                 */
+    svi_track_result epipolar_stage; /* [n] stage 3 or the regional stage 2 (all zero where neither ran)                */
+} svi_sv_frame_result;
+int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uint8_t* img_right, size_t pitch, const svi_sv_frame* in, int n,
+                                svi_sv_frame_result* out);
+
 /* Stage profiling: when enabled, every kernel of the new-landmark path is bracketed by CUDA events
  * on the stream it is launched on (the events come from a pool filled here, none is created while
  * work is being timed).  enable = 1: the lanes keep overlapping, a bracket also contains other lanes'

@@ -135,8 +135,7 @@ constexpr int kPositTerms = 28;
 constexpr int kPositTermPitch = 29;   // doubles per measurement slot: odd pitch, parked rows do not collide on one bank
 constexpr size_t kPositSmemBytes = sizeof(double) * kPositThreads * kPositTermPitch;   // dynamic: the term slots
 
-__global__ void __launch_bounds__(kPositThreads)
-stereo_posit_kernel(PositIn in, int n, PositOut* out) {
+__device__ __forceinline__ void stereo_posit_body(const PositIn& in, int n, PositOut* out) {
     extern __shared__ double s_term[];          // [kPositThreads][kPositTermPitch]
     __shared__ double s_T[16];                  // current pose WORLD->LEFT
     __shared__ double s_sum[kPositTerms];       // H upper triangle row by row | b | total error
@@ -275,6 +274,34 @@ stereo_posit_kernel(PositIn in, int n, PositOut* out) {
         for (int k = 0; k < 16; ++k) out->T[k] = ok ? s_T[k] : in.T_estimate[k];
         out->outcome = s_state;
     }
+}
+
+__global__ void __launch_bounds__(kPositThreads)
+stereo_posit_kernel(PositIn in, int n, PositOut* out) {
+    stereo_posit_body(in, n, out);
+}
+
+// The same solve with the measurement count read from device memory (svi_track_frame_stereo_only assembles the problem on the
+// device).  n <= kPositMinimumPoints is answered here as svi_solve_stereo_posit answers it on the host, without an iteration;
+// every field of *out is written, the ones an outcome does not compute as 0.
+__global__ void __launch_bounds__(kPositThreads)
+stereo_posit_count_kernel(PositIn in, const int* n_dev, PositOut* out) {
+    const int n = *n_dev;
+    if (threadIdx.x == 0) {
+        out->iterations = 0;
+        out->inliers = 0;
+        out->average_squared_error = 0.0;
+        out->risk = 0.0;
+    }
+    if (n <= kPositMinimumPoints) {   // uniform over the CTA
+        if (threadIdx.x == 0) {
+#pragma unroll
+            for (int k = 0; k < 16; ++k) out->T[k] = in.T_estimate[k];
+            out->outcome = 1;   // SVI_POSIT_TOO_FEW_POINTS
+        }
+        return;
+    }
+    stereo_posit_body(in, n, out);
 }
 
 }  // namespace svi

@@ -28,6 +28,7 @@
 #include "posit.cuh"
 #include "rectify.cuh"
 #include "select.cuh"
+#include "sv_frame.cuh"
 #include "track_plan.cuh"
 
 using namespace svi;
@@ -854,15 +855,69 @@ int track_stage2_side(svi_ctx* ctx, Lane& l, const FrameGeom& g, int n, const do
 // Stage 3 (epipolar line in LEFT): line geometry per landmark in stage3_plan_kernel (:1795-1947), sampling / matching /
 // triangulation in track_stage3_kernel, both enqueued on the lane's stream.
 int track_stage3_all(svi_ctx* ctx, Lane& l, const FrameGeom& g, int n, const double* T, double motion_scaling, const LandmarksDev& ld,
-                     const Stage3Extra& ex, const uint8_t* d_orig, const TrackOutDev& o) {
+                     const Stage3Extra& ex, const uint8_t* d_orig, const TrackOutDev& o, const int* n_dev) {
     cudaStream_t s = l.stream;
     int* n_items = ctx->roi.counters + 2;
     const TrackPlanConst k = make_plan(ctx, T, ctx->cam_l, motion_scaling);
     CK(cudaMemsetAsync(n_items, 0, sizeof(int), s));
-    stage3_plan_kernel<<<(n + 127) / 128, 128, 0, s>>>(k, ld, ex, n, o, ctx->s3_items, n_items);
+    stage3_plan_kernel<<<(n + 127) / 128, 128, 0, s>>>(k, ld, ex, n, n_dev, o, ctx->s3_items, n_items);
     track_stage3_kernel<<<(n + MATCH_WARPS - 1) / MATCH_WARPS, MATCH_WARPS * 32, MATCH_SMEM, s>>>(
         l.box_l, l.map_r, l.map_rs, g, ctx->tc, ctx->p.cutoff_stage3, ctx->p.cutoff_original, ctx->s3_items, n_items, d_orig, ld, o);
     CK(cudaGetLastError());
+    return SVI_SUCCESS;
+}
+
+// Both images of the pair into the tracking planes of lane 0 (rectified first while svi_set_rectification is set) with their box
+// sums: RIGHT goes up and gets its box sums on the side stream, beside LEFT's; lane 0's stream waits for both.
+int stage_track_pair(svi_ctx* ctx, const uint8_t* img_left, const uint8_t* img_right, size_t pitch) {
+    Lane& l = ctx->lanes[0];
+    cudaStream_t s = l.stream;
+    const size_t plane = (size_t)ctx->H * ctx->dev_pitch;
+    // both images as planes 0 / 1 of one buffer (the window-mode detector indexes them by plane)
+    CK(cudaEventRecord(ctx->fork, s));
+    CK(cudaStreamWaitEvent(ctx->side, ctx->fork, 0));
+    int rc = stage_box(ctx, img_right, pitch, ctx->trk_img + plane, l.box_r, l.box_rs, ctx->side, 1, 1);
+    if (rc == SVI_SUCCESS) rc = stage_box(ctx, img_left, pitch, ctx->trk_img, l.box_l, l.box_ls, s, 0);
+    if (cudaEventRecord(ctx->side_done, ctx->side) != cudaSuccess || cudaStreamWaitEvent(s, ctx->side_done, 0) != cudaSuccess)
+        rc = rc == SVI_SUCCESS ? fail(ctx, SVI_ERR_CUDA, "svi_track_landmarks: joining the side stream failed") : rc;
+    if (rc != SVI_SUCCESS) { cudaStreamSynchronize(ctx->side); cudaStreamSynchronize(s); }
+    return rc;
+}
+
+// The tracking cascade restricted to stage_mask on n device-resident landmarks whose outputs `o` are zeroed, entirely enqueued on
+// lane 0's stream after the images staged by stage_track_pair: every stage reads the stage / status bytes the previous one left on
+// the device and plans its own work items there.  n_dev (stage 3 alone, may be null): the landmark count when only the device
+// knows it, n is then its upper bound.
+int enqueue_cascade(svi_ctx* ctx, int n, const double* T_world_to_left, double motion_scaling, uint32_t stage_mask, const LandmarksDev& ld,
+                    const Stage3Extra& ex, const uint8_t* d_orig, const TrackOutDev& o, const int* n_dev) {
+    Lane& l = ctx->lanes[0];
+    cudaStream_t s = l.stream;
+    TrackConst k;
+    for (int i = 0; i < 12; ++i) { k.T[i] = T_world_to_left[i]; k.PL[i] = ctx->cam_l.P[i]; k.PR[i] = ctx->cam_r.P[i]; }
+    k.tri_scale = (float)(1.0 + motion_scaling);
+    k.cutoff1 = ctx->p.cutoff_stage1;
+    k.stage1_match = (stage_mask & SVI_STAGE_1) ? 1 : 0;
+    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
+    if (stage_mask & (SVI_STAGE_1 | SVI_STAGE_2)) {
+        // ---- stage 1 LEFT / RIGHT for every landmark (or only its field-of-view gate when stage 2 runs alone)
+        track_stage1_kernel<<<(n + MATCH_WARPS - 1) / MATCH_WARPS, MATCH_WARPS * 32, MATCH_SMEM, s>>>(l.box_l, l.box_r, l.map_l, l.map_ls, l.map_r, l.map_rs, g,
+                                                                                                      ctx->tc, k, ld, n, o);
+        CK(cudaGetLastError());
+    } else {
+        // stage 3 alone (trackEpipolar :828-1020): no gate, every landmark is an untracked candidate
+        CK(cudaMemsetAsync(o.status, SVI_TRK_STAGE1_DIST, (size_t)n, s));
+        CK(cudaMemsetAsync(o.stage, 0, (size_t)n, s));
+    }
+    // ---- stage 2 LEFT, then stage 2 RIGHT, for what is still untracked
+    for (int side = 0; side < 2 && (stage_mask & SVI_STAGE_2); ++side) {
+        const int rc = track_stage2_side(ctx, l, g, n, T_world_to_left, motion_scaling, side == 0, ld, o);
+        if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); return rc; }
+    }
+    // ---- stage 3 (epipolar line in LEFT)
+    if (stage_mask & SVI_STAGE_3) {
+        const int rc = track_stage3_all(ctx, l, g, n, T_world_to_left, motion_scaling, ld, ex, d_orig, o, n_dev);
+        if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); return rc; }
+    }
     return SVI_SUCCESS;
 }
 
@@ -1113,6 +1168,7 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     CK(cudaFuncSetAttribute(track_stage2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
     CK(cudaFuncSetAttribute(track_stage3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
     CK(cudaFuncSetAttribute(stereo_posit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPositSmemBytes));
+    CK(cudaFuncSetAttribute(stereo_posit_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPositSmemBytes));
     // one shared-memory carve-out for every kernel of the pipeline: back-to-back kernels with different
     // carve-outs make the SMs drain and reconfigure between launches
     {
@@ -1617,23 +1673,14 @@ int svi_track_landmarks_stages(svi_ctx* ctx, const uint8_t* img_left, const uint
     CK(cudaSetDevice(ctx->device));
     int rc = ensure_track_scratch(ctx);
     if (rc != SVI_SUCCESS) return rc;
-    Lane& l = ctx->lanes[0];
-    cudaStream_t s = l.stream;
+    cudaStream_t s = ctx->lanes[0].stream;
     ctx->arena_used = 0; ctx->pending.clear();
     using clk = std::chrono::steady_clock;
     clk::time_point tp[6];
     auto tick = [&](int i) { if (ctx->trace) tp[i] = clk::now(); };
     tick(0);
-    const size_t plane = (size_t)ctx->H * ctx->dev_pitch;
-    // both images as planes 0 / 1 of one buffer (the window-mode detector indexes them by plane)
-    // (RIGHT goes up and gets its box sums on the side stream, beside LEFT's)
-    CK(cudaEventRecord(ctx->fork, s));
-    CK(cudaStreamWaitEvent(ctx->side, ctx->fork, 0));
-    rc = stage_box(ctx, img_right, pitch, ctx->trk_img + plane, l.box_r, l.box_rs, ctx->side, 1, 1);
-    if (rc == SVI_SUCCESS) rc = stage_box(ctx, img_left, pitch, ctx->trk_img, l.box_l, l.box_ls, s, 0);
-    if (cudaEventRecord(ctx->side_done, ctx->side) != cudaSuccess || cudaStreamWaitEvent(s, ctx->side_done, 0) != cudaSuccess)
-        rc = rc == SVI_SUCCESS ? fail(ctx, SVI_ERR_CUDA, "svi_track_landmarks: joining the side stream failed") : rc;
-    if (rc != SVI_SUCCESS) { cudaStreamSynchronize(ctx->side); cudaStreamSynchronize(s); return rc; }
+    rc = stage_track_pair(ctx, img_left, img_right, pitch);
+    if (rc != SVI_SUCCESS) return rc;
     // every input array goes through the pinned mirror of the arena and up in ONE copy; the outputs form one contiguous
     // range behind them: one memset, one copy back
     double* d_xyzw; uint8_t* d_dl; uint8_t* d_dr; float* d_disp; float* d_size;
@@ -1667,35 +1714,9 @@ int svi_track_landmarks_stages(svi_ctx* ctx, const uint8_t* img_left, const uint
     UP(o.desc_r, (const uint8_t*)nullptr, (size_t)n * 32);
     const size_t out_end = ctx->arena_used;
     CK(cudaMemsetAsync(ctx->arena + out_begin, 0, out_end - out_begin, s));
-    TrackConst k;
-    for (int i = 0; i < 12; ++i) { k.T[i] = T_world_to_left[i]; k.PL[i] = ctx->cam_l.P[i]; k.PR[i] = ctx->cam_r.P[i]; }
-    k.tri_scale = (float)(1.0 + motion_scaling);
-    k.cutoff1 = ctx->p.cutoff_stage1;
-    k.stage1_match = (stage_mask & SVI_STAGE_1) ? 1 : 0;
-    LandmarksDev ld{d_xyzw, d_dl, d_dr, d_disp, d_size};
-    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, plane);
-    // The whole cascade is ONE stream of kernels: every stage reads the stage / status bytes the previous one left on
-    // the device and plans its own work items there; the host only waits once, for the results.
-    if (stage_mask & (SVI_STAGE_1 | SVI_STAGE_2)) {
-        // ---- stage 1 LEFT / RIGHT for every landmark (or only its field-of-view gate when stage 2 runs alone)
-        track_stage1_kernel<<<(n + MATCH_WARPS - 1) / MATCH_WARPS, MATCH_WARPS * 32, MATCH_SMEM, s>>>(l.box_l, l.box_r, l.map_l, l.map_ls, l.map_r, l.map_rs, g,
-                                                                                                      ctx->tc, k, ld, n, o);
-        CK(cudaGetLastError());
-    } else {
-        // stage 3 alone (trackEpipolar :828-1020): no gate, every landmark is an untracked candidate
-        CK(cudaMemsetAsync(o.status, SVI_TRK_STAGE1_DIST, (size_t)n, s));
-        CK(cudaMemsetAsync(o.stage, 0, (size_t)n, s));
-    }
-    // ---- stage 2 LEFT, then stage 2 RIGHT, for what is still untracked
-    for (int side = 0; side < 2 && (stage_mask & SVI_STAGE_2); ++side) {
-        rc = track_stage2_side(ctx, l, g, n, T_world_to_left, motion_scaling, side == 0, ld, o);
-        if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); return rc; }
-    }
-    // ---- stage 3 (epipolar line in LEFT)
-    if (stage3) {
-        rc = track_stage3_all(ctx, l, g, n, T_world_to_left, motion_scaling, ld, ex, d_orig, o);
-        if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); return rc; }
-    }
+    // The whole cascade is ONE stream of kernels; the host only waits once, for the results.
+    rc = enqueue_cascade(ctx, n, T_world_to_left, motion_scaling, stage_mask, LandmarksDev{d_xyzw, d_dl, d_dr, d_disp, d_size}, ex, d_orig, o, nullptr);
+    if (rc != SVI_SUCCESS) return rc;
     tick(2);
     int rd = SVI_SUCCESS;
     if (ctx->pin_arena) {   // one copy for the whole output range, scattered to the caller's arrays after the synchronisation
@@ -1887,6 +1908,217 @@ int svi_solve_stereo_posit(svi_ctx* ctx, const svi_posit_problem* in, svi_posit_
         std::fprintf(stderr, "svi_solve_stereo_posit n=%d: outcome %d after %d iterations | check + stage inputs %.0f us | copy up, kernel, copy back %.0f us | total %.0f us\n",
                      n, po.outcome, po.iterations, us(t_begin, t_staged), us(t_staged, t_end), us(t_begin, t_end));
     }
+    return check_overflow(ctx);
+}
+
+namespace {
+void posit_result_from(const PositOut& po, svi_posit_result* r) {
+    std::memcpy(r->T_world_to_left, po.T, sizeof(r->T_world_to_left));
+    r->outcome = (uint8_t)po.outcome;
+    r->iterations = po.iterations;
+    r->inliers = po.inliers;
+    r->average_squared_error = po.average_squared_error;
+    r->risk = po.risk;
+}
+void posit_too_few(const double* T_estimate, svi_posit_result* r) {   // svi_solve_stereo_posit's answer for n <= 25
+    std::memcpy(r->T_world_to_left, T_estimate, sizeof(r->T_world_to_left));
+    r->outcome = SVI_POSIT_TOO_FEW_POINTS;
+    r->iterations = 0;
+    r->inliers = 0;
+    r->average_squared_error = 0.0;
+    r->risk = 0.0;
+}
+bool track_result_ok(const svi_track_result& r) {
+    return r.status && r.stage && r.uv_left && r.uv_right && r.xyz_left && r.desc_left && r.desc_right;
+}
+}  // namespace
+
+int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uint8_t* img_right, size_t pitch, const svi_sv_frame* in, int n,
+                                svi_sv_frame_result* out) {
+    if (!ctx) return SVI_ERR_INVALID;
+    if (!img_left || !img_right || !in || !out || n < 0 || (int)pitch < ctx->W) return fail(ctx, SVI_ERR_INVALID, "svi_track_frame_stereo_only: bad argument");
+    const svi_landmarks& lm = in->landmarks;
+    if (n > 0 && (!lm.xyz_world || !lm.last_desc_left || !lm.last_desc_right || !lm.last_disparity || !lm.keypoint_size || !lm.uv_reference_left ||
+                  !lm.desc_reference_left || !lm.T_left_to_world_at_detection || !in->flags || !out->route || !track_result_ok(out->pose_stage) ||
+                  !track_result_ok(out->epipolar_stage)))
+        return fail(ctx, SVI_ERR_INVALID, "svi_track_frame_stereo_only: null array");
+    if (n > ctx->p.max_queries) return fail(ctx, SVI_ERR_CAPACITY, "svi_track_frame_stereo_only: n > max_queries");
+    if (!(in->motion_scaling >= 0.0 && in->motion_scaling <= 16.0))
+        return fail(ctx, SVI_ERR_INVALID, "svi_track_frame_stereo_only: motion_scaling must be within [0, 16]");
+    int n_cand = 0;
+    for (int i = 0; i < n; ++i) {
+        if (in->flags[i] & ~(SVI_SV_POSE_CANDIDATE | SVI_SV_LEAVES)) return fail(ctx, SVI_ERR_INVALID, "svi_track_frame_stereo_only: unknown flag bits");
+        n_cand += in->flags[i] & SVI_SV_POSE_CANDIDATE;
+    }
+    if (n == 0) {   // no landmark: no hit, both solves fail before an iteration, the pose is the damped prior
+        posit_too_few(in->T_estimate, &out->attempt[0]);
+        posit_too_few(in->T_estimate_damped, &out->attempt[1]);
+        out->measurements[0] = out->measurements[1] = 0;
+        out->attempts = 2;
+        out->source = SVI_SV_PRIOR;
+        std::memcpy(out->T_world_to_left, in->T_estimate_damped, sizeof(out->T_world_to_left));
+        return SVI_SUCCESS;
+    }
+    CK(cudaSetDevice(ctx->device));
+    int rc = ensure_track_scratch(ctx);
+    if (rc != SVI_SUCCESS) return rc;
+    cudaStream_t s = ctx->lanes[0].stream;
+    rc = stage_track_pair(ctx, img_left, img_right, pitch);
+    if (rc != SVI_SUCCESS) return rc;
+
+    // One device block + its pinned mirror (the staging pair of svi_solve_stereo_posit):
+    //   [inputs: the landmark arrays and flags]            one copy up
+    //   [outputs: attempts, pose stage, route, epipolar]   one memset, one copy down
+    //   [scratch: counts, index lists, gathered subset, subset results, pose problem]
+    const size_t N = (size_t)n;
+    size_t off = 0;
+    auto take = [&off](size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
+    const size_t i_xyz = take(24 * N), i_dl = take(32 * N), i_dr = take(32 * N), i_disp = take(4 * N), i_size = take(4 * N), i_uvref = take(16 * N),
+                 i_dref = take(32 * N), i_tdet = take(128 * N), i_flags = take(N);
+    const size_t in_bytes = off;
+    const size_t o_posit = take(2 * sizeof(PositOut));
+    auto take_track = [&](size_t* o7) {
+        o7[0] = take(N); o7[1] = take(N); o7[2] = take(8 * N); o7[3] = take(8 * N); o7[4] = take(24 * N); o7[5] = take(32 * N); o7[6] = take(32 * N);
+    };
+    size_t o_pose[7], o_epi[7], x_sub[7];
+    take_track(o_pose);
+    const size_t o_route = take(N);
+    take_track(o_epi);
+    const size_t out_end = off;
+    // counts: [0] candidates, [1] pose hits, [2] epipolar set, [3] regional set
+    const size_t x_cnt = take(4 * sizeof(int)), x_cand = take(4 * N), x_hits = take(4 * N), x_epi = take(4 * N), x_reg = take(4 * N);
+    const size_t x_xyz = take(24 * N), x_dl = take(32 * N), x_dr = take(32 * N), x_disp = take(4 * N), x_size = take(4 * N), x_uvref = take(16 * N),
+                 x_dref = take(32 * N), x_tdet = take(128 * N);
+    take_track(x_sub);
+    const size_t x_pxyz = take(24 * N), x_puvl = take(8 * N), x_puvr = take(8 * N);
+    if (const int r = reserve_opt(ctx, off)) return r;
+    unsigned char* hp = ctx->opt_pin;
+    unsigned char* d = ctx->opt_dev;
+    std::memcpy(hp + i_xyz, lm.xyz_world, 24 * N);
+    std::memcpy(hp + i_dl, lm.last_desc_left, 32 * N);
+    std::memcpy(hp + i_dr, lm.last_desc_right, 32 * N);
+    std::memcpy(hp + i_disp, lm.last_disparity, 4 * N);
+    std::memcpy(hp + i_size, lm.keypoint_size, 4 * N);
+    std::memcpy(hp + i_uvref, lm.uv_reference_left, 16 * N);
+    std::memcpy(hp + i_dref, lm.desc_reference_left, 32 * N);
+    std::memcpy(hp + i_tdet, lm.T_left_to_world_at_detection, 128 * N);
+    std::memcpy(hp + i_flags, in->flags, N);
+    CK(cudaMemcpyAsync(d, hp, in_bytes, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(d + o_posit, 0, out_end - o_posit, s));
+    auto dp = [d](size_t o) { return d + o; };
+    auto dd = [d](size_t o) { return reinterpret_cast<double*>(d + o); };
+    auto df = [d](size_t o) { return reinterpret_cast<float*>(d + o); };
+    auto di = [d](size_t o) { return reinterpret_cast<int*>(d + o); };
+    auto track_out = [&](const size_t* o7) { return TrackOutDev{dp(o7[0]), dp(o7[1]), df(o7[2]), df(o7[3]), dd(o7[4]), dp(o7[5]), dp(o7[6])}; };
+    const SvLandmarksDev all{dd(i_xyz), dp(i_dl), dp(i_dr), df(i_disp), df(i_size), dd(i_uvref), dp(i_dref), dd(i_tdet)};
+    const SvLandmarksDev sub{dd(x_xyz), dp(x_dl), dp(x_dr), df(x_disp), df(x_size), dd(x_uvref), dp(x_dref), dd(x_tdet)};
+    const LandmarksDev sub_ld{sub.xyz_w, sub.desc_l, sub.desc_r, sub.disparity, sub.size};
+    const Stage3Extra sub_ex{sub.uv_ref, sub.T_det};
+    const TrackOutDev pose_out = track_out(o_pose), epi_out = track_out(o_epi), sub_out = track_out(x_sub);
+    int* cnt = di(x_cnt);
+    PositOut* posit_dev = reinterpret_cast<PositOut*>(d + o_posit);
+    uint8_t* route = dp(o_route);
+    const unsigned blocks = (unsigned)((n + 127) / 128);
+    // the subset results start as a fresh tracking call's outputs: zero
+    auto clear_sub = [&]() -> int {
+        CK(cudaMemsetAsync(d + x_sub[0], 0, x_pxyz - x_sub[0], s));
+        return SVI_SUCCESS;
+    };
+
+    // ---- pose stage: the candidates (flags bit 0) in caller order, gathered once for both attempts
+    sv_compact_kernel<<<1, kCompactThreads, 0, s>>>(dp(i_flags), n, (1u << 1) | (1u << 3), di(x_cand), cnt + 0);
+    sv_gather_kernel<<<blocks, 128, 0, s>>>(all, di(x_cand), cnt + 0, n, sub);
+    CK(cudaGetLastError());
+    const double* priors[2] = {in->T_estimate, in->T_estimate_damped};
+    int accepted = -1, attempts = 0, measurements[2] = {0, 0};
+    for (int a = 0; a < 2 && accepted < 0; ++a) {
+        attempts = a + 1;
+        if (n_cand > 0) {
+            if ((rc = clear_sub()) != SVI_SUCCESS) return rc;
+            rc = enqueue_cascade(ctx, n_cand, priors[a], in->motion_scaling, SVI_STAGE_1 | SVI_STAGE_2, sub_ld, sub_ex, nullptr, sub_out, nullptr);
+            if (rc != SVI_SUCCESS) return rc;
+        }
+        // the solver's measurements: the hits in candidate order
+        sv_compact_kernel<<<1, kCompactThreads, 0, s>>>(sub_out.stage, n_cand, 0x1Eu /* stages 1..4 */, di(x_hits), cnt + 1);
+        sv_posit_assemble_kernel<<<blocks, 128, 0, s>>>(di(x_hits), cnt + 1, n, sub.xyz_w, sub_out, dd(x_pxyz), df(x_puvl), df(x_puvr));
+        PositIn pi{};
+        pi.xyz_world = dd(x_pxyz);
+        pi.uv_left = df(x_puvl);
+        pi.uv_right = df(x_puvr);
+        std::memcpy(pi.P_left, ctx->cam_l.P, sizeof(pi.P_left));
+        std::memcpy(pi.P_right, ctx->cam_r.P, sizeof(pi.P_right));
+        std::memcpy(pi.T_estimate, priors[a], sizeof(pi.T_estimate));
+        std::memcpy(pi.T_last, in->T_last, sizeof(pi.T_last));
+        std::memcpy(pi.t_imu, in->t_imu, sizeof(pi.t_imu));
+        stereo_posit_count_kernel<<<1, kPositThreads, kPositSmemBytes, s>>>(pi, cnt + 1, posit_dev + a);
+        CK(cudaGetLastError());
+        // wait: the outcome decides whether the damped attempt runs
+        CK(cudaMemcpyAsync(hp + o_posit + a * sizeof(PositOut), posit_dev + a, sizeof(PositOut), cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(hp + x_cnt + sizeof(int), cnt + 1, sizeof(int), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        PositOut po;
+        std::memcpy(&po, hp + o_posit + a * sizeof(PositOut), sizeof(po));
+        std::memcpy(&measurements[a], hp + x_cnt + sizeof(int), sizeof(int));
+        if (po.outcome == SVI_POSIT_OK) accepted = a;
+    }
+    // the stage-1/2 results of the last attempt that ran, at the candidates' places
+    if (n_cand > 0) sv_scatter_kernel<<<blocks, 128, 0, s>>>(di(x_cand), cnt + 0, n, sub_out, pose_out, nullptr);
+    double T[16];
+    if (accepted >= 0) std::memcpy(T, reinterpret_cast<const PositOut*>(hp + o_posit + accepted * sizeof(PositOut))->T, sizeof(T));
+    else std::memcpy(T, in->T_estimate_damped, sizeof(T));
+    SvPose pose;
+    std::memcpy(pose.T, T, sizeof(T));
+
+    // ---- epipolar stage: route every landmark, stage 3 on the moved ones (the count stays on the device)
+    sv_route_kernel<<<blocks, 128, 0, s>>>(n, dp(i_flags), pose_out.stage, accepted >= 0 ? 1 : 0, pose, all.T_det, route);
+    sv_compact_kernel<<<1, kCompactThreads, 0, s>>>(route, n, 1u << kRouteEpipolar, di(x_epi), cnt + 2);
+    sv_gather_kernel<<<blocks, 128, 0, s>>>(all, di(x_epi), cnt + 2, n, sub);
+    CK(cudaGetLastError());
+    if ((rc = clear_sub()) != SVI_SUCCESS) return rc;
+    rc = enqueue_cascade(ctx, n, T, in->motion_scaling, SVI_STAGE_3, sub_ld, sub_ex, sub.desc_ref, sub_out, cnt + 2);
+    if (rc != SVI_SUCCESS) return rc;
+    sv_scatter_kernel<<<blocks, 128, 0, s>>>(di(x_epi), cnt + 2, n, sub_out, epi_out, route);   // + the SVI_EPI_NO_TRANSLATION re-route
+    // ---- regional stage 2 on the unmoved ones and the re-routed ones; wait: its launch sizes need the count
+    sv_compact_kernel<<<1, kCompactThreads, 0, s>>>(route, n, (1u << kRouteRegional) | (1u << kRouteRegionalNoTranslation), di(x_reg), cnt + 3);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(hp + x_cnt, cnt, 4 * sizeof(int), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    int n_reg = 0;
+    std::memcpy(&n_reg, hp + x_cnt + 3 * sizeof(int), sizeof(int));
+    if (n_reg < 0 || n_reg > n) return fail(ctx, SVI_ERR_CUDA, "svi_track_frame_stereo_only: regional count out of range");
+    if (n_reg > 0) {
+        sv_gather_kernel<<<blocks, 128, 0, s>>>(all, di(x_reg), cnt + 3, n, sub);
+        CK(cudaGetLastError());
+        if ((rc = clear_sub()) != SVI_SUCCESS) return rc;
+        rc = enqueue_cascade(ctx, n_reg, T, in->motion_scaling, SVI_STAGE_2, sub_ld, sub_ex, nullptr, sub_out, nullptr);
+        if (rc != SVI_SUCCESS) return rc;
+        sv_scatter_kernel<<<blocks, 128, 0, s>>>(di(x_reg), cnt + 3, n, sub_out, epi_out, nullptr);
+        CK(cudaGetLastError());
+    }
+    // ---- every result in one copy
+    CK(cudaMemcpyAsync(hp + o_posit, d + o_posit, out_end - o_posit, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    for (int a = 0; a < 2; ++a) {
+        if (a < attempts) posit_result_from(*reinterpret_cast<const PositOut*>(hp + o_posit + a * sizeof(PositOut)), &out->attempt[a]);
+        else std::memset(&out->attempt[a], 0, sizeof(out->attempt[a]));
+    }
+    out->attempts = attempts;
+    out->measurements[0] = measurements[0];
+    out->measurements[1] = measurements[1];
+    out->source = accepted == 0 ? SVI_SV_POSIT : accepted == 1 ? SVI_SV_POSIT_DAMPED : SVI_SV_PRIOR;
+    std::memcpy(out->T_world_to_left, T, sizeof(T));
+    auto scatter = [&](const size_t* o7, const svi_track_result& r) {
+        std::memcpy(r.status, hp + o7[0], N);
+        std::memcpy(r.stage, hp + o7[1], N);
+        std::memcpy(r.uv_left, hp + o7[2], 8 * N);
+        std::memcpy(r.uv_right, hp + o7[3], 8 * N);
+        std::memcpy(r.xyz_left, hp + o7[4], 24 * N);
+        std::memcpy(r.desc_left, hp + o7[5], 32 * N);
+        std::memcpy(r.desc_right, hp + o7[6], 32 * N);
+    };
+    scatter(o_pose, out->pose_stage);
+    std::memcpy(out->route, hp + o_route, N);
+    scatter(o_epi, out->epipolar_stage);
     return check_overflow(ctx);
 }
 

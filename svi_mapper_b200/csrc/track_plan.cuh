@@ -165,10 +165,11 @@ __device__ inline int epipolar_plan_dev(const TrackPlanConst& k, const double* T
     return SVI_OK;
 }
 
-__global__ void stage3_plan_kernel(TrackPlanConst k, LandmarksDev lm, Stage3Extra ex, int n, TrackOutDev out,
+// n_dev (may be null): the item count when only the device knows it; n is then the capacity the grid covers
+__global__ void stage3_plan_kernel(TrackPlanConst k, LandmarksDev lm, Stage3Extra ex, int n, const int* __restrict__ n_dev, TrackOutDev out,
                                    Stage3Item* __restrict__ items, int* __restrict__ n_items) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= n) return;
+    if (q >= n || (n_dev && q >= *n_dev)) return;
     if (out.stage[q] != 0 || out.status[q] == SVI_TRK_OUT_OF_FOV) return;
     Stage3Item it;
     it.q = q;

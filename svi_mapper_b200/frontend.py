@@ -419,6 +419,65 @@ class StereoFrontend:
                      _lib.SVI_POSIT_INACCURATE: "insufficient accuracy", _lib.SVI_POSIT_HIGH_RISK: "inconsistent with prior",
                      _lib.SVI_POSIT_NOT_CONVERGED: "system did not converge"}
 
+    @staticmethod
+    def _track_out(n):
+        out = dict(status=np.zeros(n, np.uint8), stage=np.zeros(n, np.uint8), uv_l=np.zeros((n, 2), np.float32),
+                   uv_r=np.zeros((n, 2), np.float32), xyz=np.zeros((n, 3), np.float64),
+                   desc_l=np.zeros((n, 32), np.uint8), desc_r=np.zeros((n, 32), np.uint8))
+        r = _lib.TrackResult(_ptr(out["status"]), _ptr(out["stage"]), _ptr(out["uv_l"]), _ptr(out["uv_r"]), _ptr(out["xyz"]),
+                             _ptr(out["desc_l"]), _ptr(out["desc_r"]))
+        return out, r
+
+    def _posit_dict(self, res) -> dict:
+        return dict(T=np.array(res.T_world_to_left[:], np.float64).reshape(4, 4), outcome=int(res.outcome),
+                    reason=self.POSIT_REASONS[int(res.outcome)], iterations=int(res.iterations), inliers=int(res.inliers),
+                    average_squared_error=float(res.average_squared_error), risk=float(res.risk))
+
+    # -- CTrackerSV: one frame of the stereo-only tracker in one call
+    SV_SOURCES = ("posit", "posit-damped", "prior")
+
+    def track_frame_stereo_only(self, img_left, img_right, xyz_world, last_desc_left, last_desc_right, last_disparity, keypoint_size,
+                                uv_reference_left, desc_reference_left, T_left_to_world_at_detection, flags, T_estimate,
+                                T_estimate_damped, T_last=None, t_imu=None, motion_scaling: float = 1.0) -> dict:
+        """svi_track_frame_stereo_only: the pose stage (stages 1-2 and the pose solve around T_estimate, then around
+        T_estimate_damped if that fails) and the epipolar stage (stage 3, or the regional stage 2) of one frame in one call.
+        Landmark arrays as in track_landmarks (the three reference arrays are required); flags (n,) uint8: bit 0 = pose candidate
+        (bIsOptimal), bit 1 = leaves the active set in trackEpipolar.  T_last defaults to T_estimate, t_imu to zero.
+        Returns dict(T (4, 4), source ("posit" | "posit-damped" | "prior"), attempts (list of solve_stereo_posit dicts),
+        measurements (problem size of each attempt's solve), route (n,) uint8 (svi_sv_route), pose_stage and epipolar_stage
+        (track_landmarks dicts over all n landmarks))."""
+        a = self._images(img_left, "img_left")[0]
+        b = self._images(img_right, "img_right")[0]
+        xw = np.ascontiguousarray(np.asarray(xyz_world, np.float64).reshape(-1, 3))
+        n = len(xw)
+        dl = np.ascontiguousarray(np.asarray(last_desc_left, np.uint8).reshape(n, 32))
+        dr = np.ascontiguousarray(np.asarray(last_desc_right, np.uint8).reshape(n, 32))
+        disp = np.ascontiguousarray(np.asarray(last_disparity, np.float32).reshape(n))
+        size = np.ascontiguousarray(np.broadcast_to(np.asarray(keypoint_size, np.float32), (n,)).copy())
+        uvref = np.ascontiguousarray(np.asarray(uv_reference_left, np.float64).reshape(n, 2))
+        dref = np.ascontiguousarray(np.asarray(desc_reference_left, np.uint8).reshape(n, 32))
+        tdet = np.ascontiguousarray(np.broadcast_to(np.asarray(T_left_to_world_at_detection, np.float64), (n, 4, 4)).copy())
+        fl = np.ascontiguousarray(np.asarray(flags, np.uint8).reshape(n))
+        Te = np.asarray(T_estimate, np.float64).reshape(16)
+        Td = np.asarray(T_estimate_damped, np.float64).reshape(16)
+        Tl = Te if T_last is None else np.asarray(T_last, np.float64).reshape(16)
+        ti = np.zeros(3) if t_imu is None else np.asarray(t_imu, np.float64).reshape(3)
+        fr = _lib.SvFrame(_lib.Landmarks(_ptr(xw), _ptr(dl), _ptr(dr), _ptr(disp), _ptr(size), _ptr(uvref), _ptr(dref), _ptr(tdet)), _ptr(fl))
+        for i in range(16):
+            fr.T_estimate[i], fr.T_estimate_damped[i], fr.T_last[i] = float(Te[i]), float(Td[i]), float(Tl[i])
+        for i in range(3):
+            fr.t_imu[i] = float(ti[i])
+        fr.motion_scaling = float(motion_scaling)
+        pose, rp = self._track_out(n)
+        epi, re = self._track_out(n)
+        route = np.zeros(n, np.uint8)
+        res = _lib.SvFrameResult(pose_stage=rp, route=_ptr(route), epipolar_stage=re)
+        self._check(self._lib.svi_track_frame_stereo_only(self._ctx, _ptr(a), _ptr(b), self.width, C.byref(fr), n, C.byref(res)))
+        return dict(T=np.array(res.T_world_to_left[:], np.float64).reshape(4, 4), source=self.SV_SOURCES[int(res.source)],
+                    attempts=[self._posit_dict(res.attempt[k]) for k in range(int(res.attempts))],
+                    measurements=[int(res.measurements[k]) for k in range(int(res.attempts))], route=route, pose_stage=pose,
+                    epipolar_stage=epi)
+
     def solve_stereo_posit(self, xyz_world, uv_left, uv_right, T_estimate, T_last=None, t_imu=None) -> dict:
         """svi_solve_stereo_posit: CSolverStereoPosit::getTransformationWORLDtoLEFT on the GPU -- the WORLD->LEFT pose from n
         stereo measurements (xyz_world (n, 3) float64, uv_left / uv_right (n, 2) float32) starting at the prior T_estimate (4, 4).
@@ -440,9 +499,7 @@ class StereoFrontend:
             prob.t_imu[i] = float(ti[i])
         res = _lib.PositResult()
         self._check(self._lib.svi_solve_stereo_posit(self._ctx, C.byref(prob), C.byref(res)))
-        return dict(T=np.array(res.T_world_to_left[:], np.float64).reshape(4, 4), outcome=int(res.outcome),
-                    reason=self.POSIT_REASONS[int(res.outcome)], iterations=int(res.iterations), inliers=int(res.inliers),
-                    average_squared_error=float(res.average_squared_error), risk=float(res.risk))
+        return self._posit_dict(res)
 
     # -- profiling
     def set_profiling(self, enable):

@@ -617,6 +617,130 @@ public:
     }
     UIDLandmark getNumberOfTracksStage2_2() const { return m_uNumberOfTracksStage2_2; }
 
+    // Whether trackFrameStereoOnly can replace getPoseStereoPosit + trackEpipolar: a GPU context, and the GPU solve (SVI_HOST_POSIT=cpu
+    // keeps the composed calls with the CPU loop: the checker of the parity test)
+    bool canTrackFrameStereoOnly() const {
+        static const bool bCPU = [] { const char* e = std::getenv("SVI_HOST_POSIT"); return e && std::string(e) == "cpu"; }();
+        return m_pGpu && !bCPU;
+    }
+
+    // getPoseStereoPosit with the damped retry of CTrackerSV::process, then trackEpipolar, as ONE library call
+    // (svi_track_frame_stereo_only): the active landmarks are packed once, the routing, both stage subsets and the pose solves run
+    // on the device, and the bookkeeping of the composed calls follows in their order -- the pose-stage measurements (accepted solve
+    // only), the stage-3 measurements, the regional stage-2 measurements, the failed-tracking counts and the activity clean-up.
+    // Returns the frame's pose; p_uSource = svi_sv_source.
+    const Isometry3d trackFrameStereoOnly(const UIDFrame p_uFrame, const ImageView& p_matImageLEFT, const ImageView& p_matImageRIGHT,
+                                          const Isometry3d& p_matTransformationEstimateWORLDtoLEFT, const Isometry3d& p_matTransformationEstimateDampedWORLDtoLEFT,
+                                          const Isometry3d& p_matTransformationWORLDtoLEFTLAST, const CPoint3D& p_vecTranslationIMU,
+                                          const double& p_dMotionScaling, uint8_t& p_uSource) {
+        m_uNumberOfTracksStage1 = m_uNumberOfTracksStage2_1 = m_uNumberOfTracksStage3 = m_uNumberOfTracksStage2_2 = 0;
+        std::vector<CLandmark*> vecLandmarks;
+        std::vector<const CDetectionPoint*> vecDetectionPointOf;
+        for (const CDetectionPoint& cDetectionPoint : m_vecDetectionPointsActive)
+            for (CLandmark* pLandmark : *cDetectionPoint.vecLandmarks) { vecLandmarks.push_back(pLandmark); vecDetectionPointOf.push_back(&cDetectionPoint); }
+        const int n = (int)vecLandmarks.size();
+        std::vector<double> xyzW(3 * n), uvRef(2 * n), Tdet(16 * n);
+        std::vector<uint8_t> dL(32 * n), dR(32 * n), dRef(32 * n), vecFlags(n);
+        std::vector<float> disp(n), size(n);
+        for (int i = 0; i < n; ++i) {
+            const CLandmark* p = vecLandmarks[i];
+            for (int k = 0; k < 3; ++k) xyzW[3 * i + k] = p->vecPointXYZOptimized.v[k];
+            std::memcpy(&dL[32 * i], p->getLastDescriptorLEFT().data(), 32);
+            std::memcpy(&dR[32 * i], p->getLastDescriptorRIGHT().data(), 32);
+            std::memcpy(&dRef[32 * i], p->matDescriptorReferenceLEFT.data(), 32);
+            disp[i] = p->getLastDisparity();
+            size[i] = (float)p->dKeyPointSize;
+            uvRef[2 * i] = p->vecUVReferenceLEFT[0];
+            uvRef[2 * i + 1] = p->vecUVReferenceLEFT[1];
+            std::memcpy(&Tdet[16 * i], vecDetectionPointOf[i]->matTransformationLEFTtoWORLD.m, sizeof(double) * 16);
+            const bool bLeaves = 0 < p->uOptimizationsFailed || (0 < p->uOptimizationsSuccessful && !p->bIsOptimal);   // :808-825
+            vecFlags[i] = (uint8_t)((p->bIsOptimal ? SVI_SV_POSE_CANDIDATE : 0) | (bLeaves ? SVI_SV_LEAVES : 0));
+        }
+        svi_sv_frame cIn{};
+        cIn.landmarks = svi_landmarks{xyzW.data(), dL.data(), dR.data(), disp.data(), size.data(), uvRef.data(), dRef.data(), Tdet.data()};
+        cIn.flags = vecFlags.data();
+        std::memcpy(cIn.T_estimate, p_matTransformationEstimateWORLDtoLEFT.m, sizeof(cIn.T_estimate));
+        std::memcpy(cIn.T_estimate_damped, p_matTransformationEstimateDampedWORLDtoLEFT.m, sizeof(cIn.T_estimate_damped));
+        std::memcpy(cIn.T_last, p_matTransformationWORLDtoLEFTLAST.m, sizeof(cIn.T_last));
+        for (int r = 0; r < 3; ++r) cIn.t_imu[r] = p_vecTranslationIMU(r);
+        cIn.motion_scaling = p_dMotionScaling;
+        CTrackBatch p, e;
+        for (CTrackBatch* c : {&p, &e}) { c->xyz.resize(3 * n); c->oL.resize(32 * n); c->oR.resize(32 * n); c->st.resize(n); c->stage.resize(n); c->uvL.resize(2 * n); c->uvR.resize(2 * n); }
+        std::vector<uint8_t> vecRoute(n);
+        svi_sv_frame_result cOut{};
+        cOut.pose_stage = svi_track_result{p.st.data(), p.stage.data(), p.uvL.data(), p.uvR.data(), p.xyz.data(), p.oL.data(), p.oR.data()};
+        cOut.route = vecRoute.data();
+        cOut.epipolar_stage = svi_track_result{e.st.data(), e.stage.data(), e.uvL.data(), e.uvR.data(), e.xyz.data(), e.oL.data(), e.oR.data()};
+        m_pGpu->check(svi_track_frame_stereo_only(m_pGpu->ctx, p_matImageLEFT.data, p_matImageRIGHT.data, p_matImageLEFT.pitch, &cIn, n, &cOut));
+        Isometry3d matTransformationWORLDtoLEFT;
+        std::memcpy(matTransformationWORLDtoLEFT.m, cOut.T_world_to_left, sizeof(matTransformationWORLDtoLEFT.m));
+        p_uSource = cOut.source;
+        const MatrixProjection matProjectionWORLDtoLEFT(m_pCameraLEFT->m_matProjection * matTransformationWORLDtoLEFT);
+        const MatrixProjection matProjectionWORLDtoRIGHT(m_pCameraRIGHT->m_matProjection * matTransformationWORLDtoLEFT);
+        const Isometry3d matTransformationLEFTtoWORLD(inverseIsometry(matTransformationWORLDtoLEFT));
+        auto descriptors = [](const CTrackBatch& c, int i, CDescriptor& a, CDescriptor& b) {
+            std::memcpy(a.data(), &c.oL[32 * (size_t)i], 32);
+            std::memcpy(b.data(), &c.oR[32 * (size_t)i], 32);
+        };
+        // ---- getPoseStereoPosit: the hits of the last attempt, in candidate order (the counters count them even when it failed)
+        std::vector<CSolverStereoPosit::CMatch> vecMeasurementsForStereoPosit;
+        for (int i = 0; i < n; ++i) {
+            if (0 == p.stage[i]) continue;
+            CDescriptor a, b;
+            descriptors(p, i, a, b);
+            vecMeasurementsForStereoPosit.push_back(CSolverStereoPosit::CMatch(vecLandmarks[i], vecLandmarks[i]->vecPointXYZOptimized,
+                                                                               CPoint3DCAMERA(p.xyz[3 * i], p.xyz[3 * i + 1], p.xyz[3 * i + 2]),
+                                                                               Point2f(p.uvL[2 * i], p.uvL[2 * i + 1]), Point2f(p.uvR[2 * i], p.uvR[2 * i + 1]), a, b));
+            if (p.stage[i] <= 2) ++m_uNumberOfTracksStage1; else ++m_uNumberOfTracksStage2_1;
+        }
+        m_cSolverSterePosit.recordAttempts(cOut);
+        if (SVI_SV_PRIOR != cOut.source) {
+            for (const CSolverStereoPosit::CMatch& cMatchSTEREO : vecMeasurementsForStereoPosit)
+                _addMeasurementToLandmarkSTEREO(p_uFrame, cMatchSTEREO.pLandmark, cMatchSTEREO.ptUVLEFT, cMatchSTEREO.ptUVRIGHT, cMatchSTEREO.vecPointXYZLEFT,
+                                                cMatchSTEREO.matDescriptorLEFT, cMatchSTEREO.matDescriptorRIGHT, matTransformationLEFTtoWORLD,
+                                                matTransformationWORLDtoLEFT, matProjectionWORLDtoLEFT, matProjectionWORLDtoRIGHT);
+            m_vecMeasurementsStereoPositLAST.swap(vecMeasurementsForStereoPosit);
+        }
+        // ---- trackEpipolar: the landmarks that leave, then stage 3, then the regional stage 2 (unmoved ones first, then the
+        // stage-3 items without translation, both in landmark order)
+        std::vector<uint8_t> vecDropped(n, 0);
+        for (int i = 0; i < n; ++i)
+            if (vecFlags[i] & SVI_SV_LEAVES) { vecLandmarks[i]->bIsCurrentlyVisible = false; vecDropped[i] = 1; }
+        auto apply = [&](const uint8_t p_uRoute, UIDLandmark& p_uCounter) {
+            for (int i = 0; i < n; ++i) {
+                if (p_uRoute != vecRoute[i]) continue;
+                CLandmark* pLandmark = vecLandmarks[i];
+                if (0 < e.stage[i]) {
+                    CDescriptor a, b;
+                    descriptors(e, i, a, b);
+                    _addMeasurementToLandmarkSTEREO(p_uFrame, pLandmark, Point2f(e.uvL[2 * i], e.uvL[2 * i + 1]), Point2f(e.uvR[2 * i], e.uvR[2 * i + 1]),
+                                                    CPoint3DCAMERA(e.xyz[3 * i], e.xyz[3 * i + 1], e.xyz[3 * i + 2]), a, b, matTransformationLEFTtoWORLD,
+                                                    matTransformationWORLDtoLEFT, matProjectionWORLDtoLEFT, matProjectionWORLDtoRIGHT);
+                    ++p_uCounter;
+                } else {
+                    ++pLandmark->uFailedSubsequentTrackings;   // :1014-1023, :1281-1289
+                    pLandmark->bIsCurrentlyVisible = false;
+                }
+            }
+        };
+        apply(SVI_SV_ROUTE_EPIPOLAR, m_uNumberOfTracksStage3);
+        apply(SVI_SV_ROUTE_REGIONAL, m_uNumberOfTracksStage2_2);
+        apply(SVI_SV_ROUTE_REGIONAL_NO_TRANSLATION, m_uNumberOfTracksStage2_2);
+        // activity :1291-1312, as trackEpipolar
+        std::vector<CLandmark*> vecLeaving;
+        for (int i = 0; i < n; ++i)
+            if (vecDropped[i] || vecLandmarks[i]->uFailedSubsequentTrackings >= m_uMaximumFailedSubsequentTrackingsPerLandmark) vecLeaving.push_back(vecLandmarks[i]);
+        std::sort(vecLeaving.begin(), vecLeaving.end());
+        for (CDetectionPoint& cDetectionPoint : m_vecDetectionPointsActive) {
+            std::vector<CLandmark*>& v = *cDetectionPoint.vecLandmarks;
+            v.erase(std::remove_if(v.begin(), v.end(), [&](CLandmark* q) { return std::binary_search(vecLeaving.begin(), vecLeaving.end(), q); }), v.end());
+        }
+        m_vecDetectionPointsActive.erase(std::remove_if(m_vecDetectionPointsActive.begin(), m_vecDetectionPointsActive.end(),
+                                                        [](const CDetectionPoint& d) { return d.vecLandmarks->empty(); }),
+                                         m_vecDetectionPointsActive.end());
+        return matTransformationWORLDtoLEFT;
+    }
+
 private:
     const std::shared_ptr<CGpuContext> m_pGpu;
     std::shared_ptr<CTriangulator> m_pTriangulator;

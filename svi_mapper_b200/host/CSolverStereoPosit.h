@@ -76,11 +76,41 @@ public:
         m_uIterationsLAST = 0;
         if (m_pGpu && !bCPU)
             return _getTransformationWORLDtoLEFTGPU(p_matTransformationWORLDtoLEFTLAST, p_vecTranslationIMU, p_matTransformationWORLDtoLEFTESTIMATE, p_vecMeasurements);
-        return _getTransformationWORLDtoLEFTCPU(p_matTransformationWORLDtoLEFTLAST, p_vecTranslationIMU, p_matTransformationWORLDtoLEFTESTIMATE, p_vecMeasurements);
+        try {
+            return _getTransformationWORLDtoLEFTCPU(p_matTransformationWORLDtoLEFTLAST, p_vecTranslationIMU, p_matTransformationWORLDtoLEFTESTIMATE, p_vecMeasurements);
+        } catch (const CExceptionPoseOptimization& e) {
+            m_strFailureLAST = e.what();
+            throw;
+        }
     }
-    // iterations of the last successful solve; wall time of all solves so far (failed ones included)
+    // iterations of the last successful solve; wall time of all solves so far (failed ones included; the solves inside
+    // svi_track_frame_stereo_only are not timed on their own)
     uint32_t getIterationsLAST() const { return m_uIterationsLAST; }
     double getDurationSeconds() const { return m_dDurationSeconds; }
+    // what() of the last failed solve ("" while none has failed)
+    const std::string& getFailureLAST() const { return m_strFailureLAST; }
+
+    // The accounting of the solves that ran inside svi_track_frame_stereo_only, in their order, as the separate solves leave it:
+    // the text of every failed one (the last stays), the iterations of a successful last one.
+    void recordAttempts(const svi_sv_frame_result& p_cResult) {
+        m_uIterationsLAST = 0;
+        for (int a = 0; a < p_cResult.attempts && a < 2; ++a) {
+            const svi_posit_result& cAttempt = p_cResult.attempt[a];
+            if (SVI_POSIT_OK == cAttempt.outcome) m_uIterationsLAST = (uint32_t)cAttempt.iterations;
+            else m_strFailureLAST = getFailureText(cAttempt, (size_t)p_cResult.measurements[a]);
+        }
+    }
+    // the reference's exception text for a failed outcome of the library
+    static std::string getFailureText(const svi_posit_result& p_cResult, const size_t p_uNumberOfMeasurements) {
+        switch (p_cResult.outcome) {
+            case SVI_POSIT_TOO_FEW_POINTS: return "insufficient number of points: " + std::to_string(p_uNumberOfMeasurements);
+            case SVI_POSIT_INACCURATE:
+                return "insufficient accuracy (average error: " + std::to_string(p_cResult.average_squared_error) + " inliers: " +
+                       std::to_string((size_t)p_cResult.inliers) + ")";
+            case SVI_POSIT_HIGH_RISK: return "inconsistent with prior (HIGH RISK: " + std::to_string(p_cResult.risk) + ")";
+            default: return "system did not converge";
+        }
+    }
 
 private:
     struct CTimer {
@@ -114,14 +144,9 @@ private:
         for (int r = 0; r < 3; ++r) cIn.t_imu[r] = p_vecTranslationIMU(r);
         svi_posit_result cOut;
         m_pGpu->check(svi_solve_stereo_posit(m_pGpu->ctx, &cIn, &cOut));
-        switch (cOut.outcome) {
-            case SVI_POSIT_OK: break;
-            case SVI_POSIT_TOO_FEW_POINTS: throw CExceptionPoseOptimization("insufficient number of points: " + std::to_string(uNumberOfMeasurements));
-            case SVI_POSIT_INACCURATE:
-                throw CExceptionPoseOptimization("insufficient accuracy (average error: " + std::to_string(cOut.average_squared_error) +
-                                                 " inliers: " + std::to_string((size_t)cOut.inliers) + ")");
-            case SVI_POSIT_HIGH_RISK: throw CExceptionPoseOptimization("inconsistent with prior (HIGH RISK: " + std::to_string(cOut.risk) + ")");
-            default: throw CExceptionPoseOptimization("system did not converge");
+        if (SVI_POSIT_OK != cOut.outcome) {
+            m_strFailureLAST = getFailureText(cOut, uNumberOfMeasurements);
+            throw CExceptionPoseOptimization(m_strFailureLAST);
         }
         m_uIterationsLAST = (uint32_t)cOut.iterations;
         Isometry3d T;
@@ -232,6 +257,7 @@ private:
     std::vector<float> m_vecUVLEFT, m_vecUVRIGHT;
     uint32_t m_uIterationsLAST = 0;
     double m_dDurationSeconds = 0.0;
+    std::string m_strFailureLAST;
     const uint32_t m_uMinimumPointsForPoseOptimization = 25;   // CSolverStereoPosit.h:89-99
     const uint32_t m_uMinimumInliersPoseOptimization = 15;
     const uint32_t m_uCapIterationsPoseOptimization = 1000;

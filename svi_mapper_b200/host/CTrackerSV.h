@@ -54,7 +54,20 @@ public:
         m_cMatcher.resetVisibilityActiveLandmarks();                                                                           // :257
         Isometry3d matTransformationWORLDtoLEFT(matEstimate);
         m_strPoseSource = "posit";
-        try {
+        if (m_cMatcher.canTrackFrameStereoOnly()) {
+            // the pose stage, the solves and trackEpipolar in one library call: its wall time is all counted as the pose stage
+            uint8_t uSource = SVI_SV_POSIT;
+            matTransformationWORLDtoLEFT = m_cMatcher.trackFrameStereoOnly(m_uFrameCount, p_matImageLEFT, p_matImageRIGHT, matEstimate, matEstimateParallel,
+                                                                           m_matTransformationWORLDtoLEFTLAST, vecTranslationTotal, dMotionScaling, uSource);
+            if (SVI_SV_POSIT == uSource) {
+                if (0 < m_uCountInstability) --m_uCountInstability;
+            } else if (SVI_SV_POSIT_DAMPED == uSource) {
+                m_strPoseSource = "posit-damped";
+            } else {
+                if (20 > m_uCountInstability) m_uCountInstability += 5;
+                m_strPoseSource = "prior";
+            }
+        } else try {
             matTransformationWORLDtoLEFT = m_cMatcher.getPoseStereoPosit(m_uFrameCount, p_matImageLEFT, p_matImageRIGHT, matEstimate,
                                                                          m_matTransformationWORLDtoLEFTLAST, vecRotationTotal, vecTranslationTotal,
                                                                          dMotionScaling);                                      // :268-279
@@ -73,8 +86,9 @@ public:
         }
         const auto tPose = std::chrono::steady_clock::now();
         const Isometry3d matTransformationLEFTtoWORLD(inverseIsometry(matTransformationWORLDtoLEFT));
-        m_cMatcher.trackEpipolar(m_uFrameCount, p_matImageLEFT, p_matImageRIGHT, matTransformationWORLDtoLEFT, matTransformationLEFTtoWORLD,
-                                 dMotionScaling);                                                                              // :320-327
+        if (!m_cMatcher.canTrackFrameStereoOnly())
+            m_cMatcher.trackEpipolar(m_uFrameCount, p_matImageLEFT, p_matImageRIGHT, matTransformationWORLDtoLEFT, matTransformationLEFTtoWORLD,
+                                     dMotionScaling);                                                                          // :320-327
         const int64_t iVisible = (int64_t)m_cMatcher.getNumberOfVisibleLandmarks();
         if (0 < m_uNumberofVisibleLandmarksLAST &&
             0.75 < (double)((int64_t)m_uNumberofVisibleLandmarksLAST - iVisible) / (double)m_uNumberofVisibleLandmarksLAST && 20 > m_uCountInstability)
@@ -103,7 +117,8 @@ public:
     }
 
     // wall time: the pose stage (getPoseStereoPosit incl. its fallback: stages 1-2 tracking and the solves), the solves alone
-    // (CSolverStereoPosit, failed ones included), trackEpipolar, landmark optimisation, re-detection
+    // (CSolverStereoPosit, failed ones included), trackEpipolar, landmark optimisation, re-detection.  A frame tracked with
+    // trackFrameStereoOnly (the default with a GPU context) counts its solves and its epipolar stage in the pose stage.
     double getDurationPoseSeconds() const { return m_dDurationPoseSeconds; }
     double getDurationPoseSolverSeconds() const { return m_cMatcher.getSolverStereoPosit().getDurationSeconds(); }
     double getDurationTrackEpipolarSeconds() const { return m_dDurationTrackEpipolarSeconds; }

@@ -323,7 +323,9 @@ static int sequenceMain(char** argv, bool p_bRectify) {
 // SVI_HOST_POSIT=cpu: the CPU loop).  Prints, per frame, the pose source, the counters and the 12 numbers of T_WORLDtoLEFT,
 // then the M / A lines of --sequence.  With SVI_DEMO_TIMING set ONE line goes to stdout instead: the wall time of every
 // process() call (frames after the first three), split into pose stage (tracking + solves), solves alone, trackEpipolar,
-// landmark optimisation and re-detection.
+// landmark optimisation and re-detection.  By default a frame is one svi_track_frame_stereo_only call: pose_ms then holds the
+// solves and the epipolar stage too, and pose_solver_ms and track_epipolar_ms stay near zero; SVI_HOST_POSIT=cpu runs the
+// composed calls, where the three are separate.
 static int sequenceSVMain(char** argv) {
     try {
         CParameterBase::loadCameraLEFT(argv[2]);

@@ -7,7 +7,9 @@
    the C++ host layer (facade_demo --posit: GPU call, and the CPU loop under SVI_HOST_POSIT=cpu); the outputs are compared.
 2. The C3 sequence (render_sequence, vi_sensor, --frames frames) through CTrackerSV (facade_demo --sequence-sv): median frame
    time and the split pose stage / solves / trackEpipolar / optimisation / re-detection, with the GPU solve and with the CPU
-   loop, two alternating runs each; plus the pose error against the ground truth.
+   loop, two alternating runs each; plus the pose error against the ground truth.  The "gpu" runs track each frame with one
+   svi_track_frame_stereo_only call: their pose_ms holds the solves and the epipolar stage, so pose_solver_ms and
+   track_epipolar_ms are about zero there; the "cpu" runs make the composed calls, where the three are separate.
 Writes DIR/r3_posit.json (and prints it), with the card's name and power limit read in the same run."""
 from __future__ import annotations
 
