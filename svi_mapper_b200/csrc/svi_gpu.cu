@@ -141,21 +141,13 @@ struct svi_ctx {
     StereoOutDev small_out{};
     int* small_n_kp = nullptr;
     int* small_n_det = nullptr;
-    // pinned mirror of the per-query arena: uploads and result downloads of the per-query / tracking entry points bounce
-    // through it, so that pageable caller buffers never turn a transfer into a blocking staged copy
-    unsigned char* pin_arena = nullptr;
-    struct Pending { void* host; const unsigned char* pinned; size_t bytes; };
-    std::vector<Pending> pending;
     int n_sm = 148;
-    // svi_optimize_landmarks: one device buffer + its pinned mirror (inputs, then outputs), grown on demand
-    unsigned char* opt_dev = nullptr;
-    unsigned char* opt_pin = nullptr;
-    size_t opt_bytes = 0;
-    // per-query arena
-    unsigned char* arena = nullptr;
-    size_t arena_bytes = 0, arena_used = 0;
+    // the call buffer (DESIGN.md section 3): the per-call arrays of the per-query, tracking and solver entry points, one
+    // device block + its pinned mirror of the same size, grown by reserve_call
+    unsigned char* call_dev = nullptr;
+    unsigned char* call_pin = nullptr;
+    size_t call_bytes = 0;
     bool profiling = false;
-    bool batch_uploads = false;   // upload(): stage into the pinned mirror only (svi_track_landmarks sends one copy)
     bool serial = false;   // profiling mode 2: every chunk on lane 0, so that the stage events bracket ONE kernel each
     // rectification (svi_set_rectification): both cameras' maps in one device block, [camera][xy short2 | frac uint16]
     // with rect_npad (W * H rounded up to 4) entries each; off = all null, no launch, copy or allocation anywhere
@@ -196,13 +188,6 @@ FrameGeom make_geom(const svi_ctx* c, int img_pitch, size_t img_stride) {
     g.resp_pitch = c->resp_pitch;
     g.box_pitch = c->box_pitch;
     return g;
-}
-
-void* arena_alloc(svi_ctx* c, size_t bytes) {
-    size_t off = (c->arena_used + 255) & ~size_t(255);
-    if (off + bytes > c->arena_bytes) return nullptr;
-    c->arena_used = off + bytes;
-    return c->arena + off;
 }
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point lookup (no libcuda link needed).
@@ -521,7 +506,7 @@ int rectify_one(svi_ctx* ctx, int cam, const uint8_t* raw, size_t pitch, size_t 
 
 }  // namespace
 
-// ---- per-query entry points: one image (or pair) staged in lane 0, queries in the arena ----
+// ---- per-query entry points: one image (or pair) staged in lane 0, queries in the call buffer ----
 namespace {
 // Page-locked caller memory (cudaMallocHost, cudaHostRegister, a pinned torch tensor: a camera driver's DMA buffers) is
 // read by the copy engine directly; anything else goes through the library's pinned mirror, because a cudaMemcpyAsync
@@ -561,59 +546,166 @@ int stage_box(svi_ctx* ctx, const uint8_t* img, size_t pitch, uint8_t* d_img, ui
     CK(cudaGetLastError());
     return SVI_SUCCESS;
 }
-template <typename T>
-int upload(svi_ctx* ctx, T** d, const T* h, size_t count, cudaStream_t s) {
-    *d = static_cast<T*>(arena_alloc(ctx, count * sizeof(T)));
-    if (!*d) return fail(ctx, SVI_ERR_CAPACITY, "query arena exhausted: raise svi_params.max_queries");
-    if (h && ctx->pin_arena) {
-        unsigned char* mirror = ctx->pin_arena + (reinterpret_cast<unsigned char*>(*d) - ctx->arena);
-        std::memcpy(mirror, h, count * sizeof(T));
-        // batch_uploads: the caller sends the whole staged range with ONE copy once every input is in the mirror
-        if (!ctx->batch_uploads) CK(cudaMemcpyAsync(*d, mirror, count * sizeof(T), cudaMemcpyHostToDevice, s));
-    } else if (h) {
-        CK(cudaMemcpyAsync(*d, h, count * sizeof(T), cudaMemcpyHostToDevice, s));
+
+// ---- the call buffer (DESIGN.md section 3).  Every user lays out [inputs | outputs | scratch] with CallLayout, makes
+// room with reserve_call before it enqueues anything that touches the buffer, memcpys its inputs into the pinned mirror,
+// sends them up with one copy (call_send), zeroes its outputs with one memset where it needs them zeroed, and brings them
+// back with one copy and one synchronisation (call_fetch) before it memcpys them into the caller's arrays.  Pageable
+// caller arrays therefore never turn a transfer into a blocking staged copy.
+struct CallLayout {
+    size_t end = 0;
+    size_t take(size_t bytes) {   // 256-byte-aligned offset of the next `bytes`
+        const size_t o = end;
+        end = (end + bytes + 255) & ~size_t(255);
+        return o;
     }
+};
+
+// The size svi_create gives the buffer before the cap; the match entry points still bound their inputs by it.
+size_t query_bytes(const svi_ctx* c) {
+    return (size_t)c->p.max_queries * 512 + (size_t)c->p.max_corners * 64 + 3 * (size_t)c->H * c->dev_pitch + (1 << 20);
+}
+
+// Grows the buffer to twice the need (a tracker's measurement lists get longer frame by frame).  Nothing is in flight on
+// it: every user leaves lane 0 idle when it returns.
+int reserve_call(svi_ctx* ctx, size_t bytes) {
+    if (bytes <= ctx->call_bytes) return SVI_SUCCESS;
+    if (ctx->call_dev) cudaFree(ctx->call_dev);
+    if (ctx->call_pin) cudaFreeHost(ctx->call_pin);
+    ctx->call_dev = nullptr; ctx->call_pin = nullptr; ctx->call_bytes = 0;
+    const size_t want = std::max<size_t>(2 * bytes, 1u << 20);
+    CK(cudaMalloc(reinterpret_cast<void**>(&ctx->call_dev), want));
+    CK(cudaMallocHost(reinterpret_cast<void**>(&ctx->call_pin), want));
+    ctx->call_bytes = want;
     return SVI_SUCCESS;
 }
-// Result array that lives in the arena -> caller's buffer: async copy into the pinned mirror now, memcpy after the sync.
-int download(svi_ctx* ctx, void* host, const void* dev, size_t bytes, cudaStream_t s) {
-    const unsigned char* d = static_cast<const unsigned char*>(dev);
-    if (ctx->pin_arena && d >= ctx->arena && d + bytes <= ctx->arena + ctx->arena_bytes) {
-        unsigned char* mirror = ctx->pin_arena + (d - ctx->arena);
-        CK(cudaMemcpyAsync(mirror, dev, bytes, cudaMemcpyDeviceToHost, s));
-        ctx->pending.push_back({host, mirror, bytes});
-    } else {
-        CK(cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, s));
-    }
+
+template <typename T = unsigned char>
+T* dev_at(const svi_ctx* c, size_t o) { return reinterpret_cast<T*>(c->call_dev + o); }
+
+void put(svi_ctx* c, size_t o, const void* h, size_t bytes) {   // a null host array stages nothing
+    if (h) std::memcpy(c->call_pin + o, h, bytes);
+}
+
+int call_send(svi_ctx* ctx, size_t in_end, cudaStream_t s) {
+    CK(cudaMemcpyAsync(ctx->call_dev, ctx->call_pin, in_end, cudaMemcpyHostToDevice, s));
     return SVI_SUCCESS;
 }
-int flush_downloads(svi_ctx* ctx, cudaStream_t s) {
+
+int call_fetch(svi_ctx* ctx, size_t begin, size_t end, cudaStream_t s) {
+    CK(cudaMemcpyAsync(ctx->call_pin + begin, ctx->call_dev + begin, end - begin, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    for (const svi_ctx::Pending& q : ctx->pending) std::memcpy(q.host, q.pinned, q.bytes);
-    ctx->pending.clear();
     return SVI_SUCCESS;
 }
-#define UP(d, h, count)                                        \
-    do {                                                       \
-        int rc_ = upload(ctx, &(d), (h), (count), s);          \
-        if (rc_ != SVI_SUCCESS) return rc_;                    \
-    } while (0)
+
+// Declared first in every user of the buffer: a call that fails part-way still leaves lane 0 idle, so that the next
+// call may overwrite the mirror.  The successful path ends in a synchronisation of its own and sets `done`.
+struct SyncOnFailure {
+    cudaStream_t s;
+    bool done = false;
+    ~SyncOnFailure() { if (!done) cudaStreamSynchronize(s); }
+};
+
+// svi_landmarks of n landmarks, with or without the three stage-3 arrays
+struct LandmarkLayout {
+    bool stage3;
+    size_t xyz, dl, dr, disp, size, uvref = 0, dref = 0, tdet = 0;
+    LandmarkLayout(CallLayout& L, size_t n, bool with_stage3) : stage3(with_stage3) {
+        xyz = L.take(24 * n); dl = L.take(32 * n); dr = L.take(32 * n); disp = L.take(4 * n); size = L.take(4 * n);
+        if (stage3) { uvref = L.take(16 * n); dref = L.take(32 * n); tdet = L.take(128 * n); }
+    }
+    void put_all(svi_ctx* c, const svi_landmarks& lm, size_t n) const {
+        put(c, xyz, lm.xyz_world, 24 * n); put(c, dl, lm.last_desc_left, 32 * n); put(c, dr, lm.last_desc_right, 32 * n);
+        put(c, disp, lm.last_disparity, 4 * n); put(c, size, lm.keypoint_size, 4 * n);
+        if (stage3) { put(c, uvref, lm.uv_reference_left, 16 * n); put(c, dref, lm.desc_reference_left, 32 * n); put(c, tdet, lm.T_left_to_world_at_detection, 128 * n); }
+    }
+    SvLandmarksDev sv(const svi_ctx* c) const {   // the stage-3 arrays are null without them
+        return SvLandmarksDev{dev_at<double>(c, xyz), dev_at(c, dl), dev_at(c, dr), dev_at<float>(c, disp), dev_at<float>(c, size),
+                              stage3 ? dev_at<double>(c, uvref) : nullptr, stage3 ? dev_at(c, dref) : nullptr, stage3 ? dev_at<double>(c, tdet) : nullptr};
+    }
+    LandmarksDev ld(const svi_ctx* c) const {
+        const SvLandmarksDev s = sv(c);
+        return LandmarksDev{s.xyz_w, s.desc_l, s.desc_r, s.disparity, s.size};
+    }
+    Stage3Extra ex(const svi_ctx* c) const {
+        const SvLandmarksDev s = sv(c);
+        return Stage3Extra{s.uv_ref, s.T_det};
+    }
+};
+
+// The seven svi_track_result arrays of n landmarks, one contiguous range [status, end)
+struct TrackLayout {
+    size_t status, stage, uv_l, uv_r, xyz, desc_l, desc_r, end;
+    TrackLayout(CallLayout& L, size_t n) {
+        status = L.take(n); stage = L.take(n); uv_l = L.take(8 * n); uv_r = L.take(8 * n); xyz = L.take(24 * n);
+        desc_l = L.take(32 * n); desc_r = L.take(32 * n); end = L.end;
+    }
+    TrackOutDev dev(const svi_ctx* c) const {
+        return TrackOutDev{dev_at(c, status), dev_at(c, stage), dev_at<float>(c, uv_l), dev_at<float>(c, uv_r), dev_at<double>(c, xyz),
+                           dev_at(c, desc_l), dev_at(c, desc_r)};
+    }
+    void copy_out(const svi_ctx* c, size_t n, const svi_track_result& r) const {   // from the mirror, after call_fetch
+        const unsigned char* h = c->call_pin;
+        std::memcpy(r.status, h + status, n);
+        std::memcpy(r.stage, h + stage, n);
+        std::memcpy(r.uv_left, h + uv_l, 8 * n);
+        std::memcpy(r.uv_right, h + uv_r, 8 * n);
+        std::memcpy(r.xyz_left, h + xyz, 24 * n);
+        std::memcpy(r.desc_left, h + desc_l, 32 * n);
+        std::memcpy(r.desc_right, h + desc_r, 32 * n);
+    }
+};
+
+PositIn posit_in(const svi_ctx* ctx, const double* xyz, const float* uv_l, const float* uv_r, const double* T_estimate, const double* T_last,
+                 const double* t_imu) {
+    PositIn pi{};
+    pi.xyz_world = xyz;
+    pi.uv_left = uv_l;
+    pi.uv_right = uv_r;
+    std::memcpy(pi.P_left, ctx->cam_l.P, sizeof(pi.P_left));
+    std::memcpy(pi.P_right, ctx->cam_r.P, sizeof(pi.P_right));
+    std::memcpy(pi.T_estimate, T_estimate, sizeof(pi.T_estimate));
+    std::memcpy(pi.T_last, T_last, sizeof(pi.T_last));
+    std::memcpy(pi.t_imu, t_imu, sizeof(pi.t_imu));
+    return pi;
+}
+void posit_result_from(const PositOut& po, svi_posit_result* r) {
+    std::memcpy(r->T_world_to_left, po.T, sizeof(r->T_world_to_left));
+    r->outcome = (uint8_t)po.outcome;
+    r->iterations = po.iterations;
+    r->inliers = po.inliers;
+    r->average_squared_error = po.average_squared_error;
+    r->risk = po.risk;
+}
+void posit_too_few(const double* T_estimate, svi_posit_result* r) {   // svi_solve_stereo_posit's answer for n <= 25
+    std::memcpy(r->T_world_to_left, T_estimate, sizeof(r->T_world_to_left));
+    r->outcome = SVI_POSIT_TOO_FEW_POINTS;
+    r->iterations = 0;
+    r->inliers = 0;
+    r->average_squared_error = 0.0;
+    r->risk = 0.0;
+}
 }  // namespace
 
 
 namespace {
-// getMaskActiveLandmarks on the device: lane.mask (plane 0) = 255 with a radius-7 disc of zeros per centre.
+// getMaskActiveLandmarks on the device: lane.mask (plane 0) = 255 with a radius-7 disc of zeros per centre.  On success the
+// centres may still be in flight: the caller synchronises lane 0 before it returns.
 int build_mask(svi_ctx* ctx, Lane& l, const float* centres, int n_centres) {
     cudaStream_t s = l.stream;
+    SyncOnFailure idle{s};
     const size_t bytes = (size_t)ctx->H * ctx->dev_pitch;
     mask_fill_kernel<<<(unsigned)((bytes / 16 + 256) / 256), 256, 0, s>>>(l.mask, bytes);
     if (n_centres > 0) {
-        ctx->arena_used = 0; ctx->pending.clear();
-        float* d_c;
-        UP(d_c, centres, (size_t)n_centres * 2);
-        mask_discs_kernel<<<(n_centres * 15 + 255) / 256, 256, 0, s>>>(l.mask, ctx->W, ctx->H, ctx->dev_pitch, d_c, n_centres);
+        CallLayout L;
+        const size_t i_c = L.take(sizeof(float) * 2 * n_centres);
+        if (const int rc = reserve_call(ctx, L.end)) return rc;
+        put(ctx, i_c, centres, sizeof(float) * 2 * n_centres);
+        if (const int rc = call_send(ctx, L.end, s)) return rc;
+        mask_discs_kernel<<<(n_centres * 15 + 255) / 256, 256, 0, s>>>(l.mask, ctx->W, ctx->H, ctx->dev_pitch, dev_at<float>(ctx, i_c), n_centres);
     }
     CK(cudaGetLastError());
+    idle.done = true;
     return SVI_SUCCESS;
 }
 
@@ -726,38 +818,44 @@ int triangulate_common(svi_ctx* ctx, bool left_search, const uint8_t* img, size_
     CK(cudaSetDevice(ctx->device));
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
-    ctx->arena_used = 0; ctx->pending.clear();
+    SyncOnFailure idle{s};
+    const size_t N = (size_t)n;
+    CallLayout L;   // [range (left search) | top_left | uv_ref | desc_ref] -> [uv | xyz | desc | dist | idx | status]
+    const size_t i_range = left_search ? L.take(4 * N) : 0, i_tl = L.take(8 * N), i_uv = L.take(8 * N), i_desc = L.take(32 * N);
+    const size_t in_end = L.end;
+    const size_t o_uv = L.take(8 * N), o_xyz = L.take(24 * N), o_desc = L.take(32 * N), o_dist = L.take(4 * N), o_idx = L.take(4 * N),
+                 o_status = L.take(N);
+    if (const int rc = reserve_call(ctx, L.end)) return rc;
     int rc = stage_box(ctx, img, pitch, l.img_l, l.box_l, l.box_ls, s, left_search ? 0 : 1);
     if (rc != SVI_SUCCESS) return rc;
-    float* d_range = nullptr; float* d_tl; float* d_uv; uint8_t* d_desc;
-    TriOutDev o;
-    if (left_search) UP(d_range, search_range, (size_t)n);
-    UP(d_tl, top_left, (size_t)n * 2);
-    UP(d_uv, uv_ref, (size_t)n * 2);
-    UP(d_desc, desc_ref, (size_t)n * 32);
-    UP(o.uv, (const float*)nullptr, (size_t)n * 2);
-    UP(o.xyz, (const double*)nullptr, (size_t)n * 3);
-    UP(o.desc, (const uint8_t*)nullptr, (size_t)n * 32);
-    UP(o.dist, (const int*)nullptr, (size_t)n);
-    UP(o.idx, (const int*)nullptr, (size_t)n);
-    UP(o.status, (const uint8_t*)nullptr, (size_t)n);
-    CK(cudaMemsetAsync(o.uv, 0, sizeof(float) * 2 * n, s));
-    CK(cudaMemsetAsync(o.xyz, 0, sizeof(double) * 3 * n, s));
-    CK(cudaMemsetAsync(o.desc, 0, (size_t)32 * n, s));
+    if (left_search) put(ctx, i_range, search_range, 4 * N);
+    put(ctx, i_tl, top_left, 8 * N);
+    put(ctx, i_uv, uv_ref, 8 * N);
+    put(ctx, i_desc, desc_ref, 32 * N);
+    if ((rc = call_send(ctx, in_end, s)) != SVI_SUCCESS) return rc;
+    CK(cudaMemsetAsync(ctx->call_dev + in_end, 0, L.end - in_end, s));
+    const TriOutDev o{dev_at<float>(ctx, o_uv), dev_at<double>(ctx, o_xyz), dev_at(ctx, o_desc), dev_at<int>(ctx, o_dist), dev_at<int>(ctx, o_idx),
+                      dev_at(ctx, o_status)};
+    const float* d_tl = dev_at<float>(ctx, i_tl);
+    const float* d_uv = dev_at<float>(ctx, i_uv);
+    const uint8_t* d_desc = dev_at(ctx, i_desc);
     const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
     const int blocks = (n + MATCH_WARPS - 1) / MATCH_WARPS;
     if (left_search)
-        triangulate_kernel<true><<<blocks, MATCH_WARPS * 32, MATCH_SMEM, s>>>(l.map_l, l.map_ls, g, ctx->tc, n, d_range, d_tl, d_uv, d_desc, size, o);
+        triangulate_kernel<true><<<blocks, MATCH_WARPS * 32, MATCH_SMEM, s>>>(l.map_l, l.map_ls, g, ctx->tc, n, dev_at<float>(ctx, i_range), d_tl, d_uv,
+                                                                            d_desc, size, o);
     else
         triangulate_kernel<false><<<blocks, MATCH_WARPS * 32, MATCH_SMEM, s>>>(l.map_l, l.map_ls, g, ctx->tc, n, nullptr, d_tl, d_uv, d_desc, size, o);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out->uv, o.uv, sizeof(float) * 2 * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(out->xyz_left, o.xyz, sizeof(double) * 3 * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(out->desc, o.desc, (size_t)32 * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(out->distance, o.dist, sizeof(int) * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(out->match_index, o.idx, sizeof(int) * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(out->status, o.status, (size_t)n, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, in_end, L.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
+    const unsigned char* h = ctx->call_pin;
+    std::memcpy(out->uv, h + o_uv, 8 * N);
+    std::memcpy(out->xyz_left, h + o_xyz, 24 * N);
+    std::memcpy(out->desc, h + o_desc, 32 * N);
+    std::memcpy(out->distance, h + o_dist, 4 * N);
+    std::memcpy(out->match_index, h + o_idx, 4 * N);
+    std::memcpy(out->status, h + o_status, N);
     return SVI_SUCCESS;
 }
 }  // namespace
@@ -1008,12 +1106,10 @@ void svi_destroy(svi_ctx* ctx) {
     if (ctx->h_overflow) cudaFreeHost(const_cast<int*>(ctx->h_overflow));
     if (ctx->side_done) cudaEventDestroy(ctx->side_done);
     if (ctx->side) cudaStreamDestroy(ctx->side);
-    if (ctx->arena) cudaFree(ctx->arena);
-    if (ctx->opt_dev) cudaFree(ctx->opt_dev);
-    if (ctx->opt_pin) cudaFreeHost(ctx->opt_pin);
+    if (ctx->call_dev) cudaFree(ctx->call_dev);
+    if (ctx->call_pin) cudaFreeHost(ctx->call_pin);
     if (ctx->pin) cudaFreeHost(ctx->pin);
     if (ctx->small_block) cudaFree(ctx->small_block);
-    if (ctx->pin_arena) cudaFreeHost(ctx->pin_arena);
     if (ctx->trk_img) cudaFree(ctx->trk_img);
     if (ctx->s3_items) cudaFree(ctx->s3_items);
     if (ctx->resp_one) cudaFree(ctx->resp_one);
@@ -1255,9 +1351,10 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     CK(cudaStreamCreateWithFlags(&ctx->side, cudaStreamNonBlocking));
     CK(cudaEventCreateWithFlags(&ctx->side_done, cudaEventDisableTiming));
     CK(dmalloc(&ctx->trk_img, 2 * HH * ctx->dev_pitch));
-    ctx->arena_bytes = (size_t)p.max_queries * 512 + (size_t)p.max_corners * 64 + 3 * HH * ctx->dev_pitch + (1 << 20);
-    CK(cudaMalloc(reinterpret_cast<void**>(&ctx->arena), ctx->arena_bytes));
-    if (ctx->arena_bytes <= (64u << 20)) CK(cudaMallocHost(reinterpret_cast<void**>(&ctx->pin_arena), ctx->arena_bytes));
+    // sized so that the per-query and tracking calls of up to max_queries items never grow it (reserve_call)
+    ctx->call_bytes = std::min<size_t>(query_bytes(ctx), 64u << 20);
+    CK(cudaMalloc(reinterpret_cast<void**>(&ctx->call_dev), ctx->call_bytes));
+    CK(cudaMallocHost(reinterpret_cast<void**>(&ctx->call_pin), ctx->call_bytes));
     // room for kSmallFrames frames: three image planes in, every output array out
     ctx->pin_bytes = (size_t)kSmallFrames * (3 * HH * ctx->dev_pitch + (size_t)p.max_corners * kOutBytesPerSlot + 64) + 16;
     if (ctx->pin_bytes <= (64u << 20)) CK(cudaMallocHost(reinterpret_cast<void**>(&ctx->pin), ctx->pin_bytes));
@@ -1423,10 +1520,12 @@ int svi_mask_active_landmarks(svi_ctx* ctx, const float* centres_xy, int n_centr
     if (n_centres > ctx->p.max_queries) return fail(ctx, SVI_ERR_CAPACITY, "svi_mask_active_landmarks: n_centres > max_queries");
     CK(cudaSetDevice(ctx->device));
     Lane& l = ctx->lanes[0];
+    SyncOnFailure idle{l.stream};
     int rc = build_mask(ctx, l, centres_xy, n_centres);
     if (rc != SVI_SUCCESS) return rc;
     CK(cudaMemcpy2DAsync(mask, pitch, l.mask, ctx->dev_pitch, ctx->W, ctx->H, cudaMemcpyDeviceToHost, l.stream));
     CK(cudaStreamSynchronize(l.stream));
+    idle.done = true;
     return SVI_SUCCESS;
 }
 
@@ -1537,19 +1636,22 @@ int svi_describe(svi_ctx* ctx, const uint8_t* img, size_t pitch, const float* xy
     CK(cudaSetDevice(ctx->device));
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
-    ctx->arena_used = 0; ctx->pending.clear();
+    SyncOnFailure idle{s};
+    const size_t N = (size_t)n;
+    CallLayout L;   // [xy] -> [desc | kept]
+    const size_t i_xy = L.take(8 * N), o_desc = L.take(32 * N), o_kept = L.take(N);
+    if (const int rc = reserve_call(ctx, L.end)) return rc;
     int rc = stage_box(ctx, img, pitch, l.img_l, l.box_l, l.box_ls, s, 0);
     if (rc != SVI_SUCCESS) return rc;
-    float* d_xy; uint8_t* d_desc; uint8_t* d_kept;
-    UP(d_xy, xy, (size_t)n * 2);
-    UP(d_desc, (const uint8_t*)nullptr, (size_t)n * 32);
-    UP(d_kept, (const uint8_t*)nullptr, (size_t)n);
+    put(ctx, i_xy, xy, 8 * N);
+    if ((rc = call_send(ctx, o_desc, s)) != SVI_SUCCESS) return rc;
     const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
-    describe_kernel<<<(n + 3) / 4, 128, 0, s>>>(l.box_l, g, d_xy, n, d_desc, d_kept);
+    describe_kernel<<<(n + 3) / 4, 128, 0, s>>>(l.box_l, g, dev_at<float>(ctx, i_xy), n, dev_at(ctx, o_desc), dev_at(ctx, o_kept));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(desc32, d_desc, (size_t)n * 32, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(kept, d_kept, (size_t)n, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, o_desc, L.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
+    std::memcpy(desc32, ctx->call_pin + o_desc, 32 * N);
+    std::memcpy(kept, ctx->call_pin + o_kept, N);
     return SVI_SUCCESS;
 }
 
@@ -1558,21 +1660,25 @@ int svi_match_hamming(svi_ctx* ctx, const uint8_t* query32, int n_query, const u
     if (!ctx) return SVI_ERR_INVALID;
     if (!query32 || !index || !distance || n_query < 0 || n_train < 0 || (n_train > 0 && !train32))
         return fail(ctx, SVI_ERR_INVALID, "svi_match_hamming: bad argument");
-    if ((size_t)(n_query + n_train) * 40 > ctx->arena_bytes) return fail(ctx, SVI_ERR_CAPACITY, "svi_match_hamming: raise max_queries");
+    if ((size_t)(n_query + n_train) * 40 > query_bytes(ctx)) return fail(ctx, SVI_ERR_CAPACITY, "svi_match_hamming: raise max_queries");
     if (n_query == 0) return SVI_SUCCESS;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->lanes[0].stream;
-    ctx->arena_used = 0; ctx->pending.clear();
-    uint8_t* d_q; uint8_t* d_t; int* d_i; int* d_d;
-    UP(d_q, query32, (size_t)n_query * 32);
-    UP(d_t, n_train > 0 ? train32 : (const uint8_t*)nullptr, (size_t)std::max(n_train, 1) * 32);
-    UP(d_i, (const int*)nullptr, (size_t)n_query);
-    UP(d_d, (const int*)nullptr, (size_t)n_query);
-    hamming_match_kernel<<<(n_query + 3) / 4, 128, 0, s>>>(d_q, n_query, d_t, n_train, d_i, d_d);
+    SyncOnFailure idle{s};
+    const size_t Q = (size_t)n_query, T = (size_t)std::max(n_train, 1);
+    CallLayout L;   // [query | train] -> [index | distance]
+    const size_t i_q = L.take(32 * Q), i_t = L.take(32 * T), o_i = L.take(4 * Q), o_d = L.take(4 * Q);
+    if (const int rc = reserve_call(ctx, L.end)) return rc;
+    put(ctx, i_q, query32, 32 * Q);
+    put(ctx, i_t, n_train > 0 ? train32 : nullptr, 32 * T);
+    int rc = call_send(ctx, o_i, s);
+    if (rc != SVI_SUCCESS) return rc;
+    hamming_match_kernel<<<(n_query + 3) / 4, 128, 0, s>>>(dev_at(ctx, i_q), n_query, dev_at(ctx, i_t), n_train, dev_at<int>(ctx, o_i), dev_at<int>(ctx, o_d));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(index, d_i, sizeof(int) * n_query, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(distance, d_d, sizeof(int) * n_query, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, o_i, L.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
+    std::memcpy(index, ctx->call_pin + o_i, 4 * Q);
+    std::memcpy(distance, ctx->call_pin + o_d, 4 * Q);
     return SVI_SUCCESS;
 }
 
@@ -1583,27 +1689,32 @@ int svi_match_epipolar(svi_ctx* ctx, const uint8_t* query32, const float* query_
     if (!query32 || !query_xy || !index || !distance || !second_distance || n_query < 0 || n_train < 0 ||
         (n_train > 0 && (!train32 || !train_xy)))
         return fail(ctx, SVI_ERR_INVALID, "svi_match_epipolar: bad argument");
-    if ((size_t)(n_query + n_train) * 48 + (size_t)n_query * 16 > ctx->arena_bytes)
+    if ((size_t)(n_query + n_train) * 48 + (size_t)n_query * 16 > query_bytes(ctx))
         return fail(ctx, SVI_ERR_CAPACITY, "svi_match_epipolar: raise max_queries");
     if (n_query == 0) return SVI_SUCCESS;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->lanes[0].stream;
-    ctx->arena_used = 0; ctx->pending.clear();
-    uint8_t* d_q; uint8_t* d_t; float* d_qxy; float* d_txy; int* d_i; int* d_d; int* d_s;
-    UP(d_q, query32, (size_t)n_query * 32);
-    UP(d_qxy, query_xy, (size_t)n_query * 2);
-    UP(d_t, n_train > 0 ? train32 : (const uint8_t*)nullptr, (size_t)std::max(n_train, 1) * 32);
-    UP(d_txy, n_train > 0 ? train_xy : (const float*)nullptr, (size_t)std::max(n_train, 1) * 2);
-    UP(d_i, (const int*)nullptr, (size_t)n_query);
-    UP(d_d, (const int*)nullptr, (size_t)n_query);
-    UP(d_s, (const int*)nullptr, (size_t)n_query);
-    epipolar_match_kernel<<<(n_query + 3) / 4, 128, 0, s>>>(d_q, d_qxy, n_query, d_t, d_txy, n_train, band_v, min_disparity,
-                                                            max_disparity, d_i, d_d, d_s);
+    SyncOnFailure idle{s};
+    const size_t Q = (size_t)n_query, T = (size_t)std::max(n_train, 1);
+    CallLayout L;   // [query | query_xy | train | train_xy] -> [index | distance | second_distance]
+    const size_t i_q = L.take(32 * Q), i_qxy = L.take(8 * Q), i_t = L.take(32 * T), i_txy = L.take(8 * T);
+    const size_t o_i = L.take(4 * Q), o_d = L.take(4 * Q), o_s = L.take(4 * Q);
+    if (const int rc = reserve_call(ctx, L.end)) return rc;
+    put(ctx, i_q, query32, 32 * Q);
+    put(ctx, i_qxy, query_xy, 8 * Q);
+    put(ctx, i_t, n_train > 0 ? train32 : nullptr, 32 * T);
+    put(ctx, i_txy, n_train > 0 ? train_xy : nullptr, 8 * T);
+    int rc = call_send(ctx, o_i, s);
+    if (rc != SVI_SUCCESS) return rc;
+    epipolar_match_kernel<<<(n_query + 3) / 4, 128, 0, s>>>(dev_at(ctx, i_q), dev_at<float>(ctx, i_qxy), n_query, dev_at(ctx, i_t), dev_at<float>(ctx, i_txy),
+                                                            n_train, band_v, min_disparity, max_disparity, dev_at<int>(ctx, o_i), dev_at<int>(ctx, o_d),
+                                                            dev_at<int>(ctx, o_s));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(index, d_i, sizeof(int) * n_query, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(distance, d_d, sizeof(int) * n_query, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(second_distance, d_s, sizeof(int) * n_query, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, o_i, L.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
+    std::memcpy(index, ctx->call_pin + o_i, 4 * Q);
+    std::memcpy(distance, ctx->call_pin + o_d, 4 * Q);
+    std::memcpy(second_distance, ctx->call_pin + o_s, 4 * Q);
     return SVI_SUCCESS;
 }
 
@@ -1627,17 +1738,21 @@ int svi_point_in_left(svi_ctx* ctx, int n, const float* uv_left, const float* uv
     if (n == 0) return SVI_SUCCESS;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->lanes[0].stream;
-    ctx->arena_used = 0; ctx->pending.clear();
-    float* d_l; float* d_r; double* d_xyz; uint8_t* d_st;
-    UP(d_l, uv_left, (size_t)n * 2);
-    UP(d_r, uv_right, (size_t)n * 2);
-    UP(d_xyz, (const double*)nullptr, (size_t)n * 3);
-    UP(d_st, (const uint8_t*)nullptr, (size_t)n);
-    point_in_left_kernel<<<(n + 127) / 128, 128, 0, s>>>(ctx->tc, n, d_l, d_r, d_xyz, d_st);
+    SyncOnFailure idle{s};
+    const size_t N = (size_t)n;
+    CallLayout L;   // [uv_left | uv_right] -> [xyz | status]
+    const size_t i_l = L.take(8 * N), i_r = L.take(8 * N), o_xyz = L.take(24 * N), o_st = L.take(N);
+    if (const int rc = reserve_call(ctx, L.end)) return rc;
+    put(ctx, i_l, uv_left, 8 * N);
+    put(ctx, i_r, uv_right, 8 * N);
+    int rc = call_send(ctx, o_xyz, s);
+    if (rc != SVI_SUCCESS) return rc;
+    point_in_left_kernel<<<(n + 127) / 128, 128, 0, s>>>(ctx->tc, n, dev_at<float>(ctx, i_l), dev_at<float>(ctx, i_r), dev_at<double>(ctx, o_xyz), dev_at(ctx, o_st));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(xyz_left, d_xyz, sizeof(double) * 3 * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(status, d_st, (size_t)n, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, o_xyz, L.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
+    std::memcpy(xyz_left, ctx->call_pin + o_xyz, 24 * N);
+    std::memcpy(status, ctx->call_pin + o_st, N);
     return SVI_SUCCESS;
 }
 
@@ -1674,77 +1789,33 @@ int svi_track_landmarks_stages(svi_ctx* ctx, const uint8_t* img_left, const uint
     int rc = ensure_track_scratch(ctx);
     if (rc != SVI_SUCCESS) return rc;
     cudaStream_t s = ctx->lanes[0].stream;
-    ctx->arena_used = 0; ctx->pending.clear();
+    SyncOnFailure idle{s};
+    // every input array goes up in ONE copy; the outputs form one contiguous range behind them: one memset, one copy back
+    CallLayout L;
+    const LandmarkLayout li(L, (size_t)n, stage3);
+    const size_t in_end = L.end;
+    const TrackLayout lo(L, (size_t)n);
+    if ((rc = reserve_call(ctx, L.end)) != SVI_SUCCESS) return rc;
     using clk = std::chrono::steady_clock;
     clk::time_point tp[6];
     auto tick = [&](int i) { if (ctx->trace) tp[i] = clk::now(); };
     tick(0);
     rc = stage_track_pair(ctx, img_left, img_right, pitch);
     if (rc != SVI_SUCCESS) return rc;
-    // every input array goes through the pinned mirror of the arena and up in ONE copy; the outputs form one contiguous
-    // range behind them: one memset, one copy back
-    double* d_xyzw; uint8_t* d_dl; uint8_t* d_dr; float* d_disp; float* d_size;
-    ctx->batch_uploads = ctx->pin_arena != nullptr;
-    struct Unbatch { svi_ctx* c; ~Unbatch() { c->batch_uploads = false; } } unbatch{ctx};
-    UP(d_xyzw, lm->xyz_world, (size_t)n * 3);
-    UP(d_dl, lm->last_desc_left, (size_t)n * 32);
-    UP(d_dr, lm->last_desc_right, (size_t)n * 32);
-    UP(d_disp, lm->last_disparity, (size_t)n);
-    UP(d_size, lm->keypoint_size, (size_t)n);
-    Stage3Extra ex{nullptr, nullptr};
-    uint8_t* d_orig = nullptr;
-    if (stage3) {
-        double* d_uvref; double* d_tdet;
-        UP(d_uvref, lm->uv_reference_left, (size_t)n * 2);
-        UP(d_tdet, lm->T_left_to_world_at_detection, (size_t)n * 16);
-        UP(d_orig, lm->desc_reference_left, (size_t)n * 32);
-        ex.uv_ref = d_uvref; ex.T_det = d_tdet;
-    }
+    li.put_all(ctx, *lm, (size_t)n);
     tick(1);
-    if (ctx->batch_uploads) CK(cudaMemcpyAsync(ctx->arena, ctx->pin_arena, ctx->arena_used, cudaMemcpyHostToDevice, s));
-    ctx->batch_uploads = false;
-    const size_t out_begin = (ctx->arena_used + 255) & ~size_t(255);
-    TrackOutDev o;
-    UP(o.status, (const uint8_t*)nullptr, (size_t)n);
-    UP(o.stage, (const uint8_t*)nullptr, (size_t)n);
-    UP(o.uv_l, (const float*)nullptr, (size_t)n * 2);
-    UP(o.uv_r, (const float*)nullptr, (size_t)n * 2);
-    UP(o.xyz, (const double*)nullptr, (size_t)n * 3);
-    UP(o.desc_l, (const uint8_t*)nullptr, (size_t)n * 32);
-    UP(o.desc_r, (const uint8_t*)nullptr, (size_t)n * 32);
-    const size_t out_end = ctx->arena_used;
-    CK(cudaMemsetAsync(ctx->arena + out_begin, 0, out_end - out_begin, s));
+    if ((rc = call_send(ctx, in_end, s)) != SVI_SUCCESS) return rc;
+    CK(cudaMemsetAsync(ctx->call_dev + lo.status, 0, lo.end - lo.status, s));
     // The whole cascade is ONE stream of kernels; the host only waits once, for the results.
-    rc = enqueue_cascade(ctx, n, T_world_to_left, motion_scaling, stage_mask, LandmarksDev{d_xyzw, d_dl, d_dr, d_disp, d_size}, ex, d_orig, o, nullptr);
+    rc = enqueue_cascade(ctx, n, T_world_to_left, motion_scaling, stage_mask, li.ld(ctx), li.ex(ctx), li.sv(ctx).desc_ref, lo.dev(ctx), nullptr);
     if (rc != SVI_SUCCESS) return rc;
     tick(2);
-    int rd = SVI_SUCCESS;
-    if (ctx->pin_arena) {   // one copy for the whole output range, scattered to the caller's arrays after the synchronisation
-        cudaError_t e = cudaMemcpyAsync(ctx->pin_arena + out_begin, ctx->arena + out_begin, out_end - out_begin, cudaMemcpyDeviceToHost, s);
-        if (e != cudaSuccess) rd = fail(ctx, SVI_ERR_CUDA, std::string("cudaMemcpyAsync: ") + cudaGetErrorString(e));
-        auto mirror = [&](const void* d) { return ctx->pin_arena + (static_cast<const unsigned char*>(d) - ctx->arena); };
-        ctx->pending.push_back({out->status, mirror(o.status), (size_t)n});
-        ctx->pending.push_back({out->stage, mirror(o.stage), (size_t)n});
-        ctx->pending.push_back({out->uv_left, mirror(o.uv_l), sizeof(float) * 2 * n});
-        ctx->pending.push_back({out->uv_right, mirror(o.uv_r), sizeof(float) * 2 * n});
-        ctx->pending.push_back({out->xyz_left, mirror(o.xyz), sizeof(double) * 3 * n});
-        ctx->pending.push_back({out->desc_left, mirror(o.desc_l), (size_t)32 * n});
-        ctx->pending.push_back({out->desc_right, mirror(o.desc_r), (size_t)32 * n});
-    } else {
-        rd = download(ctx, out->status, o.status, (size_t)n, s);
-        if (rd == SVI_SUCCESS) rd = download(ctx, out->stage, o.stage, (size_t)n, s);
-        if (rd == SVI_SUCCESS) rd = download(ctx, out->uv_left, o.uv_l, sizeof(float) * 2 * n, s);
-        if (rd == SVI_SUCCESS) rd = download(ctx, out->uv_right, o.uv_r, sizeof(float) * 2 * n, s);
-        if (rd == SVI_SUCCESS) rd = download(ctx, out->xyz_left, o.xyz, sizeof(double) * 3 * n, s);
-        if (rd == SVI_SUCCESS) rd = download(ctx, out->desc_left, o.desc_l, (size_t)32 * n, s);
-        if (rd == SVI_SUCCESS) rd = download(ctx, out->desc_right, o.desc_r, (size_t)32 * n, s);
-    }
-    if (ctx->trace) { cudaStreamSynchronize(s); tick(3); }
-    if (rd == SVI_SUCCESS) rd = flush_downloads(ctx, s);
-    else cudaStreamSynchronize(s);
+    if ((rc = call_fetch(ctx, lo.status, lo.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
+    tick(3);
+    lo.copy_out(ctx, (size_t)n, *out);
     tick(4);
-    if (rd != SVI_SUCCESS) return rd;
-    rd = check_overflow(ctx);
+    const int rd = check_overflow(ctx);
     tick(5);
     if (ctx->trace) {
         auto us = [&](int a, int b) { return std::chrono::duration<double, std::micro>(tp[b] - tp[a]).count(); };
@@ -1754,22 +1825,6 @@ int svi_track_landmarks_stages(svi_ctx* ctx, const uint8_t* img_left, const uint
     }
     return rd;
 }
-
-namespace {
-// the staging pair of svi_optimize_landmarks / svi_solve_stereo_posit: one device buffer + its pinned mirror, grown to
-// twice the need (a tracker's measurement lists get longer frame by frame)
-int reserve_opt(svi_ctx* ctx, size_t total) {
-    if (total <= ctx->opt_bytes) return SVI_SUCCESS;
-    if (ctx->opt_dev) cudaFree(ctx->opt_dev);
-    if (ctx->opt_pin) cudaFreeHost(ctx->opt_pin);
-    ctx->opt_dev = nullptr; ctx->opt_pin = nullptr; ctx->opt_bytes = 0;
-    const size_t want = std::max<size_t>(2 * total, 1u << 20);
-    CK(cudaMalloc(reinterpret_cast<void**>(&ctx->opt_dev), want));
-    CK(cudaMallocHost(reinterpret_cast<void**>(&ctx->opt_pin), want));
-    ctx->opt_bytes = want;
-    return SVI_SUCCESS;
-}
-}  // namespace
 
 int svi_optimize_landmarks(svi_ctx* ctx, const svi_landmark_measurements* in, int n, svi_optimize_result* out) {
     if (!ctx) return SVI_ERR_INVALID;
@@ -1788,39 +1843,35 @@ int svi_optimize_landmarks(svi_ctx* ctx, const svi_landmark_measurements* in, in
     CK(cudaSetDevice(ctx->device));
     using clk = std::chrono::steady_clock;
     const clk::time_point t_begin = clk::now();
-    // layout: [xyz_guess | proj_left | proj_right | first | pose_index | uv_left | uv_right] -> [xyz | avg | iterations | outcome]
-    const size_t P = (size_t)in->n_poses;
-    size_t off = 0;
-    auto take = [&off](size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-    const size_t o_guess = take(sizeof(double) * 3 * n), o_pl = take(sizeof(double) * 12 * P), o_pr = take(sizeof(double) * 12 * P);
-    const size_t o_first = take(sizeof(int) * ((size_t)n + 1)), o_pose = take(sizeof(int) * (size_t)m);
-    const size_t o_uvl = take(sizeof(float) * 2 * (size_t)m), o_uvr = take(sizeof(float) * 2 * (size_t)m);
-    const size_t in_bytes = off;
-    const size_t o_xyz = take(sizeof(double) * 3 * n), o_avg = take(sizeof(double) * n), o_it = take(sizeof(int) * (size_t)n), o_out = take((size_t)n);
-    const size_t total = off;
-    if (const int rc = reserve_opt(ctx, total)) return rc;
-    unsigned char* hp = ctx->opt_pin;
-    std::memcpy(hp + o_guess, in->xyz_world_guess, sizeof(double) * 3 * n);
-    std::memcpy(hp + o_first, in->first, sizeof(int) * ((size_t)n + 1));
-    if (m > 0) {
-        std::memcpy(hp + o_pl, in->proj_world_to_left, sizeof(double) * 12 * P);
-        std::memcpy(hp + o_pr, in->proj_world_to_right, sizeof(double) * 12 * P);
-        std::memcpy(hp + o_pose, in->pose_index, sizeof(int) * (size_t)m);
-        std::memcpy(hp + o_uvl, in->uv_left, sizeof(float) * 2 * (size_t)m);
-        std::memcpy(hp + o_uvr, in->uv_right, sizeof(float) * 2 * (size_t)m);
-    }
     cudaStream_t s = ctx->lanes[0].stream;
+    SyncOnFailure idle{s};
+    const size_t P = (size_t)in->n_poses;
+    CallLayout L;   // [xyz_guess | proj_left | proj_right | first | pose_index | uv_left | uv_right] -> [xyz | avg | iterations | outcome]
+    const size_t o_guess = L.take(sizeof(double) * 3 * n), o_pl = L.take(sizeof(double) * 12 * P), o_pr = L.take(sizeof(double) * 12 * P);
+    const size_t o_first = L.take(sizeof(int) * ((size_t)n + 1)), o_pose = L.take(sizeof(int) * (size_t)m);
+    const size_t o_uvl = L.take(sizeof(float) * 2 * (size_t)m), o_uvr = L.take(sizeof(float) * 2 * (size_t)m);
+    const size_t o_xyz = L.take(sizeof(double) * 3 * n), o_avg = L.take(sizeof(double) * n), o_it = L.take(sizeof(int) * (size_t)n), o_out = L.take((size_t)n);
+    if (const int rc = reserve_call(ctx, L.end)) return rc;
+    put(ctx, o_guess, in->xyz_world_guess, sizeof(double) * 3 * n);
+    put(ctx, o_first, in->first, sizeof(int) * ((size_t)n + 1));
+    if (m > 0) {
+        put(ctx, o_pl, in->proj_world_to_left, sizeof(double) * 12 * P);
+        put(ctx, o_pr, in->proj_world_to_right, sizeof(double) * 12 * P);
+        put(ctx, o_pose, in->pose_index, sizeof(int) * (size_t)m);
+        put(ctx, o_uvl, in->uv_left, sizeof(float) * 2 * (size_t)m);
+        put(ctx, o_uvr, in->uv_right, sizeof(float) * 2 * (size_t)m);
+    }
     const clk::time_point t_staged = clk::now();
-    CK(cudaMemcpyAsync(ctx->opt_dev, hp, in_bytes, cudaMemcpyHostToDevice, s));
-    unsigned char* d = ctx->opt_dev;
-    LandmarkOptIn li{reinterpret_cast<const double*>(d + o_guess), reinterpret_cast<const int*>(d + o_first), reinterpret_cast<const int*>(d + o_pose),
-                     reinterpret_cast<const float*>(d + o_uvl), reinterpret_cast<const float*>(d + o_uvr), reinterpret_cast<const double*>(d + o_pl),
-                     reinterpret_cast<const double*>(d + o_pr), in->n_poses};
-    LandmarkOptOut lo{reinterpret_cast<double*>(d + o_xyz), d + o_out, reinterpret_cast<double*>(d + o_avg), reinterpret_cast<int*>(d + o_it)};
+    int rc = call_send(ctx, o_xyz, s);
+    if (rc != SVI_SUCCESS) return rc;
+    LandmarkOptIn li{dev_at<const double>(ctx, o_guess), dev_at<const int>(ctx, o_first), dev_at<const int>(ctx, o_pose), dev_at<const float>(ctx, o_uvl),
+                     dev_at<const float>(ctx, o_uvr), dev_at<const double>(ctx, o_pl), dev_at<const double>(ctx, o_pr), in->n_poses};
+    LandmarkOptOut lo{dev_at<double>(ctx, o_xyz), dev_at(ctx, o_out), dev_at<double>(ctx, o_avg), dev_at<int>(ctx, o_it)};
     optimize_landmarks_kernel<<<(n + kOptWarps - 1) / kOptWarps, kOptWarps * 32, 0, s>>>(li, n, lo);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(hp + o_xyz, d + o_xyz, total - o_xyz, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, o_xyz, L.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
+    const unsigned char* hp = ctx->call_pin;
     std::memcpy(out->xyz_world, hp + o_xyz, sizeof(double) * 3 * n);
     std::memcpy(out->average_squared_error, hp + o_avg, sizeof(double) * n);
     std::memcpy(out->outcome, hp + o_out, (size_t)n);
@@ -1854,54 +1905,33 @@ int svi_solve_stereo_posit(svi_ctx* ctx, const svi_posit_problem* in, svi_posit_
     if (!in || !out || in->n < 0) return fail(ctx, SVI_ERR_INVALID, "svi_solve_stereo_posit: bad argument");
     const int n = in->n;
     if (n > 0 && (!in->xyz_world || !in->uv_left || !in->uv_right)) return fail(ctx, SVI_ERR_INVALID, "svi_solve_stereo_posit: null array");
-    std::memcpy(out->T_world_to_left, in->T_estimate, sizeof(out->T_world_to_left));
-    out->iterations = 0;
-    out->inliers = 0;
-    out->average_squared_error = 0.0;
-    out->risk = 0.0;
     if (n <= kPositMinimumPoints) {   // !(m_uMinimumPointsForPoseOptimization < uNumberOfMeasurements): fails before any iteration
-        out->outcome = SVI_POSIT_TOO_FEW_POINTS;
+        posit_too_few(in->T_estimate, out);
         return SVI_SUCCESS;
     }
     CK(cudaSetDevice(ctx->device));
     using clk = std::chrono::steady_clock;
     const clk::time_point t_begin = clk::now();
-    // layout: [xyz | uv_left | uv_right] -> [PositOut]
-    size_t off = 0;
-    auto take = [&off](size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-    const size_t o_xyz = take(sizeof(double) * 3 * (size_t)n), o_uvl = take(sizeof(float) * 2 * (size_t)n), o_uvr = take(sizeof(float) * 2 * (size_t)n);
-    const size_t in_bytes = off;
-    const size_t o_out = take(sizeof(PositOut));
-    if (const int rc = reserve_opt(ctx, off)) return rc;
-    unsigned char* hp = ctx->opt_pin;
-    std::memcpy(hp + o_xyz, in->xyz_world, sizeof(double) * 3 * (size_t)n);
-    std::memcpy(hp + o_uvl, in->uv_left, sizeof(float) * 2 * (size_t)n);
-    std::memcpy(hp + o_uvr, in->uv_right, sizeof(float) * 2 * (size_t)n);
-    PositIn pi{};
-    unsigned char* d = ctx->opt_dev;
-    pi.xyz_world = reinterpret_cast<const double*>(d + o_xyz);
-    pi.uv_left = reinterpret_cast<const float*>(d + o_uvl);
-    pi.uv_right = reinterpret_cast<const float*>(d + o_uvr);
-    std::memcpy(pi.P_left, ctx->cam_l.P, sizeof(pi.P_left));
-    std::memcpy(pi.P_right, ctx->cam_r.P, sizeof(pi.P_right));
-    std::memcpy(pi.T_estimate, in->T_estimate, sizeof(pi.T_estimate));
-    std::memcpy(pi.T_last, in->T_last, sizeof(pi.T_last));
-    std::memcpy(pi.t_imu, in->t_imu, sizeof(pi.t_imu));
     cudaStream_t s = ctx->lanes[0].stream;
+    SyncOnFailure idle{s};
+    const size_t N = (size_t)n;
+    CallLayout L;   // [xyz | uv_left | uv_right] -> [PositOut]
+    const size_t o_xyz = L.take(24 * N), o_uvl = L.take(8 * N), o_uvr = L.take(8 * N), o_out = L.take(sizeof(PositOut));
+    if (const int rc = reserve_call(ctx, L.end)) return rc;
+    put(ctx, o_xyz, in->xyz_world, 24 * N);
+    put(ctx, o_uvl, in->uv_left, 8 * N);
+    put(ctx, o_uvr, in->uv_right, 8 * N);
+    const PositIn pi = posit_in(ctx, dev_at<double>(ctx, o_xyz), dev_at<float>(ctx, o_uvl), dev_at<float>(ctx, o_uvr), in->T_estimate, in->T_last, in->t_imu);
     const clk::time_point t_staged = clk::now();
-    CK(cudaMemcpyAsync(d, hp, in_bytes, cudaMemcpyHostToDevice, s));
-    stereo_posit_kernel<<<1, kPositThreads, kPositSmemBytes, s>>>(pi, n, reinterpret_cast<PositOut*>(d + o_out));
+    int rc = call_send(ctx, o_out, s);
+    if (rc != SVI_SUCCESS) return rc;
+    stereo_posit_kernel<<<1, kPositThreads, kPositSmemBytes, s>>>(pi, n, dev_at<PositOut>(ctx, o_out));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(hp + o_out, d + o_out, sizeof(PositOut), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, o_out, L.end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
     PositOut po;
-    std::memcpy(&po, hp + o_out, sizeof(po));
-    std::memcpy(out->T_world_to_left, po.T, sizeof(out->T_world_to_left));
-    out->outcome = (uint8_t)po.outcome;
-    out->iterations = po.iterations;
-    out->inliers = po.inliers;
-    out->average_squared_error = po.average_squared_error;
-    out->risk = po.risk;
+    std::memcpy(&po, ctx->call_pin + o_out, sizeof(po));
+    posit_result_from(po, out);
     if (ctx->trace) {
         const clk::time_point t_end = clk::now();
         auto us = [](clk::time_point a, clk::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
@@ -1912,22 +1942,6 @@ int svi_solve_stereo_posit(svi_ctx* ctx, const svi_posit_problem* in, svi_posit_
 }
 
 namespace {
-void posit_result_from(const PositOut& po, svi_posit_result* r) {
-    std::memcpy(r->T_world_to_left, po.T, sizeof(r->T_world_to_left));
-    r->outcome = (uint8_t)po.outcome;
-    r->iterations = po.iterations;
-    r->inliers = po.inliers;
-    r->average_squared_error = po.average_squared_error;
-    r->risk = po.risk;
-}
-void posit_too_few(const double* T_estimate, svi_posit_result* r) {   // svi_solve_stereo_posit's answer for n <= 25
-    std::memcpy(r->T_world_to_left, T_estimate, sizeof(r->T_world_to_left));
-    r->outcome = SVI_POSIT_TOO_FEW_POINTS;
-    r->iterations = 0;
-    r->inliers = 0;
-    r->average_squared_error = 0.0;
-    r->risk = 0.0;
-}
 bool track_result_ok(const svi_track_result& r) {
     return r.status && r.stage && r.uv_left && r.uv_right && r.xyz_left && r.desc_left && r.desc_right;
 }
@@ -1963,65 +1977,45 @@ int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uin
     int rc = ensure_track_scratch(ctx);
     if (rc != SVI_SUCCESS) return rc;
     cudaStream_t s = ctx->lanes[0].stream;
-    rc = stage_track_pair(ctx, img_left, img_right, pitch);
-    if (rc != SVI_SUCCESS) return rc;
-
-    // One device block + its pinned mirror (the staging pair of svi_solve_stereo_posit):
+    SyncOnFailure idle{s};
+    // The call buffer:
     //   [inputs: the landmark arrays and flags]            one copy up
     //   [outputs: attempts, pose stage, route, epipolar]   one memset, one copy down
     //   [scratch: counts, index lists, gathered subset, subset results, pose problem]
     const size_t N = (size_t)n;
-    size_t off = 0;
-    auto take = [&off](size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-    const size_t i_xyz = take(24 * N), i_dl = take(32 * N), i_dr = take(32 * N), i_disp = take(4 * N), i_size = take(4 * N), i_uvref = take(16 * N),
-                 i_dref = take(32 * N), i_tdet = take(128 * N), i_flags = take(N);
-    const size_t in_bytes = off;
-    const size_t o_posit = take(2 * sizeof(PositOut));
-    auto take_track = [&](size_t* o7) {
-        o7[0] = take(N); o7[1] = take(N); o7[2] = take(8 * N); o7[3] = take(8 * N); o7[4] = take(24 * N); o7[5] = take(32 * N); o7[6] = take(32 * N);
-    };
-    size_t o_pose[7], o_epi[7], x_sub[7];
-    take_track(o_pose);
-    const size_t o_route = take(N);
-    take_track(o_epi);
-    const size_t out_end = off;
+    CallLayout L;
+    const LandmarkLayout i_lm(L, N, true);
+    const size_t i_flags = L.take(N);
+    const size_t in_end = L.end;
+    const size_t o_posit = L.take(2 * sizeof(PositOut));
+    const TrackLayout o_pose(L, N);
+    const size_t o_route = L.take(N);
+    const TrackLayout o_epi(L, N);
+    const size_t out_end = L.end;
     // counts: [0] candidates, [1] pose hits, [2] epipolar set, [3] regional set
-    const size_t x_cnt = take(4 * sizeof(int)), x_cand = take(4 * N), x_hits = take(4 * N), x_epi = take(4 * N), x_reg = take(4 * N);
-    const size_t x_xyz = take(24 * N), x_dl = take(32 * N), x_dr = take(32 * N), x_disp = take(4 * N), x_size = take(4 * N), x_uvref = take(16 * N),
-                 x_dref = take(32 * N), x_tdet = take(128 * N);
-    take_track(x_sub);
-    const size_t x_pxyz = take(24 * N), x_puvl = take(8 * N), x_puvr = take(8 * N);
-    if (const int r = reserve_opt(ctx, off)) return r;
-    unsigned char* hp = ctx->opt_pin;
-    unsigned char* d = ctx->opt_dev;
-    std::memcpy(hp + i_xyz, lm.xyz_world, 24 * N);
-    std::memcpy(hp + i_dl, lm.last_desc_left, 32 * N);
-    std::memcpy(hp + i_dr, lm.last_desc_right, 32 * N);
-    std::memcpy(hp + i_disp, lm.last_disparity, 4 * N);
-    std::memcpy(hp + i_size, lm.keypoint_size, 4 * N);
-    std::memcpy(hp + i_uvref, lm.uv_reference_left, 16 * N);
-    std::memcpy(hp + i_dref, lm.desc_reference_left, 32 * N);
-    std::memcpy(hp + i_tdet, lm.T_left_to_world_at_detection, 128 * N);
-    std::memcpy(hp + i_flags, in->flags, N);
-    CK(cudaMemcpyAsync(d, hp, in_bytes, cudaMemcpyHostToDevice, s));
-    CK(cudaMemsetAsync(d + o_posit, 0, out_end - o_posit, s));
-    auto dp = [d](size_t o) { return d + o; };
-    auto dd = [d](size_t o) { return reinterpret_cast<double*>(d + o); };
-    auto df = [d](size_t o) { return reinterpret_cast<float*>(d + o); };
-    auto di = [d](size_t o) { return reinterpret_cast<int*>(d + o); };
-    auto track_out = [&](const size_t* o7) { return TrackOutDev{dp(o7[0]), dp(o7[1]), df(o7[2]), df(o7[3]), dd(o7[4]), dp(o7[5]), dp(o7[6])}; };
-    const SvLandmarksDev all{dd(i_xyz), dp(i_dl), dp(i_dr), df(i_disp), df(i_size), dd(i_uvref), dp(i_dref), dd(i_tdet)};
-    const SvLandmarksDev sub{dd(x_xyz), dp(x_dl), dp(x_dr), df(x_disp), df(x_size), dd(x_uvref), dp(x_dref), dd(x_tdet)};
-    const LandmarksDev sub_ld{sub.xyz_w, sub.desc_l, sub.desc_r, sub.disparity, sub.size};
-    const Stage3Extra sub_ex{sub.uv_ref, sub.T_det};
-    const TrackOutDev pose_out = track_out(o_pose), epi_out = track_out(o_epi), sub_out = track_out(x_sub);
+    const size_t x_cnt = L.take(4 * sizeof(int)), x_cand = L.take(4 * N), x_hits = L.take(4 * N), x_epi = L.take(4 * N), x_reg = L.take(4 * N);
+    const LandmarkLayout x_lm(L, N, true);
+    const TrackLayout x_sub(L, N);
+    const size_t x_pxyz = L.take(24 * N), x_puvl = L.take(8 * N), x_puvr = L.take(8 * N);
+    if ((rc = reserve_call(ctx, L.end)) != SVI_SUCCESS) return rc;
+    rc = stage_track_pair(ctx, img_left, img_right, pitch);
+    if (rc != SVI_SUCCESS) return rc;
+    unsigned char* hp = ctx->call_pin;
+    i_lm.put_all(ctx, lm, N);
+    put(ctx, i_flags, in->flags, N);
+    if ((rc = call_send(ctx, in_end, s)) != SVI_SUCCESS) return rc;
+    CK(cudaMemsetAsync(ctx->call_dev + o_posit, 0, out_end - o_posit, s));
+    auto dp = [ctx](size_t o) { return dev_at(ctx, o); };
+    auto di = [ctx](size_t o) { return dev_at<int>(ctx, o); };
+    const SvLandmarksDev all = i_lm.sv(ctx), sub = x_lm.sv(ctx);
+    const TrackOutDev pose_out = o_pose.dev(ctx), epi_out = o_epi.dev(ctx), sub_out = x_sub.dev(ctx);
     int* cnt = di(x_cnt);
-    PositOut* posit_dev = reinterpret_cast<PositOut*>(d + o_posit);
+    PositOut* posit_dev = dev_at<PositOut>(ctx, o_posit);
     uint8_t* route = dp(o_route);
     const unsigned blocks = (unsigned)((n + 127) / 128);
     // the subset results start as a fresh tracking call's outputs: zero
     auto clear_sub = [&]() -> int {
-        CK(cudaMemsetAsync(d + x_sub[0], 0, x_pxyz - x_sub[0], s));
+        CK(cudaMemsetAsync(ctx->call_dev + x_sub.status, 0, x_sub.end - x_sub.status, s));
         return SVI_SUCCESS;
     };
 
@@ -2035,21 +2029,14 @@ int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uin
         attempts = a + 1;
         if (n_cand > 0) {
             if ((rc = clear_sub()) != SVI_SUCCESS) return rc;
-            rc = enqueue_cascade(ctx, n_cand, priors[a], in->motion_scaling, SVI_STAGE_1 | SVI_STAGE_2, sub_ld, sub_ex, nullptr, sub_out, nullptr);
+            rc = enqueue_cascade(ctx, n_cand, priors[a], in->motion_scaling, SVI_STAGE_1 | SVI_STAGE_2, x_lm.ld(ctx), x_lm.ex(ctx), nullptr, sub_out, nullptr);
             if (rc != SVI_SUCCESS) return rc;
         }
         // the solver's measurements: the hits in candidate order
         sv_compact_kernel<<<1, kCompactThreads, 0, s>>>(sub_out.stage, n_cand, 0x1Eu /* stages 1..4 */, di(x_hits), cnt + 1);
-        sv_posit_assemble_kernel<<<blocks, 128, 0, s>>>(di(x_hits), cnt + 1, n, sub.xyz_w, sub_out, dd(x_pxyz), df(x_puvl), df(x_puvr));
-        PositIn pi{};
-        pi.xyz_world = dd(x_pxyz);
-        pi.uv_left = df(x_puvl);
-        pi.uv_right = df(x_puvr);
-        std::memcpy(pi.P_left, ctx->cam_l.P, sizeof(pi.P_left));
-        std::memcpy(pi.P_right, ctx->cam_r.P, sizeof(pi.P_right));
-        std::memcpy(pi.T_estimate, priors[a], sizeof(pi.T_estimate));
-        std::memcpy(pi.T_last, in->T_last, sizeof(pi.T_last));
-        std::memcpy(pi.t_imu, in->t_imu, sizeof(pi.t_imu));
+        const PositIn pi = posit_in(ctx, dev_at<double>(ctx, x_pxyz), dev_at<float>(ctx, x_puvl), dev_at<float>(ctx, x_puvr), priors[a], in->T_last, in->t_imu);
+        sv_posit_assemble_kernel<<<blocks, 128, 0, s>>>(di(x_hits), cnt + 1, n, sub.xyz_w, sub_out, dev_at<double>(ctx, x_pxyz), dev_at<float>(ctx, x_puvl),
+                                                        dev_at<float>(ctx, x_puvr));
         stereo_posit_count_kernel<<<1, kPositThreads, kPositSmemBytes, s>>>(pi, cnt + 1, posit_dev + a);
         CK(cudaGetLastError());
         // wait: the outcome decides whether the damped attempt runs
@@ -2075,7 +2062,7 @@ int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uin
     sv_gather_kernel<<<blocks, 128, 0, s>>>(all, di(x_epi), cnt + 2, n, sub);
     CK(cudaGetLastError());
     if ((rc = clear_sub()) != SVI_SUCCESS) return rc;
-    rc = enqueue_cascade(ctx, n, T, in->motion_scaling, SVI_STAGE_3, sub_ld, sub_ex, sub.desc_ref, sub_out, cnt + 2);
+    rc = enqueue_cascade(ctx, n, T, in->motion_scaling, SVI_STAGE_3, x_lm.ld(ctx), x_lm.ex(ctx), sub.desc_ref, sub_out, cnt + 2);
     if (rc != SVI_SUCCESS) return rc;
     sv_scatter_kernel<<<blocks, 128, 0, s>>>(di(x_epi), cnt + 2, n, sub_out, epi_out, route);   // + the SVI_EPI_NO_TRANSLATION re-route
     // ---- regional stage 2 on the unmoved ones and the re-routed ones; wait: its launch sizes need the count
@@ -2090,14 +2077,14 @@ int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uin
         sv_gather_kernel<<<blocks, 128, 0, s>>>(all, di(x_reg), cnt + 3, n, sub);
         CK(cudaGetLastError());
         if ((rc = clear_sub()) != SVI_SUCCESS) return rc;
-        rc = enqueue_cascade(ctx, n_reg, T, in->motion_scaling, SVI_STAGE_2, sub_ld, sub_ex, nullptr, sub_out, nullptr);
+        rc = enqueue_cascade(ctx, n_reg, T, in->motion_scaling, SVI_STAGE_2, x_lm.ld(ctx), x_lm.ex(ctx), nullptr, sub_out, nullptr);
         if (rc != SVI_SUCCESS) return rc;
         sv_scatter_kernel<<<blocks, 128, 0, s>>>(di(x_reg), cnt + 3, n, sub_out, epi_out, nullptr);
         CK(cudaGetLastError());
     }
     // ---- every result in one copy
-    CK(cudaMemcpyAsync(hp + o_posit, d + o_posit, out_end - o_posit, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = call_fetch(ctx, o_posit, out_end, s)) != SVI_SUCCESS) return rc;
+    idle.done = true;
     for (int a = 0; a < 2; ++a) {
         if (a < attempts) posit_result_from(*reinterpret_cast<const PositOut*>(hp + o_posit + a * sizeof(PositOut)), &out->attempt[a]);
         else std::memset(&out->attempt[a], 0, sizeof(out->attempt[a]));
@@ -2107,18 +2094,9 @@ int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uin
     out->measurements[1] = measurements[1];
     out->source = accepted == 0 ? SVI_SV_POSIT : accepted == 1 ? SVI_SV_POSIT_DAMPED : SVI_SV_PRIOR;
     std::memcpy(out->T_world_to_left, T, sizeof(T));
-    auto scatter = [&](const size_t* o7, const svi_track_result& r) {
-        std::memcpy(r.status, hp + o7[0], N);
-        std::memcpy(r.stage, hp + o7[1], N);
-        std::memcpy(r.uv_left, hp + o7[2], 8 * N);
-        std::memcpy(r.uv_right, hp + o7[3], 8 * N);
-        std::memcpy(r.xyz_left, hp + o7[4], 24 * N);
-        std::memcpy(r.desc_left, hp + o7[5], 32 * N);
-        std::memcpy(r.desc_right, hp + o7[6], 32 * N);
-    };
-    scatter(o_pose, out->pose_stage);
+    o_pose.copy_out(ctx, N, out->pose_stage);
     std::memcpy(out->route, hp + o_route, N);
-    scatter(o_epi, out->epipolar_stage);
+    o_epi.copy_out(ctx, N, out->epipolar_stage);
     return check_overflow(ctx);
 }
 
