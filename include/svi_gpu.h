@@ -206,6 +206,42 @@ int svi_match_epipolar(svi_ctx* ctx, const uint8_t* query32, const float* query_
                        float min_disparity, float max_disparity, int32_t* index, int32_t* distance,
                        int32_t* second_distance);
 
+/* Sparse stereo frames (optional mode; not a reference code path -- the reference matches by dense scan lines, as
+ * svi_stereo_frames does): addNewLandmarks with LEFT key-points matched against RIGHT key-points inside an epipolar row band,
+ * for a batch of independent pairs in one call.  Per frame:
+ *   - LEFT: detection (svi_params.detector, with the optional masks), selection, BRIEF's border filter and descriptors as in
+ *     svi_stereo_frames: n_keypoints, n_detected, uv_left and desc_left are byte-identical to that call's;
+ *   - RIGHT: the same detector without a mask, the same selection and border filter -- the list svi_detect(RIGHT) followed
+ *     by svi_describe's `kept` filter gives; match_index indexes it;
+ *   - per LEFT slot, the admissible RIGHT key-points are those svi_match_epipolar admits (fp32 tests as written there) for
+ *     this band.  None: SVI_TRI_NO_MATCH, distance = match_index = second_distance = -1.  Otherwise the first arg-min
+ *     (lowest index on ties) and the second-smallest admissible distance; !(float(distance) < params.match_cutoff) gives
+ *     SVI_TRI_DISTANCE (distance and index still written); else getPointInLEFT(uv_left, uv_right) as svi_point_in_left
+ *     gives SVI_TRI_ZERO_DISP or SVI_OK with xyz_left, uv_right and desc_right (the matched RIGHT key-point's).
+ * No ratio test is applied: second_distance is there for the caller's.  While rectification is set both images are raw.
+ * SVI_ERR_INVALID for a NaN band field or min_disparity > max_disparity.  A frame whose candidate list overflows on either
+ * side gets zero key-points on that side and the call returns SVI_ERR_CAPACITY (FAST mode: more corners than max_corners
+ * on either side is SVI_ERR_CAPACITY too).  The first call allocates the per-lane scratch of this mode. */
+typedef struct svi_sparse_band {
+    float band_v;          /* |y_L - y_R| <= band_v                       */
+    float min_disparity;   /* min_disparity <= x_L - x_R <= max_disparity */
+    float max_disparity;
+} svi_sparse_band;
+typedef struct svi_sparse_result {
+    int32_t* second_distance;    /* [frames * capacity_per_frame] second-smallest admissible distance, -1 if < 2 admissible */
+    int32_t* n_keypoints_right;  /* [frames] RIGHT key-points after BRIEF's border filter */
+} svi_sparse_result;
+int svi_stereo_frames_sparse(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride,
+                             int n_frames, const uint8_t* masks_or_null, const svi_sparse_band* band,
+                             svi_stereo_result* out, svi_sparse_result* sparse);
+
+/* Same on DEVICE pointers (images, masks and every array of *out and *sparse), enqueued after the work on `cuda_stream`
+ * like svi_stereo_frames_device; returns without synchronising.  Capacity overflows are reported by svi_check_overflow. */
+int svi_stereo_frames_sparse_device(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch,
+                                    size_t frame_stride, int n_frames, const uint8_t* masks_or_null,
+                                    const svi_sparse_band* band, const svi_stereo_result* out,
+                                    const svi_sparse_result* sparse, void* cuda_stream);
+
 /* Per-query results of the triangulating scan-line searches. */
 typedef struct svi_tri_result {
     float* uv;          /* [n*2] matched point in the searched image */

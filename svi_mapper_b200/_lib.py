@@ -21,7 +21,7 @@ SVI_ERR_INVALID, SVI_ERR_CUDA, SVI_ERR_CAPACITY, SVI_ERR_NO_DEVICE, SVI_ERR_UNSU
 
 EXPORTS = (
     "svi_params_default", "svi_status_text", "svi_brief_table_info", "svi_create", "svi_destroy", "svi_last_error", "svi_device_count",
-    "svi_stereo_frames", "svi_stereo_frames_device", "svi_check_overflow", "svi_mask_active_landmarks", "svi_stereo_frame_masked", "svi_harris_response", "svi_detect", "svi_describe",
+    "svi_stereo_frames", "svi_stereo_frames_device", "svi_stereo_frames_sparse", "svi_stereo_frames_sparse_device", "svi_check_overflow", "svi_mask_active_landmarks", "svi_stereo_frame_masked", "svi_harris_response", "svi_detect", "svi_describe",
     "svi_match_hamming", "svi_match_epipolar", "svi_triangulate_right", "svi_triangulate_left", "svi_point_in_left",
     "svi_track_landmarks", "svi_track_landmarks_stages", "svi_set_profiling", "svi_stage_timings", "svi_config", "svi_kernels_per_chunk", "svi_optimize_landmarks",
     "svi_solve_stereo_posit", "svi_track_frame_stereo_only",
@@ -55,6 +55,15 @@ class StereoResult(C.Structure):
         ("desc_left", C.c_void_p), ("desc_right", C.c_void_p), ("distance", C.c_void_p),
         ("match_index", C.c_void_p), ("status", C.c_void_p),
     ]
+
+
+class SparseBand(C.Structure):
+    """svi_sparse_band: |y_L - y_R| <= band_v and min_disparity <= x_L - x_R <= max_disparity."""
+    _fields_ = [("band_v", C.c_float), ("min_disparity", C.c_float), ("max_disparity", C.c_float)]
+
+
+class SparseResult(C.Structure):
+    _fields_ = [("second_distance", C.c_void_p), ("n_keypoints_right", C.c_void_p)]
 
 
 class TriResult(C.Structure):
@@ -147,6 +156,9 @@ def load(path=None):
     lib.svi_device_count.argtypes = []
     lib.svi_stereo_frames.argtypes = [vp, vp, vp, sz, sz, ci, vp, C.POINTER(StereoResult)]
     lib.svi_stereo_frames_device.argtypes = [vp, vp, vp, sz, sz, ci, vp, C.POINTER(StereoResult), vp]
+    lib.svi_stereo_frames_sparse.argtypes = [vp, vp, vp, sz, sz, ci, vp, C.POINTER(SparseBand), C.POINTER(StereoResult), C.POINTER(SparseResult)]
+    lib.svi_stereo_frames_sparse_device.argtypes = [vp, vp, vp, sz, sz, ci, vp, C.POINTER(SparseBand), C.POINTER(StereoResult),
+                                                    C.POINTER(SparseResult), vp]
     lib.svi_check_overflow.argtypes = [vp]
     lib.svi_mask_active_landmarks.argtypes = [vp, vp, ci, vp, sz]
     lib.svi_stereo_frame_masked.argtypes = [vp, vp, vp, sz, vp, ci, C.POINTER(StereoResult)]

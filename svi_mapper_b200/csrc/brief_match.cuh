@@ -864,46 +864,6 @@ __global__ void hamming_match_kernel(const uint8_t* __restrict__ q32, int nq, co
     }
 }
 
-// svi_match_epipolar: one warp per query; lanes stride over the trains, admissible ones (row band + disparity
-// window) are compared with XOR / popc; warp-shuffle reduction of (best key, second-best distance).
-__global__ void epipolar_match_kernel(const uint8_t* __restrict__ q32, const float* __restrict__ qxy, int nq,
-                                      const uint8_t* __restrict__ t32, const float* __restrict__ txy, int nt, float band_v,
-                                      float min_disp, float max_disp, int* __restrict__ index, int* __restrict__ distance,
-                                      int* __restrict__ second) {
-    const int lane = threadIdx.x & 31, q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (q >= nq) return;
-    uint32_t ref[kDescWords];
-    load_desc(q32 + (size_t)q * 32, ref);
-    const float xq = qxy[2 * q], yq = qxy[2 * q + 1];
-    unsigned long long best = ~0ull;   // (distance << 32 | train index): min == first arg-min
-    uint32_t second_d = 0xFFFFFFFFu;
-    for (int t = lane; t < nt; t += 32) {
-        const float d = xq - txy[2 * t];
-        if (fabsf(yq - txy[2 * t + 1]) <= band_v && d >= min_disp && d <= max_disp) {
-            uint32_t w[kDescWords];
-            load_desc(t32 + (size_t)t * 32, w);
-            const unsigned long long k = ((unsigned long long)hamming_words(ref, w) << 32) | (unsigned)t;
-            if (k < best) { second_d = min(second_d, (uint32_t)(best >> 32)); best = k; }
-            else second_d = min(second_d, (uint32_t)(k >> 32));
-        }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const unsigned long long ob = __shfl_xor_sync(0xFFFFFFFFu, best, o);
-        const uint32_t os = __shfl_xor_sync(0xFFFFFFFFu, second_d, o);
-        // merge two (best, second) pairs: the larger of the two bests competes with both seconds
-        const unsigned long long lo = min(best, ob), hi = max(best, ob);
-        second_d = min(min(second_d, os), (uint32_t)(hi >> 32));
-        best = lo;
-    }
-    if (lane == 0) {
-        const bool any = best != ~0ull;
-        index[q] = any ? (int)(best & 0xFFFFFFFFu) : -1;
-        distance[q] = any ? (int)(best >> 32) : -1;
-        second[q] = (second_d != 0xFFFFFFFFu) ? (int)second_d : -1;
-    }
-}
-
 struct TriOutDev {
     float* uv; double* xyz; uint8_t* desc; int* dist; int* idx; uint8_t* status;
 };

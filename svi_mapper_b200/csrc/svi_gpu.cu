@@ -21,6 +21,7 @@
 #include <vector>
 
 #include "../../include/svi_gpu.h"
+#include "band_match.cuh"
 #include "brief_match.cuh"
 #include "binned.cuh"
 #include "harris.cuh"
@@ -77,6 +78,20 @@ struct Lane {
     ushort2* bin_kp = nullptr;         // [chunk][max_corners]
     CUtensorMap map_l_bin{}, map_r_bin{}, map_rs_bin{};
     StereoOutDev out{};
+    // sparse frames (svi_stereo_frames_sparse): allocated at the first such call, [chunk][max_corners] lists padded by
+    // BM_ALIGN elements (band_match_kernel's copies round the streamed range out to 16-byte addresses)
+    ushort2* sp_kp_r = nullptr;        // RIGHT key-points after BRIEF's border filter, detector order
+    int* sp_n_kp_r = nullptr;          // [chunk]: their count (host path; the device path writes the caller's array)
+    int* sp_n_det_r = nullptr;         // [chunk]
+    int* sp_row_l = nullptr;           // [chunk][H + 1]: row CSR of the LEFT key-points
+    uint32_t* sp_slot_l = nullptr;     // LEFT key-points sorted by row: their slot ...
+    ushort2* sp_kp_l = nullptr;        // ... and coordinates
+    int* sp_row_r = nullptr;           // the same for RIGHT
+    uint32_t* sp_slot_r = nullptr;
+    ushort2* sp_kp_rs = nullptr;
+    uint8_t* sp_desc_r = nullptr;      // RIGHT descriptors in row order
+    int* sp_second = nullptr;          // second-smallest distance per LEFT slot (host path)
+    CUtensorMap map_r_patch{};         // RIGHT plane, box = the 56 x 49 patch of one descriptor
     std::vector<cudaEvent_t> ev;  // stage boundary events (profiling)
     size_t ev_used = 0;
     std::vector<uint8_t> ev_pre;  // per profiled chunk: did describe_left_kernel run between its two events?
@@ -287,6 +302,37 @@ int setup_binned(svi_ctx* ctx, Lane& l, size_t rows, std::string* err) {
     return SVI_SUCCESS;
 }
 
+// The detector on nf frames of one image: candidate lists in the lane's scratch (zeroed by the caller), and the image's box-sum
+// plane `box` (harris_box writes it from its own tile; in FAST mode boxsum9, without the shifted copy).  With the selection
+// below, the detection of the dense path (LEFT) and of both sides of the sparse path.
+void launch_detector(svi_ctx* ctx, Lane& l, const uint8_t* d_img, const uint8_t* d_mask, const FrameGeom& g, int nf, uint16_t* box) {
+    cudaStream_t s = l.stream;
+    const dim3 tiles((g.W + HT_W - 1) / HT_W, (g.H + HT_H - 1) / HT_H, nf);
+    if (ctx->p.detector == SVI_DETECTOR_FAST_9_16) {
+        fast_candidates_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, d_mask, g, ctx->p.fast_threshold, ctx->p.fast_nonmax, l.cand,
+                                                            l.cand_count, ctx->raw_cap);
+        boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, box, nullptr);
+    } else {
+        harris_box_kernel<<<harris_grid(g.W, g.H, nf), HT_THREADS, sizeof(HarrisSmem), s>>>(
+            d_img, d_mask, g, ctx->f1, ctx->f0, ctx->kf, ctx->p.quality_level, nullptr, box, nullptr, l.frame_max, l.cand,
+            l.cand_count, ctx->raw_cap, nullptr, nullptr, g.H);
+    }
+}
+
+// Corner selection from the lane's candidate lists: the selected corners (det_xy / n_det) and the ones that survive BRIEF's
+// border filter (kp_xy / n_kp), [nf][max_corners].
+void launch_select(svi_ctx* ctx, Lane& l, int nf, ushort2* det_xy, int* n_det, ushort2* kp_xy, int* n_kp) {
+    cudaStream_t s = l.stream;
+    const uint32_t* fmax = ctx->p.detector == SVI_DETECTOR_FAST_9_16 ? nullptr : l.frame_max;
+    if (ctx->select_smem) {
+        select_corners_kernel<true><<<nf, SEL_THREADS, 13 * SEL_SMEM_KEYS, s>>>(
+            l.cand, l.cand_count, fmax, ctx->sel, nullptr, nullptr, nullptr, det_xy, n_det, kp_xy, n_kp, ctx->d_overflow, nullptr);
+    } else {
+        select_corners_kernel<false><<<nf, SEL_THREADS, 4 * SEL_SMEM_CELLS, s>>>(
+            l.cand, l.cand_count, fmax, ctx->sel, l.g_head, l.g_next, l.g_state, det_xy, n_det, kp_xy, n_kp, ctx->d_overflow, nullptr);
+    }
+}
+
 // The kernels of the new-landmark path for `nf` frames on one lane: detector, RIGHT box sums, corner selection, then the
 // descriptor / match stages in the form that fits the call (svi_kernels_per_chunk: 4 to 6 launches).
 int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_right, const uint8_t* d_mask,
@@ -296,17 +342,8 @@ int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_
     CK(cudaMemsetAsync(l.frame_max, 0, sizeof(uint32_t) * nf, s));
     CK(cudaMemsetAsync(l.cand_count, 0, sizeof(int) * nf, s));
     const dim3 tiles((g.W + HT_W - 1) / HT_W, (g.H + HT_H - 1) / HT_H, nf);
-    const bool fast = ctx->p.detector == SVI_DETECTOR_FAST_9_16;
     mark(ctx, l);
-    if (fast) {
-        fast_candidates_kernel<<<tiles, HT_THREADS, 0, s>>>(d_left, d_mask, g, ctx->p.fast_threshold, ctx->p.fast_nonmax, l.cand,
-                                                            l.cand_count, ctx->raw_cap);
-        boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_left, g, l.box_l, nullptr);
-    } else {
-        harris_box_kernel<<<harris_grid(g.W, g.H, nf), HT_THREADS, sizeof(HarrisSmem), s>>>(
-            d_left, d_mask, g, ctx->f1, ctx->f0, ctx->kf, ctx->p.quality_level, nullptr, l.box_l, nullptr, l.frame_max, l.cand,
-            l.cand_count, ctx->raw_cap, nullptr, nullptr, g.H);
-    }
+    launch_detector(ctx, l, d_left, d_mask, g, nf, l.box_l);
     mark(ctx, l);
     // `side` (latency path): the RIGHT plane goes up on that stream -- staged by the caller's hook only now, so that the
     // host-side copy into the pinned mirror overlaps the detector -- and its box sums run there too
@@ -321,14 +358,7 @@ int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_
                                                           // one wait here keeps the stage events of the profiler in order
     }
     mark(ctx, l);
-    const uint32_t* fmax = fast ? nullptr : l.frame_max;
-    if (ctx->select_smem) {
-        select_corners_kernel<true><<<nf, SEL_THREADS, 13 * SEL_SMEM_KEYS, s>>>(
-            l.cand, l.cand_count, fmax, ctx->sel, nullptr, nullptr, nullptr, l.det_xy, n_det, l.kp_xy, n_kp, ctx->d_overflow, nullptr);
-    } else {
-        select_corners_kernel<false><<<nf, SEL_THREADS, 4 * SEL_SMEM_CELLS, s>>>(
-            l.cand, l.cand_count, fmax, ctx->sel, l.g_head, l.g_next, l.g_state, l.det_xy, n_det, l.kp_xy, n_kp, ctx->d_overflow, nullptr);
-    }
+    launch_select(ctx, l, nf, l.det_xy, n_det, l.kp_xy, n_kp);
     mark(ctx, l);
     // full batches amortise a warp's set-up over MATCH_KP_PER_WARP key-points; a small call (one pair per frame in a
     // tracker) would leave most SMs idle that way, so it spreads the key-points until two waves of warps exist
@@ -402,6 +432,69 @@ int sync_lanes(svi_ctx* ctx) {
 
 template <typename T>
 cudaError_t dmalloc(T** p, size_t count) { return cudaMalloc(reinterpret_cast<void**>(p), count * sizeof(T)); }
+
+// ---- sparse frames (svi_stereo_frames_sparse): per-lane scratch, allocated at the first sparse call; a ctx that never makes
+// one allocates nothing for it.
+int ensure_sparse_scratch(svi_ctx* ctx) {
+    // bin_keypoints_kernel sorts by row with one counter per row in shared memory
+    const int row_smem = (int)sizeof(uint32_t) * ctx->H;
+    if (row_smem > 200 * 1024) return fail(ctx, SVI_ERR_UNSUPPORTED, "svi_stereo_frames_sparse: image height above 51200 rows");
+    if (ctx->lanes[ctx->n_lanes - 1].sp_kp_r) return SVI_SUCCESS;
+    CK(cudaFuncSetAttribute(bin_keypoints_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, std::max(row_smem, 48 * 1024)));
+    const size_t C = (size_t)ctx->chunk, MC = (size_t)ctx->p.max_corners, L = C * MC + BM_ALIGN, rows = C * ((size_t)ctx->H + 1);
+    for (int i = 0; i < ctx->n_lanes; ++i) {
+        Lane& l = ctx->lanes[i];
+        if (l.sp_kp_r) continue;
+        CK(dmalloc(&l.sp_n_kp_r, C));
+        CK(dmalloc(&l.sp_n_det_r, C));
+        CK(dmalloc(&l.sp_row_l, rows));
+        CK(dmalloc(&l.sp_slot_l, L));
+        CK(dmalloc(&l.sp_kp_l, L));
+        CK(dmalloc(&l.sp_row_r, rows));
+        CK(dmalloc(&l.sp_slot_r, L));
+        CK(dmalloc(&l.sp_kp_rs, L));
+        CK(dmalloc(&l.sp_desc_r, 32 * L));
+        CK(dmalloc(&l.sp_second, L));
+        std::string merr;
+        if (!make_box_map(&l.map_r_patch, l.box_r, ctx->W, (int)(C * ctx->H), ctx->box_pitch, &merr, DL_COLS)) return fail(ctx, SVI_ERR_CUDA, merr);
+        CK(dmalloc(&l.sp_kp_r, L));   // last: marks the lane's scratch complete
+    }
+    return SVI_SUCCESS;
+}
+
+// The sparse frame of nf frames on one lane: detection and selection on LEFT (with the masks) and on RIGHT (without) -- the
+// same launches as the dense path's, RIGHT after LEFT's selection so that the candidate lists are reused --, both key-point
+// lists sorted by row (bin_keypoints_kernel with full-width bins one row high: a row CSR plus each key-point's slot), LEFT
+// descriptors into out.desc_l as on the dense path, RIGHT descriptors over the row-sorted list, then band_match_kernel.
+// second / n_kp_r: the call's second-distance slots (indexed like out) and RIGHT key-point counts (indexed by chunk frame).
+int run_sparse(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_right, const uint8_t* d_mask, const FrameGeom& g, int nf,
+               const StereoOutDev& out, int out_frame0, int* n_kp, int* n_det, int* second, int* n_kp_r, const svi_sparse_band& band) {
+    cudaStream_t s = l.stream;
+    const int MC = ctx->p.max_corners, H = ctx->H;
+    const struct { const uint8_t* img; const uint8_t* mask; uint16_t* box; int* n_det; ushort2* kp; int* n_kp; } sides[2] = {
+        {d_left, d_mask, l.box_l, n_det, l.kp_xy, n_kp}, {d_right, nullptr, l.box_r, l.sp_n_det_r, l.sp_kp_r, n_kp_r}};
+    for (const auto& sd : sides) {
+        CK(cudaMemsetAsync(l.frame_max, 0, sizeof(uint32_t) * nf, s));
+        CK(cudaMemsetAsync(l.cand_count, 0, sizeof(int) * nf, s));
+        launch_detector(ctx, l, sd.img, sd.mask, g, nf, sd.box);
+        launch_select(ctx, l, nf, l.det_xy, sd.n_det, sd.kp, sd.n_kp);   // LEFT's det_xy is not needed once it is selected
+    }
+    const size_t row_smem = sizeof(uint32_t) * H;
+    bin_keypoints_kernel<<<nf, BINK_THREADS, row_smem, s>>>(l.kp_xy, n_kp, MC, ctx->W, 1, 1, H, l.sp_row_l, l.sp_slot_l, l.sp_kp_l);
+    bin_keypoints_kernel<<<nf, BINK_THREADS, row_smem, s>>>(l.sp_kp_r, n_kp_r, MC, ctx->W, 1, 1, H, l.sp_row_r, l.sp_slot_r, l.sp_kp_rs);
+    const dim3 dgrid((MC + DL_WARPS * DL_KP_PER_WARP - 1) / (DL_WARPS * DL_KP_PER_WARP), nf);
+    describe_left_kernel<<<dgrid, DL_WARPS * 32, DL_SMEM, s>>>(l.map_l_patch, g, l.kp_xy, n_kp, MC, out.desc_l, out.cap, out_frame0);
+    describe_left_kernel<<<dgrid, DL_WARPS * 32, DL_SMEM, s>>>(l.map_r_patch, g, l.sp_kp_rs, n_kp_r, MC, l.sp_desc_r, MC, 0);
+    BandArgs a{};
+    a.band_v = band.band_v; a.min_disp = band.min_disparity; a.max_disp = band.max_disparity;
+    a.q_kp = l.sp_kp_l; a.q_slot = l.sp_slot_l; a.n_q = n_kp;
+    a.t_kp = l.sp_kp_rs; a.t_slot = l.sp_slot_r; a.t_desc = l.sp_desc_r; a.t_row = l.sp_row_r;
+    a.H = H; a.max_corners = MC;
+    a.out = out; a.out_frame0 = out_frame0; a.tc = ctx->tc; a.second = second;
+    band_match_kernel<true><<<dim3((MC + BM_THREADS - 1) / BM_THREADS, nf), BM_THREADS, BandTile<true>::SMEM, s>>>(a);
+    CK(cudaGetLastError());
+    return SVI_SUCCESS;
+}
 
 // ---- rectification
 // cvRound of OpenCV's x86 build (cvtsd2si / cvtss2si): half to even, and INT_MIN for NaN or anything outside int
@@ -1021,6 +1114,135 @@ int enqueue_cascade(svi_ctx* ctx, int n, const double* T_world_to_left, double m
 
 }  // namespace
 
+// ---- the batch frame entry points (svi_stereo_frames[_sparse][_device]): argument checks and the chunk loops they share
+namespace {
+int check_frames_args(svi_ctx* ctx, const char* name, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride,
+                      int n_frames, const svi_stereo_result* out, bool device) {
+    const std::string n(name);
+    if (!left || !right || !out || n_frames < 0 || (int)pitch < ctx->W ||
+        (device ? frame_stride < pitch * (size_t)ctx->H : (n_frames > 1 && frame_stride < pitch * (size_t)ctx->H)))
+        return fail(ctx, SVI_ERR_INVALID, n + ": bad argument");
+    if (out->capacity_per_frame < ctx->p.max_corners) return fail(ctx, SVI_ERR_CAPACITY, n + ": capacity_per_frame < max_corners");
+    if (!out->n_keypoints || !out->uv_left || !out->uv_right || !out->xyz_left || !out->desc_left || !out->desc_right ||
+        !out->distance || !out->match_index || !out->status)
+        return fail(ctx, SVI_ERR_INVALID, n + ": null output array");
+    return SVI_SUCCESS;
+}
+
+// nf frames of one per-slot array of a lane (max_corners slots per frame, elem bytes each) into the caller's host array of
+// cap slots per frame, from frame f0 on
+cudaError_t d2h_slots(void* dst, const void* src, size_t elem, int MC, int cap, int f0, int nf, cudaStream_t s) {
+    unsigned char* d = static_cast<unsigned char*>(dst) + (size_t)f0 * cap * elem;
+    if (cap == MC) return cudaMemcpyAsync(d, src, (size_t)nf * MC * elem, cudaMemcpyDeviceToHost, s);
+    return cudaMemcpy2DAsync(d, (size_t)cap * elem, src, (size_t)MC * elem, (size_t)MC * elem, nf, cudaMemcpyDeviceToHost, s);
+}
+
+// Host buffers: chunk c on lane c % n_lanes; its images (and masks) go straight from the caller's buffers into the lane's
+// staging (raw planes first while rectification is set), `run` enqueues the kernels on the lane's planes, the slot arrays and
+// counts come back into the caller's arrays, `fetch` (may be null) adds the entry point's own; one synchronisation at the end.
+using HostChunkFn = std::function<int(Lane&, const FrameGeom&, int f0, int nf)>;
+int host_frames(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride, int n_frames,
+                const uint8_t* masks, svi_stereo_result* out, const HostChunkFn& run, const HostChunkFn& fetch) {
+    const int W = ctx->W, H = ctx->H, MC = ctx->p.max_corners, cap = out->capacity_per_frame;
+    const size_t dstride = (size_t)H * ctx->dev_pitch;
+    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, dstride);
+    const bool dense = (frame_stride == pitch * (size_t)H);
+    int chunk_id = 0;
+    for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk, ++chunk_id) {
+        Lane& l = ctx->lanes[chunk_id % ctx->n_lanes];
+        cudaStream_t s = l.stream;
+        const int nf = std::min(ctx->chunk, n_frames - f0);
+        const uint8_t* srcs[3] = {left, right, masks};
+        uint8_t* dsts[3] = {ctx->rect ? l.raw_l : l.img_l, ctx->rect ? l.raw_r : l.img_r, l.mask};
+        for (int k = 0; k < 3; ++k) {
+            if (!srcs[k]) continue;
+            if (dense && (int)pitch == ctx->dev_pitch) {
+                CK(cudaMemcpyAsync(dsts[k], srcs[k] + (size_t)f0 * frame_stride, (size_t)nf * frame_stride, cudaMemcpyHostToDevice, s));
+            } else if (dense) {
+                CK(cudaMemcpy2DAsync(dsts[k], ctx->dev_pitch, srcs[k] + (size_t)f0 * frame_stride, pitch, W, (size_t)H * nf,
+                                     cudaMemcpyHostToDevice, s));
+            } else {
+                for (int f = 0; f < nf; ++f)
+                    CK(cudaMemcpy2DAsync(dsts[k] + f * dstride, ctx->dev_pitch, srcs[k] + (size_t)(f0 + f) * frame_stride,
+                                         pitch, W, H, cudaMemcpyHostToDevice, s));
+            }
+        }
+        if (ctx->rect) {
+            const int rr = rectify_pair(ctx, l.raw_l, l.raw_r, ctx->dev_pitch, dstride, l.img_l, l.img_r, nf, s);
+            if (rr != SVI_SUCCESS) return rr;
+        }
+        int rc = run(l, g, f0, nf);
+        if (rc != SVI_SUCCESS) return rc;
+        CK(d2h_slots(out->uv_left, l.out.uv_l, 2 * sizeof(float), MC, cap, f0, nf, s));
+        CK(d2h_slots(out->uv_right, l.out.uv_r, 2 * sizeof(float), MC, cap, f0, nf, s));
+        CK(d2h_slots(out->xyz_left, l.out.xyz, 3 * sizeof(double), MC, cap, f0, nf, s));
+        CK(d2h_slots(out->desc_left, l.out.desc_l, 32, MC, cap, f0, nf, s));
+        CK(d2h_slots(out->desc_right, l.out.desc_r, 32, MC, cap, f0, nf, s));
+        CK(d2h_slots(out->distance, l.out.dist, sizeof(int32_t), MC, cap, f0, nf, s));
+        CK(d2h_slots(out->match_index, l.out.idx, sizeof(int32_t), MC, cap, f0, nf, s));
+        CK(d2h_slots(out->status, l.out.status, 1, MC, cap, f0, nf, s));
+        CK(cudaMemcpyAsync(out->n_keypoints + f0, l.n_kp, sizeof(int) * nf, cudaMemcpyDeviceToHost, s));
+        if (out->n_detected) CK(cudaMemcpyAsync(out->n_detected + f0, l.n_det, sizeof(int) * nf, cudaMemcpyDeviceToHost, s));
+        if (fetch && (rc = fetch(l, g, f0, nf)) != SVI_SUCCESS) return rc;
+    }
+    int rc = sync_lanes(ctx);
+    if (rc != SVI_SUCCESS) return rc;
+    return check_overflow(ctx);
+}
+
+// Device buffers: enqueued after everything on the caller's stream, chunk c on lane c % n_lanes (lane 0 while profiling in
+// mode 2); `run` enqueues the kernels on device images and writes the caller's arrays at frame f0 (o, n_kp, n_det); the
+// lanes join the caller's stream again, no synchronisation.
+using DeviceChunkFn = std::function<int(Lane&, const uint8_t*, const uint8_t*, const uint8_t*, const FrameGeom&, int f0, int nf,
+                                        const StereoOutDev& o, int* n_kp, int* n_det)>;
+int device_frames(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride, int n_frames,
+                  const uint8_t* masks, const svi_stereo_result* out, void* cuda_stream, const DeviceChunkFn& run) {
+    cudaStream_t user = reinterpret_cast<cudaStream_t>(cuda_stream);
+    CK(cudaEventRecord(ctx->fork, user));
+    for (int i = 0; i < ctx->n_lanes; ++i) CK(cudaStreamWaitEvent(ctx->lanes[i].stream, ctx->fork, 0));
+    const FrameGeom g = make_geom(ctx, (int)pitch, frame_stride);
+    const size_t dstride = (size_t)ctx->H * ctx->dev_pitch;
+    const FrameGeom g_rect = make_geom(ctx, ctx->dev_pitch, dstride);   // rectified planes in the lane's staging
+    StereoOutDev o;
+    o.cap = out->capacity_per_frame;
+    o.uv_l = out->uv_left; o.uv_r = out->uv_right; o.xyz = out->xyz_left;
+    o.desc_l = out->desc_left; o.desc_r = out->desc_right;
+    o.dist = out->distance; o.idx = out->match_index; o.status = out->status;
+    int chunk_id = 0, rc = SVI_SUCCESS;
+    for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk, ++chunk_id) {
+        Lane& l = ctx->lanes[ctx->serial ? 0 : chunk_id % ctx->n_lanes];
+        const int nf = std::min(ctx->chunk, n_frames - f0);
+        int* n_det = out->n_detected ? out->n_detected + f0 : l.n_det;
+        const uint8_t* m = masks ? masks + (size_t)f0 * frame_stride : nullptr;
+        if (ctx->rect) {   // the caller's raw frames are read in place; the pipeline reads the rectified planes
+            rc = rectify_pair(ctx, left + (size_t)f0 * frame_stride, right + (size_t)f0 * frame_stride, pitch, frame_stride, l.img_l, l.img_r, nf,
+                              l.stream);
+            if (rc != SVI_SUCCESS) break;
+            if (m && ((int)pitch != ctx->dev_pitch || frame_stride != dstride)) {   // the masks follow the planes' layout
+                for (int f = 0; f < nf && rc == SVI_SUCCESS; ++f)
+                    if (cudaMemcpy2DAsync(l.mask + f * dstride, ctx->dev_pitch, m + (size_t)f * frame_stride, pitch, ctx->W, ctx->H,
+                                          cudaMemcpyDeviceToDevice, l.stream) != cudaSuccess)
+                        rc = fail(ctx, SVI_ERR_CUDA, "svi_stereo_frames_device: mask copy failed");
+                if (rc != SVI_SUCCESS) break;
+                m = l.mask;
+            }
+            rc = run(l, l.img_l, l.img_r, m, g_rect, f0, nf, o, out->n_keypoints + f0, n_det);
+        } else {
+            rc = run(l, left + (size_t)f0 * frame_stride, right + (size_t)f0 * frame_stride, m, g, f0, nf, o, out->n_keypoints + f0, n_det);
+        }
+        if (rc != SVI_SUCCESS) break;
+    }
+    // join the lanes back into the caller's stream -- also after a failure, so that nothing queued so far can outlive
+    // the caller's next use of its buffers
+    for (int i = 0; i < ctx->n_lanes; ++i) {
+        if (cudaEventRecord(ctx->lanes[i].done, ctx->lanes[i].stream) == cudaSuccess)
+            cudaStreamWaitEvent(user, ctx->lanes[i].done, 0);
+    }
+    return rc;
+}
+
+}  // namespace
+
 extern "C" {
 
 int svi_params_default(svi_params* p) {
@@ -1097,7 +1319,8 @@ void svi_destroy(svi_ctx* ctx) {
         void* ptrs[] = {l.box_l, l.box_r, l.box_ls, l.box_rs, l.frame_max, l.cand_count, l.cand, l.det_xy, l.kp_xy, l.n_det, l.n_kp,
                         l.g_head, l.g_next, l.g_state, l.img_l, l.img_r, l.mask, l.out.uv_l, l.out.uv_r, l.out.xyz,
                         l.out.desc_l, l.out.desc_r, l.out.dist, l.out.idx, l.out.status, l.bin_start, l.bin_slot, l.bin_kp,
-                        l.raw_l, l.raw_r};
+                        l.raw_l, l.raw_r, l.sp_kp_r, l.sp_n_kp_r, l.sp_n_det_r, l.sp_row_l, l.sp_slot_l, l.sp_kp_l, l.sp_row_r,
+                        l.sp_slot_r, l.sp_kp_rs, l.sp_desc_r, l.sp_second};
         for (void* p : ptrs) if (p) cudaFree(p);
         for (cudaEvent_t e : l.ev) cudaEventDestroy(e);
         if (l.done) cudaEventDestroy(l.done);
@@ -1278,7 +1501,8 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
                                  (const void*)triangulate_kernel<false>, (const void*)track_stage1_kernel,
                                  (const void*)track_stage2_kernel<true>, (const void*)track_stage2_kernel<false>,
                                  (const void*)track_stage3_kernel, (const void*)fast_candidates_kernel,
-                                 (const void*)describe_kernel, (const void*)hamming_match_kernel, (const void*)rectify_kernel};
+                                 (const void*)describe_kernel, (const void*)hamming_match_kernel, (const void*)rectify_kernel,
+                                 (const void*)band_match_kernel<true>, (const void*)band_match_kernel<false>};
         for (const void* k : kernels)
             CK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
@@ -1391,126 +1615,76 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
 int svi_stereo_frames_device(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride,
                              int n_frames, const uint8_t* masks, const svi_stereo_result* out, void* cuda_stream) {
     if (!ctx) return SVI_ERR_INVALID;
-    if (!left || !right || !out || n_frames < 0 || (int)pitch < ctx->W || frame_stride < pitch * (size_t)ctx->H)
-        return fail(ctx, SVI_ERR_INVALID, "svi_stereo_frames_device: bad argument");
-    if (out->capacity_per_frame < ctx->p.max_corners) return fail(ctx, SVI_ERR_CAPACITY, "svi_stereo_frames_device: capacity_per_frame < max_corners");
-    if (!out->n_keypoints || !out->uv_left || !out->uv_right || !out->xyz_left || !out->desc_left || !out->desc_right ||
-        !out->distance || !out->match_index || !out->status)
-        return fail(ctx, SVI_ERR_INVALID, "svi_stereo_frames_device: null output array");
+    const int rc = check_frames_args(ctx, "svi_stereo_frames_device", left, right, pitch, frame_stride, n_frames, out, true);
+    if (rc != SVI_SUCCESS) return rc;
     CK(cudaSetDevice(ctx->device));
-    cudaStream_t user = reinterpret_cast<cudaStream_t>(cuda_stream);
-    CK(cudaEventRecord(ctx->fork, user));
-    for (int i = 0; i < ctx->n_lanes; ++i) CK(cudaStreamWaitEvent(ctx->lanes[i].stream, ctx->fork, 0));
-    const FrameGeom g = make_geom(ctx, (int)pitch, frame_stride);
-    const size_t dstride = (size_t)ctx->H * ctx->dev_pitch;
-    const FrameGeom g_rect = make_geom(ctx, ctx->dev_pitch, dstride);   // rectified planes in the lane's staging
-    StereoOutDev o;
-    o.cap = out->capacity_per_frame;
-    o.uv_l = out->uv_left; o.uv_r = out->uv_right; o.xyz = out->xyz_left;
-    o.desc_l = out->desc_left; o.desc_r = out->desc_right;
-    o.dist = out->distance; o.idx = out->match_index; o.status = out->status;
-    int chunk_id = 0, rc = SVI_SUCCESS;
-    for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk, ++chunk_id) {
-        Lane& l = ctx->lanes[ctx->serial ? 0 : chunk_id % ctx->n_lanes];
-        const int nf = std::min(ctx->chunk, n_frames - f0);
-        int* n_det = out->n_detected ? out->n_detected + f0 : l.n_det;
-        const uint8_t* m = masks ? masks + (size_t)f0 * frame_stride : nullptr;
-        if (ctx->rect) {   // the caller's raw frames are read in place; the pipeline reads the rectified planes
-            rc = rectify_pair(ctx, left + (size_t)f0 * frame_stride, right + (size_t)f0 * frame_stride, pitch, frame_stride, l.img_l, l.img_r, nf,
-                              l.stream);
-            if (rc != SVI_SUCCESS) break;
-            if (m && ((int)pitch != ctx->dev_pitch || frame_stride != dstride)) {   // the masks follow the planes' layout
-                for (int f = 0; f < nf && rc == SVI_SUCCESS; ++f)
-                    if (cudaMemcpy2DAsync(l.mask + f * dstride, ctx->dev_pitch, m + (size_t)f * frame_stride, pitch, ctx->W, ctx->H,
-                                          cudaMemcpyDeviceToDevice, l.stream) != cudaSuccess)
-                        rc = fail(ctx, SVI_ERR_CUDA, "svi_stereo_frames_device: mask copy failed");
-                if (rc != SVI_SUCCESS) break;
-                m = l.mask;
-            }
-            rc = run_pipeline(ctx, l, l.img_l, l.img_r, m, g_rect, nf, o, f0, out->n_keypoints + f0, n_det);
-        } else {
-            rc = run_pipeline(ctx, l, left + (size_t)f0 * frame_stride, right + (size_t)f0 * frame_stride, m, g, nf, o, f0, out->n_keypoints + f0,
-                              n_det);
-        }
-        if (rc != SVI_SUCCESS) break;
-    }
-    // join the lanes back into the caller's stream -- also after a failure, so that nothing queued so far can outlive
-    // the caller's next use of its buffers
-    for (int i = 0; i < ctx->n_lanes; ++i) {
-        if (cudaEventRecord(ctx->lanes[i].done, ctx->lanes[i].stream) == cudaSuccess)
-            cudaStreamWaitEvent(user, ctx->lanes[i].done, 0);
-    }
-    return rc;
+    return device_frames(ctx, left, right, pitch, frame_stride, n_frames, masks, out, cuda_stream,
+                         [&](Lane& l, const uint8_t* dl, const uint8_t* dr, const uint8_t* dm, const FrameGeom& g, int f0, int nf,
+                             const StereoOutDev& o, int* n_kp, int* n_det) {
+                             return run_pipeline(ctx, l, dl, dr, dm, g, nf, o, f0, n_kp, n_det);
+                         });
 }
 
 int svi_stereo_frames(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride,
                       int n_frames, const uint8_t* masks, svi_stereo_result* out) {
     if (!ctx) return SVI_ERR_INVALID;
-    if (!left || !right || !out || n_frames < 0 || (int)pitch < ctx->W || (n_frames > 1 && frame_stride < pitch * (size_t)ctx->H))
-        return fail(ctx, SVI_ERR_INVALID, "svi_stereo_frames: bad argument");
-    if (out->capacity_per_frame < ctx->p.max_corners) return fail(ctx, SVI_ERR_CAPACITY, "svi_stereo_frames: capacity_per_frame < max_corners");
-    if (!out->n_keypoints || !out->uv_left || !out->uv_right || !out->xyz_left || !out->desc_left || !out->desc_right ||
-        !out->distance || !out->match_index || !out->status)
-        return fail(ctx, SVI_ERR_INVALID, "svi_stereo_frames: null output array");
+    const int rc = check_frames_args(ctx, "svi_stereo_frames", left, right, pitch, frame_stride, n_frames, out, false);
+    if (rc != SVI_SUCCESS) return rc;
     CK(cudaSetDevice(ctx->device));
-    const int W = ctx->W, H = ctx->H, MC = ctx->p.max_corners, cap = out->capacity_per_frame;
-    const size_t dstride = (size_t)H * ctx->dev_pitch;
-    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, dstride);
-    const bool dense = (frame_stride == pitch * (size_t)H);
     if (n_frames > 0 && n_frames <= std::min(kSmallFrames, ctx->chunk) && ctx->pin)
         return small_call(ctx, left, right, pitch, frame_stride, n_frames, masks, nullptr, 0, out);
-    int chunk_id = 0;
-    for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk, ++chunk_id) {
-        Lane& l = ctx->lanes[chunk_id % ctx->n_lanes];
-        cudaStream_t s = l.stream;
-        const int nf = std::min(ctx->chunk, n_frames - f0);
-        const uint8_t* srcs[3] = {left, right, masks};
-        uint8_t* dsts[3] = {ctx->rect ? l.raw_l : l.img_l, ctx->rect ? l.raw_r : l.img_r, l.mask};
-        for (int k = 0; k < 3; ++k) {
-            if (!srcs[k]) continue;
-            if (dense && (int)pitch == ctx->dev_pitch) {
-                CK(cudaMemcpyAsync(dsts[k], srcs[k] + (size_t)f0 * frame_stride, (size_t)nf * frame_stride, cudaMemcpyHostToDevice, s));
-            } else if (dense) {
-                CK(cudaMemcpy2DAsync(dsts[k], ctx->dev_pitch, srcs[k] + (size_t)f0 * frame_stride, pitch, W, (size_t)H * nf,
-                                     cudaMemcpyHostToDevice, s));
-            } else {
-                for (int f = 0; f < nf; ++f)
-                    CK(cudaMemcpy2DAsync(dsts[k] + f * dstride, ctx->dev_pitch, srcs[k] + (size_t)(f0 + f) * frame_stride,
-                                         pitch, W, H, cudaMemcpyHostToDevice, s));
-            }
-        }
-        if (ctx->rect) {
-            const int rr = rectify_pair(ctx, l.raw_l, l.raw_r, ctx->dev_pitch, dstride, l.img_l, l.img_r, nf, s);
-            if (rr != SVI_SUCCESS) return rr;
-        }
-        int rc = run_pipeline(ctx, l, l.img_l, l.img_r, masks ? l.mask : nullptr, g, nf, l.out, 0, l.n_kp, l.n_det);
-        if (rc != SVI_SUCCESS) return rc;
-        const size_t o0 = (size_t)f0 * cap;
-#define D2H(dst, src, elem)                                                                                             \
-    do {                                                                                                                \
-        if (cap == MC)                                                                                                  \
-            CK(cudaMemcpyAsync((dst) + o0 * (elem), (src), (size_t)nf * MC * (elem) * sizeof(*(dst)),                   \
-                               cudaMemcpyDeviceToHost, s));                                                             \
-        else                                                                                                            \
-            CK(cudaMemcpy2DAsync((dst) + o0 * (elem), (size_t)cap * (elem) * sizeof(*(dst)), (src),                     \
-                                 (size_t)MC * (elem) * sizeof(*(dst)), (size_t)MC * (elem) * sizeof(*(dst)), nf,        \
-                                 cudaMemcpyDeviceToHost, s));                                                           \
-    } while (0)
-        D2H(out->uv_left, l.out.uv_l, 2);
-        D2H(out->uv_right, l.out.uv_r, 2);
-        D2H(out->xyz_left, l.out.xyz, 3);
-        D2H(out->desc_left, l.out.desc_l, 32);
-        D2H(out->desc_right, l.out.desc_r, 32);
-        D2H(out->distance, l.out.dist, 1);
-        D2H(out->match_index, l.out.idx, 1);
-        D2H(out->status, l.out.status, 1);
-#undef D2H
-        CK(cudaMemcpyAsync(out->n_keypoints + f0, l.n_kp, sizeof(int) * nf, cudaMemcpyDeviceToHost, s));
-        if (out->n_detected) CK(cudaMemcpyAsync(out->n_detected + f0, l.n_det, sizeof(int) * nf, cudaMemcpyDeviceToHost, s));
-    }
-    int rc = sync_lanes(ctx);
+    return host_frames(ctx, left, right, pitch, frame_stride, n_frames, masks, out,
+                       [&](Lane& l, const FrameGeom& g, int, int nf) {
+                           return run_pipeline(ctx, l, l.img_l, l.img_r, masks ? l.mask : nullptr, g, nf, l.out, 0, l.n_kp, l.n_det);
+                       },
+                       nullptr);
+}
+
+namespace {
+int check_sparse_args(svi_ctx* ctx, const char* name, const svi_sparse_band* band, const svi_sparse_result* sparse) {
+    if (!band || !sparse) return fail(ctx, SVI_ERR_INVALID, std::string(name) + ": bad argument");
+    if (std::isnan(band->band_v) || std::isnan(band->min_disparity) || std::isnan(band->max_disparity) ||
+        band->min_disparity > band->max_disparity)
+        return fail(ctx, SVI_ERR_INVALID, std::string(name) + ": band fields must not be NaN and min_disparity <= max_disparity");
+    if (!sparse->second_distance || !sparse->n_keypoints_right) return fail(ctx, SVI_ERR_INVALID, std::string(name) + ": null output array");
+    return ensure_sparse_scratch(ctx);
+}
+}  // namespace
+
+int svi_stereo_frames_sparse(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride, int n_frames,
+                             const uint8_t* masks, const svi_sparse_band* band, svi_stereo_result* out, svi_sparse_result* sparse) {
+    if (!ctx) return SVI_ERR_INVALID;
+    int rc = check_frames_args(ctx, "svi_stereo_frames_sparse", left, right, pitch, frame_stride, n_frames, out, false);
     if (rc != SVI_SUCCESS) return rc;
-    return check_overflow(ctx);
+    CK(cudaSetDevice(ctx->device));
+    if ((rc = check_sparse_args(ctx, "svi_stereo_frames_sparse", band, sparse)) != SVI_SUCCESS) return rc;
+    const int MC = ctx->p.max_corners, cap = out->capacity_per_frame;
+    return host_frames(ctx, left, right, pitch, frame_stride, n_frames, masks, out,
+                       [&](Lane& l, const FrameGeom& g, int, int nf) {
+                           return run_sparse(ctx, l, l.img_l, l.img_r, masks ? l.mask : nullptr, g, nf, l.out, 0, l.n_kp, l.n_det, l.sp_second,
+                                             l.sp_n_kp_r, *band);
+                       },
+                       [&](Lane& l, const FrameGeom&, int f0, int nf) -> int {
+                           CK(d2h_slots(sparse->second_distance, l.sp_second, sizeof(int32_t), MC, cap, f0, nf, l.stream));
+                           CK(cudaMemcpyAsync(sparse->n_keypoints_right + f0, l.sp_n_kp_r, sizeof(int) * nf, cudaMemcpyDeviceToHost, l.stream));
+                           return SVI_SUCCESS;
+                       });
+}
+
+int svi_stereo_frames_sparse_device(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride,
+                                    int n_frames, const uint8_t* masks, const svi_sparse_band* band, const svi_stereo_result* out,
+                                    const svi_sparse_result* sparse, void* cuda_stream) {
+    if (!ctx) return SVI_ERR_INVALID;
+    int rc = check_frames_args(ctx, "svi_stereo_frames_sparse_device", left, right, pitch, frame_stride, n_frames, out, true);
+    if (rc != SVI_SUCCESS) return rc;
+    CK(cudaSetDevice(ctx->device));
+    if ((rc = check_sparse_args(ctx, "svi_stereo_frames_sparse_device", band, sparse)) != SVI_SUCCESS) return rc;
+    return device_frames(ctx, left, right, pitch, frame_stride, n_frames, masks, out, cuda_stream,
+                         [&](Lane& l, const uint8_t* dl, const uint8_t* dr, const uint8_t* dm, const FrameGeom& g, int f0, int nf,
+                             const StereoOutDev& o, int* n_kp, int* n_det) {
+                             return run_sparse(ctx, l, dl, dr, dm, g, nf, o, f0, n_kp, n_det, sparse->second_distance,
+                                               sparse->n_keypoints_right + f0, *band);
+                         });
 }
 
 int svi_mask_active_landmarks(svi_ctx* ctx, const float* centres_xy, int n_centres, uint8_t* mask, size_t pitch) {
@@ -1706,9 +1880,14 @@ int svi_match_epipolar(svi_ctx* ctx, const uint8_t* query32, const float* query_
     put(ctx, i_txy, n_train > 0 ? train_xy : nullptr, 8 * T);
     int rc = call_send(ctx, o_i, s);
     if (rc != SVI_SUCCESS) return rc;
-    epipolar_match_kernel<<<(n_query + 3) / 4, 128, 0, s>>>(dev_at(ctx, i_q), dev_at<float>(ctx, i_qxy), n_query, dev_at(ctx, i_t), dev_at<float>(ctx, i_txy),
-                                                            n_train, band_v, min_disparity, max_disparity, dev_at<int>(ctx, o_i), dev_at<int>(ctx, o_d),
-                                                            dev_at<int>(ctx, o_s));
+    // the trains in caller order as one range (band_match_kernel reads up to BM_ALIGN - 1 elements past each array: the
+    // call buffer's 256-byte alignment of every region covers them)
+    BandArgs a{};
+    a.band_v = band_v; a.min_disp = min_disparity; a.max_disp = max_disparity;
+    a.q_desc = dev_at(ctx, i_q); a.q_xy = dev_at<float2>(ctx, i_qxy); a.nq = n_query;
+    a.t_desc = dev_at(ctx, i_t); a.t_xy = dev_at<float2>(ctx, i_txy); a.nt = n_train;
+    a.index = dev_at<int>(ctx, o_i); a.distance = dev_at<int>(ctx, o_d); a.second = dev_at<int>(ctx, o_s);
+    band_match_kernel<false><<<(n_query + BM_THREADS - 1) / BM_THREADS, BM_THREADS, BandTile<false>::SMEM, s>>>(a);
     CK(cudaGetLastError());
     if ((rc = call_fetch(ctx, o_i, L.end, s)) != SVI_SUCCESS) return rc;
     idle.done = true;

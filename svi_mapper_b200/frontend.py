@@ -94,12 +94,34 @@ class StereoFrames:
     distance: np.ndarray
     match_index: np.ndarray
     status: np.ndarray
+    second_distance: np.ndarray | None = None     # sparse frames only (stereo_frames_sparse): (n_frames, capacity)
+    n_keypoints_right: np.ndarray | None = None   # sparse frames only: (n_frames,)
+
+    @classmethod
+    def empty(cls, n: int, cap: int, sparse: bool = False) -> "StereoFrames":
+        return cls(n_keypoints=np.zeros(n, np.int32), n_detected=np.zeros(n, np.int32),
+                   uv_left=np.zeros((n, cap, 2), np.float32), uv_right=np.zeros((n, cap, 2), np.float32),
+                   xyz_left=np.zeros((n, cap, 3), np.float64), desc_left=np.zeros((n, cap, 32), np.uint8),
+                   desc_right=np.zeros((n, cap, 32), np.uint8), distance=np.full((n, cap), -1, np.int32),
+                   match_index=np.full((n, cap), -1, np.int32), status=np.zeros((n, cap), np.uint8),
+                   second_distance=np.full((n, cap), -1, np.int32) if sparse else None,
+                   n_keypoints_right=np.zeros(n, np.int32) if sparse else None)
+
+    def result(self) -> _lib.StereoResult:
+        """svi_stereo_result over these (host) arrays."""
+        return _lib.StereoResult(self.uv_left.shape[1], _ptr(self.n_keypoints), _ptr(self.n_detected), _ptr(self.uv_left),
+                                 _ptr(self.uv_right), _ptr(self.xyz_left), _ptr(self.desc_left), _ptr(self.desc_right),
+                                 _ptr(self.distance), _ptr(self.match_index), _ptr(self.status))
 
     def frame(self, f: int) -> dict:
         n = int(self.n_keypoints[f])
-        return dict(uv_l=self.uv_left[f, :n], uv_r=self.uv_right[f, :n], xyz=self.xyz_left[f, :n],
-                    desc_l=self.desc_left[f, :n], desc_r=self.desc_right[f, :n], dist=self.distance[f, :n],
-                    idx=self.match_index[f, :n], status=self.status[f, :n])
+        d = dict(uv_l=self.uv_left[f, :n], uv_r=self.uv_right[f, :n], xyz=self.xyz_left[f, :n],
+                 desc_l=self.desc_left[f, :n], desc_r=self.desc_right[f, :n], dist=self.distance[f, :n],
+                 idx=self.match_index[f, :n], status=self.status[f, :n])
+        if self.second_distance is not None:
+            d["second"] = self.second_distance[f, :n]
+            d["n_right"] = int(self.n_keypoints_right[f])
+        return d
 
 
 class StereoFrontend:
@@ -211,6 +233,29 @@ class StereoFrontend:
                                                 _ptr(M), C.byref(r)))
         return out
 
+    def _band(self, band_v, min_disparity, max_disparity) -> _lib.SparseBand:
+        return _lib.SparseBand(float(band_v), float(min_disparity),
+                               float(self.params.search_range_px if max_disparity is None else max_disparity))
+
+    def stereo_frames_sparse(self, left, right, masks=None, band_v: float = 1.0, min_disparity: float = 1.0,
+                             max_disparity: float | None = None, capacity: int | None = None) -> StereoFrames:
+        """svi_stereo_frames_sparse: the batch of stereo_frames, but every LEFT key-point is matched against the RIGHT
+        key-points (same detector, no mask) with |y_L - y_R| <= band_v and min_disparity <= x_L - x_R <= max_disparity
+        (default: search_range_px) instead of by a dense scan line.  match_index indexes the frame's RIGHT key-points;
+        the result also carries second_distance (for a ratio test) and n_keypoints_right."""
+        L, R = self._images(left, "left"), self._images(right, "right")
+        if L.shape != R.shape:
+            raise ValueError("left/right batch shapes differ")
+        M = self._images(masks, "masks") if masks is not None else None
+        n, cap = L.shape[0], int(capacity or self.max_corners)
+        out = StereoFrames.empty(n, cap, sparse=True)
+        r = out.result()
+        sp = _lib.SparseResult(_ptr(out.second_distance), _ptr(out.n_keypoints_right))
+        band = self._band(band_v, min_disparity, max_disparity)
+        self._check(self._lib.svi_stereo_frames_sparse(self._ctx, _ptr(L), _ptr(R), self.width, self.width * self.height, n, _ptr(M),
+                                                       C.byref(band), C.byref(r), C.byref(sp)))
+        return out
+
     def add_new_landmarks(self, img_left, img_right, mask=None, mask_centres=None) -> dict:
         """One pair; per-key-point arrays in the reference's iteration order.  mask_centres (n, 2): the detection mask
         of getMaskActiveLandmarks is built on the GPU from these landmark centres (svi_stereo_frame_masked)."""
@@ -250,6 +295,15 @@ class StereoFrontend:
         """svi_stereo_frames_device: all addresses are DEVICE pointers; enqueues after `stream`, no sync."""
         self._check(self._lib.svi_stereo_frames_device(self._ctx, left_ptr, right_ptr, pitch, frame_stride, n_frames,
                                                        masks_ptr, C.byref(result), stream or None))
+
+    def stereo_frames_sparse_device(self, left_ptr, right_ptr, pitch, frame_stride, n_frames, result: _lib.StereoResult,
+                                    sparse: _lib.SparseResult, band_v: float = 1.0, min_disparity: float = 1.0,
+                                    max_disparity: float | None = None, masks_ptr=None, stream: int = 0):
+        """svi_stereo_frames_sparse_device: all addresses (also those in result / sparse) are DEVICE pointers; enqueues after
+        `stream`, no sync; capacity overflows surface in check_overflow()."""
+        band = self._band(band_v, min_disparity, max_disparity)
+        self._check(self._lib.svi_stereo_frames_sparse_device(self._ctx, left_ptr, right_ptr, pitch, frame_stride, n_frames, masks_ptr,
+                                                              C.byref(band), C.byref(result), C.byref(sparse), stream or None))
 
     def check_overflow(self):
         """svi_check_overflow: synchronise and raise SviError(SVI_ERR_CAPACITY) if a frame enqueued through
