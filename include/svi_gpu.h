@@ -63,7 +63,8 @@ typedef enum svi_status {
     SVI_EPI_NO_MATCHES = 21,   /* :2361 "could not find any matches (empty matches pool)"                     */
     SVI_EPI_DIST = 22,         /* :2395 "could not find a matching descriptor"                                */
     SVI_EPI_ORIG_DIST = 23,    /* :2390 "... (ORIGINAL matching distance too big)"                            */
-    SVI_EPI_NO_TRANSLATION = 24 /* :1804 detection pose == current pose: stage 3 is skipped for this landmark */
+    SVI_EPI_NO_TRANSLATION = 24, /* :1804 detection pose == current pose: stage 3 is skipped for this landmark */
+    SVI_SPARSE_NOT_MUTUAL = 25   /* sparse frames with svi_sparse_band.mutual: not a reference path (no reference text) */
 } svi_status;
 
 /* src/vision/CPinholeCamera.h:16-64: the members the hot path reads
@@ -218,14 +219,22 @@ int svi_match_epipolar(svi_ctx* ctx, const uint8_t* query32, const float* query_
  *     (lowest index on ties) and the second-smallest admissible distance; !(float(distance) < params.match_cutoff) gives
  *     SVI_TRI_DISTANCE (distance and index still written); else getPointInLEFT(uv_left, uv_right) as svi_point_in_left
  *     gives SVI_TRI_ZERO_DISP or SVI_OK with xyz_left, uv_right and desc_right (the matched RIGHT key-point's).
- * No ratio test is applied: second_distance is there for the caller's.  While rectification is set both images are raw.
- * SVI_ERR_INVALID for a NaN band field or min_disparity > max_disparity.  A frame whose candidate list overflows on either
- * side gets zero key-points on that side and the call returns SVI_ERR_CAPACITY (FAST mode: more corners than max_corners
- * on either side is SVI_ERR_CAPACITY too).  The first call allocates the per-lane scratch of this mode. */
+ * No ratio test is applied: second_distance is there for the caller's.
+ * Left-right check (band.mutual = 1, cv::BFMatcher(NORM_HAMMING, crossCheck = true)): for a slot matched to RIGHT key-point
+ *     j that passes the cut-off, the reverse arg-min of j -- the first arg-min over the frame's LEFT key-points under the
+ *     same admissibility relation, lowest LEFT slot on ties -- must be this slot, else SVI_SPARSE_NOT_MUTUAL.  Status order:
+ *     SVI_TRI_NO_MATCH, SVI_TRI_DISTANCE, SVI_SPARSE_NOT_MUTUAL, getPointInLEFT.  Every other field (LEFT fields,
+ *     n_keypoints_right, distance, match_index, second_distance) is byte-identical to mutual = 0; uv_right, xyz_left and
+ *     desc_right are valid for SVI_OK only, as always.  The first call with mutual = 1 allocates the check's per-lane scratch.
+ * While rectification is set both images are raw.
+ * SVI_ERR_INVALID for a NaN band field, min_disparity > max_disparity or mutual other than 0 or 1.  A frame whose
+ * candidate list overflows on either side gets zero key-points on that side and the call returns SVI_ERR_CAPACITY (FAST
+ * mode: more corners than max_corners on either side is SVI_ERR_CAPACITY too).  The first call allocates the per-lane scratch of this mode. */
 typedef struct svi_sparse_band {
     float band_v;          /* |y_L - y_R| <= band_v                       */
     float min_disparity;   /* min_disparity <= x_L - x_R <= max_disparity */
     float max_disparity;
+    int32_t mutual;        /* 0: no left-right check; 1: left-right check (SVI_SPARSE_NOT_MUTUAL) */
 } svi_sparse_band;
 typedef struct svi_sparse_result {
     int32_t* second_distance;    /* [frames * capacity_per_frame] second-smallest admissible distance, -1 if < 2 admissible */

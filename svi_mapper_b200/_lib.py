@@ -18,6 +18,7 @@ SVI_ERR_INVALID, SVI_ERR_CUDA, SVI_ERR_CAPACITY, SVI_ERR_NO_DEVICE, SVI_ERR_UNSU
  SVI_TRK_DEPTH, SVI_TRK_STAGE1_DIST, SVI_TRK_TRI_DESC, SVI_TRK_OUT_OF_FOV, SVI_TRK_NO_FEATURES, SVI_TRK_NO_MATCHES,
  SVI_TRK_DESC, SVI_TRK_RANGE, SVI_EPI_OUT_OF_SIGHT, SVI_EPI_VERTICAL, SVI_EPI_NEG_SLOPE, SVI_EPI_POS_SLOPE, SVI_EPI_ZERO_LEN,
  SVI_EPI_POOL_EMPTY, SVI_EPI_NO_MATCHES, SVI_EPI_DIST, SVI_EPI_ORIG_DIST, SVI_EPI_NO_TRANSLATION) = range(25)
+SVI_SPARSE_NOT_MUTUAL = 25   # sparse frames with the left-right check (SparseBand.mutual)
 
 EXPORTS = (
     "svi_params_default", "svi_status_text", "svi_brief_table_info", "svi_create", "svi_destroy", "svi_last_error", "svi_device_count",
@@ -58,8 +59,9 @@ class StereoResult(C.Structure):
 
 
 class SparseBand(C.Structure):
-    """svi_sparse_band: |y_L - y_R| <= band_v and min_disparity <= x_L - x_R <= max_disparity."""
-    _fields_ = [("band_v", C.c_float), ("min_disparity", C.c_float), ("max_disparity", C.c_float)]
+    """svi_sparse_band: |y_L - y_R| <= band_v and min_disparity <= x_L - x_R <= max_disparity; mutual = 1 adds the
+    left-right check (SVI_SPARSE_NOT_MUTUAL)."""
+    _fields_ = [("band_v", C.c_float), ("min_disparity", C.c_float), ("max_disparity", C.c_float), ("mutual", C.c_int32)]
 
 
 class SparseResult(C.Structure):

@@ -14,8 +14,17 @@
 // (distance << 32 | original index) minimum and its second-smallest distance.  Both reductions are order-independent, so the
 // result is the brute-force scan's whatever the tiles and whatever the band (a band >= H streams the whole list).
 //
-// kFrame = true (svi_stereo_frames_sparse[_device]) finishes the LEFT slot in the same kernel: cut-off, getPointInLEFT
-// (point_in_left, fp64) and the slot's outputs.  kFrame = false (svi_match_epipolar) writes index, distance and second.
+// Three modes (BandMode):
+//   BM_FRAME     svi_stereo_frames_sparse[_device]: LEFT queries against RIGHT trains; the same kernel finishes the LEFT slot:
+//                cut-off, with `mutual` set the left-right check against `rev`, getPointInLEFT (point_in_left, fp64), outputs.
+//   BM_REVERSE   the left-right check's reverse pass: RIGHT queries against LEFT trains (row-ordered descriptors gathered by
+//                gather_rows_kernel) with the bounds mirrored to (-max_disparity, -min_disparity).  x_R - x_L == -(x_L - x_R)
+//                exactly in IEEE fp32, so the test admits exactly the pairs BM_FRAME admits, NaNs included.  Writes only
+//                the (distance << 32 | LEFT slot) minimum -- the first arg-min: lowest slot on ties -- into rev[f][original
+//                RIGHT index] by 64-bit atomicMin (rev starts at ~0: no admissible LEFT key-point).  Few RIGHT queries against
+//                many LEFT trains make few, long CTAs, so gridDim.z splits each query block's train range into that many
+//                runs of tiles; the minimum is order-independent, so the result does not depend on the split.
+//   BM_EPIPOLAR  svi_match_epipolar: caller-ordered float lists; writes index, distance and second.
 #pragma once
 #include <type_traits>
 
@@ -27,7 +36,10 @@ constexpr int BM_THREADS = 128;   // queries per CTA
 constexpr int BM_TILE = 256;      // trains per shared tile (a multiple of 4: every bulk copy is a multiple of 16 bytes)
 constexpr int BM_ALIGN = 4;       // the streamed range starts and ends on a multiple of 4 elements (16-byte copy addresses)
 
-// Tile layout: [descriptors | coordinates | original indices (stereo frame only)], twice, then two mbarriers.
+enum BandMode { BM_EPIPOLAR = 0, BM_FRAME = 1, BM_REVERSE = 2 };
+
+// Tile layout: [descriptors | coordinates | original indices (row-sorted lists only)], twice, then two mbarriers.
+// kFrame: the row-sorted lists of a stereo frame (BM_FRAME and BM_REVERSE).
 template <bool kFrame>
 struct BandTile {
     using XY = typename std::conditional<kFrame, ushort2, float2>::type;   // frame: integer corners; epipolar: caller's floats
@@ -41,7 +53,8 @@ struct BandTile {
 struct BandArgs {
     float band_v, min_disp, max_disp;
     // queries.  Frame: LEFT key-points sorted by row ([f][max_corners]), their slots, per-frame counts; the descriptors are
-    // out.desc_l at the slot.  Epipolar: nq descriptors / coordinates in caller order.
+    // out.desc_l at the slot.  Reverse: the same for RIGHT, descriptors in row order ([f][max_corners]).  Epipolar: nq
+    // descriptors / coordinates in caller order.
     const ushort2* q_kp;
     const uint32_t* q_slot;
     const int* n_q;
@@ -49,7 +62,7 @@ struct BandArgs {
     const float2* q_xy;
     int nq;
     // trains.  Frame: RIGHT key-points, slots and descriptors sorted by row ([f][max_corners]) and the row CSR ([f][H + 1]).
-    // Epipolar: nt descriptors / coordinates in caller order.
+    // Reverse: the same for LEFT.  Epipolar: nt descriptors / coordinates in caller order.
     const ushort2* t_kp;
     const uint32_t* t_slot;
     const uint8_t* t_desc;
@@ -64,6 +77,11 @@ struct BandArgs {
     int* index;
     int* distance;
     int* second;
+    // left-right check.  Frame: `mutual` (CTA-uniform) applies it against rev, per-frame train counts n_t bound its index.
+    // Reverse: the output, rev[f][original RIGHT index] ([f][max_corners]), (distance << 32 | LEFT slot) or ~0.
+    unsigned long long* rev;
+    const int* n_t;
+    int mutual;
 };
 
 __device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
@@ -72,9 +90,16 @@ __device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_
                  : "memory");
 }
 
-template <bool kFrame>
+// The left-right check of LEFT slot `slot` matched to RIGHT key-point `idx`: is the reverse pass's arg-min of idx another slot?
+__device__ __forceinline__ bool not_mutual(const BandArgs& a, size_t fbase, int f, int idx, uint32_t slot) {
+    SVI_CHECK(12, idx < a.n_t[f] && idx < a.max_corners);
+    return (uint32_t)a.rev[fbase + idx] != slot;
+}
+
+template <int kMode>
 __global__ void __launch_bounds__(BM_THREADS)
 band_match_kernel(const __grid_constant__ BandArgs a) {
+    constexpr bool kFrame = kMode != BM_EPIPOLAR;   // row-sorted lists of a stereo frame
     using TL = BandTile<kFrame>;
     using XY = typename TL::XY;
     extern __shared__ __align__(128) unsigned char bm_smem[];
@@ -98,8 +123,13 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
             xq = (float)k.x;
             yq = (float)k.y;
             slot = a.q_slot[fbase + q];
-            SVI_CHECK(12, slot < (uint32_t)MC && slot < (uint32_t)a.out.cap);
-            src = a.out.desc_l + ((size_t)(a.out_frame0 + f) * a.out.cap + slot) * 32;
+            if constexpr (kMode == BM_FRAME) {
+                SVI_CHECK(12, slot < (uint32_t)MC && slot < (uint32_t)a.out.cap);
+                src = a.out.desc_l + ((size_t)(a.out_frame0 + f) * a.out.cap + slot) * 32;
+            } else {
+                SVI_CHECK(12, slot < (uint32_t)MC);
+                src = a.q_desc + (fbase + q) * 32;
+            }
         } else {
             const float2 k = a.q_xy[q];
             xq = k.x;
@@ -130,6 +160,13 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
     }
     const size_t a0 = lo & ~size_t(BM_ALIGN - 1), a1 = (hi + BM_ALIGN - 1) & ~size_t(BM_ALIGN - 1);
     const int n_tiles = (int)((a1 - a0 + BM_TILE - 1) / BM_TILE);
+    int k0 = 0, k1 = n_tiles;   // the tiles this CTA streams
+    if constexpr (kMode == BM_REVERSE) {
+        const int per = (n_tiles + (int)gridDim.z - 1) / (int)gridDim.z;
+        k0 = min(n_tiles, (int)blockIdx.z * per);
+        k1 = min(n_tiles, k0 + per);
+        if (k0 >= k1) return;   // CTA-uniform; nothing to merge
+    }
 
     const uint32_t bar0 = smem_u32(bm_smem + 2 * TL::BUF);
     if (tid == 0) {
@@ -153,8 +190,8 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
         if constexpr (kFrame) bulk_load(buf + TL::DESC + TL::XYB, a.t_slot + e0, cnt * 4u, bar);
     };
     if (tid == 0) {
-        if (n_tiles > 0) issue(0);
-        if (n_tiles > 1) issue(1);
+        if (k0 < k1) issue(k0);
+        if (k0 + 1 < k1) issue(k0 + 1);
     }
 
     const float band_v = a.band_v, dmin = a.min_disp, dmax = a.max_disp;
@@ -162,7 +199,7 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
     uint32_t second = 0xFFFFFFFFu;
     size_t best_pos = 0;               // element index of the best train (frame: its row-ordered descriptor and corner)
     uint32_t phase = 0u;               // bit b: parity of buffer b's next completion
-    for (int k = 0; k < n_tiles; ++k) {
+    for (int k = k0; k < k1; ++k) {
         const int b = k & 1;
         mbar_wait(bar0 + 8 * b, (phase >> b) & 1u);
         phase ^= 1u << b;
@@ -196,7 +233,7 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
             }
         }
         __syncthreads();   // every thread is done with buffer b
-        if (tid == 0 && k + 2 < n_tiles) issue(k + 2);
+        if (tid == 0 && k + 2 < k1) issue(k + 2);
     }
     if (!live) return;
 
@@ -204,7 +241,9 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
     const int dist = any ? (int)(best >> 32) : -1;
     const int idx = any ? (int)(uint32_t)best : -1;
     const int sec = second != 0xFFFFFFFFu ? (int)second : -1;
-    if constexpr (!kFrame) {
+    if constexpr (kMode == BM_REVERSE) {
+        if (any) atomicMin(a.rev + fbase + slot, best);
+    } else if constexpr (kMode == BM_EPIPOLAR) {
         a.index[q] = idx;
         a.distance[q] = dist;
         a.second[q] = sec;
@@ -221,6 +260,8 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
             st = SVI_TRI_NO_MATCH;
         } else if (!((float)dist < a.tc.match_cutoff)) {
             st = SVI_TRI_DISTANCE;
+        } else if (a.mutual && not_mutual(a, fbase, f, idx, slot)) {
+            st = SVI_SPARSE_NOT_MUTUAL;
         } else {
             SVI_CHECK(12, best_pos >= lo && best_pos < hi);
             const ushort2 t = a.t_kp[best_pos];
@@ -240,6 +281,19 @@ band_match_kernel(const __grid_constant__ BandArgs a) {
         }
         out.status[o] = (uint8_t)st;
     }
+}
+
+// LEFT descriptors in row order for the reverse pass: dst[f][i] = desc[frame0 + f][slot[f][i]] for the frame's n[f] key-points,
+// one thread per 16-byte half of a descriptor.
+constexpr int GR_THREADS = 256;
+__global__ void __launch_bounds__(GR_THREADS)
+gather_rows_kernel(const uint8_t* desc, int cap, int frame0, const uint32_t* slot, const int* n, int max_corners, uint8_t* dst) {
+    const int f = blockIdx.y, t = blockIdx.x * GR_THREADS + threadIdx.x, i = t >> 1;
+    if (i >= min(n[f], max_corners)) return;
+    const size_t e = (size_t)f * max_corners + i;
+    const uint32_t s = slot[e];
+    SVI_CHECK(12, s < (uint32_t)max_corners && s < (uint32_t)cap);
+    reinterpret_cast<uint4*>(dst + e * 32)[t & 1] = __ldg(reinterpret_cast<const uint4*>(desc + ((size_t)(frame0 + f) * cap + s) * 32) + (t & 1));
 }
 
 }  // namespace svi

@@ -91,6 +91,9 @@ struct Lane {
     ushort2* sp_kp_rs = nullptr;
     uint8_t* sp_desc_r = nullptr;      // RIGHT descriptors in row order
     int* sp_second = nullptr;          // second-smallest distance per LEFT slot (host path)
+    // the left-right check (svi_sparse_band.mutual): allocated at the first call that asks for it
+    uint8_t* sp_desc_lr = nullptr;     // LEFT descriptors in row order (the reverse pass's trains)
+    unsigned long long* sp_rev = nullptr;   // [chunk][max_corners]: per RIGHT key-point, (distance << 32 | best LEFT slot) or ~0
     CUtensorMap map_r_patch{};         // RIGHT plane, box = the 56 x 49 patch of one descriptor
     std::vector<cudaEvent_t> ev;  // stage boundary events (profiling)
     size_t ev_used = 0;
@@ -109,6 +112,7 @@ struct svi_ctx {
     int chunk = 0, n_lanes = 0;
     int cand_cap = 0, raw_cap = 0;
     float* resp_one = nullptr;   // svi_harris_response only: one W x H plane
+    int n_sms = 0;               // read at the first sparse call with the left-right check
     bool select_smem = true;
     int match_split = 0;     // warps per key-point in the scan-line matcher: 0 = chosen per launch; SVI_MATCH_SPLIT = 1 | 2 forces one
     bool trace = false;      // SVI_TRACE: host-side phase times of the tracking call on stderr (diagnostics)
@@ -462,10 +466,25 @@ int ensure_sparse_scratch(svi_ctx* ctx) {
     return SVI_SUCCESS;
 }
 
+// The left-right check's scratch (40 B per key-point and chunk frame): allocated at the first call with mutual = 1.
+int ensure_mutual_scratch(svi_ctx* ctx) {
+    if (!ctx->n_sms) CK(cudaDeviceGetAttribute(&ctx->n_sms, cudaDevAttrMultiProcessorCount, ctx->device));
+    const size_t C = (size_t)ctx->chunk, MC = (size_t)ctx->p.max_corners, L = C * MC + BM_ALIGN;
+    for (int i = 0; i < ctx->n_lanes; ++i) {
+        Lane& l = ctx->lanes[i];
+        if (l.sp_rev) continue;
+        CK(dmalloc(&l.sp_desc_lr, 32 * L));
+        CK(dmalloc(&l.sp_rev, C * MC));   // last: marks the lane's scratch complete
+    }
+    return SVI_SUCCESS;
+}
+
 // The sparse frame of nf frames on one lane: detection and selection on LEFT (with the masks) and on RIGHT (without) -- the
 // same launches as the dense path's, RIGHT after LEFT's selection so that the candidate lists are reused --, both key-point
 // lists sorted by row (bin_keypoints_kernel with full-width bins one row high: a row CSR plus each key-point's slot), LEFT
-// descriptors into out.desc_l as on the dense path, RIGHT descriptors over the row-sorted list, then band_match_kernel.
+// descriptors into out.desc_l as on the dense path, RIGHT descriptors over the row-sorted list, then band_match_kernel.  With
+// the left-right check, the LEFT descriptors are first gathered into row order and the reverse pass (RIGHT queries, LEFT
+// trains, mirrored bounds) writes each RIGHT key-point's best LEFT slot, which the forward pass's finish compares.
 // second / n_kp_r: the call's second-distance slots (indexed like out) and RIGHT key-point counts (indexed by chunk frame).
 int run_sparse(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_right, const uint8_t* d_mask, const FrameGeom& g, int nf,
                const StereoOutDev& out, int out_frame0, int* n_kp, int* n_det, int* second, int* n_kp_r, const svi_sparse_band& band) {
@@ -491,7 +510,22 @@ int run_sparse(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_ri
     a.t_kp = l.sp_kp_rs; a.t_slot = l.sp_slot_r; a.t_desc = l.sp_desc_r; a.t_row = l.sp_row_r;
     a.H = H; a.max_corners = MC;
     a.out = out; a.out_frame0 = out_frame0; a.tc = ctx->tc; a.second = second;
-    band_match_kernel<true><<<dim3((MC + BM_THREADS - 1) / BM_THREADS, nf), BM_THREADS, BandTile<true>::SMEM, s>>>(a);
+    const dim3 bgrid((MC + BM_THREADS - 1) / BM_THREADS, nf);
+    if (band.mutual) {
+        gather_rows_kernel<<<dim3((2 * MC + GR_THREADS - 1) / GR_THREADS, nf), GR_THREADS, 0, s>>>(out.desc_l, out.cap, out_frame0,
+                                                                                                  l.sp_slot_l, n_kp, MC, l.sp_desc_lr);
+        // splits of each RIGHT query block's LEFT range: about four CTAs per SM if every query block were full
+        const int blocks = (int)bgrid.x * nf, splits = std::min(8, std::max(1, (4 * ctx->n_sms + blocks - 1) / blocks));
+        CK(cudaMemsetAsync(l.sp_rev, 0xFF, sizeof(unsigned long long) * nf * MC, s));
+        BandArgs r{};
+        r.band_v = band.band_v; r.min_disp = -band.max_disparity; r.max_disp = -band.min_disparity;
+        r.q_kp = l.sp_kp_rs; r.q_slot = l.sp_slot_r; r.n_q = n_kp_r; r.q_desc = l.sp_desc_r;
+        r.t_kp = l.sp_kp_l; r.t_slot = l.sp_slot_l; r.t_desc = l.sp_desc_lr; r.t_row = l.sp_row_l;
+        r.H = H; r.max_corners = MC; r.rev = l.sp_rev;
+        band_match_kernel<BM_REVERSE><<<dim3(bgrid.x, nf, splits), BM_THREADS, BandTile<true>::SMEM, s>>>(r);
+        a.mutual = 1; a.rev = l.sp_rev; a.n_t = n_kp_r;
+    }
+    band_match_kernel<BM_FRAME><<<bgrid, BM_THREADS, BandTile<true>::SMEM, s>>>(a);
     CK(cudaGetLastError());
     return SVI_SUCCESS;
 }
@@ -1296,6 +1330,7 @@ const char* svi_status_text(int status) {
         case SVI_EPI_DIST: return "could not find a matching descriptor";
         case SVI_EPI_ORIG_DIST: return "could not find a matching descriptor (ORIGINAL matching distance too big)";
         case SVI_EPI_NO_TRANSLATION: return "no translation since detection: epipolar search skipped";
+        case SVI_SPARSE_NOT_MUTUAL: return "left-right check: the matched RIGHT key-point's best LEFT match is another key-point";
         default: return "unknown status";
     }
 }
@@ -1320,7 +1355,7 @@ void svi_destroy(svi_ctx* ctx) {
                         l.g_head, l.g_next, l.g_state, l.img_l, l.img_r, l.mask, l.out.uv_l, l.out.uv_r, l.out.xyz,
                         l.out.desc_l, l.out.desc_r, l.out.dist, l.out.idx, l.out.status, l.bin_start, l.bin_slot, l.bin_kp,
                         l.raw_l, l.raw_r, l.sp_kp_r, l.sp_n_kp_r, l.sp_n_det_r, l.sp_row_l, l.sp_slot_l, l.sp_kp_l, l.sp_row_r,
-                        l.sp_slot_r, l.sp_kp_rs, l.sp_desc_r, l.sp_second};
+                        l.sp_slot_r, l.sp_kp_rs, l.sp_desc_r, l.sp_second, l.sp_desc_lr, l.sp_rev};
         for (void* p : ptrs) if (p) cudaFree(p);
         for (cudaEvent_t e : l.ev) cudaEventDestroy(e);
         if (l.done) cudaEventDestroy(l.done);
@@ -1502,7 +1537,8 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
                                  (const void*)track_stage2_kernel<true>, (const void*)track_stage2_kernel<false>,
                                  (const void*)track_stage3_kernel, (const void*)fast_candidates_kernel,
                                  (const void*)describe_kernel, (const void*)hamming_match_kernel, (const void*)rectify_kernel,
-                                 (const void*)band_match_kernel<true>, (const void*)band_match_kernel<false>};
+                                 (const void*)band_match_kernel<BM_FRAME>, (const void*)band_match_kernel<BM_EPIPOLAR>,
+                                 (const void*)band_match_kernel<BM_REVERSE>, (const void*)gather_rows_kernel};
         for (const void* k : kernels)
             CK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
@@ -1646,8 +1682,11 @@ int check_sparse_args(svi_ctx* ctx, const char* name, const svi_sparse_band* ban
     if (std::isnan(band->band_v) || std::isnan(band->min_disparity) || std::isnan(band->max_disparity) ||
         band->min_disparity > band->max_disparity)
         return fail(ctx, SVI_ERR_INVALID, std::string(name) + ": band fields must not be NaN and min_disparity <= max_disparity");
+    if (band->mutual != 0 && band->mutual != 1) return fail(ctx, SVI_ERR_INVALID, std::string(name) + ": band.mutual must be 0 or 1");
     if (!sparse->second_distance || !sparse->n_keypoints_right) return fail(ctx, SVI_ERR_INVALID, std::string(name) + ": null output array");
-    return ensure_sparse_scratch(ctx);
+    const int rc = ensure_sparse_scratch(ctx);
+    if (rc != SVI_SUCCESS || !band->mutual) return rc;
+    return ensure_mutual_scratch(ctx);
 }
 }  // namespace
 
@@ -1887,7 +1926,7 @@ int svi_match_epipolar(svi_ctx* ctx, const uint8_t* query32, const float* query_
     a.q_desc = dev_at(ctx, i_q); a.q_xy = dev_at<float2>(ctx, i_qxy); a.nq = n_query;
     a.t_desc = dev_at(ctx, i_t); a.t_xy = dev_at<float2>(ctx, i_txy); a.nt = n_train;
     a.index = dev_at<int>(ctx, o_i); a.distance = dev_at<int>(ctx, o_d); a.second = dev_at<int>(ctx, o_s);
-    band_match_kernel<false><<<(n_query + BM_THREADS - 1) / BM_THREADS, BM_THREADS, BandTile<false>::SMEM, s>>>(a);
+    band_match_kernel<BM_EPIPOLAR><<<(n_query + BM_THREADS - 1) / BM_THREADS, BM_THREADS, BandTile<false>::SMEM, s>>>(a);
     CK(cudaGetLastError());
     if ((rc = call_fetch(ctx, o_i, L.end, s)) != SVI_SUCCESS) return rc;
     idle.done = true;

@@ -233,16 +233,21 @@ class StereoFrontend:
                                                 _ptr(M), C.byref(r)))
         return out
 
-    def _band(self, band_v, min_disparity, max_disparity) -> _lib.SparseBand:
+    def _band(self, band_v, min_disparity, max_disparity, mutual=False) -> _lib.SparseBand:
         return _lib.SparseBand(float(band_v), float(min_disparity),
-                               float(self.params.search_range_px if max_disparity is None else max_disparity))
+                               float(self.params.search_range_px if max_disparity is None else max_disparity), int(mutual))
 
     def stereo_frames_sparse(self, left, right, masks=None, band_v: float = 1.0, min_disparity: float = 1.0,
-                             max_disparity: float | None = None, capacity: int | None = None) -> StereoFrames:
+                             max_disparity: float | None = None, capacity: int | None = None, mutual: bool = False) -> StereoFrames:
         """svi_stereo_frames_sparse: the batch of stereo_frames, but every LEFT key-point is matched against the RIGHT
         key-points (same detector, no mask) with |y_L - y_R| <= band_v and min_disparity <= x_L - x_R <= max_disparity
         (default: search_range_px) instead of by a dense scan line.  match_index indexes the frame's RIGHT key-points;
-        the result also carries second_distance (for a ratio test) and n_keypoints_right."""
+        the result also carries second_distance (for a ratio test) and n_keypoints_right.
+
+        mutual=True adds the left-right check (cv2.BFMatcher crossCheck): a match whose RIGHT key-point has another LEFT
+        key-point as its own first arg-min in the same band gets SVI_SPARSE_NOT_MUTUAL.  Status order per slot:
+        SVI_TRI_NO_MATCH, SVI_TRI_DISTANCE (the cut-off), SVI_SPARSE_NOT_MUTUAL, then getPointInLEFT (SVI_TRI_ZERO_DISP or
+        SVI_OK).  Only status and the OK-only fields (uv_right, xyz_left, desc_right) differ from mutual=False."""
         L, R = self._images(left, "left"), self._images(right, "right")
         if L.shape != R.shape:
             raise ValueError("left/right batch shapes differ")
@@ -251,7 +256,7 @@ class StereoFrontend:
         out = StereoFrames.empty(n, cap, sparse=True)
         r = out.result()
         sp = _lib.SparseResult(_ptr(out.second_distance), _ptr(out.n_keypoints_right))
-        band = self._band(band_v, min_disparity, max_disparity)
+        band = self._band(band_v, min_disparity, max_disparity, mutual)
         self._check(self._lib.svi_stereo_frames_sparse(self._ctx, _ptr(L), _ptr(R), self.width, self.width * self.height, n, _ptr(M),
                                                        C.byref(band), C.byref(r), C.byref(sp)))
         return out
@@ -298,10 +303,11 @@ class StereoFrontend:
 
     def stereo_frames_sparse_device(self, left_ptr, right_ptr, pitch, frame_stride, n_frames, result: _lib.StereoResult,
                                     sparse: _lib.SparseResult, band_v: float = 1.0, min_disparity: float = 1.0,
-                                    max_disparity: float | None = None, masks_ptr=None, stream: int = 0):
+                                    max_disparity: float | None = None, masks_ptr=None, stream: int = 0, mutual: bool = False):
         """svi_stereo_frames_sparse_device: all addresses (also those in result / sparse) are DEVICE pointers; enqueues after
-        `stream`, no sync; capacity overflows surface in check_overflow()."""
-        band = self._band(band_v, min_disparity, max_disparity)
+        `stream`, no sync; capacity overflows surface in check_overflow().  mutual: the left-right check, with the status
+        order of stereo_frames_sparse."""
+        band = self._band(band_v, min_disparity, max_disparity, mutual)
         self._check(self._lib.svi_stereo_frames_sparse_device(self._ctx, left_ptr, right_ptr, pitch, frame_stride, n_frames, masks_ptr,
                                                               C.byref(band), C.byref(result), C.byref(sparse), stream or None))
 
