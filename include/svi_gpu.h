@@ -82,7 +82,7 @@ typedef struct svi_params {
     double quality_level;      /* 0.01  src/core/CFundamentalMatcher.cpp:18 (cv::GFTTDetector takes doubles) */
     double min_distance;       /* 7.0   ibid. */
     double harris_k;           /* 0.04  OpenCV default for GFTTDetector */
-    double min_disparity_px;   /* 0.01  src/core/CTriangulator.h:21 */
+    double min_disparity_px;   /* 0.01  src/core/CTriangulator.h:21; must be > 0 (svi_create refuses 0, negatives and NaN) */
     int32_t max_corners;       /* 1000  src/core/CFundamentalMatcher.cpp:18 */
     float keypoint_size;       /* 7.0   cv::KeyPoint::size GFTT reports (= blockSize) */
     float search_range_px;     /* 60.0  src/core/CTriangulator.h:20 */

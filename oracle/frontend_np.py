@@ -190,12 +190,27 @@ def box7_exact(c: np.ndarray) -> np.ndarray:
     return out.astype(F32)
 
 
+def harris_combine(a: np.ndarray, b: np.ndarray, c: np.ndarray, k: float) -> np.ndarray:
+    """calcHarris on the three box-summed planes.  OpenCV runs it over the plane as ONE row of W*H pixels (the planes are
+    continuous): 4-lane fp32 vectors with (float)k for all but the last (W*H) % 4 pixels, which its scalar tail computes
+    as (float)(a*c - b*b - k*(a+c)*(a+c)) with the double k -- a*c, b*b, their difference and a+c in fp32, the rest in
+    fp64.  So those 1-3 pixels at the end of the last row can differ from the vector formula in the last bit."""
+    kf = F32(k)
+    R = (a * c - b * b) - (kf * (a + c)) * (a + c)
+    n = R.size
+    if n % 4:
+        fa, fb, fc, fr = a.reshape(-1), b.reshape(-1), c.reshape(-1), R.reshape(-1)
+        for i in range(n - n % 4, n):
+            det = float(fa[i] * fc[i] - fb[i] * fb[i])
+            tr = float(fa[i] + fc[i])
+            fr[i] = F32(det - float(k) * tr * tr)
+    return R
+
+
 def harris_response(img: np.ndarray, k: float = 0.04, box=box7_opencv_order) -> np.ndarray:
     """cv::cornerHarris(img, blockSize 7, ksize 3, k) with optimisations off, fp32 bit-exact."""
     xx, xy, yy = sobel_products(np.ascontiguousarray(img))
-    a, b, c = box(xx), box(xy), box(yy)
-    kf = F32(k)
-    return (a * c - b * b) - (kf * (a + c)) * (a + c)
+    return harris_combine(box(xx), box(xy), box(yy), k)
 
 
 def harris_response_roi(img: np.ndarray, roi, k: float = 0.04, box=box7_opencv_order) -> np.ndarray:
@@ -206,8 +221,7 @@ def harris_response_roi(img: np.ndarray, roi, k: float = 0.04, box=box7_opencv_o
     x, y, w, h = roi
     xx, xy, yy = sobel_products(np.ascontiguousarray(img))
     a, b, c = (box(np.ascontiguousarray(p[y:y + h, x:x + w])) for p in (xx, xy, yy))
-    kf = F32(k)
-    return (a * c - b * b) - (kf * (a + c)) * (a + c)
+    return harris_combine(a, b, c, k)   # the response of an ROI is a fresh continuous plane: the tail is the window's
 
 
 def gftt(img: np.ndarray, max_corners=1000, quality=0.01, min_distance=7.0, mask=None,

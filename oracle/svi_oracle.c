@@ -119,6 +119,10 @@ static int harris_roi(const uint8_t* img, int w, int h, int pitch, int rx, int r
             }
         }
     }
+    /* calcHarris runs over the response as one row of rw*rh pixels (both planes are continuous): 4-lane fp32 vectors with
+     * (float)k, then a scalar tail for the last n % 4 pixels that evaluates (float)(a*c - b*b - k*(a+c)*(a+c)) with the
+     * double k (a*c, b*b, det and a+c in fp32, the rest in fp64) */
+    const size_t tail = n - n % 4;
     for (int i = 0; i < 3 * rw; ++i) col[i] = 0;
     for (int yy = -3; yy < 3; ++yy) {
         const double* d = hs + (size_t)reflect_n(yy, rh) * rw * 3;
@@ -137,6 +141,10 @@ static int harris_roi(const uint8_t* img, int w, int h, int pitch, int rx, int r
             float ac = a * c, bb = b * b;
             float det = ac - bb;
             float tr = a + c;
+            if ((size_t)y * rw + x >= tail) {
+                o[x] = (float)((double)det - k * (double)tr * (double)tr);
+                continue;
+            }
             float kt = kf * tr;
             float ktt = kt * tr;
             o[x] = det - ktt;

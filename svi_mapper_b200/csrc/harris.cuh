@@ -200,7 +200,8 @@ boxsum9_kernel(const uint8_t* __restrict__ img, FrameGeom g, uint16_t* __restric
 //                           q = (p[x-1]*f1 + p[x]*f0) + p[x+1]*f1;  Dy = q[y+1]-q[y-1]
 //   every op rounded to fp32 on its own (explicit _rn intrinsics, never an FMA).
 //   Box 7x7 (A.2): products accumulated in fp64, REFLECT_101 on the PRODUCT planes, one rounding
-//   to fp32.  Harris (A.3): R = (a*c - b*b) - (k*(a+c))*(a+c) in fp32.
+//   to fp32.  Harris (A.3): R = (a*c - b*b) - (k*(a+c))*(a+c) in fp32 (the last (W*H) % 4 pixels: k*(a+c)*(a+c) and
+//   the difference in fp64 with the double k, as calcHarris's scalar tail).
 //   Candidates (A.4): R > 0, R > thr(tile max), R >= its 8 neighbours (neighbours outside the image are
 //   ignored, as cv::dilate does), mask != 0, 1-px image border excluded.
 //   key = ordered(R) << 32 | y << 16 | x ; descending key order == cv's greaterThanPtr order
@@ -213,7 +214,7 @@ boxsum9_kernel(const uint8_t* __restrict__ img, FrameGeom g, uint16_t* __restric
 // `resp` (optional, svi_harris_response only) receives the response plane, `out_rows` rows per z.
 __global__ void __launch_bounds__(HT_THREADS, HARRIS_CTAS_PER_SM)
 harris_box_kernel(const uint8_t* __restrict__ img, const uint8_t* __restrict__ mask, FrameGeom g,
-                  float f1, float f0, float kf, double quality, float* __restrict__ resp, uint16_t* __restrict__ box,
+                  float f1, float f0, double k, double quality, float* __restrict__ resp, uint16_t* __restrict__ box,
                   uint16_t* __restrict__ box_shift, uint32_t* __restrict__ frame_max,
                   unsigned long long* __restrict__ cand, int* __restrict__ cand_count, int cand_cap,
                   const RoiItem* __restrict__ rois, const int* __restrict__ n_rois, int out_rows) {
@@ -358,24 +359,32 @@ harris_box_kernel(const uint8_t* __restrict__ img, const uint8_t* __restrict__ m
         float* rrow = resp ? resp + ((size_t)f * out_rows) * g.resp_pitch : nullptr;
         const uint8_t* mrow = mask ? mask + (size_t)f * g.img_stride : nullptr;
         const int rows_in = min(8, H - (y0 + oy0));   // rows of this thread inside the image (<= 0: none)
+        // cv::cornerHarris (calcHarris) evaluates the response plane as ONE row of W*H pixels: 4-lane fp32 vectors with
+        // (float)k, and a scalar tail for the last (W*H) % 4 pixels (the end of the last row) that computes
+        // (float)(a*c - b*b - k*(a+c)*(a+c)) with the double k: det and a+c in fp32, the rest in fp64
+        const float kf = (float)k;
+        const long long tail_start = (long long)W * H - (((W & 3) * (H & 3)) & 3);
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
+        for (int r = 0; r < 8; ++r) {
             float R = -INFINITY;   // outside the image: ignored by the neighbourhood maximum
-            if (gx < W && k < rows_in) {
-                const float a = bsum[0][k], b = bsum[1][k], c = bsum[2][k];
+            if (gx < W && r < rows_in) {
+                const float a = bsum[0][r], b = bsum[1][r], c = bsum[2][r];
                 const float det = __fsub_rn(__fmul_rn(a, c), __fmul_rn(b, b));
                 const float tr = __fadd_rn(a, c);
-                R = __fsub_rn(det, __fmul_rn(__fmul_rn(kf, tr), tr));
-                const int gy = y0 + oy0 + k;
+                const int gy = y0 + oy0 + r;
+                if ((long long)gy * W + gx < tail_start)
+                    R = __fsub_rn(det, __fmul_rn(__fmul_rn(kf, tr), tr));
+                else
+                    R = __double2float_rn(__dsub_rn((double)det, __dmul_rn(__dmul_rn(k, (double)tr), (double)tr)));
                 if (rrow) rrow[(size_t)gy * g.resp_pitch + gx] = R;
                 if (!mrow || mrow[(size_t)gy * g.img_pitch + gx]) {
                     lmax = fmaxf(lmax, R);
-                    mbits |= 1u << k;
+                    mbits |= 1u << r;
                 }
             }
-            rv[k] = R;
-            SVI_CHECK(1, oy0 + k < HT_H && x < HT_W);
-            Rs[oy0 + k][x] = R;
+            rv[r] = R;
+            SVI_CHECK(1, oy0 + r < HT_H && x < HT_W);
+            Rs[oy0 + r][x] = R;
         }
     }
     uint32_t local_max = lmax == -INFINITY ? 0u : float_to_ordered(lmax);   // 0 = no admitted pixel

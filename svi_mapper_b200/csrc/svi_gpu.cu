@@ -121,7 +121,7 @@ struct svi_ctx {
     int nbx = 0, n_bins = 0;
     SelectParams sel{};
     TriConst tc{};
-    float f1 = 0, f0 = 0, kf = 0;
+    float f1 = 0, f0 = 0;
     Lane lanes[kMaxLanes];
     // candidate-list overflow flag: one int of mapped page-locked host memory.  Kernels write it in place (only when a
     // list overflows), the host reads it after the synchronisation it does anyway -- no copy, no extra round trip per call
@@ -318,7 +318,7 @@ void launch_detector(svi_ctx* ctx, Lane& l, const uint8_t* d_img, const uint8_t*
         boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, box, nullptr);
     } else {
         harris_box_kernel<<<harris_grid(g.W, g.H, nf), HT_THREADS, sizeof(HarrisSmem), s>>>(
-            d_img, d_mask, g, ctx->f1, ctx->f0, ctx->kf, ctx->p.quality_level, nullptr, box, nullptr, l.frame_max, l.cand,
+            d_img, d_mask, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, nullptr, box, nullptr, l.frame_max, l.cand,
             l.cand_count, ctx->raw_cap, nullptr, nullptr, g.H);
     }
 }
@@ -1056,7 +1056,7 @@ int track_stage2_side(svi_ctx* ctx, Lane& l, const FrameGeom& g, int n, const do
         CK(cudaMemsetAsync(r.max, 0, sizeof(int) * ((size_t)r.items * 3 + 4), s));   // max, cand_count, defer, counters
         stage2_plan_kernel<<<(nb + 127) / 128, 128, 0, s>>>(k, left ? 0 : 1, (float)(1.0 + motion_scaling), ld, q0, q0 + nb, o, r.rois, r.s2, n_items);
         harris_box_kernel<<<harris_grid(max_w, max_h, nb), HT_THREADS, sizeof(HarrisSmem), s>>>(
-            ctx->trk_img, nullptr, g, ctx->f1, ctx->f0, ctx->kf, ctx->p.quality_level, nullptr, nullptr, nullptr, r.max, r.cand,
+            ctx->trk_img, nullptr, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, nullptr, nullptr, nullptr, r.max, r.cand,
             r.cand_count, kRoiRawCap, r.rois, n_items, 0);
         // thousands of small windows: seven small-configuration CTAs per SM; the rare window that does not fit is
         // deferred to the frame-size configuration (its CTAs return at once for every other window)
@@ -1394,6 +1394,9 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     svi_params p;
     if (params) p = *params; else svi_params_default(&p);
     if (p.max_corners <= 0 || p.max_corners > 65535) return fail(nullptr, SVI_ERR_INVALID, "svi_create: max_corners must be in [1, 65535]");
+    // CTriangulator rejects a match whose disparity is below the minimum; at 0 a zero-disparity match would pass and put
+    // the point at infinite depth (and the depth bound du / min_disparity_px would be infinite too)
+    if (!(p.min_disparity_px > 0.0)) return fail(nullptr, SVI_ERR_INVALID, "svi_create: min_disparity_px must be positive");
     if (p.max_candidates < 1024) p.max_candidates = 1024;
     if (p.max_queries < 1) p.max_queries = 1;
     {
@@ -1464,7 +1467,6 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     const double scale = 1.0 / (4.0 * 7.0 * 255.0);
     ctx->f1 = (float)scale;
     ctx->f0 = (float)(2.0 * scale);
-    ctx->kf = (float)p.harris_k;
 
     // goodFeaturesToTrack's bucket grid; cell >= minDistance keeps the 3x3 neighbourhood sufficient
     SelectParams& sp = ctx->sel;
@@ -1774,7 +1776,7 @@ int svi_harris_response(svi_ctx* ctx, const uint8_t* img, size_t pitch, float* r
     CK(cudaMemsetAsync(l.frame_max, 0, sizeof(uint32_t), s));
     if (!ctx->resp_one) CK(dmalloc(&ctx->resp_one, (size_t)ctx->H * ctx->resp_pitch));
     harris_box_kernel<<<harris_grid(g.W, g.H, 1), HT_THREADS, sizeof(HarrisSmem), s>>>(
-        l.img_l, nullptr, g, ctx->f1, ctx->f0, ctx->kf, ctx->p.quality_level, ctx->resp_one, nullptr, nullptr, l.frame_max, nullptr,
+        l.img_l, nullptr, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, ctx->resp_one, nullptr, nullptr, l.frame_max, nullptr,
         nullptr, 0, nullptr, nullptr, g.H);
     CK(cudaGetLastError());
     CK(cudaMemcpy2DAsync(response, sizeof(float) * ctx->W, ctx->resp_one, sizeof(float) * ctx->resp_pitch, sizeof(float) * ctx->W,
@@ -1817,7 +1819,7 @@ int svi_detect(svi_ctx* ctx, const uint8_t* img, size_t pitch, size_t frame_stri
                                                                 l.cand_count, ctx->raw_cap);
         } else {
             harris_box_kernel<<<harris_grid(W, H, nf), HT_THREADS, sizeof(HarrisSmem), s>>>(
-                l.img_l, d_mask, g, ctx->f1, ctx->f0, ctx->kf, ctx->p.quality_level, nullptr, nullptr, nullptr, l.frame_max, l.cand,
+                l.img_l, d_mask, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, nullptr, nullptr, nullptr, l.frame_max, l.cand,
                 l.cand_count, ctx->raw_cap, nullptr, nullptr, g.H);
         }
         const uint32_t* fmax = fast ? nullptr : l.frame_max;
