@@ -64,7 +64,8 @@ typedef enum svi_status {
     SVI_EPI_DIST = 22,         /* :2395 "could not find a matching descriptor"                                */
     SVI_EPI_ORIG_DIST = 23,    /* :2390 "... (ORIGINAL matching distance too big)"                            */
     SVI_EPI_NO_TRANSLATION = 24, /* :1804 detection pose == current pose: stage 3 is skipped for this landmark */
-    SVI_SPARSE_NOT_MUTUAL = 25   /* sparse frames with svi_sparse_band.mutual: not a reference path (no reference text) */
+    SVI_SPARSE_NOT_MUTUAL = 25,  /* sparse frames with svi_sparse_band.mutual: not a reference path (no reference text) */
+    SVI_SUBPIXEL_REJECTED = 26   /* svi_params.subpixel_window: the SAD minimum lies on the edge of the search (no reference text) */
 } svi_status;
 
 /* src/vision/CPinholeCamera.h:16-64: the members the hot path reads
@@ -100,6 +101,32 @@ typedef struct svi_params {
     int32_t detector;
     int32_t fast_threshold;    /* 10 (cv default) */
     int32_t fast_nonmax;       /* 1 */
+    /* optional sub-pixel disparity (NOT a reference code path; ORB-SLAM2's Frame::ComputeStereoMatches refinement): 0 = off
+     * (default): every output is the reference's integer-disparity result.  w = subpixel_window > 0 refines the match of every
+     * slot the new-landmark path reports SVI_OK -- svi_stereo_frames[_device] (both matchers), svi_stereo_frame_masked,
+     * svi_stereo_frames_sparse[_device] (after the left-right check when it is on) and svi_multi_stereo_frames -- with
+     * L = subpixel_search, on the images the detector read (the rectified planes while rectification is set):
+     *   1. PL = the (2w+1)^2 LEFT patch centred on (xL, y) minus its centre pixel (integers);
+     *   2. for k = -L .. L: PR(k) = the RIGHT patch centred on ((int)xR + k, y) minus its centre pixel, SAD(k) = sum |PL - PR(k)|
+     *      (int32).  y is the LEFT row for both patches (rectified images): a sparse match on a neighbouring RIGHT row is
+     *      refined on the LEFT row, and its uv_right.y stays the RIGHT key-point's row;
+     *   3. k* = the first strict minimum in increasing k; k* = +-L is SVI_SUBPIXEL_REJECTED;
+     *   4. s1, s2, s3 = SAD(k*-1), SAD(k*), SAD(k*+1); delta = float(s1 - s3) / (2 * float(s1 + s3 - 2 s2)) in fp32
+     *      (the denominator is > 0, delta is in (-0.5, 0.5]);
+     *   5. xR' = (xR + (float)k*) + delta, fp32, rounded after each addition;
+     *   6. getPointInLEFT(uv_left, (xR', y)): SVI_TRI_ZERO_DISP, or SVI_OK with uv_right.x = xR' and xyz_left.
+     * Status order: the integer path's statuses, SVI_SUBPIXEL_REJECTED, then step 6.  A slot the integer path reports
+     * SVI_TRI_ZERO_DISP (only possible with min_disparity_px >= 1 or a sparse band admitting x_R >= x_L) is not refined.
+     * Only uv_right.x, xyz_left and status change: distance, match_index, second_distance, every LEFT field and the counts are
+     * byte-identical to the mode off, and desc_right stays the descriptor at the integer match.
+     * svi_create refuses w < 0 and, for w > 0, L < 1 or w + L > 28.  BRIEF's 28-px border filter keeps every LEFT key-point
+     * and every RIGHT position either matcher reports at least 28 px inside the image, so with w + L <= 28 every patch lies
+     * inside the image: there is no border mode.  (A fractional keypoint_size or search_range_px can make the dense
+     * matcher's uv_right.x fractional; a slot whose patches would then leave the image is SVI_SUBPIXEL_REJECTED.)
+     * Not applied by the tracking cascade (svi_track_landmarks*), svi_track_frame_stereo_only or the per-query
+     * svi_triangulate_* / svi_point_in_left. */
+    int32_t subpixel_window;   /* 0 */
+    int32_t subpixel_search;   /* 0 */
 } svi_params;
 
 enum { SVI_DETECTOR_GFTT_HARRIS = 0, SVI_DETECTOR_FAST_9_16 = 1 };
@@ -453,7 +480,7 @@ int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uin
  * exclusive duration of one kernel (what the roofline record uses -- slower overall, not for timing
  * the step).  svi_set_profiling also clears the accumulators; svi_stage_timings waits for the ctx to
  * go idle and returns, per stage, the summed launch duration in ms and the number of launches
- * (arrays of length >= 5; returns the stage count; "describe_left" has launches only on the batch path, where the LEFT descriptors are a kernel of their own ahead of the matcher). */
+ * (arrays of length >= 6; returns the stage count; "describe_left" has launches only on the batch path, where the LEFT descriptors are a kernel of their own ahead of the matcher, and "subpixel" only while svi_params.subpixel_window > 0). */
 int svi_set_profiling(svi_ctx* ctx, int enable);
 int svi_stage_timings(svi_ctx* ctx, const char** names, double* total_ms, int64_t* launches, int capacity);
 
@@ -482,7 +509,7 @@ int svi_config(const svi_ctx* ctx, int32_t* chunk_frames, int32_t* n_lanes, int3
 /* Number of kernels the new-landmark path launches for one chunk of a call with n_frames frames: 4 (detector, RIGHT box
  * sums, corner selection, matcher) on the small-call path, 5 when the LEFT descriptors are a kernel of their own (batch
  * path), 6 when the batch path also sorts the key-points into image bins (dense frames); one more while rectification is
- * set (svi_set_rectification).  For launch accounting. */
+ * set (svi_set_rectification); one more while svi_params.subpixel_window > 0.  For launch accounting. */
 int svi_kernels_per_chunk(const svi_ctx* ctx, int n_frames);
 
 /* ---- undistortion + rectification of raw camera images (CStereoCamera.h:102-107, CStereoCameraIMU.h:36-51: the reference

@@ -19,6 +19,7 @@ SVI_ERR_INVALID, SVI_ERR_CUDA, SVI_ERR_CAPACITY, SVI_ERR_NO_DEVICE, SVI_ERR_UNSU
  SVI_TRK_DESC, SVI_TRK_RANGE, SVI_EPI_OUT_OF_SIGHT, SVI_EPI_VERTICAL, SVI_EPI_NEG_SLOPE, SVI_EPI_POS_SLOPE, SVI_EPI_ZERO_LEN,
  SVI_EPI_POOL_EMPTY, SVI_EPI_NO_MATCHES, SVI_EPI_DIST, SVI_EPI_ORIG_DIST, SVI_EPI_NO_TRANSLATION) = range(25)
 SVI_SPARSE_NOT_MUTUAL = 25   # sparse frames with the left-right check (SparseBand.mutual)
+SVI_SUBPIXEL_REJECTED = 26   # sub-pixel refinement (Params.subpixel_window > 0): the SAD minimum is on the edge of the search
 
 EXPORTS = (
     "svi_params_default", "svi_status_text", "svi_brief_table_info", "svi_create", "svi_destroy", "svi_last_error", "svi_device_count",
@@ -46,6 +47,7 @@ class Params(C.Structure):
         ("cutoff_stage3", C.c_float), ("cutoff_original", C.c_float),
         ("max_candidates", C.c_int32), ("chunk_frames", C.c_int32), ("max_queries", C.c_int32),
         ("detector", C.c_int32), ("fast_threshold", C.c_int32), ("fast_nonmax", C.c_int32),
+        ("subpixel_window", C.c_int32), ("subpixel_search", C.c_int32),   # sub-pixel disparity: 0 = off (default)
     ]
 
 

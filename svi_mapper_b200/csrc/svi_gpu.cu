@@ -29,6 +29,7 @@
 #include "posit.cuh"
 #include "rectify.cuh"
 #include "select.cuh"
+#include "subpixel.cuh"
 #include "sv_frame.cuh"
 #include "track_plan.cuh"
 
@@ -39,9 +40,10 @@ namespace {
 constexpr int kMaxLanes = 8;
 constexpr int kSmallFrames = 2;          // calls of up to this many frames go through the pinned bounce buffer
 constexpr size_t kOutBytesPerSlot = 8 + 8 + 24 + 32 + 32 + 4 + 4 + 1;   // uv_l uv_r xyz desc_l desc_r dist idx status
-constexpr int kStages = 5;
-const char* const kStageNames[kStages] = {"harris_box", "boxsum_right", "select_corners", "describe_left", "stereo_match"};
+constexpr int kStages = 6;
+const char* const kStageNames[kStages] = {"harris_box", "boxsum_right", "select_corners", "describe_left", "stereo_match", "subpixel"};
 constexpr int kStageDescribe = 3;   // present only on the batch path (LEFT descriptors ahead of the matcher)
+constexpr int kStageSubpixel = 5;   // present only while svi_params.subpixel_window > 0
 constexpr int kRawFactor = 4;   // the Harris kernel's list (local maxima above the TILE threshold) vs max_candidates
 
 std::string g_create_error;
@@ -266,6 +268,7 @@ void collect_timings(svi_ctx* c) {
         for (size_t i = 0, rec = 0; i + kStages < l.ev_used; i += kStages + 1, ++rec) {
             for (int s = 0; s < kStages; ++s) {
                 if (s == kStageDescribe && !(rec < l.ev_pre.size() && l.ev_pre[rec])) continue;   // no kernel in that bracket
+                if (s == kStageSubpixel && c->p.subpixel_window == 0) continue;
                 float ms = 0.f;
                 if (cudaEventElapsedTime(&ms, l.ev[i + s], l.ev[i + s + 1]) == cudaSuccess) {
                     c->stage_ms[s] += ms;
@@ -337,8 +340,22 @@ void launch_select(svi_ctx* ctx, Lane& l, int nf, ushort2* det_xy, int* n_det, u
     }
 }
 
+// Sub-pixel refinement of the chunk's SVI_OK slots (subpixel.cuh), after the matcher on the lane's stream; nothing while the
+// mode is off.  d_left / d_right: the planes the detector and the matcher read.
+int launch_subpixel(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_right, const FrameGeom& g, int nf,
+                    const StereoOutDev& out, int out_frame0, const int* n_kp) {
+    if (ctx->p.subpixel_window == 0) return SVI_SUCCESS;
+    SubpixelArgs a{};
+    a.left = d_left; a.right = d_right; a.g = g; a.n_kp = n_kp; a.max_corners = ctx->p.max_corners;
+    a.out = out; a.out_frame0 = out_frame0; a.tc = ctx->tc; a.w = ctx->p.subpixel_window; a.L = ctx->p.subpixel_search;
+    subpixel_refine_kernel<<<dim3((ctx->p.max_corners + SP_WARPS - 1) / SP_WARPS, nf), SP_WARPS * 32, 0, l.stream>>>(a);
+    CK(cudaGetLastError());
+    return SVI_SUCCESS;
+}
+
 // The kernels of the new-landmark path for `nf` frames on one lane: detector, RIGHT box sums, corner selection, then the
-// descriptor / match stages in the form that fits the call (svi_kernels_per_chunk: 4 to 6 launches).
+// descriptor / match stages in the form that fits the call, then the optional sub-pixel refinement (svi_kernels_per_chunk:
+// 4 to 7 launches).
 int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_right, const uint8_t* d_mask,
                  const FrameGeom& g, int nf, const StereoOutDev& out, int out_frame0, int* n_kp, int* n_det,
                  cudaStream_t side = nullptr, const std::function<int(cudaStream_t)>* upload_right = nullptr) {
@@ -381,7 +398,10 @@ int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_
     if (pre && ctx->match_binned && l.bin_start) {
         const int rc = run_binned<BinWide>(ctx, l, g, nf, out, out_frame0, n_kp);
         CK(cudaGetLastError());
-        return rc;
+        if (rc != SVI_SUCCESS) return rc;
+        const int rs = launch_subpixel(ctx, l, d_left, d_right, g, nf, out, out_frame0, n_kp);
+        mark(ctx, l);
+        return rs;
     }
     if (pre) {
         const dim3 dgrid((ctx->p.max_corners + DL_WARPS * DL_KP_PER_WARP - 1) / (DL_WARPS * DL_KP_PER_WARP), nf);
@@ -403,7 +423,9 @@ int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_
 #undef SVI_MATCH_ARGS
     mark(ctx, l);
     CK(cudaGetLastError());
-    return SVI_SUCCESS;
+    const int rs = launch_subpixel(ctx, l, d_left, d_right, g, nf, out, out_frame0, n_kp);
+    mark(ctx, l);
+    return rs;
 }
 
 int check_overflow(svi_ctx* ctx) {
@@ -527,7 +549,7 @@ int run_sparse(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_ri
     }
     band_match_kernel<BM_FRAME><<<bgrid, BM_THREADS, BandTile<true>::SMEM, s>>>(a);
     CK(cudaGetLastError());
-    return SVI_SUCCESS;
+    return launch_subpixel(ctx, l, d_left, d_right, g, nf, out, out_frame0, n_kp);
 }
 
 // ---- rectification
@@ -1300,6 +1322,8 @@ int svi_params_default(svi_params* p) {
     p->detector = SVI_DETECTOR_GFTT_HARRIS;
     p->fast_threshold = 10;
     p->fast_nonmax = 1;
+    p->subpixel_window = 0;
+    p->subpixel_search = 0;
     return SVI_SUCCESS;
 }
 
@@ -1331,6 +1355,7 @@ const char* svi_status_text(int status) {
         case SVI_EPI_ORIG_DIST: return "could not find a matching descriptor (ORIGINAL matching distance too big)";
         case SVI_EPI_NO_TRANSLATION: return "no translation since detection: epipolar search skipped";
         case SVI_SPARSE_NOT_MUTUAL: return "left-right check: the matched RIGHT key-point's best LEFT match is another key-point";
+        case SVI_SUBPIXEL_REJECTED: return "sub-pixel refinement: the SAD minimum lies on the edge of the search range";
         default: return "unknown status";
     }
 }
@@ -1397,6 +1422,9 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     // CTriangulator rejects a match whose disparity is below the minimum; at 0 a zero-disparity match would pass and put
     // the point at infinite depth (and the depth bound du / min_disparity_px would be infinite too)
     if (!(p.min_disparity_px > 0.0)) return fail(nullptr, SVI_ERR_INVALID, "svi_create: min_disparity_px must be positive");
+    // every patch of the refinement stays inside BRIEF's 28-px border: no border mode (include/svi_gpu.h)
+    if (p.subpixel_window < 0 || (p.subpixel_window > 0 && (p.subpixel_search < 1 || p.subpixel_window + p.subpixel_search > SP_MAX_REACH)))
+        return fail(nullptr, SVI_ERR_INVALID, "svi_create: subpixel_window must be >= 0 and, when > 0, subpixel_search >= 1 with window + search <= 28");
     if (p.max_candidates < 1024) p.max_candidates = 1024;
     if (p.max_queries < 1) p.max_queries = 1;
     {
@@ -2535,7 +2563,7 @@ int svi_kernels_per_chunk(const svi_ctx* ctx, int n_frames) {
     const long long slots = (long long)std::min(n_frames, ctx->chunk) * ctx->p.max_corners;
     const bool pre = ctx->match_pre && slots / (2LL * ctx->n_sm * 9) >= MATCH_KP_PER_WARP;
     // detector, RIGHT box sums, corner selection, matcher (+ LEFT descriptors as a kernel of their own, + the bin sort)
-    return 4 + (pre ? 1 : 0) + (pre && ctx->match_binned ? 1 : 0) + (ctx->rect ? 1 : 0);
+    return 4 + (pre ? 1 : 0) + (pre && ctx->match_binned ? 1 : 0) + (ctx->rect ? 1 : 0) + (ctx->p.subpixel_window > 0 ? 1 : 0);
 }
 
 int svi_config(const svi_ctx* ctx, int32_t* chunk_frames, int32_t* n_lanes, int32_t* select_in_smem) {
