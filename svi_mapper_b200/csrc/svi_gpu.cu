@@ -310,15 +310,15 @@ int setup_binned(svi_ctx* ctx, Lane& l, size_t rows, std::string* err) {
 }
 
 // The detector on nf frames of one image: candidate lists in the lane's scratch (zeroed by the caller), and the image's box-sum
-// plane `box` (harris_box writes it from its own tile; in FAST mode boxsum9, without the shifted copy).  With the selection
-// below, the detection of the dense path (LEFT) and of both sides of the sparse path.
+// plane `box` unless it is null (harris_box writes it from its own tile; in FAST mode boxsum9, without the shifted copy).  With
+// the selection below, the detection of svi_detect, of the dense path (LEFT) and of both sides of the sparse path.
 void launch_detector(svi_ctx* ctx, Lane& l, const uint8_t* d_img, const uint8_t* d_mask, const FrameGeom& g, int nf, uint16_t* box) {
     cudaStream_t s = l.stream;
     const dim3 tiles((g.W + HT_W - 1) / HT_W, (g.H + HT_H - 1) / HT_H, nf);
     if (ctx->p.detector == SVI_DETECTOR_FAST_9_16) {
         fast_candidates_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, d_mask, g, ctx->p.fast_threshold, ctx->p.fast_nonmax, l.cand,
                                                             l.cand_count, ctx->raw_cap);
-        boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, box, nullptr);
+        if (box) boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, box, nullptr);
     } else {
         harris_box_kernel<<<harris_grid(g.W, g.H, nf), HT_THREADS, sizeof(HarrisSmem), s>>>(
             d_img, d_mask, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, nullptr, box, nullptr, l.frame_max, l.cand,
@@ -649,14 +649,7 @@ int rectify_pair(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t
     uint8_t* dst[2] = {d_left, d_right};
     return launch_rectify(ctx, 2, cams, src, dst, pitch, stride, nf, s);
 }
-int rectify_one(svi_ctx* ctx, int cam, const uint8_t* raw, size_t pitch, size_t stride, uint8_t* d_out, int nf, cudaStream_t s) {
-    return launch_rectify(ctx, 1, &cam, &raw, &d_out, pitch, stride, nf, s);
-}
-
-}  // namespace
-
-// ---- per-query entry points: one image (or pair) staged in lane 0, queries in the call buffer ----
-namespace {
+// ---- image staging (DESIGN.md section 3): the only place where caller image and mask bytes go to the device
 // Page-locked caller memory (cudaMallocHost, cudaHostRegister, a pinned torch tensor: a camera driver's DMA buffers) is
 // read by the copy engine directly; anything else goes through the library's pinned mirror, because a cudaMemcpyAsync
 // from pageable memory is a blocking staged copy.  (One driver query per image, ~1 us; the mirror memcpy of a
@@ -667,31 +660,63 @@ bool host_is_pinned(const void* p) {
     return a.type == cudaMemoryTypeHost;
 }
 
-// One image of camera `cam` (0 = LEFT, 1 = RIGHT) into d_img plus its box sums.  While rectification is set the image is
-// raw: it goes up into lane 0's raw plane of that camera and rectify_kernel writes d_img.
-int stage_box(svi_ctx* ctx, const uint8_t* img, size_t pitch, uint8_t* d_img, uint16_t* d_box, uint16_t* d_box_shift,
-              cudaStream_t s, int cam, int pin_plane = 0) {
-    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
-    const size_t plane = (size_t)ctx->H * ctx->dev_pitch;
-    uint8_t* const d_rect = d_img;
-    if (ctx->rect) d_img = cam ? ctx->lanes[0].raw_r : ctx->lanes[0].raw_l;
-    if (host_is_pinned(img)) {
-        if ((int)pitch == ctx->dev_pitch) CK(cudaMemcpyAsync(d_img, img, plane, cudaMemcpyHostToDevice, s));
-        else CK(cudaMemcpy2DAsync(d_img, ctx->dev_pitch, img, pitch, ctx->W, ctx->H, cudaMemcpyHostToDevice, s));
-    } else if (ctx->pin && pin_plane >= 0 && (size_t)(pin_plane + 1) * plane <= ctx->pin_bytes) {
-        unsigned char* stage = ctx->pin + (size_t)pin_plane * plane;
-        if ((int)pitch == ctx->dev_pitch) std::memcpy(stage, img, plane);
-        else for (int y = 0; y < ctx->H; ++y) std::memcpy(stage + (size_t)y * ctx->dev_pitch, img + (size_t)y * pitch, ctx->W);
-        CK(cudaMemcpyAsync(d_img, stage, plane, cudaMemcpyHostToDevice, s));
+// nf planes of caller bytes (pitch bytes per row, frame_stride per frame) into the dense plane stack dst (dev_pitch per row,
+// H * dev_pitch per frame) on stream s.  A pageable source with a mirror slot (kSmallFrames planes of ctx->pin, slot k at
+// k * kSmallFrames planes) is packed into that slot and sent up with one copy; only calls that synchronise before they
+// return may pass a slot.  Anything else is copied straight from the caller, in as few copies as its layout allows.
+int upload_planes(svi_ctx* ctx, const uint8_t* src, size_t pitch, size_t frame_stride, int nf, uint8_t* dst, cudaStream_t s,
+                  int mirror_slot = -1) {
+    const int W = ctx->W, H = ctx->H, dp = ctx->dev_pitch;
+    const size_t plane = (size_t)H * dp;
+    if (mirror_slot >= 0 && ctx->pin && nf <= kSmallFrames && !host_is_pinned(src)) {
+        unsigned char* stage = ctx->pin + (size_t)mirror_slot * kSmallFrames * plane;
+        for (int f = 0; f < nf; ++f) {
+            const uint8_t* sf = src + (size_t)f * frame_stride;
+            if ((int)pitch == dp) std::memcpy(stage + f * plane, sf, plane);
+            else for (int y = 0; y < H; ++y) std::memcpy(stage + f * plane + (size_t)y * dp, sf + (size_t)y * pitch, W);
+        }
+        CK(cudaMemcpyAsync(dst, stage, nf * plane, cudaMemcpyHostToDevice, s));
+    } else if ((int)pitch == dp && (nf == 1 || frame_stride == plane)) {
+        CK(cudaMemcpyAsync(dst, src, nf * plane, cudaMemcpyHostToDevice, s));
+    } else if (frame_stride == pitch * H) {
+        CK(cudaMemcpy2DAsync(dst, dp, src, pitch, W, (size_t)H * nf, cudaMemcpyHostToDevice, s));
     } else {
-        CK(cudaMemcpy2DAsync(d_img, ctx->dev_pitch, img, pitch, ctx->W, ctx->H, cudaMemcpyHostToDevice, s));
+        for (int f = 0; f < nf; ++f)
+            CK(cudaMemcpy2DAsync(dst + f * plane, dp, src + (size_t)f * frame_stride, pitch, W, H, cudaMemcpyHostToDevice, s));
     }
-    if (ctx->rect) {
-        const int rc = rectify_one(ctx, cam, d_img, ctx->dev_pitch, plane, d_rect, 1, s);
+    return SVI_SUCCESS;
+}
+
+// Where caller bytes of camera `cam` (0 = LEFT, 1 = RIGHT) land on lane l: its raw plane of that camera while
+// rectification is set (rectify_kernel then writes dst), dst itself otherwise.
+uint8_t* landing(const svi_ctx* ctx, Lane& l, int cam, uint8_t* dst) { return !ctx->rect ? dst : cam ? l.raw_r : l.raw_l; }
+
+// The images of n_cams cameras cams[i] (nf frames each, one layout) into the dense plane stacks dst[i] of lane l: uploaded
+// to their landing planes, then, while rectification is set, one rectify_kernel launch for all of them.
+int stage_images(svi_ctx* ctx, Lane& l, int n_cams, const int* cams, const uint8_t* const* src, uint8_t* const* dst, size_t pitch,
+                 size_t frame_stride, int nf, cudaStream_t s, int mirror_slot = -1) {
+    uint8_t* land[2];
+    for (int i = 0; i < n_cams; ++i) {
+        land[i] = landing(ctx, l, cams[i], dst[i]);
+        const int rc = upload_planes(ctx, src[i], pitch, frame_stride, nf, land[i], s, mirror_slot < 0 ? -1 : mirror_slot + i);
         if (rc != SVI_SUCCESS) return rc;
     }
+    if (!ctx->rect) return SVI_SUCCESS;
+    return launch_rectify(ctx, n_cams, cams, land, dst, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch, nf, s);
+}
+
+}  // namespace
+
+// ---- per-query entry points: one image (or pair) staged in lane 0, queries in the call buffer ----
+namespace {
+// One image of camera `cam` into d_img plus its box sums, on lane 0 (stream s may be the side stream).
+int stage_box(svi_ctx* ctx, const uint8_t* img, size_t pitch, uint8_t* d_img, uint16_t* d_box, uint16_t* d_box_shift,
+              cudaStream_t s, int cam, int mirror_slot = 0) {
+    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
+    const int rc = stage_images(ctx, ctx->lanes[0], 1, &cam, &img, &d_img, pitch, pitch * ctx->H, 1, s, mirror_slot);
+    if (rc != SVI_SUCCESS) return rc;
     const dim3 tiles((g.W + HT_W - 1) / HT_W, (g.H + HT_H - 1) / HT_H, 1);
-    boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_rect, g, d_box, d_box_shift);
+    boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, d_box, d_box_shift);
     CK(cudaGetLastError());
     return SVI_SUCCESS;
 }
@@ -747,12 +772,22 @@ int call_fetch(svi_ctx* ctx, size_t begin, size_t end, cudaStream_t s) {
     return SVI_SUCCESS;
 }
 
-// Declared first in every user of the buffer: a call that fails part-way still leaves lane 0 idle, so that the next
-// call may overwrite the mirror.  The successful path ends in a synchronisation of its own and sets `done`.
+// Declared first in every user of the buffer, of the image mirror and of caller buffers read by queued copies: a call that
+// fails part-way still leaves its streams idle -- `s` (lane 0), the side stream if given, every lane of `lanes_of` if given --
+// so that the next call may overwrite the mirrors and nothing queued touches the caller's buffers after the call returned.
+// The successful path ends in a synchronisation of its own and sets `done`.
 struct SyncOnFailure {
     cudaStream_t s;
+    cudaStream_t side = nullptr;
+    const svi_ctx* lanes_of = nullptr;
     bool done = false;
-    ~SyncOnFailure() { if (!done) cudaStreamSynchronize(s); }
+    ~SyncOnFailure() {
+        if (done) return;
+        if (s) cudaStreamSynchronize(s);
+        if (side) cudaStreamSynchronize(side);
+        if (lanes_of)
+            for (int i = 0; i < lanes_of->n_lanes; ++i) cudaStreamSynchronize(lanes_of->lanes[i].stream);
+    }
 };
 
 // svi_landmarks of n landmarks, with or without the three stage-3 arrays
@@ -865,45 +900,27 @@ int build_mask(svi_ctx* ctx, Lane& l, const float* centres, int n_centres) {
 // (getMaskActiveLandmarks, CFundamentalMatcher.cpp:2043-2073): 8 bytes per landmark go up instead of a W x H plane.
 int small_call(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride, int n_frames,
                const uint8_t* masks, const float* centres, int n_centres, svi_stereo_result* out) {
-    const int W = ctx->W, H = ctx->H, MC = ctx->p.max_corners, cap = out->capacity_per_frame;
+    const int H = ctx->H, MC = ctx->p.max_corners, cap = out->capacity_per_frame;
     const size_t dstride = (size_t)H * ctx->dev_pitch;
     const FrameGeom g = make_geom(ctx, ctx->dev_pitch, dstride);
     {
         Lane& l = ctx->lanes[0];
         cudaStream_t s = l.stream;
         const int nf = n_frames;
-        const size_t plane = dstride * nf;
-        unsigned char* pin_in = ctx->pin;
         unsigned char* pin_out = ctx->pin + ((3 * (size_t)kSmallFrames * dstride + 15) & ~size_t(15));
         // upload order LEFT, mask, RIGHT: the detector starts as soon as LEFT (and the mask) is there; RIGHT goes up on the
         // side stream and its box sums run beside the detector (not while profiling: stage events live on one stream)
         cudaStream_t side = ctx->profiling ? nullptr : ctx->side;
+        SyncOnFailure idle{s, side};
         if (side) {   // whatever is still queued on the lane (an un-synchronised device-resident batch) uses the same scratch
             CK(cudaEventRecord(ctx->fork, s));
             CK(cudaStreamWaitEvent(side, ctx->fork, 0));
         }
+        // plane k goes through mirror slot k when it is pageable
         const uint8_t* srcs[3] = {left, masks, right};
-        uint8_t* dsts[3] = {ctx->rect ? l.raw_l : l.img_l, l.mask, ctx->rect ? l.raw_r : l.img_r};
+        uint8_t* dsts[3] = {landing(ctx, l, 0, l.img_l), l.mask, landing(ctx, l, 1, l.img_r)};
         auto upload_plane = [&](int k, cudaStream_t sk) -> int {
-            if (!srcs[k]) return SVI_SUCCESS;
-            if (host_is_pinned(srcs[k])) {   // the caller's buffer is page-locked: DMA straight from it
-                if ((int)pitch == ctx->dev_pitch && (nf == 1 || frame_stride == dstride)) {
-                    CK(cudaMemcpyAsync(dsts[k], srcs[k], plane, cudaMemcpyHostToDevice, sk));
-                } else {
-                    for (int f = 0; f < nf; ++f)
-                        CK(cudaMemcpy2DAsync(dsts[k] + f * dstride, ctx->dev_pitch, srcs[k] + (size_t)f * frame_stride, pitch, W, H,
-                                             cudaMemcpyHostToDevice, sk));
-                }
-                return SVI_SUCCESS;
-            }
-            unsigned char* stage = pin_in + k * (size_t)kSmallFrames * dstride;
-            for (int f = 0; f < nf; ++f) {
-                const uint8_t* src = srcs[k] + (size_t)f * frame_stride;
-                if ((int)pitch == ctx->dev_pitch) std::memcpy(stage + f * dstride, src, dstride);
-                else for (int y = 0; y < H; ++y) std::memcpy(stage + f * dstride + (size_t)y * ctx->dev_pitch, src + (size_t)y * pitch, W);
-            }
-            CK(cudaMemcpyAsync(dsts[k], stage, plane, cudaMemcpyHostToDevice, sk));
-            return SVI_SUCCESS;
+            return srcs[k] ? upload_planes(ctx, srcs[k], pitch, frame_stride, nf, dsts[k], sk, k) : SVI_SUCCESS;
         };
         for (int k = 0; k < 2; ++k) {
             const int rc = upload_plane(k, s);
@@ -914,7 +931,7 @@ int small_call(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t p
             // raw images: RIGHT goes up on the side stream beside LEFT, one launch rectifies both into img_l / img_r, and the
             // RIGHT box sums still run on the side stream beside the detector
             const int rc = upload_plane(2, side ? side : s);
-            if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); if (side) cudaStreamSynchronize(side); return rc; }
+            if (rc != SVI_SUCCESS) return rc;
             if (side) {
                 CK(cudaEventRecord(ctx->side_done, side));
                 CK(cudaStreamWaitEvent(s, ctx->side_done, 0));
@@ -934,10 +951,11 @@ int small_call(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t p
         }
         int rc = run_pipeline(ctx, l, l.img_l, l.img_r, have_mask ? l.mask : nullptr, g, nf, ctx->small_out, 0, ctx->small_n_kp, ctx->small_n_det, side,
                               ctx->rect ? nullptr : &upload_right);
-        if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); if (side) cudaStreamSynchronize(side); return rc; }
+        if (rc != SVI_SUCCESS) return rc;
         // one copy brings the whole result block back; only the live slots are scattered to the caller's arrays
         CK(cudaMemcpyAsync(pin_out, ctx->small_block, ctx->small_bytes, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
+        idle.done = true;   // the side stream joined lane 0's before the matcher
         const StereoOutDev& so = ctx->small_out;
         auto host = [&](const void* d) { return pin_out + (static_cast<const unsigned char*>(d) - ctx->small_block); };
         const int* pin_kp = reinterpret_cast<const int*>(host(ctx->small_n_kp));
@@ -1121,14 +1139,16 @@ int stage_track_pair(svi_ctx* ctx, const uint8_t* img_left, const uint8_t* img_r
     cudaStream_t s = l.stream;
     const size_t plane = (size_t)ctx->H * ctx->dev_pitch;
     // both images as planes 0 / 1 of one buffer (the window-mode detector indexes them by plane)
+    SyncOnFailure idle{s, ctx->side};
     CK(cudaEventRecord(ctx->fork, s));
     CK(cudaStreamWaitEvent(ctx->side, ctx->fork, 0));
     int rc = stage_box(ctx, img_right, pitch, ctx->trk_img + plane, l.box_r, l.box_rs, ctx->side, 1, 1);
-    if (rc == SVI_SUCCESS) rc = stage_box(ctx, img_left, pitch, ctx->trk_img, l.box_l, l.box_ls, s, 0);
-    if (cudaEventRecord(ctx->side_done, ctx->side) != cudaSuccess || cudaStreamWaitEvent(s, ctx->side_done, 0) != cudaSuccess)
-        rc = rc == SVI_SUCCESS ? fail(ctx, SVI_ERR_CUDA, "svi_track_landmarks: joining the side stream failed") : rc;
-    if (rc != SVI_SUCCESS) { cudaStreamSynchronize(ctx->side); cudaStreamSynchronize(s); }
-    return rc;
+    if (rc != SVI_SUCCESS) return rc;
+    if ((rc = stage_box(ctx, img_left, pitch, ctx->trk_img, l.box_l, l.box_ls, s, 0)) != SVI_SUCCESS) return rc;
+    CK(cudaEventRecord(ctx->side_done, ctx->side));
+    CK(cudaStreamWaitEvent(s, ctx->side_done, 0));
+    idle.done = true;   // the callers synchronise lane 0's stream, which now waits for the side stream
+    return SVI_SUCCESS;
 }
 
 // The tracking cascade restricted to stage_mask on n device-resident landmarks whose outputs `o` are zeroed, entirely enqueued on
@@ -1193,41 +1213,28 @@ cudaError_t d2h_slots(void* dst, const void* src, size_t elem, int MC, int cap, 
     return cudaMemcpy2DAsync(d, (size_t)cap * elem, src, (size_t)MC * elem, (size_t)MC * elem, nf, cudaMemcpyDeviceToHost, s);
 }
 
-// Host buffers: chunk c on lane c % n_lanes; its images (and masks) go straight from the caller's buffers into the lane's
-// staging (raw planes first while rectification is set), `run` enqueues the kernels on the lane's planes, the slot arrays and
-// counts come back into the caller's arrays, `fetch` (may be null) adds the entry point's own; one synchronisation at the end.
+// Host buffers: chunk c on lane c % n_lanes; its masks and images go straight from the caller's buffers into the lane's
+// staging (stage_images), `run` enqueues the kernels on the lane's planes, the slot arrays and counts come back into the
+// caller's arrays, `fetch` (may be null) adds the entry point's own; one synchronisation at the end.
 using HostChunkFn = std::function<int(Lane&, const FrameGeom&, int f0, int nf)>;
 int host_frames(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t pitch, size_t frame_stride, int n_frames,
                 const uint8_t* masks, svi_stereo_result* out, const HostChunkFn& run, const HostChunkFn& fetch) {
-    const int W = ctx->W, H = ctx->H, MC = ctx->p.max_corners, cap = out->capacity_per_frame;
-    const size_t dstride = (size_t)H * ctx->dev_pitch;
-    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, dstride);
-    const bool dense = (frame_stride == pitch * (size_t)H);
+    const int MC = ctx->p.max_corners, cap = out->capacity_per_frame;
+    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
+    SyncOnFailure idle{nullptr, nullptr, ctx};
     int chunk_id = 0;
     for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk, ++chunk_id) {
         Lane& l = ctx->lanes[chunk_id % ctx->n_lanes];
         cudaStream_t s = l.stream;
         const int nf = std::min(ctx->chunk, n_frames - f0);
-        const uint8_t* srcs[3] = {left, right, masks};
-        uint8_t* dsts[3] = {ctx->rect ? l.raw_l : l.img_l, ctx->rect ? l.raw_r : l.img_r, l.mask};
-        for (int k = 0; k < 3; ++k) {
-            if (!srcs[k]) continue;
-            if (dense && (int)pitch == ctx->dev_pitch) {
-                CK(cudaMemcpyAsync(dsts[k], srcs[k] + (size_t)f0 * frame_stride, (size_t)nf * frame_stride, cudaMemcpyHostToDevice, s));
-            } else if (dense) {
-                CK(cudaMemcpy2DAsync(dsts[k], ctx->dev_pitch, srcs[k] + (size_t)f0 * frame_stride, pitch, W, (size_t)H * nf,
-                                     cudaMemcpyHostToDevice, s));
-            } else {
-                for (int f = 0; f < nf; ++f)
-                    CK(cudaMemcpy2DAsync(dsts[k] + f * dstride, ctx->dev_pitch, srcs[k] + (size_t)(f0 + f) * frame_stride,
-                                         pitch, W, H, cudaMemcpyHostToDevice, s));
-            }
-        }
-        if (ctx->rect) {
-            const int rr = rectify_pair(ctx, l.raw_l, l.raw_r, ctx->dev_pitch, dstride, l.img_l, l.img_r, nf, s);
-            if (rr != SVI_SUCCESS) return rr;
-        }
-        int rc = run(l, g, f0, nf);
+        const size_t o = (size_t)f0 * frame_stride;
+        int rc = masks ? upload_planes(ctx, masks + o, pitch, frame_stride, nf, l.mask, s) : SVI_SUCCESS;
+        if (rc != SVI_SUCCESS) return rc;
+        const int cams[2] = {0, 1};
+        const uint8_t* srcs[2] = {left + o, right + o};
+        uint8_t* dsts[2] = {l.img_l, l.img_r};
+        if ((rc = stage_images(ctx, l, 2, cams, srcs, dsts, pitch, frame_stride, nf, s)) != SVI_SUCCESS) return rc;
+        rc = run(l, g, f0, nf);
         if (rc != SVI_SUCCESS) return rc;
         CK(d2h_slots(out->uv_left, l.out.uv_l, 2 * sizeof(float), MC, cap, f0, nf, s));
         CK(d2h_slots(out->uv_right, l.out.uv_r, 2 * sizeof(float), MC, cap, f0, nf, s));
@@ -1243,6 +1250,7 @@ int host_frames(svi_ctx* ctx, const uint8_t* left, const uint8_t* right, size_t 
     }
     int rc = sync_lanes(ctx);
     if (rc != SVI_SUCCESS) return rc;
+    idle.done = true;
     return check_overflow(ctx);
 }
 
@@ -1795,12 +1803,11 @@ int svi_harris_response(svi_ctx* ctx, const uint8_t* img, size_t pitch, float* r
     CK(cudaSetDevice(ctx->device));
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
+    SyncOnFailure idle{s};
     const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
-    CK(cudaMemcpy2DAsync(ctx->rect ? l.raw_l : l.img_l, ctx->dev_pitch, img, pitch, ctx->W, ctx->H, cudaMemcpyHostToDevice, s));
-    if (ctx->rect) {
-        const int rc = rectify_one(ctx, 0, l.raw_l, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch, l.img_l, 1, s);
-        if (rc != SVI_SUCCESS) return rc;
-    }
+    const int cam = 0;
+    const int rc = stage_images(ctx, l, 1, &cam, &img, &l.img_l, pitch, pitch * ctx->H, 1, s, 0);
+    if (rc != SVI_SUCCESS) return rc;
     CK(cudaMemsetAsync(l.frame_max, 0, sizeof(uint32_t), s));
     if (!ctx->resp_one) CK(dmalloc(&ctx->resp_one, (size_t)ctx->H * ctx->resp_pitch));
     harris_box_kernel<<<harris_grid(g.W, g.H, 1), HT_THREADS, sizeof(HarrisSmem), s>>>(
@@ -1810,6 +1817,7 @@ int svi_harris_response(svi_ctx* ctx, const uint8_t* img, size_t pitch, float* r
     CK(cudaMemcpy2DAsync(response, sizeof(float) * ctx->W, ctx->resp_one, sizeof(float) * ctx->resp_pitch, sizeof(float) * ctx->W,
                          ctx->H, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
+    idle.done = true;
     return SVI_SUCCESS;
 }
 
@@ -1820,44 +1828,20 @@ int svi_detect(svi_ctx* ctx, const uint8_t* img, size_t pitch, size_t frame_stri
     CK(cudaSetDevice(ctx->device));
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
-    const int W = ctx->W, H = ctx->H, MC = ctx->p.max_corners;
-    const size_t dstride = (size_t)H * ctx->dev_pitch;
-    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, dstride);
+    SyncOnFailure idle{s};
+    const int MC = ctx->p.max_corners, cam = 0;
+    const FrameGeom g = make_geom(ctx, ctx->dev_pitch, (size_t)ctx->H * ctx->dev_pitch);
     std::vector<ushort2> h_xy((size_t)ctx->chunk * MC);
     for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk) {
         const int nf = std::min(ctx->chunk, n_frames - f0);
-        for (int f = 0; f < nf; ++f) {
-            CK(cudaMemcpy2DAsync((ctx->rect ? l.raw_l : l.img_l) + f * dstride, ctx->dev_pitch, img + (size_t)(f0 + f) * frame_stride, pitch, W, H,
-                                 cudaMemcpyHostToDevice, s));
-            if (masks)
-                CK(cudaMemcpy2DAsync(l.mask + f * dstride, ctx->dev_pitch, masks + (size_t)(f0 + f) * frame_stride, pitch, W, H,
-                                     cudaMemcpyHostToDevice, s));
-        }
-        if (ctx->rect) {
-            const int rc = rectify_one(ctx, 0, l.raw_l, ctx->dev_pitch, dstride, l.img_l, nf, s);
-            if (rc != SVI_SUCCESS) return rc;
-        }
-        const uint8_t* d_mask = masks ? l.mask : nullptr;
+        const uint8_t* src = img + (size_t)f0 * frame_stride;
+        int rc = masks ? upload_planes(ctx, masks + (size_t)f0 * frame_stride, pitch, frame_stride, nf, l.mask, s) : SVI_SUCCESS;
+        if (rc != SVI_SUCCESS) return rc;
+        if ((rc = stage_images(ctx, l, 1, &cam, &src, &l.img_l, pitch, frame_stride, nf, s)) != SVI_SUCCESS) return rc;
         CK(cudaMemsetAsync(l.frame_max, 0, sizeof(uint32_t) * nf, s));
         CK(cudaMemsetAsync(l.cand_count, 0, sizeof(int) * nf, s));
-        const dim3 tiles((W + HT_W - 1) / HT_W, (H + HT_H - 1) / HT_H, nf);
-        const bool fast = ctx->p.detector == SVI_DETECTOR_FAST_9_16;
-        if (fast) {
-            fast_candidates_kernel<<<tiles, HT_THREADS, 0, s>>>(l.img_l, d_mask, g, ctx->p.fast_threshold, ctx->p.fast_nonmax, l.cand,
-                                                                l.cand_count, ctx->raw_cap);
-        } else {
-            harris_box_kernel<<<harris_grid(W, H, nf), HT_THREADS, sizeof(HarrisSmem), s>>>(
-                l.img_l, d_mask, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, nullptr, nullptr, nullptr, l.frame_max, l.cand,
-                l.cand_count, ctx->raw_cap, nullptr, nullptr, g.H);
-        }
-        const uint32_t* fmax = fast ? nullptr : l.frame_max;
-        if (ctx->select_smem)
-            select_corners_kernel<true><<<nf, SEL_THREADS, 13 * SEL_SMEM_KEYS, s>>>(l.cand, l.cand_count, fmax, ctx->sel, nullptr, nullptr,
-                                                                                  nullptr, l.det_xy, l.n_det, l.kp_xy, l.n_kp,
-                                                                                  ctx->d_overflow, nullptr);
-        else
-            select_corners_kernel<false><<<nf, SEL_THREADS, 4 * SEL_SMEM_CELLS, s>>>(l.cand, l.cand_count, fmax, ctx->sel, l.g_head, l.g_next, l.g_state,
-                                                                   l.det_xy, l.n_det, l.kp_xy, l.n_kp, ctx->d_overflow, nullptr);
+        launch_detector(ctx, l, l.img_l, masks ? l.mask : nullptr, g, nf, nullptr);
+        launch_select(ctx, l, nf, l.det_xy, l.n_det, l.kp_xy, l.n_kp);
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(h_xy.data(), l.det_xy, sizeof(ushort2) * (size_t)nf * MC, cudaMemcpyDeviceToHost, s));
         CK(cudaMemcpyAsync(counts + f0, l.n_det, sizeof(int) * nf, cudaMemcpyDeviceToHost, s));
@@ -1868,6 +1852,7 @@ int svi_detect(svi_ctx* ctx, const uint8_t* img, size_t pitch, size_t frame_stri
                 xy[((size_t)(f0 + f) * MC + i) * 2 + 1] = (float)h_xy[(size_t)f * MC + i].y;
             }
     }
+    idle.done = true;
     return check_overflow(ctx);
 }
 
@@ -2443,19 +2428,17 @@ int svi_rectify(svi_ctx* ctx, int side, const uint8_t* raw, size_t pitch, size_t
     CK(cudaSetDevice(ctx->device));
     Lane& l = ctx->lanes[0];
     cudaStream_t s = l.stream;
-    const size_t dstride = (size_t)ctx->H * ctx->dev_pitch;
-    uint8_t* d_raw = side ? l.raw_r : l.raw_l;
+    SyncOnFailure idle{s};
     for (int f0 = 0; f0 < n_frames; f0 += ctx->chunk) {
         const int nf = std::min(ctx->chunk, n_frames - f0);
-        for (int f = 0; f < nf; ++f)
-            CK(cudaMemcpy2DAsync(d_raw + f * dstride, ctx->dev_pitch, raw + (size_t)(f0 + f) * frame_stride, pitch, ctx->W, ctx->H,
-                                 cudaMemcpyHostToDevice, s));
-        const int rc = rectify_one(ctx, side, d_raw, ctx->dev_pitch, dstride, l.img_l, nf, s);
-        if (rc != SVI_SUCCESS) { cudaStreamSynchronize(s); return rc; }
+        const uint8_t* src = raw + (size_t)f0 * frame_stride;
+        const int rc = stage_images(ctx, l, 1, &side, &src, &l.img_l, pitch, frame_stride, nf, s);
+        if (rc != SVI_SUCCESS) return rc;
         CK(cudaMemcpy2DAsync(out + (size_t)f0 * ctx->H * out_pitch, out_pitch, l.img_l, ctx->dev_pitch, ctx->W, (size_t)ctx->H * nf,
                              cudaMemcpyDeviceToHost, s));
     }
     CK(cudaStreamSynchronize(s));
+    idle.done = true;
     return check_overflow(ctx);
 }
 

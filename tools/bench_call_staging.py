@@ -6,8 +6,10 @@ Each round runs one worker process per build (SVI_GPU_LIB selects the build), th
 A worker times --calls synchronous calls of each entry point (after 20 warm-up calls) on one context and reports the medians:
 describe and triangulate_right / triangulate_left at n = 1 and n = 1000, track_landmarks on a C3 landmark state (all stages),
 stereo_frame_masked with the state's landmark centres, optimize_landmarks (1000 landmarks, 6 measurements each),
-solve_stereo_posit (1000 measurements) and track_frame_stereo_only on the same state.  The inputs are seeded and shared by both
-builds; every worker's outputs are hashed, and the hashes of A and B must agree.  The run-to-run spread of a build is the range
+solve_stereo_posit (1000 measurements) and track_frame_stereo_only on the same state, and the image staging of the one- and
+two-pair calls: stereo_frames of one pair from pageable and from page-locked memory, of two pairs with padded rows, harris_response,
+detect and rectify of one frame.  The inputs are seeded and shared by both builds; every worker's outputs are hashed (the
+RIGHT-side fields of an unmatched key-point left out), and the hashes of A and B must agree.  The run-to-run spread of a build is the range
 of its round medians over their median.  Writes DIR/call_staging.json (and prints a summary), with the card's name and power
 limit read in the same run."""
 from __future__ import annotations
@@ -55,7 +57,7 @@ def make_inputs(path: pathlib.Path):
     xy = np.stack([rng.integers(28, W - 28, 1000), rng.integers(28, H - 28, 1000)], 1).astype(np.float32)
     opt = _optimize_args(cams, 1000, 6, rng)
     posit = _posit_args(cams, 1000, rng)
-    d = dict(L=L[8], R=R[8], T=T[8], T_prev=T[7], xy=xy, desc=rng.integers(0, 256, (1000, 32), dtype=np.uint8),
+    d = dict(L=L[8], R=R[8], L_prev=L[7], R_prev=R[7], T=T[8], T_prev=T[7], xy=xy, desc=rng.integers(0, 256, (1000, 32), dtype=np.uint8),
              search=rng.uniform(0.5, 90.0, 1000).astype(np.float32), **{"st_" + k: v for k, v in st.items()},
              **{f"opt_{i}": v for i, v in enumerate(opt)}, **{f"posit_{i}": v for i, v in enumerate(posit)})
     np.savez(path, **d)
@@ -63,8 +65,10 @@ def make_inputs(path: pathlib.Path):
 
 
 def worker(inputs: str, calls: int):
+    import torch
     from svi_mapper_b200 import StereoFrontend
-    from test_call_buffer import _flat
+    from svi_mapper_b200.frontend import StereoFrames
+    from test_image_staging import _flat
     d = dict(np.load(inputs))
     st = {k[3:]: v for k, v in d.items() if k.startswith("st_")}
     n_lm = len(st["uid"])
@@ -74,8 +78,25 @@ def worker(inputs: str, calls: int):
     tl_r = np.stack([np.maximum(0, xy[:, 0] - 28 - search), xy[:, 1] - 28], 1).astype(np.float32)
     tl_l = np.stack([xy[:, 0] - 28, xy[:, 1] - 28], 1).astype(np.float32)
     centres = np.ascontiguousarray(st["uv_ref"].astype(np.float32))
-    with StereoFrontend(*_cams()) as fe:
-        entries = {}
+    H, W = L.shape
+    pinned = torch.from_numpy(np.stack([L, R])).pin_memory()
+    pad = np.random.default_rng(5).integers(0, 256, (2, 2, H + 2, W + 13), dtype=np.uint8)   # [side, frame], garbage in the padding
+    pad[0, :, :H, :W] = d["L_prev"], L
+    pad[1, :, :H, :W] = d["R_prev"], R
+    with StereoFrontend(*_cams()) as fe, StereoFrontend(*_cams()) as fr:
+        fr.set_rectification(*_cams())
+        two = StereoFrames.empty(2, fe.max_corners)
+        two_r = two.result()
+
+        def two_padded():
+            fe.stereo_frames_raw(pad[0].ctypes.data, pad[1].ctypes.data, W + 13, (H + 2) * (W + 13), 2, two_r)
+            return two
+        entries = {"stereo_frames 1 pair pageable": lambda: fe.stereo_frames(L, R),
+                   "stereo_frames 1 pair page-locked": lambda: fe.stereo_frames(pinned[0].numpy(), pinned[1].numpy()),
+                   "stereo_frames 2 pairs padded rows": two_padded,
+                   "harris_response": lambda: fe.harris_response(L),
+                   "detect 1 frame": lambda: fe.detect(L),
+                   "rectify 1 frame": lambda: fr.rectify(L, 0)}
         for n in (1, 1000):
             entries[f"describe n={n}"] = lambda n=n: fe.describe(L, xy[:n])
             entries[f"triangulate_right n={n}"] = lambda n=n: fe.triangulate_right(R, tl_r[:n], xy[:n], desc[:n])
