@@ -97,6 +97,7 @@ def load(native=False):
     lib.svo_gftt_roi.argtypes = [vp, ci, ci, ci, ci, ci, ci, ci, ci, C.c_double, C.c_double, C.c_double, vp, ci]
     lib.svo_track_params_default.argtypes = [C.POINTER(TrackParams)]
     lib.svo_optimize_landmark.argtypes = [vp, ci, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.svo_solve_stereo_posit.argtypes = [vp, vp, vp, vp, vp, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.svo_track_landmarks.argtypes = [C.POINTER(Config), C.POINTER(TrackParams), vp, vp, ci, vp, C.POINTER(Landmarks), ci, C.c_double,
                                         C.c_uint, C.POINTER(TrackResult), ci]
     _libs[key] = lib
@@ -242,3 +243,26 @@ def optimize_landmark(xyz_guess, measurements, native=False) -> dict:
                                             outcome.ctypes.data, avg.ctypes.data, iters.ctypes.data)
     assert rc == 0
     return dict(xyz=xyz, outcome=int(outcome[0]), average_squared_error=float(avg[0]), iterations=int(iters[0]))
+
+
+def solve_stereo_posit(P_left, P_right, xyz_world, uv_left, uv_right, T_estimate, T_last=None, t_imu=None, native=False) -> dict:
+    """svo_solve_stereo_posit: CSolverStereoPosit::getTransformationWORLDtoLEFT for one frame's measurements (xyz_world (n, 3)
+    float64, uv_left / uv_right (n, 2) float32) from the prior T_estimate; the same arguments (plus the two 3 x 4 projection
+    matrices) and result keys as StereoFrontend.solve_stereo_posit, minus `reason`.  T_last defaults to T_estimate, t_imu to zero."""
+    P = [np.ascontiguousarray(np.asarray(m, np.float64).reshape(12)) for m in (P_left, P_right)]
+    xw = np.ascontiguousarray(np.asarray(xyz_world, np.float64).reshape(-1, 3))
+    n = len(xw)
+    ul = np.ascontiguousarray(np.asarray(uv_left, np.float32).reshape(n, 2))
+    ur = np.ascontiguousarray(np.asarray(uv_right, np.float32).reshape(n, 2))
+    Te = np.ascontiguousarray(np.asarray(T_estimate, np.float64).reshape(16))
+    Tl = Te if T_last is None else np.ascontiguousarray(np.asarray(T_last, np.float64).reshape(16))
+    ti = np.zeros(3) if t_imu is None else np.ascontiguousarray(np.asarray(t_imu, np.float64).reshape(3))
+    T = np.zeros(16, np.float64)
+    outcome, iters, inliers = np.zeros(1, np.int32), np.zeros(1, np.int32), np.zeros(1, np.int32)
+    avg, risk = np.zeros(1, np.float64), np.zeros(1, np.float64)
+    rc = load(native).svo_solve_stereo_posit(P[0].ctypes.data, P[1].ctypes.data, Te.ctypes.data, Tl.ctypes.data, ti.ctypes.data, n, xw.ctypes.data,
+                                             ul.ctypes.data, ur.ctypes.data, T.ctypes.data, outcome.ctypes.data, iters.ctypes.data,
+                                             inliers.ctypes.data, avg.ctypes.data, risk.ctypes.data)
+    assert rc == 0
+    return dict(T=T.reshape(4, 4), outcome=int(outcome[0]), iterations=int(iters[0]), inliers=int(inliers[0]),
+                average_squared_error=float(avg[0]), risk=float(risk[0]))

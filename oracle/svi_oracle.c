@@ -1058,3 +1058,144 @@ int svo_optimize_landmark(const double* xyz_guess, int m, const double* proj_lef
     *outcome = 4;
     return 0;
 }
+
+/* ---- CSolverStereoPosit::getTransformationWORLDtoLEFT (src/optimization/CSolverStereoPosit.cpp:8-170): robust Gauss-Newton on
+ * the four-dimensional stereo re-projection error of the WORLD->LEFT pose, constants of CSolverStereoPosit.h:89-99.  Written
+ * from the reference's loop: per measurement the transform into the LEFT frame (points with z <= 0 contribute nothing but still
+ * count in the average), both projections, the error, the robust weight, the 4 x 6 Jacobian of the increment (translation,
+ * quaternion vector part of CMiniVisionToolbox::getTransformationFromVector, src/vision/CMiniVisionToolbox.cpp:354-377) and the
+ * accumulation of the normal equations; then H dx = -b by Gaussian elimination with partial pivoting, the pose update
+ * T = T(dx) * T, the re-orthonormalisation R -= 0.5 R (R^T R - I), and at convergence (1e-5 on the total weighted error) the
+ * accuracy verdict, the translation clamp against T_last and the risk test against the prior's position plus t_imu.
+ * Every sum runs in measurement order and every operation rounds on its own (-ffp-contract=off), so the result is the C++ host
+ * layer's (host/CSolverStereoPosit.h) to the last bit.
+ * P_left / P_right / T_estimate / T_last row-major (3 x 4, 4 x 4); n measurements: xyz_world n x 3, uv_left / uv_right n x 2.
+ * Outputs as svi_posit_result: T_out = the solution for outcome 0, else T_estimate; outcome 0 ok / 1 too few points (n <= 25) /
+ * 2 inaccurate / 3 high risk / 4 not converged in 1000 iterations; iterations run (0 for 1); inliers of the last iteration;
+ * average_squared_error of the converged iteration (else 0); risk (0 unless the risk test ran). */
+static void svo_iso_mul(const double* A, const double* B, double* C) {   /* Isometry3d * Isometry3d: bottom row (0 0 0 1) */
+    for (int k = 0; k < 16; ++k) C[k] = (k % 5 == 0) ? 1.0 : 0.0;
+    for (int r = 0; r < 3; ++r)
+        for (int c = 0; c < 4; ++c) {
+            double s = 0.0;
+            for (int k = 0; k < 3; ++k) s += A[4 * r + k] * B[4 * k + c];
+            C[4 * r + c] = s + (c == 3 ? A[4 * r + 3] : 0.0);
+        }
+}
+
+static void svo_posit_rows(const double* P, const double a[3], double c, const double Jt[3][6], double* rowU, double* rowV) {
+    for (int k = 0; k < 6; ++k) {
+        double PJ[3];
+        for (int r = 0; r < 3; ++r) PJ[r] = P[4 * r] * Jt[0][k] + P[4 * r + 1] * Jt[1][k] + P[4 * r + 2] * Jt[2][k];
+        rowU[k] = PJ[0] / c - a[0] / (c * c) * PJ[2];
+        rowV[k] = PJ[1] / c - a[1] / (c * c) * PJ[2];
+    }
+}
+
+static void svo_posit_solve(const double H[6][6], const double b[6], double x[6]) {
+    double A[6][7];
+    for (int i = 0; i < 6; ++i) { for (int j = 0; j < 6; ++j) A[i][j] = H[i][j]; A[i][6] = -b[i]; }
+    for (int c = 0; c < 6; ++c) {
+        int piv = c;
+        for (int r = c + 1; r < 6; ++r) if (fabs(A[r][c]) > fabs(A[piv][c])) piv = r;
+        if (piv != c) for (int j = 0; j < 7; ++j) { const double t = A[c][j]; A[c][j] = A[piv][j]; A[piv][j] = t; }
+        for (int r = c + 1; r < 6; ++r) {
+            const double f = A[r][c] / A[c][c];
+            for (int j = c; j < 7; ++j) A[r][j] -= f * A[c][j];
+        }
+    }
+    for (int r = 5; r >= 0; --r) {
+        double s = A[r][6];
+        for (int j = r + 1; j < 6; ++j) s -= A[r][j] * x[j];
+        x[r] = s / A[r][r];
+    }
+}
+
+int svo_solve_stereo_posit(const double* P_left, const double* P_right, const double* T_estimate, const double* T_last, const double* t_imu,
+                           int n, const double* xyz_world, const float* uv_left, const float* uv_right, double* T_out, int32_t* outcome,
+                           int32_t* iterations, int32_t* inliers_out, double* average_squared_error, double* risk_out) {
+    const double kernel = 10.0, max_avg = 9.0, max_risk = 2.0, delta = 1e-5, min_t2 = 0.001;
+    const int min_points = 25, min_inliers = 15, cap = 1000;
+    memcpy(T_out, T_estimate, 16 * sizeof(double));
+    *iterations = 0; *inliers_out = 0; *average_squared_error = 0.0; *risk_out = 0.0;
+    if (!(min_points < n)) { *outcome = 1; return 0; }
+    double T[16];
+    memcpy(T, T_estimate, sizeof(T));
+    double prev = 0.0;
+    for (int it = 0; it < cap; ++it) {
+        double H[6][6] = {{0}}, b[6] = {0, 0, 0, 0, 0, 0}, total = 0.0;
+        int inliers = 0;
+        for (int m = 0; m < n; ++m) {
+            const double* X = xyz_world + 3 * (size_t)m;
+            const double p[3] = {T[0] * X[0] + T[1] * X[1] + T[2] * X[2] + T[3], T[4] * X[0] + T[5] * X[1] + T[6] * X[2] + T[7],
+                                 T[8] * X[0] + T[9] * X[1] + T[10] * X[2] + T[11]};
+            if (!(0.0 < p[2])) continue;
+            double aL[3], aR[3];
+            for (int r = 0; r < 3; ++r) {
+                aL[r] = P_left[4 * r] * p[0] + P_left[4 * r + 1] * p[1] + P_left[4 * r + 2] * p[2] + P_left[4 * r + 3];
+                aR[r] = P_right[4 * r] * p[0] + P_right[4 * r + 1] * p[1] + P_right[4 * r + 2] * p[2] + P_right[4 * r + 3];
+            }
+            const double cL = aL[2], cR = aR[2];
+            const double e[4] = {aL[0] / cL - (double)uv_left[2 * (size_t)m], aL[1] / cL - (double)uv_left[2 * (size_t)m + 1],
+                                 aR[0] / cR - (double)uv_right[2 * (size_t)m], aR[1] / cR - (double)uv_right[2 * (size_t)m + 1]};
+            const double e2 = e[0] * e[0] + e[1] * e[1] + e[2] * e[2] + e[3] * e[3];
+            double w = 1.0;
+            if (kernel < e2) w = kernel / e2; else ++inliers;
+            total += w * e2;
+            const double Jt[3][6] = {{1, 0, 0, 0, 2 * p[2], -2 * p[1]}, {0, 1, 0, -2 * p[2], 0, 2 * p[0]}, {0, 0, 1, 2 * p[1], -2 * p[0], 0}};
+            double J[4][6];
+            svo_posit_rows(P_left, aL, cL, Jt, J[0], J[1]);
+            svo_posit_rows(P_right, aR, cR, Jt, J[2], J[3]);
+            for (int i = 0; i < 6; ++i) {
+                for (int j = 0; j < 6; ++j) H[i][j] += w * (J[0][i] * J[0][j] + J[1][i] * J[1][j] + J[2][i] * J[2][j] + J[3][i] * J[3][j]);
+                b[i] += w * (J[0][i] * e[0] + J[1][i] * e[1] + J[2][i] * e[2] + J[3][i] * e[3]);
+            }
+        }
+        double dx[6], D[16], Tn[16];
+        svo_posit_solve(H, b, dx);
+        for (int k = 0; k < 16; ++k) D[k] = (k % 5 == 0) ? 1.0 : 0.0;
+        D[3] = dx[0]; D[7] = dx[1]; D[11] = dx[2];
+        const double x = dx[3], y = dx[4], z = dx[5], n2 = x * x + y * y + z * z;
+        if (1.0 > n2) {
+            const double qw = sqrt(1.0 - n2);
+            D[0] = 1 - 2 * (y * y + z * z); D[1] = 2 * (x * y - z * qw);     D[2] = 2 * (x * z + y * qw);
+            D[4] = 2 * (x * y + z * qw);     D[5] = 1 - 2 * (x * x + z * z); D[6] = 2 * (y * z - x * qw);
+            D[8] = 2 * (x * z - y * qw);     D[9] = 2 * (y * z + x * qw);     D[10] = 1 - 2 * (x * x + y * y);
+        }
+        svo_iso_mul(D, T, Tn);
+        double RtR[3][3], R[3][3];
+        for (int i = 0; i < 3; ++i)
+            for (int j = 0; j < 3; ++j) RtR[i][j] = Tn[i] * Tn[j] + Tn[4 + i] * Tn[4 + j] + Tn[8 + i] * Tn[8 + j] - (i == j ? 1.0 : 0.0);
+        for (int i = 0; i < 3; ++i)
+            for (int j = 0; j < 3; ++j) R[i][j] = Tn[4 * i + j] - 0.5 * (Tn[4 * i] * RtR[0][j] + Tn[4 * i + 1] * RtR[1][j] + Tn[4 * i + 2] * RtR[2][j]);
+        for (int i = 0; i < 3; ++i)
+            for (int j = 0; j < 3; ++j) Tn[4 * i + j] = R[i][j];
+        memcpy(T, Tn, sizeof(T));
+        *iterations = it + 1;
+        *inliers_out = inliers;
+        if (delta > fabs(prev - total)) {
+            const double avg = total / (double)n;
+            *average_squared_error = avg;
+            if (max_avg < avg && min_inliers > inliers) { *outcome = 2; return 0; }
+            double d2 = 0.0;
+            for (int r = 0; r < 3; ++r) { const double d = T[4 * r + 3] - T_last[4 * r + 3]; d2 += d * d; }
+            if (min_t2 > d2)
+                for (int r = 0; r < 3; ++r) T[4 * r + 3] = T_last[4 * r + 3];   /* the translational part is not integrated */
+            double risk = 0.0;
+            for (int r = 0; r < 3; ++r) {   /* position of the solution minus the prior's, minus t_imu (inverseIsometry's translation) */
+                const double ti = -(T[r] * T[3] + T[4 + r] * T[7] + T[8 + r] * T[11]);
+                const double te = -(T_estimate[r] * T_estimate[3] + T_estimate[4 + r] * T_estimate[7] + T_estimate[8 + r] * T_estimate[11]);
+                const double d = ti - te - t_imu[r];
+                risk += d * d;
+            }
+            *risk_out = risk;
+            if (max_risk < risk) { *outcome = 3; return 0; }
+            memcpy(T_out, T, sizeof(T));
+            *outcome = 0;
+            return 0;
+        }
+        prev = total;
+    }
+    *outcome = 4;
+    return 0;
+}
