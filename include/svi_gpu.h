@@ -65,7 +65,8 @@ typedef enum svi_status {
     SVI_EPI_ORIG_DIST = 23,    /* :2390 "... (ORIGINAL matching distance too big)"                            */
     SVI_EPI_NO_TRANSLATION = 24, /* :1804 detection pose == current pose: stage 3 is skipped for this landmark */
     SVI_SPARSE_NOT_MUTUAL = 25,  /* sparse frames with svi_sparse_band.mutual: not a reference path (no reference text) */
-    SVI_SUBPIXEL_REJECTED = 26   /* svi_params.subpixel_window: the SAD minimum lies on the edge of the search (no reference text) */
+    SVI_SUBPIXEL_REJECTED = 26,  /* svi_params.subpixel_window: the SAD minimum lies on the edge of the search (no reference text) */
+    SVI_LR_INCONSISTENT = 27     /* svi_params.lr_max_diff: the reverse search does not lead back to the LEFT key-point (no reference text) */
 } svi_status;
 
 /* src/vision/CPinholeCamera.h:16-64: the members the hot path reads
@@ -103,7 +104,8 @@ typedef struct svi_params {
     int32_t fast_nonmax;       /* 1 */
     /* optional sub-pixel disparity (NOT a reference code path; ORB-SLAM2's Frame::ComputeStereoMatches refinement): 0 = off
      * (default): every output is the reference's integer-disparity result.  w = subpixel_window > 0 refines the match of every
-     * slot the new-landmark path reports SVI_OK -- svi_stereo_frames[_device] (both matchers), svi_stereo_frame_masked,
+     * slot the new-landmark path reports SVI_OK (after the left-right check of lr_max_diff when it is on) --
+     * svi_stereo_frames[_device] (both matchers), svi_stereo_frame_masked,
      * svi_stereo_frames_sparse[_device] (after the left-right check when it is on) and svi_multi_stereo_frames -- with
      * L = subpixel_search, on the images the detector read (the rectified planes while rectification is set):
      *   1. PL = the (2w+1)^2 LEFT patch centred on (xL, y) minus its centre pixel (integers);
@@ -127,6 +129,25 @@ typedef struct svi_params {
      * svi_triangulate_* / svi_point_in_left. */
     int32_t subpixel_window;   /* 0 */
     int32_t subpixel_search;   /* 0 */
+    /* optional left-right consistency check of the dense scan-line matches (NOT a reference code path; the convention of
+     * cv::StereoSGBM's disp12MaxDiff): -1 = off (default): every output, launch and allocation is the reference path's.
+     * With lr_max_diff = t >= 0, every slot the dense matcher reports SVI_OK, with LEFT key-point (xL, y), match (xR, y) and
+     * RIGHT descriptor desc_right, is searched back with the reference's own reverse search, the 7-argument
+     * CTriangulator::getPointTriangulatedInLEFT (CTriangulator.cpp:255-324, what svi_triangulate_left runs):
+     *   r = getPointTriangulatedInLEFT(LEFT image, search_range_px, u_tl = xR - 4 * keypoint_size,
+     *                                  v_tl = y - 4 * keypoint_size, keypoint_size, (xR, y), desc_right)   (fp32 corners)
+     *   the slot stays SVI_OK iff r.status == SVI_OK and |r.uv.x - xL| <= t (fp32), otherwise it is SVI_LR_INCONSISTENT.
+     * The LEFT image is the plane the detector read (the rectified one while rectification is set).  The reverse pool
+     * xR+1 .. xR+search_range+1 holds xL, so the reverse minimum distance is at most the forward one; with the default
+     * parameters the reverse search cannot fail the cut-off, and it fails only through the rule above (for example through
+     * getPointInLEFT with a raised min_disparity_px).  Status order: every forward status unchanged, the check on forward
+     * SVI_OK slots only, then the sub-pixel refinement (subpixel_window) on the slots that survive it.  status is the only
+     * field the check writes: every other output byte is identical to the call with the check off.
+     * Applied by svi_stereo_frames[_device] (both matchers, both detectors), svi_stereo_frame_masked and
+     * svi_multi_stereo_frames.  Not applied by the sparse frames (svi_sparse_band.mutual is their check), the tracking
+     * cascade (svi_track_landmarks*), svi_track_frame_stereo_only or the per-query svi_triangulate_* / svi_point_in_left.
+     * svi_create refuses values below -1. */
+    int32_t lr_max_diff;       /* -1 */
 } svi_params;
 
 enum { SVI_DETECTOR_GFTT_HARRIS = 0, SVI_DETECTOR_FAST_9_16 = 1 };
@@ -480,7 +501,8 @@ int svi_track_frame_stereo_only(svi_ctx* ctx, const uint8_t* img_left, const uin
  * exclusive duration of one kernel (what the roofline record uses -- slower overall, not for timing
  * the step).  svi_set_profiling also clears the accumulators; svi_stage_timings waits for the ctx to
  * go idle and returns, per stage, the summed launch duration in ms and the number of launches
- * (arrays of length >= 6; returns the stage count; "describe_left" has launches only on the batch path, where the LEFT descriptors are a kernel of their own ahead of the matcher, and "subpixel" only while svi_params.subpixel_window > 0). */
+ * (arrays of length >= 6; returns the stage count; "describe_left" has launches only on the batch path, where the LEFT descriptors are a kernel of their own ahead of the matcher, and "subpixel" only while svi_params.subpixel_window > 0; "lr_check", listed between "stereo_match" and "subpixel", is
+ * listed only while svi_params.lr_max_diff >= 0, so the arrays need length >= 7 then and the count is 6 otherwise). */
 int svi_set_profiling(svi_ctx* ctx, int enable);
 int svi_stage_timings(svi_ctx* ctx, const char** names, double* total_ms, int64_t* launches, int capacity);
 
@@ -509,7 +531,8 @@ int svi_config(const svi_ctx* ctx, int32_t* chunk_frames, int32_t* n_lanes, int3
 /* Number of kernels the new-landmark path launches for one chunk of a call with n_frames frames: 4 (detector, RIGHT box
  * sums, corner selection, matcher) on the small-call path, 5 when the LEFT descriptors are a kernel of their own (batch
  * path), 6 when the batch path also sorts the key-points into image bins (dense frames); one more while rectification is
- * set (svi_set_rectification); one more while svi_params.subpixel_window > 0.  For launch accounting. */
+ * set (svi_set_rectification); one more while svi_params.subpixel_window > 0; one more while svi_params.lr_max_diff >= 0.
+ * For launch accounting. */
 int svi_kernels_per_chunk(const svi_ctx* ctx, int n_frames);
 
 /* ---- undistortion + rectification of raw camera images (CStereoCamera.h:102-107, CStereoCameraIMU.h:36-51: the reference

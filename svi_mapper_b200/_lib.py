@@ -20,6 +20,7 @@ SVI_ERR_INVALID, SVI_ERR_CUDA, SVI_ERR_CAPACITY, SVI_ERR_NO_DEVICE, SVI_ERR_UNSU
  SVI_EPI_POOL_EMPTY, SVI_EPI_NO_MATCHES, SVI_EPI_DIST, SVI_EPI_ORIG_DIST, SVI_EPI_NO_TRANSLATION) = range(25)
 SVI_SPARSE_NOT_MUTUAL = 25   # sparse frames with the left-right check (SparseBand.mutual)
 SVI_SUBPIXEL_REJECTED = 26   # sub-pixel refinement (Params.subpixel_window > 0): the SAD minimum is on the edge of the search
+SVI_LR_INCONSISTENT = 27     # dense left-right check (Params.lr_max_diff >= 0): the reverse search does not lead back
 
 EXPORTS = (
     "svi_params_default", "svi_status_text", "svi_brief_table_info", "svi_create", "svi_destroy", "svi_last_error", "svi_device_count",
@@ -48,6 +49,7 @@ class Params(C.Structure):
         ("max_candidates", C.c_int32), ("chunk_frames", C.c_int32), ("max_queries", C.c_int32),
         ("detector", C.c_int32), ("fast_threshold", C.c_int32), ("fast_nonmax", C.c_int32),
         ("subpixel_window", C.c_int32), ("subpixel_search", C.c_int32),   # sub-pixel disparity: 0 = off (default)
+        ("lr_max_diff", C.c_int32),   # left-right check of the dense matches, in px: -1 = off (default)
     ]
 
 

@@ -26,6 +26,7 @@
 #include "binned.cuh"
 #include "harris.cuh"
 #include "landmark_opt.cuh"
+#include "lr_check.cuh"
 #include "posit.cuh"
 #include "rectify.cuh"
 #include "select.cuh"
@@ -40,10 +41,13 @@ namespace {
 constexpr int kMaxLanes = 8;
 constexpr int kSmallFrames = 2;          // calls of up to this many frames go through the pinned bounce buffer
 constexpr size_t kOutBytesPerSlot = 8 + 8 + 24 + 32 + 32 + 4 + 4 + 1;   // uv_l uv_r xyz desc_l desc_r dist idx status
-constexpr int kStages = 6;
-const char* const kStageNames[kStages] = {"harris_box", "boxsum_right", "select_corners", "describe_left", "stereo_match", "subpixel"};
+// in launch order; svi_stage_timings lists "lr_check" only while the check is on
+constexpr int kStages = 7;
+const char* const kStageNames[kStages] = {"harris_box", "boxsum_right", "select_corners", "describe_left", "stereo_match", "lr_check",
+                                          "subpixel"};
 constexpr int kStageDescribe = 3;   // present only on the batch path (LEFT descriptors ahead of the matcher)
-constexpr int kStageSubpixel = 5;   // present only while svi_params.subpixel_window > 0
+constexpr int kStageLrCheck = 5;    // present only while svi_params.lr_max_diff >= 0
+constexpr int kStageSubpixel = 6;   // present only while svi_params.subpixel_window > 0
 constexpr int kRawFactor = 4;   // the Harris kernel's list (local maxima above the TILE threshold) vs max_candidates
 
 std::string g_create_error;
@@ -269,6 +273,7 @@ void collect_timings(svi_ctx* c) {
             for (int s = 0; s < kStages; ++s) {
                 if (s == kStageDescribe && !(rec < l.ev_pre.size() && l.ev_pre[rec])) continue;   // no kernel in that bracket
                 if (s == kStageSubpixel && c->p.subpixel_window == 0) continue;
+                if (s == kStageLrCheck && c->p.lr_max_diff < 0) continue;
                 float ms = 0.f;
                 if (cudaEventElapsedTime(&ms, l.ev[i + s], l.ev[i + s + 1]) == cudaSuccess) {
                     c->stage_ms[s] += ms;
@@ -310,18 +315,20 @@ int setup_binned(svi_ctx* ctx, Lane& l, size_t rows, std::string* err) {
 }
 
 // The detector on nf frames of one image: candidate lists in the lane's scratch (zeroed by the caller), and the image's box-sum
-// plane `box` unless it is null (harris_box writes it from its own tile; in FAST mode boxsum9, without the shifted copy).  With
-// the selection below, the detection of svi_detect, of the dense path (LEFT) and of both sides of the sparse path.
-void launch_detector(svi_ctx* ctx, Lane& l, const uint8_t* d_img, const uint8_t* d_mask, const FrameGeom& g, int nf, uint16_t* box) {
+// plane `box` unless it is null (harris_box writes it from its own tile; in FAST mode boxsum9), with its shifted copy
+// `box_shift` when that is not null (only the dense path's left-right check reads it).  With the selection below, the
+// detection of svi_detect, of the dense path (LEFT) and of both sides of the sparse path.
+void launch_detector(svi_ctx* ctx, Lane& l, const uint8_t* d_img, const uint8_t* d_mask, const FrameGeom& g, int nf, uint16_t* box,
+                     uint16_t* box_shift = nullptr) {
     cudaStream_t s = l.stream;
     const dim3 tiles((g.W + HT_W - 1) / HT_W, (g.H + HT_H - 1) / HT_H, nf);
     if (ctx->p.detector == SVI_DETECTOR_FAST_9_16) {
         fast_candidates_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, d_mask, g, ctx->p.fast_threshold, ctx->p.fast_nonmax, l.cand,
                                                             l.cand_count, ctx->raw_cap);
-        if (box) boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, box, nullptr);
+        if (box) boxsum9_kernel<<<tiles, HT_THREADS, 0, s>>>(d_img, g, box, box_shift);
     } else {
         harris_box_kernel<<<harris_grid(g.W, g.H, nf), HT_THREADS, sizeof(HarrisSmem), s>>>(
-            d_img, d_mask, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, nullptr, box, nullptr, l.frame_max, l.cand,
+            d_img, d_mask, g, ctx->f1, ctx->f0, ctx->p.harris_k, ctx->p.quality_level, nullptr, box, box_shift, l.frame_max, l.cand,
             l.cand_count, ctx->raw_cap, nullptr, nullptr, g.H);
     }
 }
@@ -353,9 +360,22 @@ int launch_subpixel(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t*
     return SVI_SUCCESS;
 }
 
+// Left-right check of the chunk's SVI_OK slots (lr_check.cuh), after the matcher on the lane's stream; nothing while the check
+// is off.  It reads the LEFT planes the detector wrote (box_l and, only while the check is on, box_ls).
+int launch_lr_check(svi_ctx* ctx, Lane& l, const FrameGeom& g, int nf, const StereoOutDev& out, int out_frame0, const int* n_kp) {
+    if (ctx->p.lr_max_diff < 0) return SVI_SUCCESS;
+    LrCheckArgs a{};
+    a.g = g; a.tc = ctx->tc; a.size = ctx->p.keypoint_size; a.search_range = ctx->p.search_range_px;
+    a.max_diff = (float)ctx->p.lr_max_diff; a.n_kp = n_kp; a.max_corners = ctx->p.max_corners;
+    a.out = out; a.out_frame0 = out_frame0;
+    lr_check_kernel<<<dim3((ctx->p.max_corners + MATCH_WARPS - 1) / MATCH_WARPS, nf), MATCH_WARPS * 32, MATCH_SMEM, l.stream>>>(l.map_l, l.map_ls, a);
+    CK(cudaGetLastError());
+    return SVI_SUCCESS;
+}
+
 // The kernels of the new-landmark path for `nf` frames on one lane: detector, RIGHT box sums, corner selection, then the
-// descriptor / match stages in the form that fits the call, then the optional sub-pixel refinement (svi_kernels_per_chunk:
-// 4 to 7 launches).
+// descriptor / match stages in the form that fits the call, then the optional left-right check and the optional sub-pixel
+// refinement (svi_kernels_per_chunk: 4 to 8 launches).
 int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_right, const uint8_t* d_mask,
                  const FrameGeom& g, int nf, const StereoOutDev& out, int out_frame0, int* n_kp, int* n_det,
                  cudaStream_t side = nullptr, const std::function<int(cudaStream_t)>* upload_right = nullptr) {
@@ -364,7 +384,7 @@ int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_
     CK(cudaMemsetAsync(l.cand_count, 0, sizeof(int) * nf, s));
     const dim3 tiles((g.W + HT_W - 1) / HT_W, (g.H + HT_H - 1) / HT_H, nf);
     mark(ctx, l);
-    launch_detector(ctx, l, d_left, d_mask, g, nf, l.box_l);
+    launch_detector(ctx, l, d_left, d_mask, g, nf, l.box_l, ctx->p.lr_max_diff >= 0 ? l.box_ls : nullptr);
     mark(ctx, l);
     // `side` (latency path): the RIGHT plane goes up on that stream -- staged by the caller's hook only now, so that the
     // host-side copy into the pinned mirror overlaps the detector -- and its box sums run there too
@@ -399,6 +419,9 @@ int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_
         const int rc = run_binned<BinWide>(ctx, l, g, nf, out, out_frame0, n_kp);
         CK(cudaGetLastError());
         if (rc != SVI_SUCCESS) return rc;
+        const int rl = launch_lr_check(ctx, l, g, nf, out, out_frame0, n_kp);
+        mark(ctx, l);
+        if (rl != SVI_SUCCESS) return rl;
         const int rs = launch_subpixel(ctx, l, d_left, d_right, g, nf, out, out_frame0, n_kp);
         mark(ctx, l);
         return rs;
@@ -423,6 +446,9 @@ int run_pipeline(svi_ctx* ctx, Lane& l, const uint8_t* d_left, const uint8_t* d_
 #undef SVI_MATCH_ARGS
     mark(ctx, l);
     CK(cudaGetLastError());
+    const int rl = launch_lr_check(ctx, l, g, nf, out, out_frame0, n_kp);
+    mark(ctx, l);
+    if (rl != SVI_SUCCESS) return rl;
     const int rs = launch_subpixel(ctx, l, d_left, d_right, g, nf, out, out_frame0, n_kp);
     mark(ctx, l);
     return rs;
@@ -1332,6 +1358,7 @@ int svi_params_default(svi_params* p) {
     p->fast_nonmax = 1;
     p->subpixel_window = 0;
     p->subpixel_search = 0;
+    p->lr_max_diff = -1;
     return SVI_SUCCESS;
 }
 
@@ -1364,6 +1391,7 @@ const char* svi_status_text(int status) {
         case SVI_EPI_NO_TRANSLATION: return "no translation since detection: epipolar search skipped";
         case SVI_SPARSE_NOT_MUTUAL: return "left-right check: the matched RIGHT key-point's best LEFT match is another key-point";
         case SVI_SUBPIXEL_REJECTED: return "sub-pixel refinement: the SAD minimum lies on the edge of the search range";
+        case SVI_LR_INCONSISTENT: return "left-right check: the reverse search from the RIGHT match does not lead back to the LEFT key-point";
         default: return "unknown status";
     }
 }
@@ -1433,6 +1461,7 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     // every patch of the refinement stays inside BRIEF's 28-px border: no border mode (include/svi_gpu.h)
     if (p.subpixel_window < 0 || (p.subpixel_window > 0 && (p.subpixel_search < 1 || p.subpixel_window + p.subpixel_search > SP_MAX_REACH)))
         return fail(nullptr, SVI_ERR_INVALID, "svi_create: subpixel_window must be >= 0 and, when > 0, subpixel_search >= 1 with window + search <= 28");
+    if (p.lr_max_diff < -1) return fail(nullptr, SVI_ERR_INVALID, "svi_create: lr_max_diff must be -1 (off) or >= 0");
     if (p.max_candidates < 1024) p.max_candidates = 1024;
     if (p.max_queries < 1) p.max_queries = 1;
     {
@@ -1554,6 +1583,7 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
     CK(cudaFuncSetAttribute(stereo_match_binned_kernel<BinWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, BinWide::M_SMEM));
     CK(cudaFuncSetAttribute(describe_left_binned_kernel<BinWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, BinWide::D_SMEM));
     CK(cudaFuncSetAttribute(triangulate_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
+    CK(cudaFuncSetAttribute(lr_check_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
     CK(cudaFuncSetAttribute(triangulate_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
     CK(cudaFuncSetAttribute(track_stage1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
     CK(cudaFuncSetAttribute(track_stage2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MATCH_SMEM));
@@ -1570,7 +1600,7 @@ int svi_create(const svi_camera* left, const svi_camera* right, const svi_params
                                  (const void*)stereo_match_split_kernel<2, true>, (const void*)stereo_match_split_kernel<2, false>,
                                  (const void*)describe_left_kernel, (const void*)stereo_match_binned_kernel<BinWide>,
                                  (const void*)describe_left_binned_kernel<BinWide>, (const void*)bin_keypoints_kernel,
-                                 (const void*)triangulate_kernel<true>,
+                                 (const void*)triangulate_kernel<true>, (const void*)lr_check_kernel,
                                  (const void*)triangulate_kernel<false>, (const void*)track_stage1_kernel,
                                  (const void*)track_stage2_kernel<true>, (const void*)track_stage2_kernel<false>,
                                  (const void*)track_stage3_kernel, (const void*)fast_candidates_kernel,
@@ -2356,11 +2386,13 @@ int svi_stage_timings(svi_ctx* ctx, const char** names, double* total_ms, int64_
     if (!ctx || !names || !total_ms || !launches) return SVI_ERR_INVALID;
     for (int i = 0; i < ctx->n_lanes; ++i) cudaStreamSynchronize(ctx->lanes[i].stream);
     collect_timings(ctx);
-    int n = std::min(capacity, kStages);
-    for (int i = 0; i < n; ++i) {
-        names[i] = kStageNames[i];
-        total_ms[i] = ctx->stage_ms[i];
-        launches[i] = ctx->stage_launches[i];
+    int n = 0;
+    for (int i = 0; i < kStages && n < capacity; ++i) {
+        if (i == kStageLrCheck && ctx->p.lr_max_diff < 0) continue;
+        names[n] = kStageNames[i];
+        total_ms[n] = ctx->stage_ms[i];
+        launches[n] = ctx->stage_launches[i];
+        ++n;
     }
     return n;
 }
@@ -2546,7 +2578,8 @@ int svi_kernels_per_chunk(const svi_ctx* ctx, int n_frames) {
     const long long slots = (long long)std::min(n_frames, ctx->chunk) * ctx->p.max_corners;
     const bool pre = ctx->match_pre && slots / (2LL * ctx->n_sm * 9) >= MATCH_KP_PER_WARP;
     // detector, RIGHT box sums, corner selection, matcher (+ LEFT descriptors as a kernel of their own, + the bin sort)
-    return 4 + (pre ? 1 : 0) + (pre && ctx->match_binned ? 1 : 0) + (ctx->rect ? 1 : 0) + (ctx->p.subpixel_window > 0 ? 1 : 0);
+    return 4 + (pre ? 1 : 0) + (pre && ctx->match_binned ? 1 : 0) + (ctx->rect ? 1 : 0) + (ctx->p.subpixel_window > 0 ? 1 : 0) +
+           (ctx->p.lr_max_diff >= 0 ? 1 : 0);
 }
 
 int svi_config(const svi_ctx* ctx, int32_t* chunk_frames, int32_t* n_lanes, int32_t* select_in_smem) {
